@@ -3,14 +3,14 @@
 inference with 8x mirror TTA + Gaussian aggregation on a synthetic 182x218x182 FLAIR volume,
 Generic_UNet random-init, patch 128^3 (config[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1: cohort sharding, every rank runs K subjects, no collective on
 the data path -> "scaling": "weak").  A step = one volume through z-score -> 12 tiles x 8 mirrors of
 Generic_UNet -> overlap-add -> finalize.  `value` is timed with the raw volume already in HBM; `e2e` goes
 through the C-ABI host-buffer call (dwmh_predict_volume_host) with pinned host memory, H2D + D2H inside.
 `--impl reference` times the CPU oracle (the reference's PyTorch arithmetic, oracle/) on the host cores.
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  `--dump-outputs DIR` also writes what the last timed step returned (see dump_outputs).
 """
 import argparse
 import json
@@ -223,6 +223,19 @@ def conv_algorithmic_bytes(plans, raw32_max_edge=64):
 
 
 V2_SHAPE = (512, 512, 320)
+DUMP_VOXELS = 1 << 22
+
+
+def dump_outputs(out_dir, seg, probs):
+    """The argmax [X,Y,Z] and softmax [2,X,Y,Z] of a timed step on a fixed, seeded sample of DUMP_VOXELS voxels (the same
+    voxels in every run), as DIR/seg.npy [N] and DIR/softmax.npy [2,N] in float32: 48 MiB, so that two builds can be
+    compared output for output."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(0).choice(seg.numel(), size=DUMP_VOXELS, replace=False))
+    i = torch.from_numpy(idx).to(seg.device)
+    np.save(os.path.join(out_dir, "seg.npy"), seg.reshape(-1)[i].float().cpu().numpy())
+    np.save(os.path.join(out_dir, "softmax.npy"), probs.reshape(2, -1)[:, i].float().cpu().numpy())
 
 
 def run_b200(args):
@@ -281,6 +294,7 @@ def run_b200(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps, warmup, net=None):
+        """-> (ms, kernel launches, what the last timed step returned)"""
         net = net or n
         for i in range(warmup):
             fn(i)
@@ -289,7 +303,7 @@ def run_b200(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(steps):
-            fn(i)
+            last = fn(i)
         e1.record()
         barrier()
         ms = e0.elapsed_time(e1)
@@ -298,14 +312,17 @@ def run_b200(args):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, k1 - k0
+        return ms, k1 - k0, last
 
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    ms_dev, launches = timed(step_device, args.steps, args.warmup)
+    ms_dev, launches, last = timed(step_device, args.steps, args.warmup)
     clocks = sampler.stop() if rank == 0 else None
-    ms_e2e, _ = timed(step_e2e, max(1, args.steps), 1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)     # before the next step overwrites agg, which holds the softmax
+    del last
+    ms_e2e, _, _ = timed(step_e2e, args.steps, 1)
 
     # roofline of the dominant kernel family (conv stack): device time of the conv stack, CUDA events
     # recorded by the library on the launching stream around the launches of one more volume
@@ -346,7 +363,7 @@ def run_b200(args):
             n.normalize_(vol, None, 2, return_stats=False)
             return PAR.predict_volume_ensemble(trs, vol)
         es = max(1, min(args.steps, 3))
-        ms_ens, _ = timed(step_ens, es, 1)
+        ms_ens, _, _ = timed(step_ens, es, 1)
         ens = {"models": args.ensemble, "value": world * es / (ms_ens / 1e3), "unit": "volumes/s", "ms_per_volume": ms_ens / es,
                "forwards_per_volume": args.ensemble * N_TILES * N_MIRRORS, "steps": es,
                "note": "BASELINE config 5: every subject through %d resident random-init models (seeds 1234+k), 8x TTA each, softmax mean + argmax on the device; cohort sharded over %d GPU(s), no collective" % (args.ensemble, world)}
@@ -427,7 +444,7 @@ def run_b200(args):
             n_alt = tr_alt.network
             s_ref, _ = step_device(0)
             s_ref = s_ref.clone()
-            ms_alt, _ = timed(lambda i: step_device(i, n_alt), 3, 2, n_alt)
+            ms_alt, _, _ = timed(lambda i: step_device(i, n_alt), 3, 2, n_alt)
             s_alt, _ = step_device(0, n_alt)
             alt = {"dtype": other, "value": 3 / (ms_alt / 1e3), "unit": "volumes/s", "ms_per_step": ms_alt / 3,
                    "argmax_agreement_with_%s_run" % args.dtype: float((s_alt == s_ref).float().mean().item())}
@@ -443,7 +460,7 @@ def run_b200(args):
         return
 
     vps = world * args.steps / (ms_dev / 1e3)
-    vps_e2e = world * max(1, args.steps) / (ms_e2e / 1e3)
+    vps_e2e = world * args.steps / (ms_e2e / 1e3)
     tflop_vol = flops_fwd * N_TILES * N_MIRRORS / 1e12
     n_batches = -(-N_TILES * N_MIRRORS // args.max_batch)
     tc_launches = tc_launches_per_fwd * n_batches
@@ -512,7 +529,7 @@ def run_b200(args):
         "cpu_baseline": cpu,
         "incumbent_cudnn": inc,
         "e2e": {"value": vps_e2e, "unit": "volumes/s", "h2d_bytes_per_step": 4 * V, "d2h_bytes_per_step": 9 * V,
-                "ms_per_step": ms_e2e / max(1, args.steps), "api": "dwmh_predict_volume_host (C ABI, pinned host buffers)"},
+                "ms_per_step": ms_e2e / args.steps, "api": "dwmh_predict_volume_host (C ABI, pinned host buffers)"},
         "ensemble5": ens,
         "tile_sharded": big,
         "alt_dtype": alt,
@@ -538,7 +555,12 @@ def main():
     ap.add_argument("--big-steps", type=int, default=2)
     ap.add_argument("--reduce", default="reduce", choices=["reduce", "allreduce", "allreduce2"], help="collective of the tile-sharded block")
     ap.add_argument("--alt-dtype", type=int, default=1, help="N = 1: also time the other operand type (bf16 beside fp16)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's seg / softmax to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the b200 path's outputs; the reference arm times single tiles")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -3,9 +3,9 @@ the oracle itself is `parity unpinned`, see oracle/__init__.py).
 
   v1_tta.npz : BASELINE.json config 2 -- synthetic 182x218x182 volume (seed 0), benchmark network
                (model 0), z-score (nonzero mask), step 0.5, Gaussian, 8x mirror TTA, fp32 oracle.
-               Holds the full argmax as packed bits and the class-1 probability on a stride-3 lattice
-               plus a dense 48^3 block (fp32), so the full-size GPU run is checked without the
-               7-minute CPU oracle.
+               Holds the argmax of a seeded half of the voxels as packed bits, the class-1 probability on
+               a stride-6 lattice and both probabilities in a dense 32^3 block (fp32; tests/golden/fixtures.py
+               save_v1 / load_v1), so the full-size GPU run is checked without the 7-minute CPU oracle.
   small_*.npz: tiny networks / volumes the oracle also re-computes live in the tests.
 
 usage: python tests/golden/make_golden.py [v1_tta|v1_notta|all]
@@ -19,7 +19,9 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
+sys.path.insert(0, os.path.dirname(HERE))
 import oracle as O  # noqa: E402
+from golden import fixtures as F  # noqa: E402
 
 
 def v1(tta: bool):
@@ -34,14 +36,9 @@ def v1(tta: bool):
                                                                      use_gaussian=True)
     dt = time.time() - t0
     name = "v1_tta.npz" if tta else "v1_notta.npz"
-    np.savez_compressed(
-        os.path.join(HERE, name),
-        seg_bits=np.packbits(seg.astype(np.uint8).ravel()), shape=np.array(seg.shape),
-        p1_lattice=probs[1, ::3, ::3, ::3].astype(np.float32),
-        p1_block=probs[1, 60:108, 80:128, 60:108].astype(np.float32),
-        p0_block=probs[0, 60:108, 80:128, 60:108].astype(np.float32),
-        zscore_mean_std=np.array([raw[0][raw[0] != 0].mean(), raw[0][raw[0] != 0].std()], dtype=np.float64),
-        oracle_seconds=np.array([dt]), fg_frac=np.array([seg.mean()]))
+    F.save_v1(os.path.join(HERE, name), seg.astype(np.uint8), probs,
+              zscore_mean_std=np.array([raw[0][raw[0] != 0].mean(), raw[0][raw[0] != 0].std()], dtype=np.float64),
+              oracle_seconds=np.array([dt]))
     print(name, "done in %.1fs, fg=%.4f" % (dt, seg.mean()))
 
 

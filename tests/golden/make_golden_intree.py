@@ -10,7 +10,9 @@ engine these rows CAN be pinned: this script imports
 
 unmodified (third-party modules that are absent here and not touched by these functions -- nibabel, skimage,
 matplotlib, ... -- are replaced by inert stand-ins; NIfTI file access of the two stage-2 workers is redirected to an
-in-memory dict) and stores their outputs on seeded inputs in tests/golden/intree_v1.npz.
+in-memory dict) and stores their outputs on seeded inputs in tests/golden/intree_v1.npz.  The seeded inputs come from
+tests/golden/fixtures.py, which also writes the file (inputs as digests; volumes the tests compare with a tolerance on
+a fixed voxel sample).
 
 usage: python tests/golden/make_golden_intree.py                 -> intree_v1.npz
        python tests/golden/make_golden_intree.py nll_analysis    -> nll_analysis_v1.npz (the whole nll_analysis, end to end)
@@ -22,7 +24,15 @@ from unittest.mock import MagicMock
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("DEEPWMH_REFERENCE", "/root/reference")
+sys.path.insert(0, os.path.dirname(HERE))
+from golden import fixtures as F  # noqa: E402
+
+REF = os.environ.get("DEEPWMH_REFERENCE", "DeepWMH")          # a checkout of the original DeepWMH project
+SAMPLED_INTREE = ["zscore_plain", "group_mean", "group_std", "nll_none", "nll_neg", "nll_mu", "nll_sigma", "nll_eps",
+                  "pipe_x_prime", "pipe_local_mu", "pipe_anomaly", "pipe_mean", "pipe_std", "pipe_ref_anomaly0", "pipe_anomaly_cf",
+                  "group_mean_masked", "group_std_masked", "nll_usemask", "nll_usemask_mu", "nll_usemask_sigma"] + \
+                 ["msg_%s_%s" % (a, t) for t in ("p12", "p50", "podd", "nomask") for a in ("mean", "std")]
+SAMPLED_NLL = ["%s_%s" % (n, t) for t in ("pos", "none") for n in ("normalized_input", "intensity_thr", "local_mean", "mean_value", "std_value")]
 
 
 def import_reference():
@@ -43,34 +53,20 @@ def import_reference():
     raise RuntimeError("could not import the reference")
 
 
-def inputs(seed=7, shape=(40, 46, 38), k=5):
-    """Seeded stage-1 inputs: a target, k registered references, a rough brain mask, a valid-score mask."""
-    rng = np.random.default_rng(seed)
-    g = np.stack(np.meshgrid(*[np.linspace(-1, 1, s) for s in shape], indexing="ij"))
-    brain = ((g ** 2).sum(0) < 0.8).astype("float32")
-    base = (100 + 30 * g[0] + 20 * np.sin(3 * g[1]) * g[2]).astype("float32")
-    refs = [(base * rng.uniform(0.8, 1.2) + rng.normal(0, 8, shape)).astype("float32") * brain for _ in range(k)]
-    target = (base + rng.normal(0, 8, shape)).astype("float32")
-    target[12:16, 20:25, 15:19] += 80.0                          # a hyper-intense lesion
-    target *= brain
-    valid = (brain * (rng.random(shape) > 0.1)).astype("float32")
-    return target, refs, brain, valid
-
-
 def main():
     io, la, mt, ms, stubbed = import_reference()
     out = {"stubbed_modules": np.array(stubbed)}
-    rng = np.random.default_rng(11)
+    inp = F.intree_inputs()
 
     # ---- z_score / masked_mean / masked_std (image_ops.py:13-21,172-179)
-    target, refs, brain, valid = inputs()
+    target, refs, brain, valid = inp["in_target"], list(inp["in_refs"]), inp["in_brain"], inp["in_valid"]
     out["in_target"], out["in_refs"], out["in_brain"], out["in_valid"] = target, np.stack(refs), brain, valid
     out["zscore_masked"] = io.z_score(target, mask=brain)
     out["zscore_plain"] = io.z_score(target)
     out["masked_mean_std"] = np.array([io.masked_mean(target, brain), io.masked_std(target, brain)], dtype=np.float64)
 
     # ---- remove_sparks / remove_3mm_sparks (image_ops.py:325-367)
-    sp = (rng.random((30, 34, 28)) > 0.8).astype("float32")
+    sp = inp["sparks_in"]
     out["sparks_in"] = sp
     for name, vox in (("iso1", [1.0, 1.0, 1.0]), ("iso05", [0.5, 0.5, 0.5]), ("iso2", [2.0, 2.0, 2.0]),
                       ("thick", [1.0, 1.0, 6.0]), ("aniso", [0.9, 0.9, 2.5])):
@@ -87,9 +83,7 @@ def main():
     ms.try_load_nifti = lambda p: False
     ms.file_exist = lambda p: False
     shape = (33, 40, 29)
-    xs = [np.clip(rng.normal(0.5, 0.35, size=shape), 0, 1).astype(np.float32) for _ in range(5)]
-    xs[2][:4] = 0.5
-    m = (rng.random(shape) > 0.3).astype(np.float32)
+    xs, m = list(inp["ens_x"]), inp["ens_mask"]
     store["mask"] = m
     masked = []
     for i, x in enumerate(xs):
@@ -102,8 +96,7 @@ def main():
     out["ens_y0_dtype"] = np.array(str(store["y0"].dtype))
 
     # ---- Dice (analysis/metrics.py:26-32)
-    a = (rng.random((20, 20, 20)) > 0.6).astype("float32")
-    b = (rng.random((20, 20, 20)) > 0.6).astype("float32")
+    a, b = inp["dice_in"]
     dice_fn = [getattr(mt, n) for n in dir(mt) if "dice" in n.lower() and callable(getattr(mt, n))]
     out["dice_in"] = np.stack([a, b])
     out["dice_names"] = np.array([f.__name__ for f in dice_fn])
@@ -162,9 +155,7 @@ def main():
     out["pipe_ref_anomaly0"] = la.nll(x_i[0], x_i, min_std=0.03, side="+") * valid
 
     # ---- component_filtering (image_ops.py:253-306): per-slice erosion + largest component, three orientations
-    speck = valid.copy()
-    speck[2:4, 3:6, 4:6] = 1.0                                      # sparks outside the brain, to be filtered away
-    speck[36:39, 40:43, 30:34] = 1.0
+    speck = inp["cf_in"]                                            # the valid mask plus sparks outside the brain
     out["cf_in"] = speck
     for vox, tag in (([1.0, 1.0, 1.0], "iso"), ([0.9, 0.9, 4.0], "thick_z"), ([5.0, 1.0, 1.0], "thick_x")):
         out["cf_" + tag] = io.component_filtering(speck, vox).astype(np.float32)
@@ -176,9 +167,7 @@ def main():
     # ---- group_mean / group_std with masks (image_ops.py:197-231) and the Otsu branch of nll (lesion_analysis.py:87-92).
     # skimage is absent, so for nll(use_mask=True) the restated threshold_otsu (oracle/intree_oracle.py, unpinned) is
     # injected into the reference module; everything else on that path is the reference's own code.
-    rng2 = np.random.default_rng(31)
-    gm = [(rng2.random(zt.shape) > 0.35).astype("float32") for _ in zr]
-    gm[0][5:9] = 0; gm[1][5:9] = 0; gm[2][5:9] = 0; gm[3][5:9] = 0; gm[4][5:9] = 0     # a slab no reference covers -> NaN
+    gm = list(inp["gmask"])                                         # with a slab no reference covers -> NaN
     out["gmask"] = np.stack(gm)
     out["group_mean_masked"] = io.group_mean(zr, masks=gm)
     out["group_std_masked"] = io.group_std(zr, masks=gm)
@@ -192,7 +181,7 @@ def main():
     for k_, v in out.items():
         v = np.asarray(v)
         conv[k_] = v.astype(np.float32) if v.dtype == np.float64 and v.ndim >= 3 else v   # volumes: fp32 on disk
-    np.savez_compressed(os.path.join(HERE, "intree_v1.npz"), **conv)
+    F.save(os.path.join(HERE, "intree_v1.npz"), {k: v for k, v in conv.items() if k not in inp}, {k: conv[k] for k in inp}, SAMPLED_INTREE)
     print("wrote intree_v1.npz:", len(conv), "arrays;", "stubbed:", ", ".join(stubbed))
 
 
@@ -205,28 +194,11 @@ def nll_analysis_fixture():
     its NIfTI readers / writers are redirected to a dict, the plot is a no-op, apply_otsu=False (skimage is absent).
     -> tests/golden/nll_analysis_v1.npz"""
     io, la, mt, ms, stubbed = import_reference()
-    rng = np.random.default_rng(23)
-    shape, k = (44, 52, 40), 6
-    g = np.stack(np.meshgrid(*[np.linspace(-1, 1, s) for s in shape], indexing="ij"))
-    r2 = (g ** 2).sum(0)
-    base = (100 + 25 * g[0] + 15 * np.cos(2 * g[1]) * g[2]).astype("float32")
-    store, brains, tissues, refs = {}, [], [], []
+    inp = F.nll_analysis_inputs()
+    k = len(inp["in_refs"])
+    store = {"x": inp["in_target"]}
     for i in range(k):
-        rad = 0.78 + 0.04 * rng.random()
-        brain = (r2 < rad).astype("float32")
-        # tissue labels 0..3 (background / cerebrum / cerebellum + brainstem / cortex), slightly different per reference
-        t = np.zeros(shape, "float32")
-        t[r2 < rad] = 3
-        t[r2 < rad - 0.12] = 1
-        t[(r2 < rad - 0.05) & (g[2] < -0.35 + 0.03 * rng.random()) & (g[1] < 0.1)] = 2
-        img = ((base * rng.uniform(0.85, 1.15) + rng.normal(0, 7, shape)) * brain).astype("float32")
-        store["r%d" % i], store["m%d" % i], store["y%d" % i] = img, brain, t
-        refs.append(img); brains.append(brain); tissues.append(t)
-    target = (base + rng.normal(0, 7, shape)).astype("float32")
-    target[14:18, 22:27, 20:24] += 70.0                              # lesion in the cerebrum
-    target[20:23, 12:15, 6:9] += 60.0                                # lesion in the cerebellum (median-filtered region)
-    target *= (r2 < 0.8)
-    store["x"] = target
+        store["r%d" % i], store["m%d" % i], store["y%d" % i] = inp["in_refs"][i], inp["in_label1"][i], inp["in_label2"][i].astype("float32")
     vox = (1.0, 1.2, 1.1)
     la.get_nifti_pixdim = lambda p: list(vox)
     la.load_nifti_simple = lambda p: np.asarray(store[p]).astype("float32")
@@ -235,8 +207,7 @@ def nll_analysis_fixture():
     la.hist_plot = lambda *a, **kw: None
     la.mkdir = lambda p: p
     case = {"x": "x", "r": ["r%d" % i for i in range(k)], "m": ["m%d" % i for i in range(k)], "y": ["y%d" % i for i in range(k)]}
-    out = {"in_target": target, "in_refs": np.stack(refs), "in_label1": np.stack(brains), "in_label2": np.stack(tissues).astype(np.uint8),
-           "voxel_size": np.array(vox)}
+    out = {"voxel_size": np.array(vox)}
     for prior, tag in (("+", "pos"), (None, "none")):
         an, valid, cx, cy, cr, thr = la.nll_analysis(case, apply_otsu=False, intensity_prior=prior, case_output_folder="o", debug=True)
         out["anomaly_" + tag], out["valid_" + tag] = np.asarray(an, np.float32), np.asarray(valid, np.float32)
@@ -244,7 +215,7 @@ def nll_analysis_fixture():
         out["threshold_" + tag] = np.array(thr)
         for name in ("normalized_input", "intensity_thr", "rough_brain", "local_mean", "mean_value", "std_value", "averaged_label"):
             out[name + "_" + tag] = np.asarray(store["out:" + name + ".nii.gz"], np.float32)
-    np.savez_compressed(os.path.join(HERE, "nll_analysis_v1.npz"), **out)
+    F.save(os.path.join(HERE, "nll_analysis_v1.npz"), out, inp, SAMPLED_NLL)
     print("wrote nll_analysis_v1.npz:", {k_: (v.shape if hasattr(v, "shape") else v) for k_, v in out.items() if k_.startswith(("thr", "curve_x"))})
 
 

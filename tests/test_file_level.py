@@ -13,6 +13,7 @@ from scipy.ndimage import binary_fill_holes, label
 import oracle as O
 from conftest import small_plans
 from deepwmh_b200 import cli, nifti, preprocess
+from golden.fixtures import intree as intree_fixture
 
 
 def test_nifti_round_trip_and_header(tmp_path):
@@ -206,7 +207,7 @@ def test_device_remove_sparks_matches_scipy_components():
     got = net.remove_sparks(torch.from_numpy(s).cuda(), 3).cpu().numpy()
     assert np.array_equal(got, preprocess.remove_sparks(s, 3).astype(np.uint8))
     # outputs of the reference's own remove_sparks / remove_3mm_sparks (tests/golden/make_golden_intree.py)
-    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "intree_v1.npz"))
+    g = intree_fixture()
     sp = torch.from_numpy((g["sparks_in"] > 0.5).astype(np.uint8)).cuda()
     for tag in ("iso1", "iso05", "iso2", "thick", "aniso"):
         got = net.remove_3mm_sparks(sp, g["sparks_vox_" + tag].tolist()).cpu().numpy()
@@ -247,7 +248,7 @@ def test_device_masked_ensemble_is_bit_exact():
         assert np.array_equal(acc.cpu().numpy(), f_ref)
         assert np.array_equal(clean.cpu().numpy(), l_ref)
     # the reference's own two workers on seeded inputs (tests/golden/make_golden_intree.py)
-    g = np.load(os.path.join(os.path.dirname(__file__), "golden", "intree_v1.npz"))
+    g = intree_fixture()
     acc = torch.zeros(g["ens_field"].shape, dtype=torch.float32, device="cuda")
     md = torch.from_numpy(g["ens_mask"]).cuda()
     for x in g["ens_x"]:

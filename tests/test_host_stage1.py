@@ -1,14 +1,11 @@
 """Host-side logic of deepwmh_b200/stage1.py (no GPU): kernel-size / patch-size rules, the Otsu scan and the threshold
 search, against the reference-pinned oracle (oracle/intree_oracle.py) and the reference's own end-to-end output."""
-import os
-
 import numpy as np
 import pytest
 
 from oracle import intree_oracle as I
 from deepwmh_b200 import stage1 as S
-
-GOLD = os.path.dirname(__file__) + "/golden/"
+from golden import fixtures as F
 
 
 @pytest.mark.parametrize("vox", [[1, 1, 1], [0.7, 0.7, 0.7], [0.5, 0.6, 1.5], [0.9, 0.9, 5.0], [6.0, 1.0, 1.0], [0.4, 3.0, 0.4], [2, 2, 2]])
@@ -17,7 +14,7 @@ def test_median_kernel_rule(vox):
 
 
 def test_median_kernel_rule_matches_reference_fixture():
-    g = np.load(GOLD + "intree_v1.npz")
+    g = F.intree()
     for tag, ks in (("iso1", [3, 3, 3]), ("iso07", [4, 4, 4]), ("mixed", [6, 5, 3]), ("thick", [3, 3, 1])):
         assert S.median_kernel_size(g["median_vox_" + tag].tolist()) == ks
 
@@ -38,7 +35,7 @@ def test_otsu_scan_equals_the_restatement():
 
 
 def test_threshold_search_on_the_reference_curves():
-    f = np.load(GOLD + "nll_analysis_v1.npz")
+    f = F.nll_analysis()
     for tag, prior in (("pos", "+"), ("none", None)):
         _, _, cx, _, _, thr, _ = I.nll_analysis_arrays(f["in_target"], list(f["in_refs"]), list(f["in_label1"]),
                                                        [t.astype(np.float32) for t in f["in_label2"]], f["voxel_size"].tolist(), prior)

@@ -11,6 +11,7 @@ from hypothesis import given, settings, strategies as st
 
 import oracle as O
 from conftest import small_plans
+from golden import fixtures as F
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 
@@ -177,13 +178,14 @@ def test_dice_definition():
 @pytest.mark.skipif(not os.path.exists(os.path.join(GOLD, "v1_tta.npz")), reason="fixture not generated")
 def test_golden_fixture_consistent_with_oracle_pieces():
     """The committed full-size fixture must agree with cheap pieces of the oracle recomputed now."""
-    g = np.load(os.path.join(GOLD, "v1_tta.npz"))
+    g = F.load_v1(os.path.join(GOLD, "v1_tta.npz"))
     assert tuple(g["shape"]) == (182, 218, 182)
     raw = O.synthetic_flair((182, 218, 182), seed=0)[0]
     m = raw != 0
     assert np.allclose(g["zscore_mean_std"], [raw[m].mean(), raw[m].std()], rtol=1e-6)
-    seg = np.unpackbits(g["seg_bits"])[: 182 * 218 * 182].reshape(182, 218, 182)
-    assert abs(seg.mean() - float(g["fg_frac"][0])) < 1e-9
-    blk = seg[60:108, 80:128, 60:108]
-    assert np.array_equal(blk, (g["p1_block"] > g["p0_block"]).astype(np.uint8))
+    assert abs(g["seg"].mean() - float(g["fg_frac"][0])) < 1e-9
+    seg = np.zeros((182, 218, 182), np.uint8)
+    seg[g["seg_sample"]] = g["seg"]
+    blk_sample = g["seg_sample"][F.V1_BLOCK]
+    assert np.array_equal(seg[F.V1_BLOCK][blk_sample], (g["p1_block"] > g["p0_block"]).astype(np.uint8)[blk_sample])
     assert np.allclose(g["p1_block"] + g["p0_block"], 1.0, atol=1e-5)

@@ -13,8 +13,11 @@ import numpy as np
 import torch
 import torch.nn.functional as F
 
-sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
+ROOT = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 import oracle as O  # noqa: E402
+from golden import fixtures as GF  # noqa: E402
 
 torch.backends.cudnn.allow_tf32 = False
 torch.backends.cuda.matmul.allow_tf32 = False
@@ -142,11 +145,10 @@ def main():
     t0 = time.time()
     seg_r, p_r = predict(net, data)
     print("fp32 oracle on GPU: %.1fs, fg=%.4f" % (time.time() - t0, seg_r.mean()))
-    gpath = os.path.join(os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))), "tests", "golden", "v1_tta.npz")
+    gpath = os.path.join(ROOT, "tests", "golden", "v1_tta.npz")
     if os.path.exists(gpath):
-        g = np.load(gpath)
-        seg_g = np.unpackbits(g["seg_bits"])[: seg_r.size].reshape(seg_r.shape)
-        print("GPU fp32 oracle vs committed CPU golden: agree %.6f" % np.mean(seg_g == seg_r))
+        g = GF.load_v1(gpath)               # the argmax of a seeded half of the voxels
+        print("GPU fp32 oracle vs committed CPU golden: agree %.6f" % np.mean(g["seg"] == seg_r[g["seg_sample"]]))
     head = raw[0] != 0
     print("near-boundary mass: frac |p-0.5|<1e-3: all %.5f  head %.5f  background %.5f" % (
         np.mean(np.abs(p_r[1] - 0.5) < 1e-3), np.mean(np.abs(p_r[1][head] - 0.5) < 1e-3), np.mean(np.abs(p_r[1][~head] - 0.5) < 1e-3)))
