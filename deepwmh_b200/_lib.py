@@ -68,6 +68,8 @@ SYMBOLS = {
     "dwmh_s1_apply_priors": (C.c_int, [C.c_int32, _P, _P, _P, _P, C.c_int32, C.c_int64, _P]),
     "dwmh_resample_workspace": (C.c_int, [C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.POINTER(C.c_int64)]),
     "dwmh_resample": (C.c_int, [C.c_int32, _P, C.POINTER(C.c_int32), _P, C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.c_int32, _P, _P]),
+    "dwmh_n4_workspace": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int64)]),
+    "dwmh_n4": (C.c_int, [C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int32), _P, _P, _P, _P]),
     "dwmh_predict_volume_host": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_int32,
                                            C.c_int32, C.c_int32, _P, _P, _P]),
     "dwmh_predict_volume_host_masked": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_int32,

@@ -22,7 +22,8 @@ NVCC_FLAGS = [
 
 
 def _sources():
-    srcs = [os.path.join(CSRC, "api.cu"), os.path.join(CSRC, "stage1.cu"), os.path.join(CSRC, "resample.cu")]
+    srcs = [os.path.join(CSRC, "api.cu"), os.path.join(CSRC, "stage1.cu"), os.path.join(CSRC, "resample.cu"),
+            os.path.join(CSRC, "n4.cu")]
     deps = [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC))] + [os.path.join(ROOT, "include", "deepwmh_b200.h")]
     return srcs, deps
 

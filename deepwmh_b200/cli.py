@@ -4,9 +4,10 @@
 Same flags (-i -n -m -o -g --skip-bfc --custom-task-name), same output tree
 (<out>/001_Preprocessed_Images/<case>_0000.nii.gz, <out>/002_Segmentations/{001_raw,002_postproc_3mm,003_postproc_fov}),
 same fail-fast behaviour (any error -> non-zero exit); the 3 mm spark removal (predict.py:158-163) runs on the device.  Additive: --gpus a,b,... shards the cases over GPUs
-(one worker process per GPU, no collective).  Out of scope and therefore external, exactly as in the reference:
-N4 bias-field correction (ANTs binary; use --skip-bfc or have N4BiasFieldCorrection on PATH), ROBEX FOV masking
-(skipped with a notice unless ROBEX_DIR is set) and GIF previews.
+(one worker process per GPU, no collective); --device-bfc runs N4 bias-field correction on the first of those GPUs
+(deepwmh_b200.n4, same -s 2 and 50x50x50x50 schedule) instead of the ANTs binary.  By default, as in the reference,
+N4 is the external ANTs program (use --skip-bfc, --device-bfc or have N4BiasFieldCorrection on PATH).  External, exactly as in
+the reference: ROBEX FOV masking (skipped with a notice unless ROBEX_DIR is set) and GIF previews.
 """
 from __future__ import annotations
 
@@ -140,7 +141,10 @@ def main(argv=None):
     ap.add_argument("-o", "--output-folder", type=str, required=True,
                     help="Folder where pre-processed input images and predicted segmentations will be stored.")
     ap.add_argument("-g", "--gpu", type=int, default=0, help="GPU id.")
-    ap.add_argument("--skip-bfc", action="store_true", help="[Advanced] Skip bias field correction.")
+    bfc = ap.add_mutually_exclusive_group()
+    bfc.add_argument("--skip-bfc", action="store_true", help="[Advanced] Skip bias field correction.")
+    bfc.add_argument("--device-bfc", action="store_true",
+                     help="[B200] N4 bias-field correction on the GPU instead of the ANTs binary.")
     ap.add_argument("--custom-task-name", type=str, required=False, help="[Advanced] Find model in specified task to segment image.")
     ap.add_argument("--gpus", type=str, default=None, help="[B200] comma-separated GPU ids: shard the cases over several GPUs.")
     args = ap.parse_args(argv)
@@ -159,10 +163,15 @@ def main(argv=None):
     for d in (image_folder, raw_seg, post_3mm, post_fov):
         os.makedirs(d, exist_ok=True)
 
+    gpus = [int(g) for g in args.gpus.split(",")] if args.gpus else [args.gpu]
     print("Pre-processing test images for prediction.")
     for case, src in zip(args.case_names, images):
         dst = os.path.join(image_folder, "%s_0000.nii.gz" % case)
-        if args.skip_bfc:
+        if args.device_bfc:
+            from .n4 import n4_bias_field_correction
+            d, h = nifti.read_nifti(src)
+            nifti.write_nifti(dst, n4_bias_field_correction(d, 2, (50, 50, 50, 50), device=gpus[0]), h, dtype=np.float32)
+        elif args.skip_bfc:
             if src.endswith(".gz"):
                 shutil.copyfile(src, dst)
             else:
@@ -179,7 +188,6 @@ def main(argv=None):
 
     work = [(c, os.path.join(image_folder, "%s_0000.nii.gz" % c), os.path.join(raw_seg, "%s.nii.gz" % c),
              os.path.join(post_3mm, "%s.nii.gz" % c)) for c in args.case_names]
-    gpus = [int(g) for g in args.gpus.split(",")] if args.gpus else [args.gpu]
     if len(gpus) == 1:
         _worker(gpus[0], work, model)
     else:

@@ -222,6 +222,17 @@ int dwmh_resample_workspace(const int32_t in_shape[3], int32_t order, int32_t se
 int dwmh_resample(int32_t device, const float* src_dev, const int32_t in_shape[3], void* dst_dev, const int32_t out_shape[3],
                   int32_t order, int32_t separate_axis, int32_t out_mode, void* workspace_dev, void* stream);
 
+/* --- N4 bias-field correction (the `N4BiasFieldCorrection -d 3 -c [50x50x50x50,0.0] -s 2` step of DeepWMH_predict,
+ * deepwmh/main/predict.py:117-126) on the device, context-free.  Restated from Tustison et al. 2010 with 200 bins, FWHM 0.15,
+ * Wiener noise 0.01, cubic B-splines on an initial 1 x 1 x 1 mesh doubled per level, convergence threshold 0
+ * (oracle/n4_oracle.py, DESIGN.md).  in_dev fp32 [X][Y][Z]; voxels <= 0 take no part in the fit.  Shrink by `shrink` per axis
+ * (floor(N / shrink) points, at least 2 per axis), num_levels <= 8 fitting levels with iterations_host[level] iterations each
+ * (HOST array).  out_dev = in / exp(B); log_field_dev (may be NULL) = B.  in_dev may alias out_dev.  Deterministic: two calls
+ * are bit-identical.  No host synchronisation.  workspace_dev: dwmh_n4_workspace() bytes of device memory. */
+int dwmh_n4_workspace(int32_t X, int32_t Y, int32_t Z, int32_t shrink, int32_t num_levels, int64_t* bytes);
+int dwmh_n4(int32_t device, const float* in_dev, int32_t X, int32_t Y, int32_t Z, int32_t shrink, int32_t num_levels,
+            const int32_t* iterations_host, float* out_dev, float* log_field_dev, void* workspace_dev, void* stream);
+
 /* --- a6 end to end with HOST buffers (what predict_preprocessed_data_return_seg_and_softmax does):
  * raw fp32 volume [X][Y][Z] in host memory -> (optional z-score, mask_mode as above, <0 = skip)
  * -> tiled prediction -> host softmax fp32 [2][X][Y][Z] and seg uint8 [X][Y][Z].  H2D/D2H inside. */
