@@ -7,6 +7,7 @@
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
+#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <string>
@@ -55,6 +56,9 @@ extern "C" int dwmh_version(void) { return 100; }
 // ------------------------------------------------------------------------------------------------
 enum LayerKind { L_FIRST = 0, L_CONV = 1, L_TCONV = 2 };
 
+// largest output edge of a normalised conv whose raw output is stored in fp32 (Layer::raw32)
+constexpr int RAW32_MAX_EDGE = 64;
+
 struct Layer {
   LayerKind kind;
   std::string name;                 // nnU-Net module prefix
@@ -100,7 +104,6 @@ struct dwmh_ctx {
   std::vector<float> w_head; bool have_head = false; float* w_head_dev = nullptr;
   bool committed = false;
   bool force_generic = false;
-  int raw32_max_edge = 64;
   // workspaces
   double* stats_arena = nullptr; size_t stats_bytes = 0;
   StatPartial* stat_partials = nullptr; size_t stat_partials_cap = 0;   // per-CTA Welford partials of the layer in flight
@@ -215,7 +218,6 @@ extern "C" int dwmh_create(dwmh_ctx** out, int device, const dwmh_net_desc* desc
   dwmh_ctx* c = new dwmh_ctx();
   c->device = device; c->d = *desc; c->bf16 = desc->act_dtype == 1; c->num_sms = prop.multiProcessorCount;
   c->max_batch = desc->max_batch > 0 ? desc->max_batch : 8;
-  if (const char* e = getenv("DWMH_RAW32_MAX_EDGE")) c->raw32_max_edge = atoi(e);
   if (build_plan(c)) { delete c; return 1; }
   for (int i = 0; i < 4; ++i) cudaEventCreate(&c->ev[i]);
   *out = c;
@@ -228,7 +230,7 @@ extern "C" int dwmh_create_like(dwmh_ctx** out, dwmh_ctx* parent) {
   if (!parent->buffers_ready) return fail("dwmh_create_like: commit the parent's weights first (its workspaces do not exist yet)");
   dwmh_ctx* c = nullptr;
   DW_TRY(dwmh_create(&c, parent->device, &parent->d));
-  c->max_batch = parent->max_batch; c->raw32_max_edge = parent->raw32_max_edge;
+  c->max_batch = parent->max_batch;
   c->lender = parent;
   *out = c;
   return 0;
@@ -349,7 +351,7 @@ extern "C" int dwmh_commit_weights(dwmh_ctx* c) {
     // fp32 raw storage of conv outputs (profiles/precision_full_r01.txt): those layers then round once
     // (operand) instead of twice (storage + operand)
     L.raw32 = L.kind == L_CONV && L.has_norm && (int)(&L - c->layers.data()) != c->last_conv &&
-              std::max(L.out_sp[0], std::max(L.out_sp[1], L.out_sp[2])) <= c->raw32_max_edge;
+              std::max(L.out_sp[0], std::max(L.out_sp[1], L.out_sp[2])) <= RAW32_MAX_EDGE;
     std::vector<float> pk;
     if (L.kind == L_FIRST) {
       pk.resize((size_t)taps * L.cout);
@@ -414,9 +416,7 @@ extern "C" int dwmh_commit_weights(dwmh_ctx* c) {
     tc_free(L.tc);
     std::string why;
     if (L.kind == L_FIRST) {
-      static int allow_first = -1;
-      if (allow_first < 0) { const char* e = getenv("DWMH_TC_FIRST"); allow_first = e ? atoi(e) : 1; }
-      if (allow_first && L.k[0] == 3 && L.k[1] == 3 && L.k[2] == 3 && L.c0 == 1) {
+      if (L.k[0] == 3 && L.k[1] == 3 && L.k[2] == 3 && L.c0 == 1) {
         std::vector<float> w27((size_t)27 * L.cout);
         for (int co = 0; co < L.cout; ++co) for (int t = 0; t < 27; ++t) w27[(size_t)t * L.cout + co] = L.w[(size_t)co * 27 + t];
         if (tc_prepare_first(L.tc, w27, L.cout, L.out_sp, c->bf16, L.raw, &why))
@@ -451,15 +451,13 @@ extern "C" int dwmh_commit_weights(dwmh_ctx* c) {
     }
   }
   // norm-on-load fusion: producer P feeds exactly one consumer, a tcgen05 layer whose shape supports the in-kernel
-  // transform, and P's raw output is fp16 (the transform works in place on the landed TMA box)
+  // transform, and P's raw output is fp16 (the consumer's loaders read it into registers and transform it there)
   {
-    static int allow = -1;
-    if (allow < 0) { const char* e = getenv("DWMH_FUSE_NORM"); allow = e ? atoi(e) : 1; }
     std::vector<int> uses(nL, 0);
     for (auto& L : c->layers) { if (L.in0 >= 0) uses[L.in0]++; if (L.in1 >= 0) uses[L.in1]++; }
     for (auto& L : c->layers) L.fused_norm = false;
     for (auto& L : c->layers) {
-      if (!allow || L.kind != L_CONV || !L.tc.enabled || !L.tc.xform_ok || L.in0 < 0) continue;
+      if (L.kind != L_CONV || !L.tc.enabled || !L.tc.xform_ok || L.in0 < 0) continue;
       Layer& P = c->layers[L.in0];
       if (P.has_norm && !P.raw32 && uses[L.in0] == 1 && P.s2d_s[0] * P.s2d_s[1] * P.s2d_s[2] == 1 && P.cout <= 64) P.fused_norm = true;
     }

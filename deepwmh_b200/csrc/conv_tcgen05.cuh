@@ -13,20 +13,22 @@
 //     accumulators sit in neighbouring TMEM column blocks, so one tcgen05.mma of N = 3*CB consumes an
 //     A window once for three taps (narrow layers, Cout = 32, would otherwise be bound by the
 //     128 B/clk shared-memory operand bandwidth at ~40 % of the tensor peak).
-//   * accumulators form a ring of R = 512/CB TMEM slots; the epilogue warps drain a finished plane
-//     (tcgen05.ld -> fp16/bf16 pack -> coalesced 16-B stores, InstanceNorm sum / sum-of-squares by a
-//     transposing warp-shuffle reduction), zero the slot (tcgen05.st) and hand it back, so every MMA
-//     accumulates and no per-slot first-touch flag is needed.
+//   * accumulators form a ring of R = 512/CB TMEM slots; the first MMA into an output plane overwrites
+//     its slot (accumulate = 0), the later ones accumulate.  The epilogue warps drain a finished plane
+//     (tcgen05.ld -> fp16/bf16 pack -> coalesced 16-B stores, InstanceNorm Welford partials (count,
+//     mean, M2) per warp, merged in fp64 by stats_reduce_kernel) and hand the slot back.
 //   * weights are pre-packed on the host as ready-made K-major operand tiles [kc][tap_yx][k8][3*CB][8]
 //     and either stay resident in shared memory for the whole CTA or stream through a ring of bulk
 //     copies.
-// Warp roles: 0 = TMA producer (activations), 1 = MMA issuer + TMEM owner, 2..5 = epilogue,
-// 6 = bulk-copy producer (weights).  All hand-offs are mbarriers; nothing spins on __syncthreads.
+// Warp roles of a group: 0 = TMA producer (activations), 1 = MMA issuer, 2..5 = epilogue, 6 = bulk-copy
+// producer (weights); the norm-on-load kernels load through roles 0, 6, 7 and the first-conv kernels
+// build their operand in roles 0, 6 with role 7 fetching input slices.  Which hardware warp takes which
+// role is set by the kRole / kGroup tables in the kernel (epilogue warps first, issuers last); warp 1
+// of the CTA allocates TMEM.  All hand-offs are mbarriers; nothing spins on __syncthreads.
 #pragma once
 #include <cuda.h>
 #include <algorithm>
-#include <cstdio>
-#include <cstdlib>
+#include <cstring>
 #include <string>
 #include <type_traits>
 #include <vector>
@@ -64,16 +66,13 @@ struct TcKParams {
   TcClassDesc cls[8];
   int D, H, W, tilesH, tilesW, ZB, nzb, ncb;
   int SA, NB, resident, R, fmt;
-  // norm-on-load (XFORM kernels): the input tensor is the producer's RAW fp16 output; InstanceNorm + LeakyReLU of the
-  // producer are applied to each landed plane in shared memory by the two producer warps before the MMA reads it
+  // norm-on-load (XFORM kernels): the input tensor is the producer's RAW fp16 output; three loader warps per group read each
+  // plane from global memory into registers, apply InstanceNorm + LeakyReLU of the producer and store it into the activation stage
   const double* xf_sums; const float* xf_gamma; const float* xf_beta; double xf_inv_count; int xform; const void* xf_src;
   // FIRST kernels (Cin = 1 first conv): loader warps build an im2col operand from the fp32 volume / patches
   const float* fc_src; const SampleMeta* fc_metas; int fc_patch_mode, fc_SY, fc_SZ, first;
-  int stagger;        // cycles by which the second issuer of a dual-group CTA starts late (DWMH_TC_STAGGER: -1 = one burst, 0 = off)
   int G;              // work-item pipelines ("groups") per CTA: 2 = two tiles share the resident weights, each with 256 TMEM columns
   int total_items;
-  unsigned long long* prof;   // dbg & 8: per-role wait/total cycle counters
-  int dbg;            // profiling knobs (env DWMH_TC_DEBUG): 1 = no activation TMA, 2 = no MMA, 4 = no epilogue stores
   uint32_t a_stage_bytes, b_tile_bytes, off_b, off_bar;
 };
 
@@ -107,8 +106,6 @@ struct RingPos {
   __device__ __forceinline__ void advance(uint32_t n) { if (++idx == n) { idx = 0; phase ^= 1; } }
   __device__ __forceinline__ RingPos next(uint32_t n) const { RingPos r = *this; r.advance(n); return r; }
 };
-
-#define DWMH_TIMED_WAIT(acc, ...) do { if (prof_on) { const long long t__ = clock64(); __VA_ARGS__; acc += clock64() - t__; } else { __VA_ARGS__; } } while (0)
 
 __device__ __forceinline__ uint64_t tc_desc(uint32_t hi, uint32_t lo) { return ((uint64_t)hi << 32) | lo; }
 
@@ -227,9 +224,6 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
   __syncthreads();
   tc::tc_fence_after();
   const uint32_t tmem = *tmem_ptr_smem + (uint32_t)g * 256u;       // group 1 owns TMEM columns 256..511
-  const bool prof_on = (p.dbg & 8) != 0;
-  long long w0_ = 0, w1_ = 0, w2_ = 0, w3_ = 0;      // profiling (dbg & 8): barrier waits, issue bursts, general-path time
-  const long long tstart_ = clock64();
 
   if (idle) {
     // odd item count: the second group of the last CTA has nothing to do
@@ -306,7 +300,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     tc::mbar_wait(s_full + 8, 0, 11);
     RingPos xf;
     for (int j = 0; j < z_end - z_lo; ++j) {                    // plane t = z_lo + j reads slices j, j+1, j+2
-      DWMH_TIMED_WAIT(w1_, tc::mbar_wait(s_full + 8 * ((j + 2) & 3), ((j + 2) >> 2) & 1, 11));
+      tc::mbar_wait(s_full + 8 * ((j + 2) & 3), ((j + 2) >> 2) & 1, 11);
       tc::mbar_wait(a_empty + 8 * xf.idx, xf.phase ^ 1, 9);
       uint4* stage = reinterpret_cast<uint4*>(smem + (size_t)g * SA * p.a_stage_bytes + (size_t)xf.idx * p.a_stage_bytes);
       const uint32_t* sl[3] = {ring + (j & 3) * TC_FIRST_SLICE, ring + ((j + 1) & 3) * TC_FIRST_SLICE, ring + ((j + 2) & 3) * TC_FIRST_SLICE};
@@ -421,7 +415,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     }
     for (int t_use = t_first; t_use <= t_last; ++t_use) {
       for (int kc_use = 0; kc_use < p.nkc; ++kc_use) {
-        DWMH_TIMED_WAIT(w0_, tc::mbar_wait(a_empty + 8 * xf.idx, xf.phase ^ 1, 8));
+        tc::mbar_wait(a_empty + 8 * xf.idx, xf.phase ^ 1, 8);
         const uint4* sp_next = next_src();
         uint32_t stage = smem_a + xf.idx * p.a_stage_bytes + slot0;        // 32-bit shared address, kept opaque so that it stays in ONE
         asm volatile("" : "+r"(stage));                                     // register (under pressure ptxas rebuilt it per slot from S2R / LDC chains)
@@ -436,7 +430,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
           }
           float f[8];
           unpack8<T>(buf[i], f);
-          if (i == NIT - 1 && sp_next && !(p.dbg & 1)) {
+          if (i == NIT - 1 && sp_next) {
 #pragma unroll
             for (int q = 0; q < NIT; ++q)
               if (pin[q & 1]) buf[q] = ld_stream(sp_next + (size_t)(q >> 1) * V4 + poff[q & 1]);
@@ -448,7 +442,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
           }
           if (pin[i & 1]) st_shared_128(stage + ((i >> 1) * NPOS + 32 * (i & 1)) * 16, pack8<T>(f));
         }
-        DWMH_TIMED_WAIT(w1_, tc::fence_proxy_async());          // generic-proxy stores -> async-proxy (UMMA) reads
+        tc::fence_proxy_async();          // generic-proxy stores -> async-proxy (UMMA) reads
         __syncwarp();
         if (lane == 0) tc::mbar_arrive(a_ready + 8 * xf.idx);
         xf.advance(SA);
@@ -463,9 +457,8 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
       for (int c = 0; c < p.nclass; ++c) {
         if (max(t + p.cls[c].jlo, z_lo) > min(t + p.cls[c].jlo + p.cls[c].jcnt - 1, z_end - 1)) continue;
         for (int kc = 0; kc < p.nkc; ++kc) {
-          DWMH_TIMED_WAIT(w0_, tc::mbar_wait(a_empty + 8 * a.idx, a.phase ^ 1, 1));
-          if (leader && (p.dbg & 1)) tc::mbar_arrive(a_full + 8 * a.idx);
-          if (leader && !(p.dbg & 1)) {
+          tc::mbar_wait(a_empty + 8 * a.idx, a.phase ^ 1, 1);
+          if (leader) {
             tc::mbar_arrive_expect_tx(a_full + 8 * a.idx, p.a_stage_bytes);
             const bool first = kc < p.nkc0;
             const int c8 = first ? (n * p.nclass + c) * (p.C0 >> 3) + kc * (2 * KSTEPS) : n * (p.C1 >> 3) + (kc - p.nkc0) * (2 * KSTEPS);
@@ -496,7 +489,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
           for (int kc = 0; kc < p.nkc; ++kc)
             for (int ti = 0; ti < ntaps; ++ti) {
               const int tile = kc * p.tiles_per_kc + p.cls[c].tile0 + ti;
-              DWMH_TIMED_WAIT(w0_, tc::mbar_wait(b_empty + 8 * b.idx, b.phase ^ 1, 2));
+              tc::mbar_wait(b_empty + 8 * b.idx, b.phase ^ 1, 2);
               if (leader) {
                 tc::mbar_arrive_expect_tx(b_full + 8 * b.idx, p.b_tile_bytes);
                 tc::bulk_load(smem_base + p.off_b + b.idx * p.b_tile_bytes, wsrc + (size_t)tile * p.b_tile_bytes, p.b_tile_bytes, b_full + 8 * b.idx);
@@ -512,7 +505,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     // between two MMAs is kept to a descriptor add: ring cursors instead of div/mod, and a straight-line
     // unrolled burst of 9 taps x KSTEPS per channel chunk in the steady state of a stride-1 layer.
     const bool elected = tc::elect_one();
-    const bool leader = elected && !(p.dbg & 2);
+    const bool leader = elected;
     if constexpr (FIRST) {
       // one output plane per step: 6 MMAs (hi*w_hi, lo*w_hi, hi*w_lo; K = 32 each) into the plane's own slot
       const uint32_t idesc = tc::instr_desc_f16(p.fmt, 128, (int)CB);
@@ -552,14 +545,6 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     const bool plain = p.nclass == 1 && p.Jlo == -1 && p.Jhi == 1;     // stride-1 3x3x3
     if (p.resident)
       for (int t = 0; t < p.nkc * p.tiles_per_kc; ++t) tc::mbar_wait(b_full + 8 * t, 0, 5);
-    if (DUAL && g == 1 && p.stagger > 0) {
-      // The two issuers of a CTA run identical work and otherwise stay in phase: both burst at once (each MMA then takes two
-      // slots of the shared tensor pipe) and both do their per-plane bookkeeping at once (pipe idle).  The lag between them is
-      // preserved from plane to plane, so group 1 starts one burst late and the bursts of one group cover the gaps of the other.
-      tc::mbar_wait(a_mma, 0, 4);                          // its first plane is there: the delay is not hidden behind a load
-      const long long t0_ = clock64();
-      while (clock64() - t0_ < (long long)p.stagger) { }
-    }
     RingPos a, b, fresh, done;
     bool b_peek = false;      // same for the weight ring
     bool a_peek = false;      // a_full of the CURRENT stage already observed complete (prefetched try_wait)
@@ -571,7 +556,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
       if (zo_lo != zo_lo_prev) { lo_slot = (lo_slot + 1 == R) ? 0 : lo_slot + 1; zo_lo_prev = zo_lo; }
       const int fresh_from = next_fresh;        // output planes >= fresh_from are first touched in this step
       while (next_fresh <= zo_hi) {             // the epilogue must have drained the slot's previous use
-        DWMH_TIMED_WAIT(w1_, tc::mbar_wait(acc_empty + 8 * fresh.idx, fresh.phase ^ 1, 3));
+        tc::mbar_wait(acc_empty + 8 * fresh.idx, fresh.phase ^ 1, 3);
         fresh.advance(R);
         ++next_fresh;
       }
@@ -592,16 +577,15 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         const uint32_t idA = wrapA ? id2 : idesc1, idB = wrapA ? idesc1 : id2, offB = wrapA ? 2 * CB : CB;
         const uint32_t col1 = (lo_slot + 1 == R) ? tmem : col + CB, col2 = wrapA ? tmem : tmem + CB;      // slots lo+1, lo+2 when wrapping
         for (int kc = 0; kc < p.nkc; ++kc) {
-          if (!a_peek) DWMH_TIMED_WAIT(w0_, tc::mbar_wait(a_mma + 8 * a.idx, a.phase, 4));
+          if (!a_peek) tc::mbar_wait(a_mma + 8 * a.idx, a.phase, 4);
           tc::tc_fence_after();
           { const RingPos an = a.next(SA); a_peek = tc::mbar_test_wait(a_mma + 8 * an.idx, an.phase); }   // result consumed after the burst
-          const long long tb_ = prof_on ? clock64() : 0;
           if constexpr (!RES) {
             // streamed weight tiles: one ring slot per tap, shared by the groups of the CTA
             const uint32_t a_lo0 = ((smem_a_d + a.idx * p.a_stage_bytes) >> 4) | a_lbo_field;
 #pragma unroll
             for (int sft = 0; sft < 9; ++sft) {
-              if (!b_peek) DWMH_TIMED_WAIT(w1_, tc::mbar_wait(b_full + 8 * b.idx, b.phase, 6));
+              if (!b_peek) tc::mbar_wait(b_full + 8 * b.idx, b.phase, 6);
               tc::tc_fence_after();
               const uint32_t b_lo0 = ((smem_b_d + b.idx * p.b_tile_bytes) >> 4) | (b_lbo16 << 16);
               { const RingPos bn = b.next(NB); b_peek = tc::mbar_test_wait(b_full + 8 * bn.idx, bn.phase); }
@@ -667,7 +651,6 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
               bl += tile16;
             }
           }
-          if (prof_on) w2_ += clock64() - tb_;
           if (elected) tc::umma_commit(a_empty + 8 * a.idx);
           a.advance(SA);
         }
@@ -680,7 +663,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         ++t;
         lo_slot = (lo_slot + 1 == R) ? 0 : lo_slot + 1;           // the oldest live output plane is now t - 1
         zo_lo_prev = t - 1;
-        DWMH_TIMED_WAIT(w1_, tc::mbar_wait(acc_empty + 8 * fresh.idx, fresh.phase ^ 1, 3));      // output plane t + 1 starts
+        tc::mbar_wait(acc_empty + 8 * fresh.idx, fresh.phase ^ 1, 3);      // output plane t + 1 starts
         fresh.advance(R);
         ++next_fresh;
         }
@@ -693,7 +676,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         // KSTEPS MMAs of N = CB per channel chunk into the plane's own slot; the first MMA overwrites it.
         const uint32_t col = tmem + lo_slot * CB;
         for (int kc = 0; kc < p.nkc; ++kc) {
-          if (!a_peek) DWMH_TIMED_WAIT(w0_, tc::mbar_wait(a_mma + 8 * a.idx, a.phase, 4));
+          if (!a_peek) tc::mbar_wait(a_mma + 8 * a.idx, a.phase, 4);
           tc::tc_fence_after();
           { const RingPos an = a.next(SA); a_peek = tc::mbar_test_wait(a_mma + 8 * an.idx, an.phase); }
           const uint32_t a_lo0 = ((smem_a_d + a.idx * p.a_stage_bytes) >> 4) | a_lbo_field;
@@ -702,7 +685,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
           for (int sft = 0; sft < 9; ++sft) {
             uint32_t b_lo0 = bl;
             if (!p.resident) {
-              if (!b_peek) DWMH_TIMED_WAIT(w1_, tc::mbar_wait(b_full + 8 * b.idx, b.phase, 6));
+              if (!b_peek) tc::mbar_wait(b_full + 8 * b.idx, b.phase, 6);
               tc::tc_fence_after();
               b_lo0 = ((smem_b_d + b.idx * p.b_tile_bytes) >> 4) | (b_lbo16 << 16);
               { const RingPos bn = b.next(NB); b_peek = tc::mbar_test_wait(b_full + 8 * bn.idx, bn.phase); }
@@ -741,12 +724,14 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         const uint32_t id2 = idesc0 | (((2 * CB) >> 3) << 17);
         auto s222_step = [&](auto res_c, auto wrap_c) {
           constexpr bool RES = decltype(res_c)::value, WRAP = decltype(wrap_c)::value;
+          uint32_t kstep = kstep_b;        // opaque: otherwise the offsets of all tiles x K steps are hoisted into the issuer's prologue and spill
+          asm volatile("" : "+r"(kstep));
 #pragma unroll
           for (int c = 0; c < 8; ++c) {
             const int cd = c >> 2, ph = (c >> 1) & 1, pw = c & 1;
             const int tile0 = cd * 9 + (ph ? (pw ? 5 : 3) : (pw ? 1 : 0));
             for (int kc = 0; kc < p.nkc; ++kc) {
-              if (!a_peek) DWMH_TIMED_WAIT(w0_, tc::mbar_wait(a_mma + 8 * a.idx, a.phase, 4));
+              if (!a_peek) tc::mbar_wait(a_mma + 8 * a.idx, a.phase, 4);
               tc::tc_fence_after();
               { const RingPos an = a.next(SA); a_peek = tc::mbar_test_wait(a_mma + 8 * an.idx, an.phase); }
               const uint32_t a_lo0 = ((smem_a_d + a.idx * p.a_stage_bytes) >> 4) | a_lbo_field;
@@ -759,7 +744,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
                   uint32_t b_lo0;
                   if constexpr (RES) b_lo0 = b_res + ti * tile16;
                   else {
-                    if (!b_peek) DWMH_TIMED_WAIT(w1_, tc::mbar_wait(b_full + 8 * b.idx, b.phase, 6));
+                    if (!b_peek) tc::mbar_wait(b_full + 8 * b.idx, b.phase, 6);
                     tc::tc_fence_after();
                     b_lo0 = ((smem_b_d + b.idx * p.b_tile_bytes) >> 4) | (b_lbo16 << 16);
                     { const RingPos bn = b.next(NB); b_peek = tc::mbar_test_wait(b_full + 8 * bn.idx, bn.phase); }
@@ -768,7 +753,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
 #pragma unroll
                     for (int kk = 0; kk < KSTEPS; ++kk) {
                       const uint64_t adesc = tc_desc(a_hi, a_lo0 + dy * TC_PW + dx + kk * (2 * TC_PLANE_BYTES >> 4));
-                      const uint32_t bl = b_lo0 + kk * kstep_b;
+                      const uint32_t bl = b_lo0 + kk * kstep;
                       if (cd == 0) {
                         const bool first_site = c == 0 && kk == 0;             // the step's first MMA overwrites output t+1
                         if (WRAP || (first_site && kc == 0)) {
@@ -807,7 +792,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         for (int c = 0; c < p.nclass; ++c) {
           const int jc = p.cls[c].jcnt, tapmask = p.cls[c].tapmask;
           for (int kc = 0; kc < p.nkc; ++kc) {
-            if (!a_peek) DWMH_TIMED_WAIT(w0_, tc::mbar_wait(a_mma + 8 * a.idx, a.phase, 4));
+            if (!a_peek) tc::mbar_wait(a_mma + 8 * a.idx, a.phase, 4);
             tc::tc_fence_after();
             { const RingPos an = a.next(SA); a_peek = tc::mbar_test_wait(a_mma + 8 * an.idx, an.phase); }
             const uint32_t a_lo0 = ((smem_a_d + a.idx * p.a_stage_bytes) >> 4) | a_lbo_field;
@@ -817,7 +802,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
               uint32_t b_lo0;
               if (p.resident) { b_lo0 = b_res; b_res += tile16; }
               else {
-                if (!b_peek) DWMH_TIMED_WAIT(w1_, tc::mbar_wait(b_full + 8 * b.idx, b.phase, 6));
+                if (!b_peek) tc::mbar_wait(b_full + 8 * b.idx, b.phase, 6);
                 tc::tc_fence_after();
                 b_lo0 = ((smem_b_d + b.idx * p.b_tile_bytes) >> 4) | (b_lbo16 << 16);
                 { const RingPos bn = b.next(NB); b_peek = tc::mbar_test_wait(b_full + 8 * bn.idx, bn.phase); }
@@ -854,7 +839,6 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         continue;
       }
       // ---- general path: parity classes, ring wrap, block edges, streamed weights -------------------
-      const long long tg_ = prof_on ? clock64() : 0;
       bool first_mma = true;
       for (int c = 0; c < p.nclass; ++c) {
         const int dlo = max(t + p.cls[c].jlo, z_lo), dhi = min(t + p.cls[c].jlo + p.cls[c].jcnt - 1, z_end - 1);
@@ -877,7 +861,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         }
         const int tapmask = p.cls[c].tapmask;
         for (int kc = 0; kc < p.nkc; ++kc) {
-          if (!a_peek) DWMH_TIMED_WAIT(w0_, tc::mbar_wait(a_mma + 8 * a.idx, a.phase, 4));
+          if (!a_peek) tc::mbar_wait(a_mma + 8 * a.idx, a.phase, 4);
           a_peek = false;
           tc::tc_fence_after();
           const uint32_t a_lo0 = ((smem_a_d + a.idx * p.a_stage_bytes) >> 4) | a_lbo_field;
@@ -887,7 +871,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
             uint32_t b_lo0;
             if (p.resident) { b_lo0 = b_res; b_res += tile16; }
             else {
-              if (!b_peek) DWMH_TIMED_WAIT(w1_, tc::mbar_wait(b_full + 8 * b.idx, b.phase, 6));
+              if (!b_peek) tc::mbar_wait(b_full + 8 * b.idx, b.phase, 6);
               tc::tc_fence_after();
               b_lo0 = ((smem_b_d + b.idx * p.b_tile_bytes) >> 4) | (b_lbo16 << 16);
               { const RingPos bn = b.next(NB); b_peek = tc::mbar_test_wait(b_full + 8 * bn.idx, bn.phase); }   // consumed at the next tap
@@ -929,7 +913,6 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         ++next_done;
       }
       __syncwarp();
-      if (prof_on) w3_ += clock64() - tg_;
     }
     }   // !FIRST
   } else {
@@ -937,7 +920,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     const int q = warp_abs & 3;       // TMEM lane quarter is fixed by the hardware warp id
     const int row = q * 32 + lane;
     const int h = h0 + (row >> 3), w = w0 + (row & 7);
-    const bool valid = h < p.H && w < p.W && !(p.dbg & 4);
+    const bool valid = h < p.H && w < p.W;
     const uint32_t tm_lane = tmem + ((uint32_t)(q * 32) << 16);
     const int nch = CB >> 4;
     if constexpr (TCONV) {
@@ -948,7 +931,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
       uint4* out_n = reinterpret_cast<uint4*>(p.out) + (size_t)n * (p.Cout_t >> 3) * Vo;
       uint32_t slot = 0, phase = 0;
       for (int t = z_lo; t < z_end; ++t) {
-        DWMH_TIMED_WAIT(w0_, tc::mbar_wait(acc_full + 8 * slot, phase, 7));
+        tc::mbar_wait(acc_full + 8 * slot, phase, 7);
         tc::tc_fence_after();
         if (p.osw == 2) {
           // W-doubling (the usual case): the two W parities of a voxel are adjacent in memory, so a lane stores 32
@@ -1019,7 +1002,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     uint4* out_base = reinterpret_cast<uint4*>(p.out) + ((size_t)n * (p.Cout >> 3) + (size_t)cb * (CB >> 3)) * V;
     uint32_t slot = 0, phase = 0;
     for (int zo = z_lo; zo < z_end; ++zo) {
-      DWMH_TIMED_WAIT(w0_, tc::mbar_wait(acc_full + 8 * slot, phase, 7));
+      tc::mbar_wait(acc_full + 8 * slot, phase, 7);
       tc::tc_fence_after();
       uint4* outp = out_base + ((size_t)zo * p.H + h) * p.W + w;
       float wgt_new, cnt_prev = cnt;
@@ -1133,14 +1116,6 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     }
     }   // !TCONV
   }
-  if (prof_on && lane == 0 && g == 0 && (warp <= 2 || warp == 6)) {
-    const int role = warp == 6 ? 3 : warp;          // 0 act producer, 1 mma, 2 epilogue (warp 2), 3 weight producer
-    atomicAdd(p.prof + role * 4 + 0, (unsigned long long)w0_);
-    atomicAdd(p.prof + role * 4 + 1, (unsigned long long)w1_);
-    atomicAdd(p.prof + role * 4 + 2, (unsigned long long)(clock64() - tstart_));
-    atomicAdd(p.prof + role * 4 + 3, (unsigned long long)w2_);
-    if (role == 1) atomicAdd(p.prof + 3, (unsigned long long)w3_);
-  }
   tc::tc_fence_before();
   __syncthreads();
   if constexpr (!TCONV) {
@@ -1179,13 +1154,6 @@ inline void tc_free(TcLayer& t) {
   if (t.wpack) cudaFree(t.wpack);
   t.wpack = nullptr;
   t.enabled = false;
-}
-
-// activation-ring depth of the resident-weight plans (DWMH_TC_MAX_SA, default 4; <= 8: the barrier block has room for it)
-inline int tc_max_sa() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("DWMH_TC_MAX_SA"); v = e ? std::max(2, std::min(8, atoi(e))) : TC_MAX_SA; }
-  return v;
 }
 
 typedef CUresult (*PFN_tmapEncodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
@@ -1304,10 +1272,8 @@ inline int tc_prepare(TcLayer& t, const std::vector<float>& w, int c0, int c1, i
   while (KC0 > 16 && (c0 % KC0 || c1 % KC0)) KC0 >>= 1;
   const int budget = TC_SMEM_MAX - TC_SMEM_RESERVED;
   int KC = 0, CB = 0, SA = 0, NB = 0, resident = 0, G = 1;
-  static int allow_dual = -1;
-  if (allow_dual < 0) { const char* e = getenv("DWMH_TC_DUAL"); allow_dual = e ? atoi(e) : 1; }
   // (1) dual-group resident plan: two tile pipelines share the resident weights (each gets 256 TMEM columns)
-  for (int kc = KC0; kc >= 16 && !CB && allow_dual; kc >>= 1) {
+  for (int kc = KC0; kc >= 16 && !CB; kc >>= 1) {
     const int a_stage = kc * 360, ntile = (cin / kc) * kp.tiles_per_kc;
     if (ntile > TC_MAX_NB) continue;
     for (int cbt = std::min(cout, 64); cbt >= 32; cbt -= 16) {
@@ -1315,13 +1281,13 @@ inline int tc_prepare(TcLayer& t, const std::vector<float>& w, int c0, int c1, i
       const long long btot = (long long)ntile * kp.jmax * cbt * kc * 2;
       if (btot + 2LL * 3 * a_stage <= budget) {
         KC = kc; CB = cbt; resident = 1; NB = ntile; G = 2;
-        SA = (int)std::min<long long>(tc_max_sa(), (budget - btot) / (2LL * a_stage));
+        SA = (int)std::min<long long>(TC_MAX_SA, (budget - btot) / (2LL * a_stage));
         break;
       }
     }
   }
   // (1b) dual-group streaming plan: both groups consume ONE shared ring of weight tiles in lockstep (M = 256 per tile fetched)
-  for (int kc = KC0; kc >= 32 && !CB && allow_dual; kc >>= 1) {
+  for (int kc = KC0; kc >= 32 && !CB; kc >>= 1) {
     const int a_stage = kc * 360;
     for (int cbt = std::min(cout, 64); cbt >= 32; cbt -= 16) {
       if (cout % cbt) continue;
@@ -1341,7 +1307,7 @@ inline int tc_prepare(TcLayer& t, const std::vector<float>& w, int c0, int c1, i
         const long long btot = (long long)ntile * kp.jmax * cbt * kc * 2;
         if (btot + 2LL * a_stage <= budget) {
           KC = kc; CB = cbt; resident = 1; NB = ntile;
-          SA = (int)std::min<long long>(tc_max_sa(), (budget - btot) / a_stage);
+          SA = (int)std::min<long long>(TC_MAX_SA, (budget - btot) / a_stage);
           break;
         }
       }
@@ -1546,9 +1512,7 @@ struct TcFirstSrc { const float* src; const SampleMeta* metas; int patch_mode, S
 // planes per z-block: split D until the grid fills the machine about twice
 inline int tc_plan_zb(const TcKParams& kp, int nb, int num_sms) {
   const int tiles = kp.tilesH * kp.tilesW;
-  static int model = -1;
-  if (model < 0) { const char* e = getenv("DWMH_TC_ZB_MODEL"); model = e ? atoi(e) : 1; }
-  if (model && !kp.first && !kp.tconv && kp.D >= 16) {
+  if (!kp.first && !kp.tconv && kp.D >= 16) {
     // 3-D convs on >= 16 planes: minimise waves x input planes per CTA (block + depth halo).  16^3 layers then run 128 CTAs of 18
     // planes in one wave instead of 256 CTAs of 10 planes in two, dec3-a 1024 CTAs in 7 waves instead of 512 in 4 (3.46 rounded up):
     // -6 % on dec3-a, -5..9 % on the 16^3 and the strided layers (profiles/ab_loader_r02b.txt).  The first conv, the transposed
@@ -1592,15 +1556,6 @@ int tc_launch(TcLayer& t, int nb, double* sums, StatPartial* partials, int num_s
   const int tiles = kp.tilesH * kp.tilesW;
   const int ZB = tc_plan_zb(kp, nb, num_sms);
   kp.ZB = ZB; kp.nzb = (kp.D + ZB - 1) / ZB;
-  { static int dbg = -1; if (dbg < 0) { const char* e = getenv("DWMH_TC_DEBUG"); dbg = e ? atoi(e) : 0; } kp.dbg = dbg; }
-  {
-    static int stg = -2;
-    if (stg == -2) { const char* e = getenv("DWMH_TC_STAGGER"); stg = e ? atoi(e) : 0; }
-    // one burst = the MMAs of one input plane at the shared-memory-bound rate
-    const int n3 = kp.jmax * kp.CB;
-    const int per_mma = std::max(n3 / 2, (4096 + 32 * n3) / 128);
-    kp.stagger = stg < 0 ? kp.nkc * 9 * (kp.KC / 16) * per_mma * (-stg) / 1 : stg;
-  }
   const long long items = (long long)nb * kp.ncb * kp.nzb * tiles;
   // both groups of a CTA must share the cout block whose weights are resident: pairs (2k, 2k+1) stay inside
   // one (n, cb) when the tiles x z-blocks count is even
@@ -1608,12 +1563,6 @@ int tc_launch(TcLayer& t, int nb, double* sums, StatPartial* partials, int num_s
   kp.total_items = (int)items;
   const unsigned grid = (unsigned)((items + kp.G - 1) / kp.G);
   const unsigned threads = TC_THREADS * kp.G;
-  static unsigned long long* prof_dev = nullptr;
-  if (kp.dbg & 8) {
-    if (!prof_dev) cudaMalloc((void**)&prof_dev, 16 * sizeof(unsigned long long));
-    cudaMemsetAsync(prof_dev, 0, 16 * sizeof(unsigned long long), st);
-  }
-  kp.prof = prof_dev;
   const int ks = kp.KC / 16;
   const bool small = kp.CB <= 32 && !kp.tconv;
 #define DWMH_TC_LAUNCH(K, S, C, D) conv3_tc_kernel<T, K, S, C, D, false><<<grid, threads, t.smem_bytes, st>>>(t.tm0, t.tm1, kp)
@@ -1635,14 +1584,6 @@ int tc_launch(TcLayer& t, int nb, double* sums, StatPartial* partials, int num_s
     stats_reduce_kernel<<<nb * kp.ncb, kp.CB * jn, 0, st>>>(partials, sums, kp.ncb, kp.CB, kp.Cout, kp.nzb * tiles, jn);
     e = cudaGetLastError();
     if (e != cudaSuccess) { if (err) *err = std::string("stats_reduce_kernel launch failed: ") + cudaGetErrorString(e); return 1; }
-  }
-  if (kp.dbg & 8) {
-    unsigned long long h[16];
-    cudaStreamSynchronize(st);
-    cudaMemcpy(h, prof_dev, sizeof h, cudaMemcpyDeviceToHost);
-    const double g = (double)grid;
-    fprintf(stderr, "tcprof C0=%d C1=%d Cout=%d CB=%d KC=%d D=%d res=%d grid=%u planes/cta=%d | act-prod wait_empty %.0f w1 %.0f tot %.0f | mma wait_a %.0f wait_acc/b %.0f burst %.0f general-path %.0f tot %.0f | epi wait_full %.0f tot %.0f | w-prod wait %.0f tot %.0f (cycles per CTA)\n",
-            kp.C0, kp.C1, kp.Cout, kp.CB, kp.KC, kp.D, kp.resident, grid, kp.ZB, h[0] / g, h[1] / g, h[2] / g, h[4] / g, h[5] / g, h[7] / g, h[3] / g, h[6] / g, h[8] / g, h[10] / g, h[12] / g, h[14] / g);
   }
   return 0;
 }

@@ -32,7 +32,6 @@ The GPU cases reach the kernel paths DESIGN section 4 describes; the CPU test ru
 of the device's fp16 scheme, which pins the tolerance model and the hook plumbing without a GPU.
 """
 import copy
-import os
 
 import pytest
 import torch
@@ -43,7 +42,7 @@ from conftest import small_plans
 
 U = {"fp16": 2.0 ** -11, "bf16": 2.0 ** -8}
 SENS_MIN = 4.0
-RAW32_MAX_EDGE = int(os.environ.get("DWMH_RAW32_MAX_EDGE", "64"))    # the library's rule for fp32 raw storage
+RAW32_MAX_EDGE = 64    # mirrors RAW32_MAX_EDGE in csrc/api.cu: the largest edge whose raw conv output is stored in fp32
 
 
 def round_act(t, act):
