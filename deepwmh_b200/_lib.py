@@ -10,6 +10,8 @@ import numpy as np
 from . import build as _build
 
 DWMH_MAX_POOL = 7
+DWMH_MAX_IN_CHANNELS = 4
+DWMH_MAX_CLASSES = 8
 
 
 class NetDesc(C.Structure):
@@ -43,6 +45,7 @@ SYMBOLS = {
     "dwmh_finalize": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, _P]),
     "dwmh_axpy": (C.c_int, [_P, _P, _P, C.c_float, C.c_int64, _P]),
     "dwmh_argmax2": (C.c_int, [_P, _P, _P, C.c_int64, _P]),
+    "dwmh_argmax": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int64, _P]),
     "dwmh_ensemble_masked_add": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P]),
     "dwmh_ensemble_refine": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int64, _P]),
     "dwmh_remove_sparks": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P]),

@@ -73,12 +73,13 @@ def _check_cases(case_names: List[str], images: List[str]):
             sys.exit(1)
 
 
-def predict_case(trainer, plans: Dict, in_file: str, out_file: str, softmax_file: str = None, post3mm_file: str = None,
+def predict_case(trainer, plans: Dict, in_file, out_file: str, softmax_file: str = None, post3mm_file: str = None,
                  do_mirroring: bool = True):
-    """One case the way nnUNet_predict's predict_cases does it for a single modality (SURVEY.md A7/A10): preprocess_patient
-    (crop -> transpose -> resample -> z-score), tiled prediction, transpose back, resample back, argmax, paste back, NIfTI.
-    Everything between the file read and the file write stays on the device."""
-    data, _, props = trainer.preprocess_patient([in_file], as_numpy=False)
+    """One case the way nnUNet_predict's predict_cases does it (SURVEY.md A7/A10): preprocess_patient (crop -> transpose ->
+    resample -> z-score), tiled prediction, transpose back, resample back, argmax, paste back, NIfTI.  in_file: the image, or
+    the list of its modality files in channel order.  Everything between the file read and the file write stays on the device."""
+    files = [in_file] if isinstance(in_file, str) else list(in_file)
+    data, _, props = trainer.preprocess_patient(files, as_numpy=False)
     _, softmax = trainer.predict_preprocessed_data_return_seg_and_softmax(
         data, do_mirroring=do_mirroring, mirror_axes=trainer.data_aug_params["mirror_axes"], use_sliding_window=True,
         step_size=0.5, use_gaussian=True, all_in_gpu=False, mixed_precision=True, return_device_tensors=True)
@@ -153,6 +154,10 @@ def main(argv=None):
     _check_cases(args.case_names, images)
     os.environ["RESULTS_FOLDER"] = os.path.abspath(args.trained_model)
     model = find_model(args.trained_model, args.custom_task_name)
+    n_mod = int(load_plans(model["plans"]).get("num_modalities", 1))
+    if n_mod != 1:
+        raise RuntimeError("the model in %s takes %d input modalities; DeepWMH_predict takes one image per case. Run "
+                           "nnUNet_predict with <case>_0000 ... <case>_%04d.nii.gz input files instead." % (args.trained_model, n_mod, n_mod - 1))
     print("model file is valid.")
 
     out = os.path.abspath(args.output_folder)

@@ -199,8 +199,23 @@ static int build_plan(dwmh_ctx* c) {
 // ------------------------------------------------------------------------------------------------
 // life cycle
 // ------------------------------------------------------------------------------------------------
+// Model shapes this library runs; checked before any device work, so an unsupported model fails the same way everywhere.
+static int check_model_bounds(const dwmh_net_desc* d) {
+  if (d->in_channels < 1 || d->in_channels > DWMH_MAX_IN_CHANNELS)
+    return fail("dwmh_create: in_channels=%d unsupported (1 <= in_channels <= %d: the first conv keeps 4 input slices and one "
+                "weight tile per modality in one SM's shared memory)", d->in_channels, DWMH_MAX_IN_CHANNELS);
+  if (d->num_classes < 2 || d->num_classes > DWMH_MAX_CLASSES)
+    return fail("dwmh_create: num_classes=%d unsupported (2 <= num_classes <= %d: the head keeps every class's logits of two "
+                "voxels in registers)", d->num_classes, DWMH_MAX_CLASSES);
+  if (d->in_channels > 1 && d->base_num_features > 32)
+    return fail("dwmh_create: base_num_features=%d with in_channels=%d unsupported (the multi-modality first conv has at most 32 "
+                "output channels)", d->base_num_features, d->in_channels);
+  return 0;
+}
+
 extern "C" int dwmh_create(dwmh_ctx** out, int device, const dwmh_net_desc* desc) {
   if (!out || !desc) return fail("dwmh_create: null argument");
+  if (desc->struct_size == (int32_t)sizeof(dwmh_net_desc)) DW_TRY(check_model_bounds(desc));
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
     return fail("dwmh_create: no CUDA device visible (this library has no CPU fallback)");
@@ -212,8 +227,6 @@ extern "C" int dwmh_create(dwmh_ctx** out, int device, const dwmh_net_desc* desc
   cudaDeviceProp prop;
   CU_TRY(cudaGetDeviceProperties(&prop, device));
   if (prop.major != 10) return fail("dwmh_create: device %d is sm_%d%d; this build targets sm_100a (B200) only", device, prop.major, prop.minor);
-  if (desc->in_channels != 1) return fail("in_channels=%d unsupported (DeepWMH uses one FLAIR modality)", desc->in_channels);
-  if (desc->num_classes != 2) return fail("num_classes=%d unsupported (DeepWMH: background + WMH)", desc->num_classes);
   if (desc->num_pool < 1 || desc->num_pool > DWMH_MAX_POOL) return fail("num_pool out of range");
   dwmh_ctx* c = new dwmh_ctx();
   c->device = device; c->d = *desc; c->bf16 = desc->act_dtype == 1; c->num_sms = prop.multiProcessorCount;
@@ -354,8 +367,10 @@ extern "C" int dwmh_commit_weights(dwmh_ctx* c) {
               std::max(L.out_sp[0], std::max(L.out_sp[1], L.out_sp[2])) <= RAW32_MAX_EDGE;
     std::vector<float> pk;
     if (L.kind == L_FIRST) {
-      pk.resize((size_t)taps * L.cout);
-      for (int co = 0; co < L.cout; ++co) for (int t = 0; t < taps; ++t) pk[(size_t)t * L.cout + co] = L.w[(size_t)co * taps + t];
+      // [modality][tap][Cout] from PyTorch's [Cout][modality][tap]
+      pk.resize((size_t)L.c0 * taps * L.cout);
+      for (int co = 0; co < L.cout; ++co) for (int m = 0; m < L.c0; ++m) for (int t = 0; t < taps; ++t)
+        pk[((size_t)m * taps + t) * L.cout + co] = L.w[((size_t)co * L.c0 + m) * taps + t];
     } else if (L.kind == L_CONV) {
       const int cin = L.c0 + L.c1, ncob = L.cout / GC_COB;
       pk.resize((size_t)cin * L.cout * taps);
@@ -398,7 +413,7 @@ extern "C" int dwmh_commit_weights(dwmh_ctx* c) {
   }
   if (!c->buffers_ready) {
     CU_TRY(cudaMalloc((void**)&c->stats_arena, c->stats_bytes));
-    CU_TRY(cudaMalloc((void**)&c->probs, (size_t)maxN * 2 * c->P() * sizeof(float)));
+    CU_TRY(cudaMalloc((void**)&c->probs, (size_t)maxN * c->d.num_classes * c->P() * sizeof(float)));
     size_t off = 0;
     for (int i = 0; i < nL; ++i) {
       Layer& L = c->layers[i];
@@ -416,10 +431,11 @@ extern "C" int dwmh_commit_weights(dwmh_ctx* c) {
     tc_free(L.tc);
     std::string why;
     if (L.kind == L_FIRST) {
-      if (L.k[0] == 3 && L.k[1] == 3 && L.k[2] == 3 && L.c0 == 1) {
-        std::vector<float> w27((size_t)27 * L.cout);
-        for (int co = 0; co < L.cout; ++co) for (int t = 0; t < 27; ++t) w27[(size_t)t * L.cout + co] = L.w[(size_t)co * 27 + t];
-        if (tc_prepare_first(L.tc, w27, L.cout, L.out_sp, c->bf16, L.raw, &why))
+      if (L.k[0] == 3 && L.k[1] == 3 && L.k[2] == 3 && L.c0 <= DWMH_MAX_IN_CHANNELS) {
+        std::vector<float> w27((size_t)L.c0 * 27 * L.cout);      // [modality][tap][Cout]
+        for (int co = 0; co < L.cout; ++co) for (int m = 0; m < L.c0; ++m) for (int t = 0; t < 27; ++t)
+          w27[((size_t)m * 27 + t) * L.cout + co] = L.w[((size_t)co * L.c0 + m) * 27 + t];
+        if (tc_prepare_first(L.tc, w27, L.cout, L.out_sp, c->bf16, L.raw, &why, L.c0))
           if (!why.empty()) return fail("tcgen05 setup for %s failed: %s", L.name.c_str(), why.c_str());
       }
       continue;
@@ -588,6 +604,18 @@ extern "C" int dwmh_zscore(dwmh_ctx* c, float* vol, const int8_t* seg, int64_t n
 // ------------------------------------------------------------------------------------------------
 // forward
 // ------------------------------------------------------------------------------------------------
+// head of a model with NC = 3 .. DWMH_MAX_CLASSES classes
+template <typename T>
+static int launch_head_c(int NC, dim3 grid, cudaStream_t st, const T* y, NormParams np, const float* w, float* probs, int C, int64_t V) {
+  const size_t smem = (size_t)(2 + NC) * C * sizeof(float);
+  switch (NC) {
+#define DWMH_HEAD_C(K) case K: head_softmax_c_kernel<T, K><<<grid, 256, smem, st>>>(y, np, w, probs, C, V); return 0
+    DWMH_HEAD_C(3); DWMH_HEAD_C(4); DWMH_HEAD_C(5); DWMH_HEAD_C(6); DWMH_HEAD_C(7); DWMH_HEAD_C(8);
+#undef DWMH_HEAD_C
+    default: return fail("internal: no head for %d classes", NC);
+  }
+}
+
 // One batch of forwards on one stream.  Every conv / transposed conv is a conv3_tc_kernel launch (tcgen05) unless the layer
 // shape is unsupported or dwmh_set_force_generic is on (CUDA-core cross-check kernels).
 template <typename T>
@@ -620,16 +648,20 @@ static int forward_impl(dwmh_ctx* c, const float* src, int patch_mode, int SX, i
     const bool use_tc = L.tc.enabled && !c->force_generic;
     L.stats_mean_var = use_tc && L.has_norm;
     if (L.kind == L_FIRST && use_tc) {
-      TcFirstSrc fs{src, metas, patch_mode, SY, SZ};
+      TcFirstSrc fs{src, metas, patch_mode, SY, SZ, patch_mode ? c->P() : (int64_t)SX * SY * SZ};
       DW_TRY(tc_timed(L, [&] { return tc_launch<T>(L.tc, nb, L.sums, c->stat_partials, c->num_sms, st, &g_err, nullptr, &fs); }));
     } else if (L.kind == L_FIRST) {
       FirstConvParams p;
       p.src = src; p.metas = metas; p.w = L.w_dev; p.out = L.raw; p.sums = L.sums; p.patch_mode = patch_mode;
       p.SX = SX; p.SY = SY; p.SZ = SZ; p.px = L.out_sp[0]; p.py = L.out_sp[1]; p.pz = L.out_sp[2];
       p.kd = L.k[0]; p.kh = L.k[1]; p.kw = L.k[2]; p.Cout = L.cout;
+      p.Cin = L.c0; p.mstride = (int64_t)SX * SY * SZ;
       dim3 grid((unsigned)((L.vout() + 256 * FC_VPT - 1) / (256 * FC_VPT)), nb);
-      const size_t smem = ((size_t)taps * L.cout + 2 * L.cout) * sizeof(float);
-      if (taps == 27 && L.cout <= 32 && L.out_sp[2] % 2 == 0) {
+      const size_t smem = ((size_t)L.c0 * taps * L.cout + 2 * L.cout) * sizeof(float);
+      if (L.c0 > 1) {
+        if (taps == 27) conv_first_mm_kernel<T, true><<<grid, 256, smem, st>>>(p);
+        else conv_first_mm_kernel<T, false><<<grid, 256, smem, st>>>(p);
+      } else if (taps == 27 && L.cout <= 32 && L.out_sp[2] % 2 == 0) {
         dim3 grid2((unsigned)((L.vout() / 2 + 128 * FC_VPT - 1) / (128 * FC_VPT)), nb);
         conv_first_k3x2_kernel<T><<<grid2, 128, smem, st>>>(p);
       } else if (taps == 27) conv_first_kernel<T, true><<<grid, 256, smem, st>>>(p);
@@ -682,8 +714,13 @@ static int forward_impl(dwmh_ctx* c, const float* src, int patch_mode, int SX, i
   Layer& L = c->layers[c->last_conv];
   const int64_t head_items = (L.cout == 32 && (L.vout() & 1) == 0) ? L.vout() / 2 : L.vout();      // two voxels per thread in the usual head
   dim3 grid((unsigned)((head_items + 255) / 256), nb);
-  DW_TRY(cls_timed(2, (double)nb * L.vout() * (2.0 * L.cout + 8.0), [&] {
-    head_softmax_kernel<T><<<grid, 256, 4 * L.cout * sizeof(float), st>>>((const T*)L.out, norm_of(L), c->w_head_dev, c->probs, L.cout, L.vout()); return 0; }));
+  const int NC = c->d.num_classes;
+  DW_TRY(cls_timed(2, (double)nb * L.vout() * (2.0 * L.cout + 4.0 * NC), [&] {
+    if (NC == 2) {
+      head_softmax_kernel<T><<<grid, 256, 4 * L.cout * sizeof(float), st>>>((const T*)L.out, norm_of(L), c->w_head_dev, c->probs, L.cout, L.vout());
+      return 0;
+    }
+    return launch_head_c<T>(NC, grid, st, (const T*)L.out, norm_of(L), c->w_head_dev, c->probs, L.cout, L.vout()); }));
   c->launches++;
   c->conv_flops += 2.0 * L.vout() * L.cout * c->d.num_classes * nb;
   CU_TRY(cudaGetLastError());
@@ -701,10 +738,11 @@ extern "C" int dwmh_forward_patches(dwmh_ctx* c, const float* patches, int32_t n
   cudaStream_t st = (cudaStream_t)stream_;
   DEV_GUARD(c->device);
   const int64_t P = c->P();
+  const int NM = c->d.in_channels, NC = c->d.num_classes;
   for (int b = 0; b < n; b += c->max_batch) {
     const int nb = std::min(c->max_batch, n - b);
-    DW_TRY(forward(c, patches + (size_t)b * P, 1, 0, 0, 0, nullptr, nb, st));
-    CU_TRY(cudaMemcpyAsync(probs_out + (size_t)b * 2 * P, c->probs, (size_t)nb * 2 * P * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    DW_TRY(forward(c, patches + (size_t)b * NM * P, 1, 0, 0, 0, nullptr, nb, st));
+    CU_TRY(cudaMemcpyAsync(probs_out + (size_t)b * NC * P, c->probs, (size_t)nb * NC * P * sizeof(float), cudaMemcpyDeviceToDevice, st));
   }
   return 0;
 }
@@ -780,6 +818,7 @@ extern "C" int dwmh_predict_3d(dwmh_ctx* c, const float* vol, int32_t X, int32_t
   CU_TRY(cudaMemcpyAsync(c->metas_dev, metas.data(), metas.size() * sizeof(SampleMeta), cudaMemcpyHostToDevice, st));
   const int tiles_per_batch = std::max(1, c->max_batch / M);
   const int64_t P = c->P();
+  const int NC = c->d.num_classes;
   float conv_ms = 0.f, agg_ms = 0.f;
   if (c->stage_timing) {
     while (c->tcev.size() < 256) { cudaEvent_t e; CU_TRY(cudaEventCreate(&e)); c->tcev.push_back(e); }
@@ -794,9 +833,14 @@ extern "C" int dwmh_predict_3d(dwmh_ctx* c, const float* vol, int32_t X, int32_t
     DW_TRY(forward(c, vol, 0, X, Y, Z, c->metas_dev + (size_t)t0 * M, tb * M, st));
     if (c->stage_timing) CU_TRY(cudaEventRecord(c->ev[1], st));
     for (int t = 0; t < tb; ++t) {
-      aggregate_tile_kernel<<<(unsigned)((P + 255) / 256), 256, 0, st>>>(
-          c->probs + (size_t)t * M * 2 * P, c->metas_dev + (size_t)(t0 + t) * M, M, gauss ? c->gauss_dev : nullptr,
-          agg, wgt, ps[0], ps[1], ps[2], X, Y, Z);
+      if (NC == 2)
+        aggregate_tile_kernel<<<(unsigned)((P + 255) / 256), 256, 0, st>>>(
+            c->probs + (size_t)t * M * 2 * P, c->metas_dev + (size_t)(t0 + t) * M, M, gauss ? c->gauss_dev : nullptr,
+            agg, wgt, ps[0], ps[1], ps[2], X, Y, Z);
+      else
+        aggregate_tile_c_kernel<<<(unsigned)((P + 255) / 256), 256, 0, st>>>(
+            c->probs + (size_t)t * M * NC * P, c->metas_dev + (size_t)(t0 + t) * M, M, NC, gauss ? c->gauss_dev : nullptr,
+            agg, wgt, ps[0], ps[1], ps[2], X, Y, Z);
       c->launches++;
     }
     if (c->stage_timing) {
@@ -847,6 +891,12 @@ extern "C" int dwmh_finalize(dwmh_ctx* c, const float* agg, const float* wgt, fl
   cudaStream_t st = (cudaStream_t)stream_;
   DEV_GUARD(c->device);
   const int64_t V = (int64_t)X * Y * Z;
+  if (c->d.num_classes != 2) {
+    finalize_c_kernel<<<c->num_sms * 8, 256, 0, st>>>(agg, wgt, softmax, seg, c->d.num_classes, V);
+    c->launches++;
+    CU_TRY(cudaGetLastError());
+    return 0;
+  }
   const bool vec = (V & 3) == 0 && !((reinterpret_cast<uintptr_t>(agg) | reinterpret_cast<uintptr_t>(wgt) | reinterpret_cast<uintptr_t>(softmax)) & 15) &&
                    !(reinterpret_cast<uintptr_t>(seg) & 3);
   if (vec) finalize_kernel<true><<<c->num_sms * 8, 256, 0, st>>>(agg, wgt, softmax, seg, V);
@@ -869,6 +919,16 @@ extern "C" int dwmh_argmax2(dwmh_ctx* c, const float* p, uint8_t* seg, int64_t V
   if (!c || !p || !seg) return fail("dwmh_argmax2: null argument");
   DEV_GUARD(c->device);
   argmax2_kernel<<<c->num_sms * 8, 256, 0, (cudaStream_t)stream_>>>(p, seg, V);
+  c->launches++;
+  CU_TRY(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int dwmh_argmax(dwmh_ctx* c, const float* p, int32_t num_classes, uint8_t* seg, int64_t V, void* stream_) {
+  if (!c || !p || !seg) return fail("dwmh_argmax: null argument");
+  if (num_classes < 1 || num_classes > 255) return fail("dwmh_argmax: num_classes=%d outside 1..255 (uint8 labels)", num_classes);
+  DEV_GUARD(c->device);
+  argmax_c_kernel<<<c->num_sms * 8, 256, 0, (cudaStream_t)stream_>>>(p, num_classes, seg, V);
   c->launches++;
   CU_TRY(cudaGetLastError());
   return 0;
@@ -963,40 +1023,48 @@ static int predict_volume_host_impl(dwmh_ctx* c, const float* vol_host, const in
   const int bx = (PX - X) / 2, by = (PY - Y) / 2, bz = (PZ - Z) / 2;
   const bool padded = PX != X || PY != Y || PZ != Z;
   const int64_t PV = (int64_t)PX * PY * PZ;
-  DW_TRY(grow(&c->hv_vol, &c->hv_vol_cap, (size_t)V));
-  DW_TRY(grow(&c->hv_agg, &c->hv_agg_cap, (size_t)2 * PV));
+  // modalities: vol_host [NM][X][Y][Z]; on the device each channel starts 16-byte aligned (z-score's vector accesses)
+  const int NM = c->d.in_channels, NC = c->d.num_classes;
+  const int64_t Vp = NM == 1 ? V : (V + 3) & ~(int64_t)3;
+  DW_TRY(grow(&c->hv_vol, &c->hv_vol_cap, (size_t)NM * Vp));
+  DW_TRY(grow(&c->hv_agg, &c->hv_agg_cap, (size_t)NC * PV));
   DW_TRY(grow(&c->hv_wgt, &c->hv_wgt_cap, (size_t)PV));
   DW_TRY(grow(&c->hv_seg, &c->hv_seg_cap, (size_t)PV));
-  CU_TRY(cudaMemcpyAsync(c->hv_vol, vol_host, V * sizeof(float), cudaMemcpyHostToDevice, st));
+  for (int m = 0; m < NM; ++m)
+    CU_TRY(cudaMemcpyAsync(c->hv_vol + (size_t)m * Vp, vol_host + (size_t)m * V, V * sizeof(float), cudaMemcpyHostToDevice, st));
   const int8_t* mask_dev = nullptr;
   if (seg_mask_host) {
     // the crop mask rides in the (not yet used) label buffer: 1 byte per voxel, 4-byte aligned
     CU_TRY(cudaMemcpyAsync(c->hv_seg, seg_mask_host, V, cudaMemcpyHostToDevice, st));
     mask_dev = reinterpret_cast<const int8_t*>(c->hv_seg);
   }
-  if (zscore_mask_mode >= 0) DW_TRY(dwmh_zscore(c, c->hv_vol, mask_dev, V, zscore_mask_mode, nullptr, st));
+  // nnU-Net normalises every modality on its own (same mask for all of them here)
+  if (zscore_mask_mode >= 0)
+    for (int m = 0; m < NM; ++m) DW_TRY(dwmh_zscore(c, c->hv_vol + (size_t)m * Vp, mask_dev, V, zscore_mask_mode, nullptr, st));
   const float* vol_dev = c->hv_vol;
-  if (padded) {
-    DW_TRY(grow(&c->hv_pad, &c->hv_pad_cap, (size_t)PV));
-    CU_TRY(cudaMemsetAsync(c->hv_pad, 0, PV * sizeof(float), st));
-    cudaMemcpy3DParms cp = {};
-    cp.srcPtr = make_cudaPitchedPtr(c->hv_vol, Z * sizeof(float), Z, Y);
-    cp.dstPtr = make_cudaPitchedPtr(c->hv_pad, PZ * sizeof(float), PZ, PY);
-    cp.dstPos = make_cudaPos(bz * sizeof(float), by, bx);
-    cp.extent = make_cudaExtent(Z * sizeof(float), Y, X);
-    cp.kind = cudaMemcpyDeviceToDevice;
-    CU_TRY(cudaMemcpy3DAsync(&cp, st));
+  if (padded || Vp != V) {
+    DW_TRY(grow(&c->hv_pad, &c->hv_pad_cap, (size_t)NM * PV));
+    if (padded) CU_TRY(cudaMemsetAsync(c->hv_pad, 0, NM * PV * sizeof(float), st));
+    for (int m = 0; m < NM; ++m) {
+      cudaMemcpy3DParms cp = {};
+      cp.srcPtr = make_cudaPitchedPtr(c->hv_vol + (size_t)m * Vp, Z * sizeof(float), Z, Y);
+      cp.dstPtr = make_cudaPitchedPtr(c->hv_pad + (size_t)m * PV, PZ * sizeof(float), PZ, PY);
+      cp.dstPos = make_cudaPos(bz * sizeof(float), by, bx);
+      cp.extent = make_cudaExtent(Z * sizeof(float), Y, X);
+      cp.kind = cudaMemcpyDeviceToDevice;
+      CU_TRY(cudaMemcpy3DAsync(&cp, st));
+    }
     vol_dev = c->hv_pad;
   }
-  CU_TRY(cudaMemsetAsync(c->hv_agg, 0, 2 * PV * sizeof(float), st));
+  CU_TRY(cudaMemsetAsync(c->hv_agg, 0, NC * PV * sizeof(float), st));
   CU_TRY(cudaMemsetAsync(c->hv_wgt, 0, PV * sizeof(float), st));
   DW_TRY(dwmh_predict_3d(c, vol_dev, PX, PY, PZ, step_size, do_mirroring, mirror_axes_mask, use_gaussian, c->hv_agg, c->hv_wgt, 0, -1, st));
   DW_TRY(dwmh_finalize(c, c->hv_agg, c->hv_wgt, c->hv_agg, c->hv_seg, PX, PY, PZ, st));
   if (!padded) {
-    if (softmax_host) CU_TRY(cudaMemcpyAsync(softmax_host, c->hv_agg, 2 * V * sizeof(float), cudaMemcpyDeviceToHost, st));
+    if (softmax_host) CU_TRY(cudaMemcpyAsync(softmax_host, c->hv_agg, NC * V * sizeof(float), cudaMemcpyDeviceToHost, st));
     if (seg_host) CU_TRY(cudaMemcpyAsync(seg_host, c->hv_seg, V, cudaMemcpyDeviceToHost, st));
   } else {
-    for (int ch = 0; ch < 2 && softmax_host; ++ch) {
+    for (int ch = 0; ch < NC && softmax_host; ++ch) {
       cudaMemcpy3DParms cp = {};
       cp.srcPtr = make_cudaPitchedPtr(c->hv_agg + (size_t)ch * PV, PZ * sizeof(float), PZ, PY);
       cp.srcPos = make_cudaPos(bz * sizeof(float), by, bx);

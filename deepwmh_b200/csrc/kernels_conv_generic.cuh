@@ -27,6 +27,8 @@ struct FirstConvParams {
   int px, py, pz;
   int kd, kh, kw;
   int Cout;
+  int Cin;                     // modalities (conv_first_mm_kernel; the single-modality kernels ignore it)
+  int64_t mstride;             // floats between two modalities of the volume (patch_mode 0)
 };
 
 // K3: kernel is 3x3x3 (fully unrolled taps, inputs stay in registers).  Each thread walks FC_VPT voxels
@@ -214,6 +216,114 @@ __global__ void __launch_bounds__(128) conv_first_k3x2_kernel(FirstConvParams p)
       }
     }
   }
+#pragma unroll
+  for (int k = 16; k >= 1; k >>= 1) {
+    const bool up = (lane & k) != 0;
+#pragma unroll
+    for (int i = 0; i < k; ++i) {
+      const float sa_ = up ? rs[i] : rs[i + k], ka_ = up ? rs[i + k] : rs[i];
+      const float sb_ = up ? rq[i] : rq[i + k], kb_ = up ? rq[i + k] : rq[i];
+      rs[i] = ka_ + __shfl_xor_sync(0xffffffffu, sa_, k);
+      rq[i] = kb_ + __shfl_xor_sync(0xffffffffu, sb_, k);
+    }
+  }
+  if (lane < p.Cout) { atomicAdd(&sstat[lane * 2], rs[0]); atomicAdd(&sstat[lane * 2 + 1], rq[0]); }
+  __syncthreads();
+  for (int c = threadIdx.x; c < 2 * p.Cout; c += blockDim.x)
+    atomicAdd(p.sums + (size_t)n * p.Cout * 2 + c, (double)sstat[c]);
+}
+
+// ---------------------------------------------------------------------------------------------
+// First conv with Cin = p.Cin > 1 modalities (nnU-Net models with several input images): the volume is [Cin][SX][SY][SZ]
+// (patch_mode 0, modalities p.mstride floats apart) or patches [n][Cin][px][py][pz].  One thread per output voxel; per
+// 8-channel output chunk the taps of modality 0, 1, ... accumulate in that order into one fp32 sum.  w: [Cin][taps][Cout].
+// Statistics as in conv_first_kernel.  Requires Cout <= 32.
+// ---------------------------------------------------------------------------------------------
+template <typename T, bool K3>
+__global__ void __launch_bounds__(256) conv_first_mm_kernel(FirstConvParams p) {
+  extern __shared__ float smf[];                 // weights [Cin][taps][Cout], then stats [Cout][2]
+  const int kd = K3 ? 3 : p.kd, kh = K3 ? 3 : p.kh, kw = K3 ? 3 : p.kw;
+  const int taps = kd * kh * kw;
+  float* sw = smf;
+  float* sstat = smf + p.Cin * taps * p.Cout;
+  for (int i = threadIdx.x; i < p.Cin * taps * p.Cout; i += blockDim.x) sw[i] = p.w[i];
+  for (int i = threadIdx.x; i < 2 * p.Cout; i += blockDim.x) sstat[i] = 0.f;
+  __syncthreads();
+  const int n = blockIdx.y;
+  const int64_t P = (int64_t)p.px * p.py * p.pz;
+  int ox = 0, oy = 0, oz = 0, flip = 0;
+  const float* src = p.src;
+  int SY = p.SY, SZ = p.SZ;
+  int64_t mstride = p.mstride;
+  if (p.patch_mode) { src += (size_t)n * p.Cin * P; SY = p.py; SZ = p.pz; mstride = P; }
+  else { const SampleMeta m = p.metas[n]; ox = m.ox; oy = m.oy; oz = m.oz; flip = m.flip; }
+  const int lane = threadIdx.x & 31;
+  float rs[32], rq[32];
+#pragma unroll
+  for (int q = 0; q < 32; ++q) { rs[q] = 0.f; rq[q] = 0.f; }
+  for (int it = 0; it < FC_VPT; ++it) {
+    const int64_t v = ((int64_t)blockIdx.x * FC_VPT + it) * blockDim.x + threadIdx.x;
+    const bool active = v < P;
+    const int k = (int)(v % p.pz), j = (int)((v / p.pz) % p.py), i = (int)(v / ((int64_t)p.pz * p.py));
+    float acc[4][8];
+#pragma unroll
+    for (int cc = 0; cc < 4; ++cc)
+#pragma unroll
+      for (int q = 0; q < 8; ++q) acc[cc][q] = 0.f;
+    for (int m = 0; m < p.Cin; ++m) {
+      float xin[27];
+#pragma unroll
+      for (int a = 0; a < 3; ++a)
+#pragma unroll
+        for (int b = 0; b < 3; ++b)
+#pragma unroll
+          for (int c = 0; c < 3; ++c) {
+            float val = 0.f;
+            if (a < kd && b < kh && c < kw) {
+              const int ii = i + a - (kd >> 1), jj = j + b - (kh >> 1), kk = k + c - (kw >> 1);
+              if (active && ii >= 0 && ii < p.px && jj >= 0 && jj < p.py && kk >= 0 && kk < p.pz) {
+                const int si = ox + ((flip & 4) ? p.px - 1 - ii : ii);
+                const int sj = oy + ((flip & 2) ? p.py - 1 - jj : jj);
+                const int sk = oz + ((flip & 1) ? p.pz - 1 - kk : kk);
+                val = __ldg(src + (size_t)m * mstride + ((size_t)si * SY + sj) * SZ + sk);
+              }
+            }
+            xin[(a * 3 + b) * 3 + c] = val;
+          }
+      const float* wm = sw + (size_t)m * taps * p.Cout;
+#pragma unroll
+      for (int cc = 0; cc < 4; ++cc) {
+        if (cc < (p.Cout >> 3)) {
+#pragma unroll
+          for (int a = 0; a < 3; ++a)
+#pragma unroll
+            for (int b = 0; b < 3; ++b)
+#pragma unroll
+              for (int c = 0; c < 3; ++c) {
+                if (a < kd && b < kh && c < kw) {
+                  const int t = (a * kh + b) * kw + c;
+                  const float4 w0 = *reinterpret_cast<const float4*>(wm + t * p.Cout + cc * 8);
+                  const float4 w1 = *reinterpret_cast<const float4*>(wm + t * p.Cout + cc * 8 + 4);
+                  const float x = xin[(a * 3 + b) * 3 + c];
+                  float* ac = acc[cc];
+                  ac[0] = fmaf(x, w0.x, ac[0]); ac[1] = fmaf(x, w0.y, ac[1]); ac[2] = fmaf(x, w0.z, ac[2]); ac[3] = fmaf(x, w0.w, ac[3]);
+                  ac[4] = fmaf(x, w1.x, ac[4]); ac[5] = fmaf(x, w1.y, ac[5]); ac[6] = fmaf(x, w1.z, ac[6]); ac[7] = fmaf(x, w1.w, ac[7]);
+                }
+              }
+        }
+      }
+    }
+    uint4* outp = reinterpret_cast<uint4*>(p.out) + (size_t)n * (p.Cout >> 3) * P + v;
+#pragma unroll
+    for (int cc = 0; cc < 4; ++cc) {
+      if (cc < (p.Cout >> 3) && active) {
+        outp[(size_t)cc * P] = pack8<T>(acc[cc]);
+#pragma unroll
+        for (int q = 0; q < 8; ++q) { rs[cc * 8 + q] += acc[cc][q]; rq[cc * 8 + q] = fmaf(acc[cc][q], acc[cc][q], rq[cc * 8 + q]); }
+      }
+    }
+  }
+  // transposing butterfly: lane l ends with the warp total of channel l
 #pragma unroll
   for (int k = 16; k >= 1; k >>= 1) {
     const bool up = (lane & k) != 0;

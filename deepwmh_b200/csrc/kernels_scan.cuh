@@ -203,6 +203,106 @@ __global__ void __launch_bounds__(256) head_softmax_kernel(const T* __restrict__
 }
 
 // ---------------------------------------------------------------------------------------------
+// The same head for NC = 3..8 classes (models with more than background + one label): logits l_k = sum_c w[k][c] x_c,
+// p_k = exp(l_k - max) / sum_k' exp(l_k' - max) in fp32, summed in class order.  probs: [n][NC][V].  Loads and shared
+// coefficient reads as in head_softmax_kernel (two voxels per thread and 256-bit loads when C == 32 and V is even).
+// ---------------------------------------------------------------------------------------------
+template <int NC>
+__device__ __forceinline__ void softmax_nc(const float (&l)[NC], float (&p)[NC]) {
+  float m = l[0];
+#pragma unroll
+  for (int k = 1; k < NC; ++k) m = fmaxf(m, l[k]);
+  float e[NC], s = 0.f;
+#pragma unroll
+  for (int k = 0; k < NC; ++k) { e[k] = expf(l[k] - m); s += e[k]; }
+#pragma unroll
+  for (int k = 0; k < NC; ++k) p[k] = e[k] / s;
+}
+
+template <typename T, int NC>
+__global__ void __launch_bounds__(256) head_softmax_c_kernel(const T* __restrict__ y, NormParams np,
+                                                             const float* __restrict__ w_head,   // [NC][C]
+                                                             float* __restrict__ probs, int C, int64_t V) {
+  extern __shared__ __align__(16) float sm[];          // a[C], b[C], w[NC][C]
+  float* sa = sm; float* sb = sm + C; float* sw = sm + 2 * C;
+  const int n = blockIdx.y;
+  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+    float a = 1.f, b = 0.f;
+    if (np.sums) norm_coeffs(np, n, C, c, a, b);
+    sa[c] = a; sb[c] = b;
+  }
+  for (int i = threadIdx.x; i < NC * C; i += blockDim.x) sw[i] = w_head[i];
+  __syncthreads();
+  if (C == 32 && (V & 1) == 0) {
+    const int64_t v2 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (2 * v2 >= V) return;
+    const uint4* yp2 = reinterpret_cast<const uint4*>(y) + (size_t)n * 4 * V + 2 * v2;
+    uint4 q[4][2];
+#pragma unroll
+    for (int cc = 0; cc < 4; ++cc) ld_global_256(yp2 + (size_t)cc * V, q[cc][0], q[cc][1]);
+    float l[2][NC];
+#pragma unroll
+    for (int e = 0; e < 2; ++e)
+#pragma unroll
+      for (int k = 0; k < NC; ++k) l[e][k] = 0.f;
+    const float4* sa4 = reinterpret_cast<const float4*>(sa); const float4* sb4 = reinterpret_cast<const float4*>(sb);
+    const float4* sw4 = reinterpret_cast<const float4*>(sw);
+#pragma unroll
+    for (int cc = 0; cc < 4; ++cc) {
+      float f[2][8];
+      unpack8<T>(q[cc][0], f[0]); unpack8<T>(q[cc][1], f[1]);
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const float4 a4 = sa4[cc * 2 + h], b4 = sb4[cc * 2 + h];
+        const float ca[4] = {a4.x, a4.y, a4.z, a4.w}, cb[4] = {b4.x, b4.y, b4.z, b4.w};
+        float x[2][4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+#pragma unroll
+          for (int e = 0; e < 2; ++e) x[e][j] = np.sums ? lrelu(fmaf(ca[j], f[e][h * 4 + j], cb[j])) : f[e][h * 4 + j];
+#pragma unroll
+        for (int k = 0; k < NC; ++k) {
+          const float4 u4 = sw4[k * 8 + cc * 2 + h];
+          const float cu[4] = {u4.x, u4.y, u4.z, u4.w};
+#pragma unroll
+          for (int j = 0; j < 4; ++j)
+#pragma unroll
+            for (int e = 0; e < 2; ++e) l[e][k] = fmaf(cu[j], x[e][j], l[e][k]);
+        }
+      }
+    }
+    float p[2][NC];
+    softmax_nc<NC>(l[0], p[0]);
+    softmax_nc<NC>(l[1], p[1]);
+#pragma unroll
+    for (int k = 0; k < NC; ++k)
+      *reinterpret_cast<float2*>(probs + ((size_t)n * NC + k) * V + 2 * v2) = make_float2(p[0][k], p[1][k]);
+    return;
+  }
+  const int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (v >= V) return;
+  const uint4* yp = reinterpret_cast<const uint4*>(y) + (size_t)n * (C >> 3) * V + v;
+  float l[NC];
+#pragma unroll
+  for (int k = 0; k < NC; ++k) l[k] = 0.f;
+  for (int cc = 0; cc < (C >> 3); ++cc) {
+    float f[8];
+    unpack8<T>(ld_stream(yp + (size_t)cc * V), f);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const int c = cc * 8 + j;
+      const float x = np.sums ? lrelu(fmaf(sa[c], f[j], sb[c])) : f[j];
+#pragma unroll
+      for (int k = 0; k < NC; ++k) l[k] = fmaf(sw[k * C + c], x, l[k]);
+    }
+  }
+  float p[NC];
+  softmax_nc<NC>(l, p);
+#pragma unroll
+  for (int k = 0; k < NC; ++k) probs[((size_t)n * NC + k) * V + v] = p[k];
+}
+
+// ---------------------------------------------------------------------------------------------
 // a11/a12  One tile: result = sum_m (1/M) * unflip_m(p_m); result *= gaussian; agg[:, tile] += result;
 // wgt[tile] += gaussian.  Same fp32 operation order as the reference.  Tiles are aggregated by
 // consecutive launches on one stream, so the overlap-add is deterministic (no atomics).
@@ -236,6 +336,45 @@ __global__ void __launch_bounds__(256) aggregate_tile_kernel(const float* __rest
   const int64_t dst = ((int64_t)(metas[0].ox + i) * Y + (metas[0].oy + j)) * Z + (metas[0].oz + k);
   agg[dst] += r0;
   agg[V + dst] += r1;
+  wgt[dst] += g;
+}
+
+// The same for NC <= 8 classes: probs [M][NC][P]; per class the operation order of aggregate_tile_kernel.
+__global__ void __launch_bounds__(256) aggregate_tile_c_kernel(const float* __restrict__ probs,
+                                                               const SampleMeta* __restrict__ metas, int M, int NC,
+                                                               const float* __restrict__ gauss,   // [P] or nullptr
+                                                               float* __restrict__ agg, float* __restrict__ wgt,
+                                                               int px, int py, int pz, int X, int Y, int Z) {
+  const int64_t P = (int64_t)px * py * pz;
+  const int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (v >= P) return;
+  const int k = (int)(v % pz);
+  const int j = (int)((v / pz) % py);
+  const int i = (int)(v / ((int64_t)pz * py));
+  const float inv = 1.0f / (float)M;
+  float r[8];
+#pragma unroll
+  for (int c = 0; c < 8; ++c) r[c] = 0.f;
+  for (int m = 0; m < M; ++m) {
+    const int f = metas[m].flip;
+    const int kk = (f & 1) ? pz - 1 - k : k;
+    const int jj = (f & 2) ? py - 1 - j : j;
+    const int ii = (f & 4) ? px - 1 - i : i;
+    const int64_t src = ((int64_t)ii * py + jj) * pz + kk;
+#pragma unroll
+    for (int c = 0; c < 8; ++c)
+      if (c < NC) r[c] += inv * probs[((size_t)m * NC + c) * P + src];
+  }
+  const float g = gauss ? gauss[v] : 1.0f;
+  const int64_t V = (int64_t)X * Y * Z;
+  const int64_t dst = ((int64_t)(metas[0].ox + i) * Y + (metas[0].oy + j)) * Z + (metas[0].oz + k);
+#pragma unroll
+  for (int c = 0; c < 8; ++c) {
+    if (c < NC) {
+      if (gauss) r[c] *= g;
+      agg[(size_t)c * V + dst] += r[c];
+    }
+  }
   wgt[dst] += g;
 }
 
@@ -302,6 +441,38 @@ __global__ void __launch_bounds__(256) finalize_kernel(const float* agg, const f
     const float p0 = agg[i] / w, p1 = agg[V + i] / w;
     if (softmax_out) { softmax_out[i] = p0; softmax_out[V + i] = p1; }
     if (seg) seg[i] = p1 > p0 ? 1 : 0;
+  }
+}
+
+// NC classes: softmax_out [NC][V] (may alias agg) = agg / wgt; seg = the first class holding the maximum (numpy.argmax).
+__global__ void __launch_bounds__(256) finalize_c_kernel(const float* agg, const float* __restrict__ wgt, float* softmax_out,
+                                                         uint8_t* __restrict__ seg, int NC, int64_t V) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < V; i += stride) {
+    const float w = wgt[i];
+    float best = agg[i] / w;
+    int arg = 0;
+    if (softmax_out) softmax_out[i] = best;
+    for (int c = 1; c < NC; ++c) {
+      const float p = agg[(size_t)c * V + i] / w;
+      if (softmax_out) softmax_out[(size_t)c * V + i] = p;
+      if (p > best) { best = p; arg = c; }
+    }
+    if (seg) seg[i] = (uint8_t)arg;
+  }
+}
+
+// argmax over NC classes of p [NC][V], first maximum (numpy.argmax)
+__global__ void __launch_bounds__(256) argmax_c_kernel(const float* __restrict__ p, int NC, uint8_t* __restrict__ seg, int64_t V) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < V; i += stride) {
+    float best = p[i];
+    int arg = 0;
+    for (int c = 1; c < NC; ++c) {
+      const float x = p[(size_t)c * V + i];
+      if (x > best) { best = x; arg = c; }
+    }
+    seg[i] = (uint8_t)arg;
   }
 }
 

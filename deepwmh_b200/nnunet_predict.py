@@ -8,7 +8,8 @@ DeepWMH reaches the hot path by spawning `nnUNet_predict` with exactly these com
     nnUNet_predict ... -chk model_best                                           (DCNN_multistage.py:531-535)
 
 with RESULTS_FOLDER / CUDA_VISIBLE_DEVICES in the environment (predict.py:101,150).  This module accepts those flags with
-the same meaning: inputs `<in>/<case>_0000.nii.gz`, outputs `<out>/<case>.nii.gz` (uint8 labels), `<out>/<case>_0.nii.gz`
+the same meaning: inputs `<in>/<case>_0000.nii.gz` (models with M modalities: `<case>_0000 ... <case>_000{M-1}.nii.gz`, the
+modality order of the training data), outputs `<out>/<case>.nii.gz` (uint8 labels 0 .. C-1), `<out>/<case>_0.nii.gz`
 (background probability, the fork's --save_softmax, read back at DCNN_multistage.py:359) and a copy of plans.pkl
 (upstream copies it; DeepWMH ignores it, predict.py:159-162).  Any failure raises -> non-zero exit, which is what
 `run_shell` turns into `exit(msg)` (deepwmh/utilities/external_call.py:63-72).  Flags of upstream nnUNet_predict that
@@ -29,9 +30,19 @@ def _cases_in(folder: str) -> List[str]:
     return sorted({f[:-len("_0000.nii.gz")] for f in os.listdir(folder) if f.endswith("_0000.nii.gz")})
 
 
+def case_files(folder: str, case: str, num_modalities: int) -> List[str]:
+    """`<folder>/<case>_0000.nii.gz ... <case>_%04d.nii.gz` (modality order); raises if one of them is missing."""
+    files = [os.path.join(folder, "%s_%04d.nii.gz" % (case, m)) for m in range(num_modalities)]
+    missing = [os.path.basename(f) for f in files if not os.path.isfile(f)]
+    if missing:
+        raise RuntimeError("case %s lacks modality file(s) %s in %s (the model takes %d modalities: %s_0000 ... %s_%04d.nii.gz)"
+                           % (case, ", ".join(missing), folder, num_modalities, case, case, num_modalities - 1))
+    return files
+
+
 def main(argv=None) -> int:
     ap = argparse.ArgumentParser(prog="nnUNet_predict", description="nnU-Net v1 inference on B200 (DeepWMH drop-in subset).")
-    ap.add_argument("-i", "--input_folder", required=True, help="folder with <case>_0000.nii.gz files")
+    ap.add_argument("-i", "--input_folder", required=True, help="folder with <case>_0000.nii.gz (... <case>_000{M-1}.nii.gz) files")
     ap.add_argument("-o", "--output_folder", required=True)
     ap.add_argument("-t", "--task_name", required=True, help="task name or id, e.g. Task002_FinalModel")
     ap.add_argument("-tr", "--trainer_class_name", default="nnUNetTrainerV2")
@@ -88,6 +99,9 @@ def main(argv=None) -> int:
             raise RuntimeError("selected cases without an input file <case>_0000.nii.gz: %s" % ", ".join(missing))
         cases = [c for c in cases if c in set(args.selected_cases)]
     cases = cases[args.part_id::args.num_parts]                  # upstream's --part_id / --num_parts sharding
+    plans = _cli.load_plans(plans_path)
+    n_mod = int(plans.get("num_modalities", 1))
+    inputs = {c: case_files(args.input_folder, c, n_mod) for c in cases}     # every modality present before any GPU work
     os.makedirs(args.output_folder, exist_ok=True)
     shutil.copy(plans_path, args.output_folder)
     todo = []
@@ -102,14 +116,13 @@ def main(argv=None) -> int:
     import torch
 
     import deepwmh_b200
-    plans = _cli.load_plans(plans_path)
     trainer = deepwmh_b200.nnUNetTrainerV2(plans, device=0, max_batch=32 if not args.disable_tta else 16)   # CUDA_VISIBLE_DEVICES selects the GPU
     trainer.load_checkpoint_ram(torch.load(ckpt_path, map_location="cpu", weights_only=False), False)
     if args.step_size != 0.5:
         raise NotImplementedError("--step_size other than 0.5 is not passed by DeepWMH")
     for c in todo:
         print("predicting", c)
-        _cli.predict_case(trainer, plans, os.path.join(args.input_folder, c + "_0000.nii.gz"), os.path.join(args.output_folder, c + ".nii.gz"),
+        _cli.predict_case(trainer, plans, inputs[c], os.path.join(args.output_folder, c + ".nii.gz"),
                           softmax_file=os.path.join(args.output_folder, c + "_0.nii.gz") if args.save_softmax else None,
                           do_mirroring=not args.disable_tta)
     trainer.network.close()

@@ -74,27 +74,27 @@ def predict_volume_tile_sharded(trainer, data, do_mirroring=True, mirror_axes=(0
                                 use_gaussian=True, group=None, reduce: str = "reduce", timings: Optional[Dict] = None):
     """Tile-sharded predict_preprocessed_data_return_seg_and_softmax: every rank passes the same (c,x,y,z) array
     (numpy or a CUDA tensor) and the ranks holding the complete sum (rank 0, or all with an all-reduce) get
-    (seg uint8 [x,y,z], softmax fp32 [2,x,y,z]) back as device tensors; the others get (None, None).
+    (seg uint8 [x,y,z], softmax fp32 [C,x,y,z]) back as device tensors; the others get (None, None).
     timings (optional dict) receives device milliseconds of the stages {tiles, collective, finalize} (adds syncs)."""
     from .predictor import pad_nd_image
     net = trainer.network
     rank, world = _world(group)
     with torch.cuda.device(net.device):
         if isinstance(data, torch.Tensor) and data.is_cuda:
-            vol = data.detach()[0].to(device=net.device, dtype=torch.float32)
-            diff = [max(p - s, 0) for p, s in zip(net.patch_size, vol.shape)]
+            vol = data.detach().to(device=net.device, dtype=torch.float32)
+            diff = [max(p - s, 0) for p, s in zip(net.patch_size, vol.shape[1:])]
             pads = [(d // 2, d // 2 + d % 2) for d in diff]
             if any(diff):
                 vol = torch.nn.functional.pad(vol, (pads[2][0], pads[2][1], pads[1][0], pads[1][1], pads[0][0], pads[0][1]))
             vol = vol.contiguous()
-            sl = tuple(slice(b, vol.shape[i] - a) for i, (b, a) in enumerate(pads))
+            sl = tuple(slice(b, vol.shape[i + 1] - a) for i, (b, a) in enumerate(pads))
         else:
             padded, slicer = pad_nd_image(np.asarray(data, dtype=np.float32), net.patch_size)
-            vol = torch.from_numpy(np.ascontiguousarray(padded[0])).to(net.device)
+            vol = torch.from_numpy(np.ascontiguousarray(padded)).to(net.device)
             sl = tuple(slicer[1:])
-        X, Y, Z = vol.shape
+        X, Y, Z = vol.shape[1:]
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)] if timings is not None else None
-        agg = torch.zeros((2, X, Y, Z), dtype=torch.float32, device=net.device)
+        agg = torch.zeros((net.num_classes, X, Y, Z), dtype=torch.float32, device=net.device)
         n_tiles = net.num_tiles((X, Y, Z), step_size)
         b, e = shard_tiles(n_tiles, rank, world)
         # use_gaussian must be decided on the GLOBAL tile count (the reference: num_tiles > 1)
@@ -148,22 +148,24 @@ def make_ensemble(plans: Dict, state_dicts: Sequence[Dict], device: int = 0, act
 
 def predict_volume_ensemble(trainers: Sequence, vol: torch.Tensor, do_mirroring=True, mirror_axes=(0, 1, 2), step_size=0.5,
                             use_gaussian=True):
-    """predict_cases' `for p in params` loop (a13) with every model resident: vol = normalised fp32 [X,Y,Z] on the device
-    (each extent >= patch) -> (seg uint8 [X,Y,Z], mean softmax fp32 [2,X,Y,Z]), all on the device: per model tiled
-    prediction + finalize, running mean by dwmh_axpy (mean = sum_k softmax_k / k in model order), argmax by dwmh_argmax2."""
+    """predict_cases' `for p in params` loop (a13) with every model resident: vol = normalised fp32 [X,Y,Z] (one modality) or
+    [M,X,Y,Z] on the device (each extent >= patch) -> (seg uint8 [X,Y,Z], mean softmax fp32 [C,X,Y,Z]), all on the device: per
+    model tiled prediction + finalize, running mean by dwmh_axpy (mean = sum_k softmax_k / k in model order), argmax by
+    dwmh_argmax2 (two classes) or dwmh_argmax."""
     net0 = trainers[0].network
     k = len(trainers)
     with torch.cuda.device(net0.device):
-        X, Y, Z = vol.shape
-        mean = torch.zeros((2, X, Y, Z), dtype=torch.float32, device=net0.device)
-        agg = torch.empty((2, X, Y, Z), dtype=torch.float32, device=net0.device)
+        X, Y, Z = vol.shape[-3:]
+        C = net0.num_classes
+        mean = torch.zeros((C, X, Y, Z), dtype=torch.float32, device=net0.device)
+        agg = torch.empty((C, X, Y, Z), dtype=torch.float32, device=net0.device)
         wgt = torch.empty((X, Y, Z), dtype=torch.float32, device=net0.device)
         for tr in trainers:
             agg.zero_(); wgt.zero_()
             tr.network.accumulate_tiles(vol, agg, wgt, step_size, do_mirroring, mirror_axes, use_gaussian)
             _, probs = tr.network.finalize(agg, wgt)
             net0.axpy_(mean, probs, 1.0 / k)
-        seg = net0.argmax2(mean)
+        seg = net0.argmax(mean)
     return seg, mean
 
 

@@ -166,6 +166,16 @@ class SegmentationNetwork:
         check(self._lib.dwmh_argmax2(self._ctx, _ptr(softmax), _ptr(seg), seg.numel(), self._st()))
         return seg
 
+    def argmax(self, softmax: torch.Tensor) -> torch.Tensor:
+        """Class map uint8 [x,y,z] of fp32 probabilities [C,x,y,z] on the device; ties go to the lower class (numpy.argmax).
+        Two classes take dwmh_argmax2, more take dwmh_argmax."""
+        assert softmax.is_cuda and softmax.dtype == torch.float32 and softmax.is_contiguous()
+        if softmax.shape[0] == 2:
+            return self.argmax2(softmax)
+        seg = torch.empty(tuple(softmax.shape[1:]), dtype=torch.uint8, device=softmax.device)
+        check(self._lib.dwmh_argmax(self._ctx, _ptr(softmax), int(softmax.shape[0]), _ptr(seg), seg.numel(), self._st()))
+        return seg
+
     def normalize_(self, vol: torch.Tensor, seg: Optional[torch.Tensor] = None, mask_mode: int = 2, return_stats: bool = True):
         """In-place z-score of a device fp32 volume (a2).  mask_mode: 0 all, 1 seg>=0, 2 vol!=0.
         return_stats: (mean, std, count) on the host -- this synchronises the stream; False keeps the call asynchronous."""
@@ -180,8 +190,13 @@ class SegmentationNetwork:
     def accumulate_tiles(self, vol: torch.Tensor, agg: torch.Tensor, wgt: torch.Tensor, step_size: float,
                          do_mirroring: bool, mirror_axes: Sequence[int], use_gaussian: bool,
                          tile_begin: int = 0, tile_end: int = -1):
-        """dwmh_predict_3d on device tensors: vol [X,Y,Z] fp32, agg [2,X,Y,Z], wgt [X,Y,Z] (accumulated into)."""
-        X, Y, Z = vol.shape
+        """dwmh_predict_3d on device tensors: vol [M,X,Y,Z] fp32 (or [X,Y,Z] for one modality), agg [C,X,Y,Z], wgt [X,Y,Z]
+        (accumulated into)."""
+        X, Y, Z = vol.shape[-3:]
+        if (vol.shape[0] if vol.dim() == 4 else 1) != self.input_channels or vol.dim() not in (3, 4):
+            raise ValueError("vol must be [%d, X, Y, Z]" % self.input_channels)
+        if tuple(agg.shape) != (self.num_classes, X, Y, Z):
+            raise ValueError("agg must be [%d, X, Y, Z]" % self.num_classes)
         check(self._lib.dwmh_predict_3d(self._ctx, _ptr(vol), X, Y, Z, float(step_size), int(bool(do_mirroring)),
                                         mirror_axes_mask(mirror_axes), int(bool(use_gaussian)), _ptr(agg), _ptr(wgt),
                                         int(tile_begin), int(tile_end), self._st()))
@@ -229,10 +244,12 @@ class SegmentationNetwork:
         return len(s[0]) * len(s[1]) * len(s[2])
 
     def forward_patches(self, patches: torch.Tensor) -> torch.Tensor:
-        """softmax(Generic_UNet(x)) for x [n,1,px,py,pz] fp32 on device -> [n,2,px,py,pz] fp32."""
+        """softmax(Generic_UNet(x)) for x [n,M,px,py,pz] fp32 on device -> [n,C,px,py,pz] fp32."""
         assert patches.is_cuda and patches.dtype == torch.float32 and patches.is_contiguous()
         n = patches.shape[0]
-        out = torch.empty((n, 2) + tuple(self.patch_size), dtype=torch.float32, device=patches.device)
+        if patches.numel() != n * self.input_channels * int(np.prod(self.patch_size)):
+            raise ValueError("patches must be [n, %d, %d, %d, %d]" % ((self.input_channels,) + self.patch_size))
+        out = torch.empty((n, self.num_classes) + tuple(self.patch_size), dtype=torch.float32, device=patches.device)
         check(self._lib.dwmh_forward_patches(self._ctx, _ptr(patches), n, _ptr(out), self._st()))
         return out
 
@@ -272,7 +289,7 @@ class SegmentationNetwork:
                    use_gaussian: bool = False, pad_border_mode: str = "constant", pad_kwargs: dict = None,
                    all_in_gpu: bool = False, verbose: bool = True, mixed_precision: bool = True,
                    return_device_tensors: bool = False):
-        """[U:SegmentationNetwork.predict_3D].  x: (c, x, y, z) numpy fp32 or CUDA tensor.
+        """[U:SegmentationNetwork.predict_3D].  x: (M, x, y, z) numpy fp32 or CUDA tensor, M = input modalities.
         Returns (seg int64 [x,y,z], class_probabilities fp32 [classes,x,y,z]) as numpy arrays, or -- additive flag
         return_device_tensors -- (seg uint8, probabilities fp32) as CUDA tensors without the device-to-host copies."""
         assert step_size <= 1, "step_size must be smaller than 1. Otherwise there will be a gap between consecutive predictions"
@@ -297,19 +314,19 @@ class SegmentationNetwork:
         with torch.cuda.device(self.device):
             if isinstance(x, torch.Tensor) and x.is_cuda:
                 # device input stays on the device: zero padding (a10) with the same below / above split as pad_nd_image
-                vol = x.detach()[0].to(device=self.device, dtype=torch.float32)
-                diff = [max(p - s, 0) for p, s in zip(self.patch_size, vol.shape)]
+                vol = x.detach().to(device=self.device, dtype=torch.float32)
+                diff = [max(p - s, 0) for p, s in zip(self.patch_size, vol.shape[1:])]
                 pads = [(d // 2, d // 2 + d % 2) for d in diff]
                 if any(diff):
                     vol = torch.nn.functional.pad(vol, (pads[2][0], pads[2][1], pads[1][0], pads[1][1], pads[0][0], pads[0][1]))
                 vol = vol.contiguous()
-                slicer = (slice(None),) + tuple(slice(b, vol.shape[i] - a) for i, (b, a) in enumerate(pads))
+                slicer = (slice(None),) + tuple(slice(b, vol.shape[i + 1] - a) for i, (b, a) in enumerate(pads))
             else:
                 if isinstance(x, torch.Tensor):
                     x = x.detach().float().numpy()
                 data, slicer = pad_nd_image(np.asarray(x, dtype=np.float32), self.patch_size, pad_border_mode, pad_kwargs)
-                vol = torch.from_numpy(np.ascontiguousarray(data[0])).to(self.device, non_blocking=False)
-            X, Y, Z = vol.shape
+                vol = torch.from_numpy(np.ascontiguousarray(data)).to(self.device, non_blocking=False)
+            X, Y, Z = vol.shape[1:]
             agg = torch.zeros((self.num_classes, X, Y, Z), dtype=torch.float32, device=self.device)
             wgt = torch.zeros((X, Y, Z), dtype=torch.float32, device=self.device)
             self.accumulate_tiles(vol, agg, wgt, step_size, do_mirroring, mirror_axes, use_gaussian)
@@ -396,16 +413,18 @@ class nnUNetTrainerV2:
                                 mirror_axes=(0, 1, 2), step_size: float = 0.5, use_gaussian: bool = True,
                                 out_softmax: Optional[np.ndarray] = None, out_seg: Optional[np.ndarray] = None,
                                 seg_mask: Optional[np.ndarray] = None):
-        """raw fp32 [X,Y,Z] host volume -> (seg uint8 [X,Y,Z], softmax fp32 [2,X,Y,Z]); z-score, H2D,
-        tiled prediction, finalize and D2H all inside dwmh_predict_volume_host.  seg_mask: nnU-Net's crop mask
-        (int8, >= 0 inside) -> normalisation over that mask (dwmh_predict_volume_host_masked)."""
-        assert vol.dtype == np.float32 and vol.ndim == 3 and vol.flags.c_contiguous
-        X, Y, Z = vol.shape
-        sm = out_softmax if out_softmax is not None else np.empty((2, X, Y, Z), dtype=np.float32)
+        """raw fp32 [X,Y,Z] (one modality) or [M,X,Y,Z] host volume -> (seg uint8 [X,Y,Z], softmax fp32 [C,X,Y,Z]); z-score
+        of every modality, H2D, tiled prediction, finalize and D2H all inside dwmh_predict_volume_host.  seg_mask: nnU-Net's
+        crop mask (int8, >= 0 inside) -> normalisation over that mask (dwmh_predict_volume_host_masked)."""
+        M = self.network.input_channels
+        assert vol.dtype == np.float32 and vol.flags.c_contiguous
+        assert (vol.ndim == 3 and M == 1) or (vol.ndim == 4 and vol.shape[0] == M), "vol must be [%d, X, Y, Z]" % M
+        X, Y, Z = vol.shape[-3:]
+        sm = out_softmax if out_softmax is not None else np.empty((self.network.num_classes, X, Y, Z), dtype=np.float32)
         sg = out_seg if out_seg is not None else np.empty((X, Y, Z), dtype=np.uint8)
         net = self.network
         if seg_mask is not None:
-            assert seg_mask.dtype == np.int8 and seg_mask.shape == vol.shape and seg_mask.flags.c_contiguous
+            assert seg_mask.dtype == np.int8 and seg_mask.shape == (X, Y, Z) and seg_mask.flags.c_contiguous
             with torch.cuda.device(net.device):
                 check(net._lib.dwmh_predict_volume_host_masked(
                     net._ctx, vol.ctypes.data_as(C.c_void_p), seg_mask.ctypes.data_as(C.c_void_p), X, Y, Z, float(step_size),

@@ -1,6 +1,6 @@
 """File-level steps either side of the hot path (SURVEY.md section 8f-1/8f-2), host side.
 
-Restates, for the single-modality case DeepWMH uses, what nnU-Net v1 does around predict_3D:
+Restates, for DeepWMH's single modality and for models with up to four, what nnU-Net v1 does around predict_3D:
   * crop_to_nonzero                      [U:preprocessing/cropping.py]      (scipy binary_fill_holes, as upstream)
   * paste-back export                    [U:inference/segmentation_export.py]
   * remove_3mm_sparks                    deepwmh/analysis/image_ops.py:325-367 (scipy.ndimage.label, as the reference)
@@ -148,17 +148,41 @@ def remove_3mm_sparks(mask: np.ndarray, voxel_size: Sequence[float]) -> np.ndarr
     return remove_sparks(mask, max(mv, 2))
 
 
+def read_modalities(input_files: Sequence[str]):
+    """The M modality files of one case (`<case>_0000 ... <case>_000{M-1}`) -> (data fp32 [M, z, y, x] in SimpleITK axis order,
+    header of the first file).  The files must agree in shape, spacing and orientation, as nnU-Net requires."""
+    from . import nifti
+    vols, hdr0 = [], None
+    for i, f in enumerate(input_files):
+        vol_xyz, hdr = nifti.read_nifti(f)
+        if hdr0 is None:
+            hdr0 = hdr
+        else:
+            if tuple(hdr["shape"]) != tuple(hdr0["shape"]):
+                raise ValueError("modality %d (%s) has shape %s, modality 0 has %s" % (i, f, tuple(hdr["shape"]), tuple(hdr0["shape"])))
+            if not np.allclose(hdr["spacing"], hdr0["spacing"], rtol=1e-5, atol=1e-6) or not np.allclose(hdr["srow"], hdr0["srow"], rtol=1e-5, atol=1e-5):
+                raise ValueError("modality %d (%s) does not share the geometry (spacing / affine) of modality 0 (%s)" % (i, f, input_files[0]))
+        vols.append(np.transpose(vol_xyz, (2, 1, 0)))
+    return np.ascontiguousarray(np.stack(vols)).astype(np.float32), hdr0
+
+
 def preprocess_test_case(network, plans: Dict, input_files: Sequence[str], force_separate_z=None):
-    """[U:GenericPreprocessor.preprocess_test_case] for DeepWMH's single FLAIR modality (`<case>_0000.nii.gz`):
-    read (SimpleITK axis order z, y, x) -> crop_to_nonzero -> transpose_forward -> NaN -> 0 -> resample to the plans'
-    spacing (device) -> masked z-score (device).  Returns (data fp32 CUDA [1, x, y, z], seg int8 CUDA [1, x, y, z], properties)."""
+    """[U:GenericPreprocessor.preprocess_test_case] for M = plans['num_modalities'] modalities (`<case>_0000 ...`; DeepWMH: one
+    FLAIR): read (SimpleITK axis order z, y, x) -> crop_to_nonzero (nonzero mask over all modalities, holes filled) ->
+    transpose_forward -> NaN -> 0 -> resample every modality to the plans' spacing (device) -> z-score of every modality with
+    its own use_mask_for_norm (device).  Only the non-CT scheme exists here.  Returns (data fp32 CUDA [M, x, y, z],
+    seg int8 CUDA [1, x, y, z], properties)."""
     import torch
 
-    from . import nifti
-    if len(input_files) != 1:
-        raise NotImplementedError("DeepWMH models take one modality (FLAIR); got %d input files" % len(input_files))
-    vol_xyz, hdr = nifti.read_nifti(input_files[0])
-    data = np.ascontiguousarray(np.transpose(vol_xyz, (2, 1, 0)))[None].astype(np.float32)
+    M = int(plans.get("num_modalities", 1))
+    if len(input_files) != M:
+        raise ValueError("the model takes %d modalities; got %d input files" % (M, len(input_files)))
+    schemes = plans.get("normalization_schemes") or {}
+    for m in range(M):
+        if schemes.get(m, "nonCT") != "nonCT":
+            raise NotImplementedError("normalization scheme %r of modality %d: only nnU-Net's non-CT z-score is implemented"
+                                      % (schemes.get(m), m))
+    data, hdr = read_modalities(input_files)
     stage = max(plans["plans_per_stage"].keys())
     target_spacing = np.array(plans["plans_per_stage"][stage]["current_spacing"], dtype=np.float64)
     tf = list(plans.get("transpose_forward", [0, 1, 2]))
@@ -172,24 +196,37 @@ def preprocess_test_case(network, plans: Dict, input_files: Sequence[str], force
     seg = np.ascontiguousarray(seg.transpose([0] + [i + 1 for i in tf]))
     cropped[np.isnan(cropped)] = 0
     original_spacing_transposed = props["original_spacing"][tf]
-    use_mask = bool(plans.get("use_mask_for_norm", {0: False})[0])
+    mask_for_norm = plans.get("use_mask_for_norm", {0: False})
+    use_mask = [bool(mask_for_norm[m]) for m in range(M)]
     with torch.cuda.device(network.device):
         d = torch.from_numpy(cropped).to(network.device)
         sg = torch.from_numpy(seg).to(network.device)
         d, sg = resample_patient_device(d, sg, original_spacing_transposed, target_spacing, force_separate_z)
         props["size_after_resampling"] = tuple(d.shape[1:])
         props["spacing_after_resampling"] = target_spacing
-        props["use_nonzero_mask_for_norm"] = {0: use_mask}
-        v = d[0].contiguous()
-        network.normalize_(v, sg[0].contiguous() if use_mask else None, 1 if use_mask else 0, return_stats=False)
-        d = v[None]
+        props["use_nonzero_mask_for_norm"] = {m: use_mask[m] for m in range(M)}
+        if M == 1:
+            v = d[0].contiguous()
+            network.normalize_(v, sg[0].contiguous() if use_mask[0] else None, 1 if use_mask[0] else 0, return_stats=False)
+            d = v[None]
+        else:
+            d = d.contiguous()
+            mask = sg[0].contiguous()
+            # each channel of d starts 16-byte aligned only if X*Y*Z % 4 == 0: normalise a padded copy otherwise
+            chans = []
+            for m in range(M):
+                v = d[m].clone() if d[0].numel() % 4 else d[m]
+                network.normalize_(v, mask if use_mask[m] else None, 1 if use_mask[m] else 0, return_stats=False)
+                chans.append(v)
+            d = torch.stack(chans) if d[0].numel() % 4 else d
     return d, sg, props
 
 
 def save_segmentation_nifti_from_softmax(network, softmax, out_fname: str, properties: Dict, order: int = 1, force_separate_z=None,
                                          softmax_fname: Optional[str] = None, post3mm_fname: Optional[str] = None):
     """[U:inference/segmentation_export.py::save_segmentation_nifti_from_softmax]: softmax [classes, x, y, z] (ALREADY
-    transposed back; CUDA tensor or numpy) -> resample back to the cropped grid (order 1, device) -> argmax -> paste into
+    transposed back; CUDA tensor or numpy) -> resample back to the cropped grid (order 1, device) -> argmax (labels
+    0 .. classes-1, ties to the lower class) -> paste into
     zeros(original size) at the crop box -> uint8 NIfTI with the input's header.  softmax_fname: the fork's
     `--save_softmax` (background probability as `<case>_0.nii.gz`, DCNN_multistage.py:340-343,359: 1 outside the crop);
     post3mm_fname: `remove_3mm_sparks` of the label map on the device (deepwmh/main/predict.py:19-26,158-163)."""
@@ -202,7 +239,7 @@ def save_segmentation_nifti_from_softmax(network, softmax, out_fname: str, prope
         sm = sm.to(device=network.device, dtype=torch.float32).contiguous()
         sm = resample_softmax_back_device(sm, properties["size_after_cropping"], properties["original_spacing"],
                                           properties["spacing_after_resampling"], force_separate_z, order)
-        seg = network.argmax2(sm.contiguous())
+        seg = network.argmax(sm.contiguous())
         full_shape = tuple(int(v) for v in properties["original_size_of_raw_data"])
         sl = tuple(slice(b[0], b[1]) for b in properties["crop_bbox"])
         full = torch.zeros(full_shape, dtype=torch.uint8, device=network.device)

@@ -12,7 +12,9 @@
  * the thread-local message.  One dwmh_ctx per GPU, not re-entrant; distinct contexts are
  * independent.  Device pointers are plain CUDA device addresses owned by the caller; `stream` is
  * a cudaStream_t passed as void* (NULL = default stream).  Volumes are C-ordered [X][Y][Z]
- * (Z fastest), exactly the (c, x, y, z) numpy arrays nnU-Net hands to predict_3D with c == 1.
+ * (Z fastest); inputs of M = in_channels modalities are channel-major [M][X][Y][Z] and class maps
+ * [C][X][Y][Z] with C = num_classes, exactly the (c, x, y, z) numpy arrays nnU-Net hands to and
+ * returns from predict_3D.  DeepWMH's own model has M = 1 and C = 2.
  * No torch types, no exceptions and no Python objects cross this line.
  */
 #ifndef DEEPWMH_B200_H_
@@ -25,14 +27,17 @@ extern "C" {
 #endif
 
 #define DWMH_MAX_POOL 7
+#define DWMH_MAX_IN_CHANNELS 4   /* modalities: the multi-modality first conv keeps 4 input slices per modality and one
+                                    weight tile per modality in one SM's shared memory */
+#define DWMH_MAX_CLASSES 8       /* classes (incl. background): the head keeps every class's logit of two voxels in registers */
 
 typedef struct dwmh_ctx dwmh_ctx;
 
 /* Generic_UNet hyper-parameters, i.e. what nnUNetTrainerV2.process_plans reads from plans.pkl
  * (SURVEY.md Appendix A1/A6).  Replaces nnUNetTrainerV2.initialize_network [U]. */
 typedef struct dwmh_net_desc {
-  int32_t in_channels;                        /* plans['num_modalities']; only 1 is supported        */
-  int32_t num_classes;                        /* plans['num_classes'] + 1; only 2 is supported       */
+  int32_t in_channels;                        /* plans['num_modalities']: 1 .. DWMH_MAX_IN_CHANNELS  */
+  int32_t num_classes;                        /* plans['num_classes'] + 1: 2 .. DWMH_MAX_CLASSES     */
   int32_t base_num_features;                  /* 32                                                  */
   int32_t max_num_features;                   /* 320                                                 */
   int32_t num_pool;                           /* len(pool_op_kernel_sizes)                           */
@@ -49,7 +54,9 @@ typedef struct dwmh_net_desc {
 const char* dwmh_last_error(void);
 int dwmh_version(void);
 
-/* --- life cycle (replaces load_model_and_checkpoint_files + trainer.initialize(False)) ---------- */
+/* --- life cycle (replaces load_model_and_checkpoint_files + trainer.initialize(False)) ----------
+ * dwmh_create fails for in_channels or num_classes outside the bounds above, and for in_channels > 1 with
+ * base_num_features > 32. */
 int dwmh_create(dwmh_ctx** out, int device, const dwmh_net_desc* desc);
 int dwmh_destroy(dwmh_ctx* ctx);
 /* A further model on the same device that BORROWS the activation workspaces of `parent` (k resident models of the
@@ -67,7 +74,8 @@ int dwmh_set_weight(dwmh_ctx* ctx, const char* nnunet_key, const float* data, co
 int dwmh_commit_weights(dwmh_ctx* ctx);
 
 /* --- a2: GenericPreprocessor.resample_and_normalize, non-CT scheme [U] -------------------------
- * In place on a device fp32 volume of n voxels.
+ * In place on a device fp32 volume of n voxels: ONE modality (nnU-Net normalises each modality on its own,
+ * so a multi-modality input takes one call per channel, each channel 16-byte aligned).
  * mask_mode 0: use_mask_for_norm False -> statistics over all voxels, all voxels normalised.
  * mask_mode 1: mask = (seg[i] >= 0), seg = device int8 array (nnU-Net's nonzero mask); outside -> 0.
  * mask_mode 2: mask = (vol[i] != 0)   (the benchmark's definition, SURVEY.md section 8d).
@@ -85,8 +93,8 @@ int dwmh_gaussian_map(const int32_t patch[3], double sigma_scale, float* out_hos
 int dwmh_set_importance_map(dwmh_ctx* ctx, const float* map_host);
 
 /* --- a7/a11/a12: SegmentationNetwork.predict_3D, tiled branch -----------------------------------
- * vol_dev: normalised fp32 [X][Y][Z], each extent >= patch (caller pads, a10).
- * Accumulates into agg_dev fp32 [2][X][Y][Z] and wgt_dev fp32 [X][Y][Z] (caller zero-initialises):
+ * vol_dev: normalised fp32 [M][X][Y][Z], each extent >= patch (caller pads, a10).
+ * Accumulates into agg_dev fp32 [C][X][Y][Z] and wgt_dev fp32 [X][Y][Z] (caller zero-initialises):
  *   agg[:, tile] += gaussian * sum_m (1/M) unflip_m(softmax(net(flip_m(tile)))),  wgt[tile] += gaussian
  * for the tiles with linear index in [tile_begin, tile_end) in x-outer / y / z-inner order
  * (tile_end < 0 = all).  mirror_axes_mask: bit a set = axis a in mirror_axes; do_mirroring = 0 -> M = 1.
@@ -103,13 +111,16 @@ int dwmh_weight_map(dwmh_ctx* ctx, int32_t X, int32_t Y, int32_t Z, double step_
                     float* wgt_dev, void* stream);
 
 /* class_probabilities = agg / wgt ; seg = argmax over classes (first maximum wins).
- * softmax_dev fp32 [2][X][Y][Z] (may alias agg_dev), seg_dev uint8 [X][Y][Z]; either may be NULL. */
+ * softmax_dev fp32 [C][X][Y][Z] (may alias agg_dev), seg_dev uint8 [X][Y][Z] with values 0 .. C-1; either may be NULL. */
 int dwmh_finalize(dwmh_ctx* ctx, const float* agg_dev, const float* wgt_dev, float* softmax_dev,
                   uint8_t* seg_dev, int32_t X, int32_t Y, int32_t Z, void* stream);
 
 /* a13 ensemble: acc += softmax / k  (k-model mean of predict_cases), n floats. */
 int dwmh_axpy(dwmh_ctx* ctx, float* acc_dev, const float* x_dev, float alpha, int64_t n, void* stream);
 int dwmh_argmax2(dwmh_ctx* ctx, const float* softmax_dev, uint8_t* seg_dev, int64_t nvox, void* stream);
+/* seg = argmax over num_classes (1 .. 255) of softmax_dev fp32 [num_classes][nvox]; the first maximum wins (ties go to the
+ * lower class, as numpy.argmax).  dwmh_argmax2 is the same for two classes. */
+int dwmh_argmax(dwmh_ctx* ctx, const float* softmax_dev, int32_t num_classes, uint8_t* seg_dev, int64_t nvox, void* stream);
 
 /* --- SURVEY 8f-3: checkpoint ensemble with softmax masking (deepwmh/pipeline/DCNN_multistage.py:102-125,317-394).
  * dwmh_ensemble_masked_add: acc += 1 - m (1 - x) for one checkpoint's BACKGROUND probability x (the fork's
@@ -234,22 +245,22 @@ int dwmh_n4(int32_t device, const float* in_dev, int32_t X, int32_t Y, int32_t Z
             const int32_t* iterations_host, float* out_dev, float* log_field_dev, void* workspace_dev, void* stream);
 
 /* --- a6 end to end with HOST buffers (what predict_preprocessed_data_return_seg_and_softmax does):
- * raw fp32 volume [X][Y][Z] in host memory -> (optional z-score, mask_mode as above, <0 = skip)
- * -> tiled prediction -> host softmax fp32 [2][X][Y][Z] and seg uint8 [X][Y][Z].  H2D/D2H inside. */
+ * raw fp32 volume [M][X][Y][Z] in host memory -> (optional z-score of every modality, mask_mode as above, <0 = skip)
+ * -> tiled prediction -> host softmax fp32 [C][X][Y][Z] and seg uint8 [X][Y][Z].  H2D/D2H inside. */
 int dwmh_predict_volume_host(dwmh_ctx* ctx, const float* vol_host, int32_t X, int32_t Y, int32_t Z,
                              int32_t zscore_mask_mode, double step_size, int32_t do_mirroring,
                              int32_t mirror_axes_mask, int32_t use_gaussian,
                              float* softmax_host, uint8_t* seg_host, void* stream);
 
 /* The same with nnU-Net's own normalisation mask (mask_mode 1): seg_mask_host int8 [X][Y][Z], >= 0 inside the
- * hole-filled non-zero crop mask (crop_to_nonzero [U:preprocessing/cropping.py]), -1 outside. */
+ * hole-filled non-zero crop mask (crop_to_nonzero [U:preprocessing/cropping.py]), -1 outside; one mask for all modalities. */
 int dwmh_predict_volume_host_masked(dwmh_ctx* ctx, const float* vol_host, const int8_t* seg_mask_host,
                                     int32_t X, int32_t Y, int32_t Z, double step_size, int32_t do_mirroring,
                                     int32_t mirror_axes_mask, int32_t use_gaussian,
                                     float* softmax_host, uint8_t* seg_host, void* stream);
 
 /* --- test / profiling hooks ----------------------------------------------------------------------
- * Generic_UNet.forward + softmax on n patches: patches_dev fp32 [n][px][py][pz] -> probs_dev fp32 [n][2][px][py][pz]. */
+ * Generic_UNet.forward + softmax on n patches: patches_dev fp32 [n][M][px][py][pz] -> probs_dev fp32 [n][C][px][py][pz]. */
 int dwmh_forward_patches(dwmh_ctx* ctx, const float* patches_dev, int32_t n, float* probs_dev, void* stream);
 /* Copy the (normalised, activated) output of layer `layer_index` of the last forward, converted to
  * fp32 NCDHW, into out_dev (capacity in floats); dims_out = {n, c, d, h, w}.  Layer order = execution order. */
