@@ -106,6 +106,7 @@ struct dwmh_ctx {
   bool force_generic = false;
   // workspaces
   double* stats_arena = nullptr; size_t stats_bytes = 0;
+  float* fc_partials = nullptr;      // block statistics of the CUDA-core first conv (in stats_arena, past stats_bytes)
   StatPartial* stat_partials = nullptr; size_t stat_partials_cap = 0;   // per-CTA Welford partials of the layer in flight
   float* probs = nullptr;            // [maxN][2][P]
   bool buffers_ready = false;
@@ -400,10 +401,14 @@ extern "C" int dwmh_commit_weights(dwmh_ctx* c) {
   size_t stat_doubles = 0;
   for (auto& L : c->layers) if (L.has_norm) stat_doubles += (size_t)maxN * L.cout * 2;
   c->stats_bytes = stat_doubles * sizeof(double);
+  // the CUDA-core first-conv kernels leave [n][block][Cout][2] partial statistics (not cleared per forward: every slot is written)
+  const Layer& L0 = c->layers[0];
+  const int64_t fc_blocks = std::max((L0.vout() + 256 * FC_VPT - 1) / (256 * FC_VPT), (L0.vout() / 2 + 128 * FC_VPT - 1) / (128 * FC_VPT));
+  const size_t fc_bytes = (size_t)maxN * fc_blocks * 2 * L0.cout * sizeof(float);
   if (!c->buffers_ready && c->lender) {
     dwmh_ctx* o = c->lender;
     if (o->layers.size() != c->layers.size() || o->max_batch != maxN) return fail("dwmh_commit_weights: lender context does not match");
-    c->stats_arena = o->stats_arena; c->probs = o->probs;
+    c->stats_arena = o->stats_arena; c->fc_partials = o->fc_partials; c->probs = o->probs;
     for (int i = 0; i < nL; ++i) {
       Layer& L = c->layers[i]; const Layer& S = o->layers[i];
       if (L.raw32 != S.raw32) return fail("dwmh_commit_weights: lender context does not match (raw storage of %s)", L.name.c_str());
@@ -412,7 +417,8 @@ extern "C" int dwmh_commit_weights(dwmh_ctx* c) {
     c->buffers_ready = true;
   }
   if (!c->buffers_ready) {
-    CU_TRY(cudaMalloc((void**)&c->stats_arena, c->stats_bytes));
+    CU_TRY(cudaMalloc((void**)&c->stats_arena, c->stats_bytes + fc_bytes));
+    c->fc_partials = reinterpret_cast<float*>(reinterpret_cast<char*>(c->stats_arena) + c->stats_bytes);
     CU_TRY(cudaMalloc((void**)&c->probs, (size_t)maxN * c->d.num_classes * c->P() * sizeof(float)));
     size_t off = 0;
     for (int i = 0; i < nL; ++i) {
@@ -655,18 +661,19 @@ static int forward_impl(dwmh_ctx* c, const float* src, int patch_mode, int SX, i
       p.src = src; p.metas = metas; p.w = L.w_dev; p.out = L.raw; p.sums = L.sums; p.patch_mode = patch_mode;
       p.SX = SX; p.SY = SY; p.SZ = SZ; p.px = L.out_sp[0]; p.py = L.out_sp[1]; p.pz = L.out_sp[2];
       p.kd = L.k[0]; p.kh = L.k[1]; p.kw = L.k[2]; p.Cout = L.cout;
-      p.Cin = L.c0; p.mstride = (int64_t)SX * SY * SZ;
+      p.Cin = L.c0; p.mstride = (int64_t)SX * SY * SZ; p.partials = c->fc_partials;
       dim3 grid((unsigned)((L.vout() + 256 * FC_VPT - 1) / (256 * FC_VPT)), nb);
-      const size_t smem = ((size_t)L.c0 * taps * L.cout + 2 * L.cout) * sizeof(float);
+      const size_t smem = ((size_t)L.c0 * taps * L.cout + 8 * 2 * L.cout) * sizeof(float);     // weights, 8 warps' statistics
       if (L.c0 > 1) {
         if (taps == 27) conv_first_mm_kernel<T, true><<<grid, 256, smem, st>>>(p);
         else conv_first_mm_kernel<T, false><<<grid, 256, smem, st>>>(p);
       } else if (taps == 27 && L.cout <= 32 && L.out_sp[2] % 2 == 0) {
-        dim3 grid2((unsigned)((L.vout() / 2 + 128 * FC_VPT - 1) / (128 * FC_VPT)), nb);
-        conv_first_k3x2_kernel<T><<<grid2, 128, smem, st>>>(p);
+        grid.x = (unsigned)((L.vout() / 2 + 128 * FC_VPT - 1) / (128 * FC_VPT));
+        conv_first_k3x2_kernel<T><<<grid, 128, smem, st>>>(p);
       } else if (taps == 27) conv_first_kernel<T, true><<<grid, 256, smem, st>>>(p);
       else conv_first_kernel<T, false><<<grid, 256, smem, st>>>(p);
-      c->launches++;
+      first_stats_reduce_kernel<<<nb, 128, 0, st>>>(c->fc_partials, L.sums, (int)grid.x, 2 * L.cout);
+      c->launches += 2;
     } else if (L.kind == L_CONV && use_tc) {
       Layer& P = c->layers[L.in0];
       NormParams pn = norm_of(P);

@@ -29,7 +29,32 @@ struct FirstConvParams {
   int Cout;
   int Cin;                     // modalities (conv_first_mm_kernel; the single-modality kernels ignore it)
   int64_t mstride;             // floats between two modalities of the volume (patch_mode 0)
+  float* partials;             // [n][gridDim.x][Cout][2]: each block's statistics, summed by first_stats_reduce_kernel
 };
+
+// Statistics of the first-conv kernels without atomics, so that a forward gives the same bits on every run: sstat holds
+// one [Cout][2] slot per warp, written by that warp alone; each block sums its warps' slots in warp order into its own
+// slot of p.partials, and first_stats_reduce_kernel adds the blocks of a sample in block order in fp64.
+__device__ __forceinline__ void first_conv_block_partials(const float* sstat, float* partials, int n, int Cout) {
+  __syncthreads();
+  const int nw = blockDim.x >> 5;
+  for (int c = threadIdx.x; c < 2 * Cout; c += blockDim.x) {
+    float s = 0.f;
+    for (int w = 0; w < nw; ++w) s += sstat[w * 2 * Cout + c];
+    partials[((size_t)n * gridDim.x + blockIdx.x) * 2 * Cout + c] = s;
+  }
+}
+
+// grid: one block per sample; sums [n][C2] (C2 = 2 Cout) = sum over the nblk blocks of partials [n][nblk][C2], in order
+__global__ void __launch_bounds__(128) first_stats_reduce_kernel(const float* __restrict__ partials, double* __restrict__ sums,
+                                                                 int nblk, int C2) {
+  const int n = blockIdx.x;
+  for (int c = threadIdx.x; c < C2; c += blockDim.x) {
+    double s = 0.0;
+    for (int b = 0; b < nblk; ++b) s += (double)partials[((size_t)n * nblk + b) * C2 + c];
+    sums[(size_t)n * C2 + c] = s;
+  }
+}
 
 // K3: kernel is 3x3x3 (fully unrolled taps, inputs stay in registers).  Each thread walks FC_VPT voxels
 // (stride = blockDim) and keeps per-channel running statistics in registers (Cout <= 32) so the warp
@@ -38,13 +63,13 @@ constexpr int FC_VPT = 4;
 
 template <typename T, bool K3>
 __global__ void __launch_bounds__(256) conv_first_kernel(FirstConvParams p) {
-  extern __shared__ float smf[];                 // weights [taps][Cout], then stats [Cout][2]
+  extern __shared__ float smf[];                 // weights [taps][Cout], then stats [warp][Cout][2]
   const int kd = K3 ? 3 : p.kd, kh = K3 ? 3 : p.kh, kw = K3 ? 3 : p.kw;
   const int taps = kd * kh * kw;
   float* sw = smf;
   float* sstat = smf + taps * p.Cout;
   for (int i = threadIdx.x; i < taps * p.Cout; i += blockDim.x) sw[i] = p.w[i];
-  for (int i = threadIdx.x; i < 2 * p.Cout; i += blockDim.x) sstat[i] = 0.f;
+  for (int i = threadIdx.x; i < (blockDim.x >> 5) * 2 * p.Cout; i += blockDim.x) sstat[i] = 0.f;
   __syncthreads();
   const int n = blockIdx.y;
   const int64_t P = (int64_t)p.px * p.py * p.pz;
@@ -54,6 +79,7 @@ __global__ void __launch_bounds__(256) conv_first_kernel(FirstConvParams p) {
   if (p.patch_mode) { src += (size_t)n * P; SY = p.py; SZ = p.pz; }
   else { const SampleMeta m = p.metas[n]; ox = m.ox; oy = m.oy; oz = m.oz; flip = m.flip; }
   const int lane = threadIdx.x & 31;
+  float* wst = sstat + (threadIdx.x >> 5) * 2 * p.Cout;     // this warp's statistics slot
   const bool reg_stats = p.Cout <= 32;
   float rs[32], rq[32];
 #pragma unroll
@@ -115,7 +141,7 @@ __global__ void __launch_bounds__(256) conv_first_kernel(FirstConvParams p) {
         for (int q = 0; q < 8; ++q) {
           const float a_ = active ? acc[q] : 0.f;
           const float s = warp_sum(a_), ss = warp_sum(a_ * a_);
-          if (lane == 0) { atomicAdd(&sstat[(cc * 8 + q) * 2], s); atomicAdd(&sstat[(cc * 8 + q) * 2 + 1], ss); }
+          if (lane == 0) { wst[(cc * 8 + q) * 2] += s; wst[(cc * 8 + q) * 2 + 1] += ss; }
         }
       }
     }
@@ -133,11 +159,9 @@ __global__ void __launch_bounds__(256) conv_first_kernel(FirstConvParams p) {
         rq[i] = kb_ + __shfl_xor_sync(0xffffffffu, sb_, k);
       }
     }
-    if (lane < p.Cout) { atomicAdd(&sstat[lane * 2], rs[0]); atomicAdd(&sstat[lane * 2 + 1], rq[0]); }
+    if (lane < p.Cout) { wst[lane * 2] = rs[0]; wst[lane * 2 + 1] = rq[0]; }
   }
-  __syncthreads();
-  for (int c = threadIdx.x; c < 2 * p.Cout; c += blockDim.x)
-    atomicAdd(p.sums + (size_t)n * p.Cout * 2 + c, (double)sstat[c]);
+  first_conv_block_partials(sstat, p.partials, n, p.Cout);
 }
 
 // 3x3x3 specialisation with TWO z-adjacent voxels per thread: one broadcast weight load feeds 16 FMAs
@@ -145,11 +169,11 @@ __global__ void __launch_bounds__(256) conv_first_kernel(FirstConvParams p) {
 // 3x3x4 input neighbourhood.  Requires pz even and Cout <= 32.
 template <typename T>
 __global__ void __launch_bounds__(128) conv_first_k3x2_kernel(FirstConvParams p) {
-  extern __shared__ float smf[];                 // weights [27][Cout], then stats [Cout][2]
+  extern __shared__ float smf[];                 // weights [27][Cout], then stats [warp][Cout][2]
   float* sw = smf;
   float* sstat = smf + 27 * p.Cout;
   for (int i = threadIdx.x; i < 27 * p.Cout; i += blockDim.x) sw[i] = p.w[i];
-  for (int i = threadIdx.x; i < 2 * p.Cout; i += blockDim.x) sstat[i] = 0.f;
+  for (int i = threadIdx.x; i < (blockDim.x >> 5) * 2 * p.Cout; i += blockDim.x) sstat[i] = 0.f;
   __syncthreads();
   const int n = blockIdx.y;
   const int64_t P = (int64_t)p.px * p.py * p.pz, P2 = P >> 1;
@@ -159,6 +183,7 @@ __global__ void __launch_bounds__(128) conv_first_k3x2_kernel(FirstConvParams p)
   if (p.patch_mode) { src += (size_t)n * P; SY = p.py; SZ = p.pz; }
   else { const SampleMeta m = p.metas[n]; ox = m.ox; oy = m.oy; oz = m.oz; flip = m.flip; }
   const int lane = threadIdx.x & 31;
+  float* wst = sstat + (threadIdx.x >> 5) * 2 * p.Cout;     // this warp's statistics slot
   const int pz2 = p.pz >> 1;
   float rs[32], rq[32];
 #pragma unroll
@@ -227,10 +252,8 @@ __global__ void __launch_bounds__(128) conv_first_k3x2_kernel(FirstConvParams p)
       rq[i] = kb_ + __shfl_xor_sync(0xffffffffu, sb_, k);
     }
   }
-  if (lane < p.Cout) { atomicAdd(&sstat[lane * 2], rs[0]); atomicAdd(&sstat[lane * 2 + 1], rq[0]); }
-  __syncthreads();
-  for (int c = threadIdx.x; c < 2 * p.Cout; c += blockDim.x)
-    atomicAdd(p.sums + (size_t)n * p.Cout * 2 + c, (double)sstat[c]);
+  if (lane < p.Cout) { wst[lane * 2] = rs[0]; wst[lane * 2 + 1] = rq[0]; }
+  first_conv_block_partials(sstat, p.partials, n, p.Cout);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -241,13 +264,13 @@ __global__ void __launch_bounds__(128) conv_first_k3x2_kernel(FirstConvParams p)
 // ---------------------------------------------------------------------------------------------
 template <typename T, bool K3>
 __global__ void __launch_bounds__(256) conv_first_mm_kernel(FirstConvParams p) {
-  extern __shared__ float smf[];                 // weights [Cin][taps][Cout], then stats [Cout][2]
+  extern __shared__ float smf[];                 // weights [Cin][taps][Cout], then stats [warp][Cout][2]
   const int kd = K3 ? 3 : p.kd, kh = K3 ? 3 : p.kh, kw = K3 ? 3 : p.kw;
   const int taps = kd * kh * kw;
   float* sw = smf;
   float* sstat = smf + p.Cin * taps * p.Cout;
   for (int i = threadIdx.x; i < p.Cin * taps * p.Cout; i += blockDim.x) sw[i] = p.w[i];
-  for (int i = threadIdx.x; i < 2 * p.Cout; i += blockDim.x) sstat[i] = 0.f;
+  for (int i = threadIdx.x; i < (blockDim.x >> 5) * 2 * p.Cout; i += blockDim.x) sstat[i] = 0.f;
   __syncthreads();
   const int n = blockIdx.y;
   const int64_t P = (int64_t)p.px * p.py * p.pz;
@@ -258,6 +281,7 @@ __global__ void __launch_bounds__(256) conv_first_mm_kernel(FirstConvParams p) {
   if (p.patch_mode) { src += (size_t)n * p.Cin * P; SY = p.py; SZ = p.pz; mstride = P; }
   else { const SampleMeta m = p.metas[n]; ox = m.ox; oy = m.oy; oz = m.oz; flip = m.flip; }
   const int lane = threadIdx.x & 31;
+  float* wst = sstat + (threadIdx.x >> 5) * 2 * p.Cout;     // this warp's statistics slot
   float rs[32], rq[32];
 #pragma unroll
   for (int q = 0; q < 32; ++q) { rs[q] = 0.f; rq[q] = 0.f; }
@@ -335,10 +359,8 @@ __global__ void __launch_bounds__(256) conv_first_mm_kernel(FirstConvParams p) {
       rq[i] = kb_ + __shfl_xor_sync(0xffffffffu, sb_, k);
     }
   }
-  if (lane < p.Cout) { atomicAdd(&sstat[lane * 2], rs[0]); atomicAdd(&sstat[lane * 2 + 1], rq[0]); }
-  __syncthreads();
-  for (int c = threadIdx.x; c < 2 * p.Cout; c += blockDim.x)
-    atomicAdd(p.sums + (size_t)n * p.Cout * 2 + c, (double)sstat[c]);
+  if (lane < p.Cout) { wst[lane * 2] = rs[0]; wst[lane * 2 + 1] = rq[0]; }
+  first_conv_block_partials(sstat, p.partials, n, p.Cout);
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -187,22 +187,41 @@ class SegmentationNetwork:
         check(self._lib.dwmh_zscore(self._ctx, _ptr(vol), _ptr(seg), vol.numel(), mask_mode, stats, self._st()))
         return tuple(stats)
 
+    def _check_buffers(self, agg: torch.Tensor, wgt: torch.Tensor, vol: Optional[torch.Tensor] = None):
+        """The kernels take raw pointers: every tensor must be contiguous CUDA fp32 on this network's device, vol
+        [M,X,Y,Z] (or [X,Y,Z] for one modality), agg [C,X,Y,Z] and wgt [X,Y,Z] of one volume."""
+        named = (("vol", vol), ("agg", agg), ("wgt", wgt)) if vol is not None else (("agg", agg), ("wgt", wgt))
+        for name, t in named:
+            if not isinstance(t, torch.Tensor) or t.device != self.device or t.dtype != torch.float32:
+                raise ValueError("%s must be a float32 tensor on %s" % (name, self.device))
+            if not t.is_contiguous():
+                raise ValueError("%s must be contiguous" % name)
+        if wgt.dim() != 3:
+            raise ValueError("wgt must be [X, Y, Z]")
+        X, Y, Z = wgt.shape
+        if vol is not None:
+            one = vol.dim() == 3 and self.input_channels == 1
+            if not one and (vol.dim() != 4 or vol.shape[0] != self.input_channels):
+                raise ValueError("vol must be [%d, X, Y, Z]" % self.input_channels)
+            if tuple(vol.shape[-3:]) != (X, Y, Z):
+                raise ValueError("vol %s and wgt %s cover different volumes" % (tuple(vol.shape), tuple(wgt.shape)))
+        if tuple(agg.shape) != (self.num_classes, X, Y, Z):
+            raise ValueError("agg must be [%d, %d, %d, %d]" % (self.num_classes, X, Y, Z))
+        return X, Y, Z
+
     def accumulate_tiles(self, vol: torch.Tensor, agg: torch.Tensor, wgt: torch.Tensor, step_size: float,
                          do_mirroring: bool, mirror_axes: Sequence[int], use_gaussian: bool,
                          tile_begin: int = 0, tile_end: int = -1):
         """dwmh_predict_3d on device tensors: vol [M,X,Y,Z] fp32 (or [X,Y,Z] for one modality), agg [C,X,Y,Z], wgt [X,Y,Z]
         (accumulated into)."""
-        X, Y, Z = vol.shape[-3:]
-        if (vol.shape[0] if vol.dim() == 4 else 1) != self.input_channels or vol.dim() not in (3, 4):
-            raise ValueError("vol must be [%d, X, Y, Z]" % self.input_channels)
-        if tuple(agg.shape) != (self.num_classes, X, Y, Z):
-            raise ValueError("agg must be [%d, X, Y, Z]" % self.num_classes)
+        X, Y, Z = self._check_buffers(agg, wgt, vol)
         check(self._lib.dwmh_predict_3d(self._ctx, _ptr(vol), X, Y, Z, float(step_size), int(bool(do_mirroring)),
                                         mirror_axes_mask(mirror_axes), int(bool(use_gaussian)), _ptr(agg), _ptr(wgt),
                                         int(tile_begin), int(tile_end), self._st()))
 
     def finalize(self, agg: torch.Tensor, wgt: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
-        X, Y, Z = wgt.shape
+        """agg [C,X,Y,Z] / wgt [X,Y,Z] in place -> (seg uint8 [X,Y,Z], agg as the probabilities)."""
+        X, Y, Z = self._check_buffers(agg, wgt)
         seg = torch.empty((X, Y, Z), dtype=torch.uint8, device=agg.device)
         check(self._lib.dwmh_finalize(self._ctx, _ptr(agg), _ptr(wgt), _ptr(agg), _ptr(seg), X, Y, Z, self._st()))
         return seg, agg

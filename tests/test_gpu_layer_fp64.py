@@ -13,7 +13,7 @@ and u the unit roundoff of the activation type (2^-11 fp16, 2^-8 bf16):
 
     conv + InstanceNorm + LeakyReLU   |dev - ref| <= 2u|ref| + s (|gamma| / sigma)(eps_raw |y| + 2^-14 A) + 2^-24
     transposed conv                   |dev - ref| <= 2u|ref| + 2^-14 A
-    head (1x1x1 + softmax)            |p_dev - p_ref| <= 1e-6 + 2^-14 (A_0 + A_1)
+    head (1x1x1 + softmax)            |p_dev - p_ref| <= 1e-6 + 2^-14 sum_k A_k    (A_k: the logit of class k on |x|, |w|)
 
 eps_raw = u where the raw conv output is stored in the activation type (the first conv, the last conv and every layer
 with an edge above 64 voxels) and 2^-23 where it is kept in fp32.  2u|ref| covers the output rounding, 2^-14 A the fp32
@@ -26,7 +26,9 @@ halves, and it drops to 4.2 on the 128-channel decoder conv of the 32^3 plan alr
 A tolerance is only worth something if it can see a wrong kernel.  Each layer therefore also recomputes its reference
 with one piece of the operation removed -- the centre tap of every input channel for a conv, one of the output parity
 classes for a transposed conv -- and requires the median of |perturbed - ref| / tol to be at least 4 (on the affected
-elements).  Only the host reference is perturbed.
+elements).  The head's reference is recomputed with the last class's weights of channels 0-3 and 4-7 exchanged -- the
+error of a coefficient chunk index that is off by one -- and the median over that class must reach the same 4.  Only the
+host reference is perturbed.
 
 The GPU cases reach the kernel paths DESIGN section 4 describes; the CPU test runs the same harness against an emulation
 of the device's fp16 scheme, which pins the tolerance model and the hook plumbing without a GPU.
@@ -112,17 +114,30 @@ def tconv_report(m, x, ref, dev, u):
     return err, sens
 
 
+def swap_last_class_chunks(w):
+    """The head weights [C, c, 1, 1, 1] with the last class's channels 0-3 and 4-7 exchanged: what the two-voxel head
+    computes if its float4 coefficient index (k * 8 + cc * 2 + h) is off by one chunk for that class."""
+    w = w.clone()
+    w[-1, 0:8] = torch.cat([w[-1, 4:8], w[-1, 0:4]])
+    return w
+
+
 def head_report(net, last, probs):
+    """max |p_dev - p_ref| / tol of the head, and the median of |p_swapped - p_ref| / tol over the last class, with
+    p_swapped the reference computed from swap_last_class_chunks's weights."""
     w = net.seg_outputs[-1].weight
     p_ref = torch.softmax(F.conv3d(last, w), 1)
     a = F.conv3d(last.abs(), w.abs()).sum(1, keepdim=True)
-    return ((probs - p_ref).abs() / (1e-6 + 2.0 ** -14 * a)).max().item()
+    tol = 1e-6 + 2.0 ** -14 * a
+    p_swap = torch.softmax(F.conv3d(last, swap_last_class_chunks(w)), 1)
+    sens = torch.median(_sub((p_swap - p_ref)[:, -1:].abs() / tol)).item()
+    return ((probs - p_ref).abs() / tol).max().item(), sens
 
 
 def layer_fp64_reports(net, dev, x, act="fp16", ref_device=None):
     """Run `dev` (a SegmentationNetwork, or the CPU emulation below) on x [n, 1, *patch] and compare each of its layers with
     the float64 reference fed the device's previous outputs.  Returns one dict per device layer, in device order (the
-    execution order of the network), and the head's ratio."""
+    execution order of the network), and the head's (ratio, sensitivity)."""
     ref_device = ref_device if ref_device is not None else x.device
     n, u = x.shape[0], U[act]
     probs = dev.forward_patches(x).to(ref_device, torch.float64)
@@ -173,16 +188,18 @@ def print_reports(name, reports, head):
         print("%-22s layer %2d %-12s %-18s%s max err/tol %.3f  sensitivity %8.1f" % (
             name, r["layer"], r["kind"], "x".join(map(str, r["shape"])), " nol" if r["norm_on_load"] else "    ",
             r["err"], r["sens"]))
-    print("%-22s head                                  max err/tol %.3f" % (name, head))
+    print("%-22s head                                  max err/tol %.3f  sensitivity %8.1f" % ((name,) + head))
 
 
 def check_reports(name, reports, head):
+    """head: (max err/tol, sensitivity) of head_report."""
     print_reports(name, reports, head)
     bad = [(r["layer"], r["kind"], round(r["err"], 3)) for r in reports if not r["err"] <= 1.0]
     blind = [(r["layer"], r["kind"], round(r["sens"], 2)) for r in reports if not r["sens"] >= SENS_MIN]
     assert not bad, (name, "above tolerance", bad)
     assert not blind, (name, "tolerance cannot see a one-tap error", blind)
-    assert head <= 1.0, (name, "head", head)
+    assert head[0] <= 1.0, (name, "head", head)
+    assert head[1] >= SENS_MIN, (name, "head tolerance cannot see a swapped coefficient chunk", head)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -257,6 +274,23 @@ def test_tolerance_flags_an_emulated_device_that_drops_the_centre_tap():
     reports, _ = layer_fp64_reports(net, dev, x, "fp16", "cpu")
     errs = [r["err"] for r in reports]
     assert errs[3] > SENS_MIN and max(errs[:3]) <= 1.0 and max(errs[4:]) <= 1.0, errs
+
+
+def test_tolerance_flags_an_emulated_head_with_a_swapped_coefficient_chunk():
+    """Eight classes: a device head that reads the last class's channels 0-3 where 4-7 belong fails the head bound,
+    while every layer before it still passes."""
+    plans = small_plans()
+    plans["num_classes"] = 7
+    net = O.build_benchmark_network(0, plans)
+    broken = copy.deepcopy(net)
+    with torch.no_grad():
+        broken.seg_outputs[-1].weight.copy_(swap_last_class_chunks(broken.seg_outputs[-1].weight))
+    x = torch.randn(1, 1, 32, 32, 32, generator=torch.Generator().manual_seed(13))
+    reports, head = layer_fp64_reports(net, EmulatedDevice(broken), x, "fp16", "cpu")
+    assert max(r["err"] for r in reports) <= 1.0
+    assert head[0] > SENS_MIN, head
+    _, head_ok = layer_fp64_reports(net, EmulatedDevice(net), x, "fp16", "cpu")
+    assert head_ok[0] <= 1.0 and head_ok[1] >= SENS_MIN, head_ok
 
 
 # ------------------------------------------------------------------------------------------------
