@@ -49,6 +49,7 @@ SYMBOLS = {
     "dwmh_ensemble_masked_add": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P]),
     "dwmh_ensemble_refine": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int64, _P]),
     "dwmh_remove_sparks": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P]),
+    "dwmh_keep_largest_components": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_uint32, C.c_double, C.c_double, _P]),
     "dwmh_s1_zscore": (C.c_int, [C.c_int32, _P, _P, C.c_int64, C.c_int32, _P, C.POINTER(C.c_double), _P]),
     "dwmh_s1_zscore_batch": (C.c_int, [C.c_int32, C.POINTER(_P), C.c_int32, _P, C.c_int64, C.c_int32, _P, _P]),
     "dwmh_s1_local_mean_align_workspace": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_int64)]),

@@ -74,10 +74,11 @@ def _check_cases(case_names: List[str], images: List[str]):
 
 
 def predict_case(trainer, plans: Dict, in_file, out_file: str, softmax_file: str = None, post3mm_file: str = None,
-                 do_mirroring: bool = True):
+                 do_mirroring: bool = True, for_which_classes=None, min_valid_object_sizes=None):
     """One case the way nnUNet_predict's predict_cases does it (SURVEY.md A7/A10): preprocess_patient (crop -> transpose ->
     resample -> z-score), tiled prediction, transpose back, resample back, argmax, paste back, NIfTI.  in_file: the image, or
-    the list of its modality files in channel order.  Everything between the file read and the file write stays on the device."""
+    the list of its modality files in channel order.  Everything between the file read and the file write stays on the device.
+    for_which_classes / min_valid_object_sizes: a loaded postprocessing.json for the label file (postprocessing.py)."""
     files = [in_file] if isinstance(in_file, str) else list(in_file)
     data, _, props = trainer.preprocess_patient(files, as_numpy=False)
     _, softmax = trainer.predict_preprocessed_data_return_seg_and_softmax(
@@ -85,7 +86,8 @@ def predict_case(trainer, plans: Dict, in_file, out_file: str, softmax_file: str
         step_size=0.5, use_gaussian=True, all_in_gpu=False, mixed_precision=True, return_device_tensors=True)
     tb = list(plans.get("transpose_backward", [0, 1, 2]))
     softmax = softmax.permute([0] + [i + 1 for i in tb])
-    preprocess.save_segmentation_nifti_from_softmax(trainer.network, softmax, out_file, props, 1, None, softmax_file, post3mm_file)
+    preprocess.save_segmentation_nifti_from_softmax(trainer.network, softmax, out_file, props, 1, None, softmax_file, post3mm_file,
+                                                    for_which_classes, min_valid_object_sizes)
 
 
 def robex_fov_masking(case_names: List[str], image_folder: str, post_3mm_folder: str, post_fov_folder: str, robex_dir: str):

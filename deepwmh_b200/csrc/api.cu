@@ -116,6 +116,7 @@ struct dwmh_ctx {
   double* zs_acc = nullptr;          // z-score: [0..2] totals for the host, [4 ...] one {sum, sum of squares, count} slot per CTA
   unsigned long long* zs_barrier = nullptr; unsigned long long zs_target = 0; int zs_grid = 0;
   int* ccl_labels = nullptr; int* ccl_sizes = nullptr; size_t ccl_cap_l = 0, ccl_cap_s = 0;   // dwmh_remove_sparks workspace
+  int* ccl_max = nullptr; size_t ccl_cap_m = 0;                                                 // dwmh_keep_largest_components
   // host-buffer path (grow only)
   float* hv_vol = nullptr; float* hv_pad = nullptr; float* hv_agg = nullptr; float* hv_wgt = nullptr; uint8_t* hv_seg = nullptr;
   size_t hv_vol_cap = 0, hv_pad_cap = 0, hv_agg_cap = 0, hv_wgt_cap = 0, hv_seg_cap = 0;
@@ -263,7 +264,7 @@ extern "C" int dwmh_destroy(dwmh_ctx* c) {
   if (!c->lender) { free_dev(c->stats_arena); free_dev(c->probs); free_dev(c->stat_partials); }
   free_dev(c->w_head_dev); free_dev(c->gauss_dev); free_dev(c->metas_dev); free_dev(c->zs_acc); free_dev(c->zs_barrier);
   free_dev(c->hv_vol); free_dev(c->hv_pad); free_dev(c->hv_agg); free_dev(c->hv_wgt); free_dev(c->hv_seg);
-  free_dev(c->ccl_labels); free_dev(c->ccl_sizes);
+  free_dev(c->ccl_labels); free_dev(c->ccl_sizes); free_dev(c->ccl_max);
   for (int i = 0; i < 4; ++i) if (c->ev[i]) cudaEventDestroy(c->ev[i]);
   for (auto e : c->tcev) cudaEventDestroy(e);
   delete c;
@@ -990,6 +991,35 @@ extern "C" int dwmh_remove_sparks(dwmh_ctx* c, const uint8_t* seg, int32_t X, in
   ccl_count_kernel<<<grid, 256, 0, st>>>(c->ccl_labels, c->ccl_sizes, V);
   ccl_filter_kernel<<<grid, 256, 0, st>>>(c->ccl_labels, c->ccl_sizes, out, min_volume, V);
   c->launches += 4;
+  CU_TRY(cudaGetLastError());
+  return 0;
+}
+
+// nnU-Net v1 postprocessing.json, one entry of for_which_classes, in place (DESIGN §11).  The values are checked before the
+// pointers and nothing is dereferenced before both pass, so every refusal can be seen without a device (and without a context).
+extern "C" int dwmh_keep_largest_components(dwmh_ctx* c, uint8_t* seg, int32_t X, int32_t Y, int32_t Z, uint32_t class_mask,
+                                            double volume_per_voxel, double min_valid_mm3, void* stream_) {
+  if (X <= 0 || Y <= 0 || Z <= 0) return fail("dwmh_keep_largest_components: empty volume %d x %d x %d", X, Y, Z);
+  const int64_t V = (int64_t)X * Y * Z;
+  if (V >= (int64_t)1 << 31) return fail("dwmh_keep_largest_components: volume of %lld voxels exceeds the 32-bit label range", (long long)V);
+  if (class_mask == 0) return fail("dwmh_keep_largest_components: class_mask selects no class");
+  if (class_mask & 1u) return fail("dwmh_keep_largest_components: class_mask 0x%x selects class 0 (cannot remove background)", class_mask);
+  if (!(volume_per_voxel > 0.0) || !std::isfinite(volume_per_voxel))
+    return fail("dwmh_keep_largest_components: volume_per_voxel %g is not a positive finite number", volume_per_voxel);
+  if (std::isnan(min_valid_mm3)) return fail("dwmh_keep_largest_components: min_valid_mm3 is NaN (< 0 means no minimum)");
+  if (!c || !seg) return fail("dwmh_keep_largest_components: null argument");
+  DEV_GUARD(c->device);
+  DW_TRY(grow(&c->ccl_labels, &c->ccl_cap_l, (size_t)V));
+  DW_TRY(grow(&c->ccl_sizes, &c->ccl_cap_s, (size_t)V));
+  DW_TRY(grow(&c->ccl_max, &c->ccl_cap_m, (size_t)1));
+  cudaStream_t st = (cudaStream_t)stream_;
+  const int grid = c->num_sms * 8;
+  ccl_init_classes_kernel<<<grid, 256, 0, st>>>(seg, c->ccl_labels, c->ccl_sizes, c->ccl_max, class_mask, V, Z);
+  ccl_merge_kernel<<<grid, 256, 0, st>>>(c->ccl_labels, X, Y, Z);
+  ccl_count_kernel<<<grid, 256, 0, st>>>(c->ccl_labels, c->ccl_sizes, V);
+  ccl_max_size_kernel<<<grid, 256, 0, st>>>(c->ccl_sizes, c->ccl_max, V);
+  ccl_keep_largest_kernel<<<grid, 256, 0, st>>>(c->ccl_labels, c->ccl_sizes, c->ccl_max, seg, volume_per_voxel, min_valid_mm3, V);
+  c->launches += 5;
   CU_TRY(cudaGetLastError());
   return 0;
 }

@@ -2,6 +2,7 @@
 // 3-D connected components with 6-connectivity (scipy.ndimage.label's default structuring element) by lock-free
 // union-find on voxel indices, then a component-size filter.  Integer work: the result is bit-identical to the
 // reference's loop (components smaller than min_volume voxels are discarded, the rest become 1).
+// The same labelling serves nnU-Net's postprocessing.json (keep the largest component of a class set, DESIGN §11).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -76,6 +77,46 @@ static __global__ void __launch_bounds__(256) ccl_filter_kernel(const int* __res
   for (int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; v < V; v += (int64_t)gridDim.x * blockDim.x) {
     const int r = L[v];
     out[v] = (r >= 0 && size[r] >= min_volume) ? 1 : 0;
+  }
+}
+
+// ---- nnU-Net v1 postprocessing (remove_all_but_the_largest_connected_component), one entry of postprocessing.json ----
+// The mask is class-set membership: bit seg[v] of class_mask (labels >= 32 are never in the set).  Same labels as
+// ccl_init_kernel otherwise, so ccl_merge_kernel / ccl_count_kernel run unchanged.  Also clears the maximum for this call.
+static __global__ void __launch_bounds__(256) ccl_init_classes_kernel(const uint8_t* __restrict__ seg, int* __restrict__ L, int* __restrict__ size,
+                                                                      int* __restrict__ max_size, uint32_t class_mask, int64_t V, int Z) {
+  if (blockIdx.x == 0 && threadIdx.x == 0) *max_size = 0;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t v0 = (int64_t)blockIdx.x * blockDim.x + (threadIdx.x & ~31); v0 < V; v0 += stride) {   // warp-uniform trip count
+    const int64_t v = v0 + (threadIdx.x & 31);
+    const bool in = v < V;
+    const unsigned s = in ? seg[v] : 32u;
+    const int l = ccl_run_start(s < 32u && ((class_mask >> s) & 1u), in && v % Z == 0, v);
+    if (in) { L[v] = l; size[v] = 0; }
+  }
+}
+
+// largest component: size[] is non-zero at roots only; integer max, so the result does not depend on the order
+static __global__ void __launch_bounds__(256) ccl_max_size_kernel(const int* __restrict__ size, int* __restrict__ max_size, int64_t V) {
+  int m = 0;
+  for (int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; v < V; v += (int64_t)gridDim.x * blockDim.x) m = max(m, size[v]);
+  for (int o = 16; o; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0 && m > 0) atomicMax(max_size, m);
+}
+
+// Zero the voxels of the mask whose component is not of the largest size and, when min_valid_mm3 >= 0, is smaller than
+// min_valid_mm3 (count * volume_per_voxel in fp64, as upstream compares its sizes).  Voxels outside the mask are not written.
+static __global__ void __launch_bounds__(256) ccl_keep_largest_kernel(const int* __restrict__ L, const int* __restrict__ size,
+                                                                      const int* __restrict__ max_size, uint8_t* __restrict__ seg,
+                                                                      double volume_per_voxel, double min_valid_mm3, int64_t V) {
+  const int keep = *max_size;
+  for (int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; v < V; v += (int64_t)gridDim.x * blockDim.x) {
+    const int r = L[v];
+    if (r < 0) continue;
+    const int n = size[r];
+    if (n == keep) continue;
+    if (min_valid_mm3 >= 0.0 && (double)n * volume_per_voxel >= min_valid_mm3) continue;
+    seg[v] = 0;
   }
 }
 

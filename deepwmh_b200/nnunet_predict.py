@@ -11,7 +11,9 @@ with RESULTS_FOLDER / CUDA_VISIBLE_DEVICES in the environment (predict.py:101,15
 the same meaning: inputs `<in>/<case>_0000.nii.gz` (models with M modalities: `<case>_0000 ... <case>_000{M-1}.nii.gz`, the
 modality order of the training data), outputs `<out>/<case>.nii.gz` (uint8 labels 0 .. C-1), `<out>/<case>_0.nii.gz`
 (background probability, the fork's --save_softmax, read back at DCNN_multistage.py:359) and a copy of plans.pkl
-(upstream copies it; DeepWMH ignores it, predict.py:159-162).  Any failure raises -> non-zero exit, which is what
+(upstream copies it; DeepWMH ignores it, predict.py:159-162).  Unless --disable_post_processing is given, a
+`postprocessing.json` in the trainer folder is applied to each label file on the device and copied to the output folder,
+as upstream's predict_cases does (DESIGN §11; DeepWMH passes the flag).  Any failure raises -> non-zero exit, which is what
 `run_shell` turns into `exit(msg)` (deepwmh/utilities/external_call.py:63-72).  Flags of upstream nnUNet_predict that
 DeepWMH never passes and this path does not implement are rejected loudly rather than ignored.
 """
@@ -24,6 +26,7 @@ import sys
 from typing import List
 
 from . import cli as _cli
+from . import postprocessing as _pp
 
 
 def _cases_in(folder: str) -> List[str]:
@@ -53,7 +56,7 @@ def main(argv=None) -> int:
     ap.add_argument("-z", "--save_npz", action="store_true")
     ap.add_argument("--save_softmax", action="store_true", help="[fork] also write the background probability as <case>_0.nii.gz")
     ap.add_argument("--disable_tta", action="store_true", help="no mirroring (8x faster)")
-    ap.add_argument("--disable_post_processing", action="store_true", help="accepted; no postprocessing.json is ever applied here")
+    ap.add_argument("--disable_post_processing", action="store_true", help="do not apply the trainer folder's postprocessing.json (keep the largest component of its classes) to the label files")
     ap.add_argument("--selected_cases", nargs="+", default=None, help="[fork] only predict these case names")
     ap.add_argument("--overwrite_existing", action="store_true")
     ap.add_argument("--step_size", type=float, default=0.5)
@@ -102,8 +105,18 @@ def main(argv=None) -> int:
     plans = _cli.load_plans(plans_path)
     n_mod = int(plans.get("num_modalities", 1))
     inputs = {c: case_files(args.input_folder, c, n_mod) for c in cases}     # every modality present before any GPU work
+    pp_file = os.path.join(tdir, "postprocessing.json")
+    for_which_classes, min_sizes = None, None
+    if not args.disable_post_processing:
+        if os.path.isfile(pp_file):
+            for_which_classes, min_sizes = _pp.load_postprocessing(pp_file)   # a malformed json fails before any GPU work
+        else:
+            print("WARNING! Cannot run postprocessing because the postprocessing file is missing. Make sure to run "
+                  "consolidate_folds in the output folder of the model first!\nThe folder you need to run this in is %s" % tdir)
     os.makedirs(args.output_folder, exist_ok=True)
     shutil.copy(plans_path, args.output_folder)
+    if for_which_classes is not None:
+        shutil.copy(pp_file, args.output_folder)
     todo = []
     for c in cases:
         out = os.path.join(args.output_folder, c + ".nii.gz")
@@ -124,7 +137,7 @@ def main(argv=None) -> int:
         print("predicting", c)
         _cli.predict_case(trainer, plans, inputs[c], os.path.join(args.output_folder, c + ".nii.gz"),
                           softmax_file=os.path.join(args.output_folder, c + "_0.nii.gz") if args.save_softmax else None,
-                          do_mirroring=not args.disable_tta)
+                          do_mirroring=not args.disable_tta, for_which_classes=for_which_classes, min_valid_object_sizes=min_sizes)
     trainer.network.close()
     return 0
 

@@ -250,6 +250,16 @@ class SegmentationNetwork:
         check(self._lib.dwmh_remove_sparks(self._ctx, _ptr(seg), X, Y, Z, int(min_volume), _ptr(out), self._st()))
         return out
 
+    def keep_largest_components_(self, seg: torch.Tensor, class_mask: int, volume_per_voxel: float, min_valid_mm3: float = -1.0) -> torch.Tensor:
+        """One entry of nnU-Net's postprocessing.json in place on a uint8 label map [X,Y,Z] (deepwmh_b200/postprocessing.py):
+        of the 6-connected components of the classes in class_mask (bit c = class c), the largest stay and so do those of at
+        least min_valid_mm3 (if >= 0); the voxels of every other one become 0."""
+        assert seg.is_cuda and seg.dtype == torch.uint8 and seg.is_contiguous() and seg.dim() == 3
+        X, Y, Z = seg.shape
+        check(self._lib.dwmh_keep_largest_components(self._ctx, _ptr(seg), X, Y, Z, int(class_mask), float(volume_per_voxel),
+                                                     float(min_valid_mm3), self._st()))
+        return seg
+
     def remove_3mm_sparks(self, seg: torch.Tensor, voxel_size: Sequence[float]) -> torch.Tensor:
         """`remove_3mm_sparks` (image_ops.py:346-367): the voxel-size rule on the host, the component filter on the device."""
         vs = [float(v) for v in voxel_size]

@@ -223,16 +223,20 @@ def preprocess_test_case(network, plans: Dict, input_files: Sequence[str], force
 
 
 def save_segmentation_nifti_from_softmax(network, softmax, out_fname: str, properties: Dict, order: int = 1, force_separate_z=None,
-                                         softmax_fname: Optional[str] = None, post3mm_fname: Optional[str] = None):
+                                         softmax_fname: Optional[str] = None, post3mm_fname: Optional[str] = None,
+                                         for_which_classes=None, min_valid_object_sizes=None):
     """[U:inference/segmentation_export.py::save_segmentation_nifti_from_softmax]: softmax [classes, x, y, z] (ALREADY
     transposed back; CUDA tensor or numpy) -> resample back to the cropped grid (order 1, device) -> argmax (labels
     0 .. classes-1, ties to the lower class) -> paste into
     zeros(original size) at the crop box -> uint8 NIfTI with the input's header.  softmax_fname: the fork's
     `--save_softmax` (background probability as `<case>_0.nii.gz`, DCNN_multistage.py:340-343,359: 1 outside the crop);
-    post3mm_fname: `remove_3mm_sparks` of the label map on the device (deepwmh/main/predict.py:19-26,158-163)."""
+    post3mm_fname: `remove_3mm_sparks` of the label map on the device (deepwmh/main/predict.py:19-26,158-163).
+    for_which_classes / min_valid_object_sizes: a postprocessing.json (deepwmh_b200/postprocessing.py), applied on the
+    device to the label file only, as upstream's predict_cases rewrites that file; the other outputs do not see it.
+    Returns the label map as written."""
     import torch
 
-    from . import nifti
+    from . import nifti, postprocessing
     hdr = properties["nifti_header"]
     with torch.cuda.device(network.device):
         sm = softmax if isinstance(softmax, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(softmax))
@@ -244,7 +248,13 @@ def save_segmentation_nifti_from_softmax(network, softmax, out_fname: str, prope
         sl = tuple(slice(b[0], b[1]) for b in properties["crop_bbox"])
         full = torch.zeros(full_shape, dtype=torch.uint8, device=network.device)
         full[sl] = seg
-        nifti.write_nifti(out_fname, np.transpose(full.cpu().numpy(), (2, 1, 0)), hdr, dtype=np.uint8)
+        labels = full
+        if for_which_classes:
+            # [U:inference/predict.py::predict_cases -> load_remove_save]: sizes in mm^3 of the written image's spacing
+            volume_per_voxel = float(np.prod(np.asarray(hdr["spacing"], dtype=np.float64)))
+            labels = postprocessing.remove_all_but_the_largest_connected_component(network, full.clone(), for_which_classes,
+                                                                                    volume_per_voxel, min_valid_object_sizes)
+        nifti.write_nifti(out_fname, np.transpose(labels.cpu().numpy(), (2, 1, 0)), hdr, dtype=np.uint8)
         if post3mm_fname is not None:
             clean = network.remove_3mm_sparks(full.contiguous(), list(hdr["spacing"][::-1])).cpu().numpy()
             nifti.write_nifti(post3mm_fname, np.transpose(clean, (2, 1, 0)).astype(np.float32), hdr, dtype=np.float32)
@@ -252,4 +262,4 @@ def save_segmentation_nifti_from_softmax(network, softmax, out_fname: str, prope
             bg = torch.ones(full_shape, dtype=torch.float32, device=network.device)
             bg[sl] = sm[0]
             nifti.write_nifti(softmax_fname, np.transpose(bg.cpu().numpy(), (2, 1, 0)), hdr, dtype=np.float32)
-    return full
+    return labels

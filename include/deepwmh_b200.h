@@ -137,6 +137,16 @@ int dwmh_ensemble_refine(dwmh_ctx* ctx, float* acc_dev, int32_t k, uint8_t* labe
 int dwmh_remove_sparks(dwmh_ctx* ctx, const uint8_t* seg_dev, int32_t X, int32_t Y, int32_t Z, int32_t min_volume,
                        uint8_t* out_dev, void* stream);
 
+/* nnU-Net v1 postprocessing, one entry of postprocessing.json: mask = label is in the class set (bit c of class_mask, bit 0 must be
+ * clear); 6-connected components of mask; the components with the largest voxel count are kept, every other one is set to 0
+ * unless min_valid_mm3 >= 0 and count * volume_per_voxel >= min_valid_mm3 (fp64).  No host synchronisation.
+ * seg_dev: uint8 [X][Y][Z], modified in place; voxels outside the mask are never written.  Five launches, all on `stream`.
+ * Refused before any device work: null ctx / seg_dev, an empty volume, X*Y*Z >= 2^31, class_mask == 0 or with bit 0 set,
+ * volume_per_voxel <= 0 or not finite, min_valid_mm3 NaN.  Applying a whole for_which_classes list is one call per entry,
+ * in order (deepwmh_b200/postprocessing.py). */
+int dwmh_keep_largest_components(dwmh_ctx* ctx, uint8_t* seg_dev, int32_t X, int32_t Y, int32_t Z, uint32_t class_mask,
+                                 double volume_per_voxel, double min_valid_mm3, void* stream);
+
 /* --- SURVEY 8f-4: stage-1 NLL anomaly map (deepwmh/analysis/lesion_analysis.py:84-176) ---------------------------
  * Context-free (no network involved): `device` is the CUDA ordinal; every buffer is a caller-owned device pointer,
  * volumes fp32 [X][Y][Z], masks fp32 with the reference's `> 0.5` convention.  fp64 arithmetic per voxel, fp32 storage.
