@@ -44,7 +44,6 @@ SYMBOLS = {
     "dwmh_weight_map": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_int32, _P, _P]),
     "dwmh_finalize": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, _P]),
     "dwmh_axpy": (C.c_int, [_P, _P, _P, C.c_float, C.c_int64, _P]),
-    "dwmh_argmax2": (C.c_int, [_P, _P, _P, C.c_int64, _P]),
     "dwmh_argmax": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int64, _P]),
     "dwmh_ensemble_masked_add": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P]),
     "dwmh_ensemble_refine": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int64, _P]),

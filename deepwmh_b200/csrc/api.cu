@@ -11,6 +11,7 @@
 #include <cstring>
 #include <map>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "common.cuh"
@@ -49,7 +50,7 @@ struct DevGuard {
 
 extern "C" const char* dwmh_last_error(void) { return g_err.c_str(); }
 extern "C" void dwmh_internal_set_error(const char* msg) { g_err = msg ? msg : ""; }   // for the other translation units (stage1.cu)
-extern "C" int dwmh_version(void) { return 100; }
+extern "C" int dwmh_version(void) { return 101; }
 
 // ------------------------------------------------------------------------------------------------
 // network plan
@@ -611,15 +612,19 @@ extern "C" int dwmh_zscore(dwmh_ctx* c, float* vol, const int8_t* seg, int64_t n
 // ------------------------------------------------------------------------------------------------
 // forward
 // ------------------------------------------------------------------------------------------------
-// head of a model with NC = 3 .. DWMH_MAX_CLASSES classes
-template <typename T>
-static int launch_head_c(int NC, dim3 grid, cudaStream_t st, const T* y, NormParams np, const float* w, float* probs, int C, int64_t V) {
-  const size_t smem = (size_t)(2 + NC) * C * sizeof(float);
+// The kernels after the last conv (head, overlap-add, finalize) are instantiated for each class count 2 .. DWMH_MAX_CLASSES:
+// f(std::integral_constant<int, NC>) launches them for the model's count.
+template <typename F>
+static int with_num_classes(int NC, F&& f) {
   switch (NC) {
-#define DWMH_HEAD_C(K) case K: head_softmax_c_kernel<T, K><<<grid, 256, smem, st>>>(y, np, w, probs, C, V); return 0
-    DWMH_HEAD_C(3); DWMH_HEAD_C(4); DWMH_HEAD_C(5); DWMH_HEAD_C(6); DWMH_HEAD_C(7); DWMH_HEAD_C(8);
-#undef DWMH_HEAD_C
-    default: return fail("internal: no head for %d classes", NC);
+    case 2: return f(std::integral_constant<int, 2>{});
+    case 3: return f(std::integral_constant<int, 3>{});
+    case 4: return f(std::integral_constant<int, 4>{});
+    case 5: return f(std::integral_constant<int, 5>{});
+    case 6: return f(std::integral_constant<int, 6>{});
+    case 7: return f(std::integral_constant<int, 7>{});
+    case 8: return f(std::integral_constant<int, 8>{});
+    default: return fail("internal: no kernels for %d classes", NC);
   }
 }
 
@@ -724,11 +729,11 @@ static int forward_impl(dwmh_ctx* c, const float* src, int patch_mode, int SX, i
   dim3 grid((unsigned)((head_items + 255) / 256), nb);
   const int NC = c->d.num_classes;
   DW_TRY(cls_timed(2, (double)nb * L.vout() * (2.0 * L.cout + 4.0 * NC), [&] {
-    if (NC == 2) {
-      head_softmax_kernel<T><<<grid, 256, 4 * L.cout * sizeof(float), st>>>((const T*)L.out, norm_of(L), c->w_head_dev, c->probs, L.cout, L.vout());
-      return 0;
-    }
-    return launch_head_c<T>(NC, grid, st, (const T*)L.out, norm_of(L), c->w_head_dev, c->probs, L.cout, L.vout()); }));
+    return with_num_classes(NC, [&](auto nc) {
+      constexpr int K = decltype(nc)::value;
+      head_softmax_kernel<T, K><<<grid, 256, (2 + K) * L.cout * sizeof(float), st>>>((const T*)L.out, norm_of(L), c->w_head_dev, c->probs,
+                                                                                    L.cout, L.vout());
+      return 0; }); }));
   c->launches++;
   c->conv_flops += 2.0 * L.vout() * L.cout * c->d.num_classes * nb;
   CU_TRY(cudaGetLastError());
@@ -840,17 +845,14 @@ extern "C" int dwmh_predict_3d(dwmh_ctx* c, const float* vol, int32_t X, int32_t
     if (c->stage_timing) CU_TRY(cudaEventRecord(c->ev[0], st));
     DW_TRY(forward(c, vol, 0, X, Y, Z, c->metas_dev + (size_t)t0 * M, tb * M, st));
     if (c->stage_timing) CU_TRY(cudaEventRecord(c->ev[1], st));
-    for (int t = 0; t < tb; ++t) {
-      if (NC == 2)
-        aggregate_tile_kernel<<<(unsigned)((P + 255) / 256), 256, 0, st>>>(
-            c->probs + (size_t)t * M * 2 * P, c->metas_dev + (size_t)(t0 + t) * M, M, gauss ? c->gauss_dev : nullptr,
+    DW_TRY(with_num_classes(NC, [&](auto nc) {
+      constexpr int K = decltype(nc)::value;
+      for (int t = 0; t < tb; ++t)
+        aggregate_tile_kernel<K><<<(unsigned)((P + 255) / 256), 256, 0, st>>>(
+            c->probs + (size_t)t * M * K * P, c->metas_dev + (size_t)(t0 + t) * M, M, gauss ? c->gauss_dev : nullptr,
             agg, wgt, ps[0], ps[1], ps[2], X, Y, Z);
-      else
-        aggregate_tile_c_kernel<<<(unsigned)((P + 255) / 256), 256, 0, st>>>(
-            c->probs + (size_t)t * M * NC * P, c->metas_dev + (size_t)(t0 + t) * M, M, NC, gauss ? c->gauss_dev : nullptr,
-            agg, wgt, ps[0], ps[1], ps[2], X, Y, Z);
-      c->launches++;
-    }
+      return 0; }));
+    c->launches += tb;
     if (c->stage_timing) {
       CU_TRY(cudaEventRecord(c->ev[2], st));
       CU_TRY(cudaEventSynchronize(c->ev[2]));
@@ -899,16 +901,13 @@ extern "C" int dwmh_finalize(dwmh_ctx* c, const float* agg, const float* wgt, fl
   cudaStream_t st = (cudaStream_t)stream_;
   DEV_GUARD(c->device);
   const int64_t V = (int64_t)X * Y * Z;
-  if (c->d.num_classes != 2) {
-    finalize_c_kernel<<<c->num_sms * 8, 256, 0, st>>>(agg, wgt, softmax, seg, c->d.num_classes, V);
-    c->launches++;
-    CU_TRY(cudaGetLastError());
-    return 0;
-  }
   const bool vec = (V & 3) == 0 && !((reinterpret_cast<uintptr_t>(agg) | reinterpret_cast<uintptr_t>(wgt) | reinterpret_cast<uintptr_t>(softmax)) & 15) &&
                    !(reinterpret_cast<uintptr_t>(seg) & 3);
-  if (vec) finalize_kernel<true><<<c->num_sms * 8, 256, 0, st>>>(agg, wgt, softmax, seg, V);
-  else finalize_kernel<false><<<c->num_sms * 8, 256, 0, st>>>(agg, wgt, softmax, seg, V);
+  DW_TRY(with_num_classes(c->d.num_classes, [&](auto nc) {
+    constexpr int K = decltype(nc)::value;
+    if (vec) finalize_kernel<K, true><<<c->num_sms * 8, 256, 0, st>>>(agg, wgt, softmax, seg, V);
+    else finalize_kernel<K, false><<<c->num_sms * 8, 256, 0, st>>>(agg, wgt, softmax, seg, V);
+    return 0; }));
   c->launches++;
   CU_TRY(cudaGetLastError());
   return 0;
@@ -923,20 +922,11 @@ extern "C" int dwmh_axpy(dwmh_ctx* c, float* acc, const float* x, float alpha, i
   return 0;
 }
 
-extern "C" int dwmh_argmax2(dwmh_ctx* c, const float* p, uint8_t* seg, int64_t V, void* stream_) {
-  if (!c || !p || !seg) return fail("dwmh_argmax2: null argument");
-  DEV_GUARD(c->device);
-  argmax2_kernel<<<c->num_sms * 8, 256, 0, (cudaStream_t)stream_>>>(p, seg, V);
-  c->launches++;
-  CU_TRY(cudaGetLastError());
-  return 0;
-}
-
 extern "C" int dwmh_argmax(dwmh_ctx* c, const float* p, int32_t num_classes, uint8_t* seg, int64_t V, void* stream_) {
   if (!c || !p || !seg) return fail("dwmh_argmax: null argument");
   if (num_classes < 1 || num_classes > 255) return fail("dwmh_argmax: num_classes=%d outside 1..255 (uint8 labels)", num_classes);
   DEV_GUARD(c->device);
-  argmax_c_kernel<<<c->num_sms * 8, 256, 0, (cudaStream_t)stream_>>>(p, num_classes, seg, V);
+  argmax_kernel<<<c->num_sms * 8, 256, 0, (cudaStream_t)stream_>>>(p, num_classes, seg, V);
   c->launches++;
   CU_TRY(cudaGetLastError());
   return 0;

@@ -102,110 +102,10 @@ __global__ void __launch_bounds__(256) zscore_fused_kernel(float* __restrict__ v
 }
 
 // ---------------------------------------------------------------------------------------------
-// Head: InstanceNorm+LeakyReLU of the last decoder conv applied on load, 1x1x1 conv to 2 logits
-// (seg_outputs[-1], no bias), softmax over classes (inference_apply_nonlin).  One thread per voxel,
-// grid.y = sample.  y: [n][C/8][V][8] raw conv output; probs: [n][2][V] fp32.
-// ---------------------------------------------------------------------------------------------
-template <typename T>
-__global__ void __launch_bounds__(256) head_softmax_kernel(const T* __restrict__ y, NormParams np,
-                                                           const float* __restrict__ w_head,   // [2][C]
-                                                           float* __restrict__ probs, int C, int64_t V) {
-  extern __shared__ __align__(16) float sm[];          // a[C], b[C], w0[C], w1[C]
-  float* sa = sm; float* sb = sm + C; float* w0 = sm + 2 * C; float* w1 = sm + 3 * C;
-  const int n = blockIdx.y;
-  for (int c = threadIdx.x; c < C; c += blockDim.x) {
-    float a = 1.f, b = 0.f;
-    if (np.sums) norm_coeffs(np, n, C, c, a, b);
-    sa[c] = a; sb[c] = b; w0[c] = w_head[c]; w1[c] = w_head[C + c];
-  }
-  __syncthreads();
-  if (C == 32 && (V & 1) == 0) {
-    // the usual head, two voxels per thread (grid sized for V / 2): four 256-bit loads in flight, coefficients read from shared
-    // memory as float4 and used for both voxels -- one voxel per thread with scalar coefficient reads was bound by instruction
-    // issue (~330 instructions per voxel, 4.9 TB/s), not by HBM.  Same arithmetic order per voxel.
-    const int64_t v2 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (2 * v2 >= V) return;
-    const uint4* yp2 = reinterpret_cast<const uint4*>(y) + (size_t)n * 4 * V + 2 * v2;
-    uint4 q[4][2];
-#pragma unroll
-    for (int cc = 0; cc < 4; ++cc) ld_global_256(yp2 + (size_t)cc * V, q[cc][0], q[cc][1]);
-    float l[2][2] = {{0.f, 0.f}, {0.f, 0.f}};
-    const float4* sa4 = reinterpret_cast<const float4*>(sa); const float4* sb4 = reinterpret_cast<const float4*>(sb);
-    const float4* w04 = reinterpret_cast<const float4*>(w0); const float4* w14 = reinterpret_cast<const float4*>(w1);
-#pragma unroll
-    for (int cc = 0; cc < 4; ++cc) {
-      float f[2][8];
-      unpack8<T>(q[cc][0], f[0]); unpack8<T>(q[cc][1], f[1]);
-#pragma unroll
-      for (int h = 0; h < 2; ++h) {
-        const float4 a4 = sa4[cc * 2 + h], b4 = sb4[cc * 2 + h], u4 = w04[cc * 2 + h], v4 = w14[cc * 2 + h];
-        const float ca[4] = {a4.x, a4.y, a4.z, a4.w}, cb[4] = {b4.x, b4.y, b4.z, b4.w};
-        const float cu[4] = {u4.x, u4.y, u4.z, u4.w}, cv[4] = {v4.x, v4.y, v4.z, v4.w};
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            const float x = np.sums ? lrelu(fmaf(ca[j], f[e][h * 4 + j], cb[j])) : f[e][h * 4 + j];
-            l[e][0] = fmaf(cu[j], x, l[e][0]);
-            l[e][1] = fmaf(cv[j], x, l[e][1]);
-          }
-      }
-    }
-    float p0[2], p1[2];
-#pragma unroll
-    for (int e = 0; e < 2; ++e) {
-      const float m = fmaxf(l[e][0], l[e][1]);
-      const float e0 = expf(l[e][0] - m), e1 = expf(l[e][1] - m);
-      const float s_ = e0 + e1;
-      p0[e] = e0 / s_; p1[e] = e1 / s_;
-    }
-    *reinterpret_cast<float2*>(probs + ((size_t)n * 2 + 0) * V + 2 * v2) = make_float2(p0[0], p0[1]);
-    *reinterpret_cast<float2*>(probs + ((size_t)n * 2 + 1) * V + 2 * v2) = make_float2(p1[0], p1[1]);
-    return;
-  }
-  const int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (v >= V) return;
-  const uint4* yp = reinterpret_cast<const uint4*>(y) + (size_t)n * (C >> 3) * V + v;
-  float l0 = 0.f, l1 = 0.f;
-  if (C == 32) {          // all four channel chunks in flight before the first use
-    uint4 q[4];
-#pragma unroll
-    for (int cc = 0; cc < 4; ++cc) q[cc] = ld_stream(yp + (size_t)cc * V);
-#pragma unroll
-    for (int cc = 0; cc < 4; ++cc) {
-      float f[8];
-      unpack8<T>(q[cc], f);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const int c = cc * 8 + j;
-        const float x = np.sums ? lrelu(fmaf(sa[c], f[j], sb[c])) : f[j];
-        l0 = fmaf(w0[c], x, l0);
-        l1 = fmaf(w1[c], x, l1);
-      }
-    }
-  } else
-  for (int cc = 0; cc < (C >> 3); ++cc) {
-    float f[8];
-    unpack8<T>(ld_stream(yp + (size_t)cc * V), f);
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const int c = cc * 8 + j;
-      const float x = np.sums ? lrelu(fmaf(sa[c], f[j], sb[c])) : f[j];
-      l0 = fmaf(w0[c], x, l0);
-      l1 = fmaf(w1[c], x, l1);
-    }
-  }
-  const float m = fmaxf(l0, l1);
-  const float e0 = expf(l0 - m), e1 = expf(l1 - m);
-  const float s = e0 + e1;
-  probs[((size_t)n * 2 + 0) * V + v] = e0 / s;
-  probs[((size_t)n * 2 + 1) * V + v] = e1 / s;
-}
-
-// ---------------------------------------------------------------------------------------------
-// The same head for NC = 3..8 classes (models with more than background + one label): logits l_k = sum_c w[k][c] x_c,
-// p_k = exp(l_k - max) / sum_k' exp(l_k' - max) in fp32, summed in class order.  probs: [n][NC][V].  Loads and shared
-// coefficient reads as in head_softmax_kernel (two voxels per thread and 256-bit loads when C == 32 and V is even).
+// Head: InstanceNorm+LeakyReLU of the last decoder conv applied on load, 1x1x1 conv to NC = 2..8 logits
+// (seg_outputs[-1], no bias), softmax over classes (inference_apply_nonlin): l_k = sum_c w[k][c] x_c,
+// p_k = exp(l_k - max) / sum_k' exp(l_k' - max) in fp32, summed in class order.  One thread per voxel (two when
+// C == 32 and V is even), grid.y = sample.  y: [n][C/8][V][8] raw conv output; probs: [n][NC][V] fp32.
 // ---------------------------------------------------------------------------------------------
 template <int NC>
 __device__ __forceinline__ void softmax_nc(const float (&l)[NC], float (&p)[NC]) {
@@ -220,9 +120,9 @@ __device__ __forceinline__ void softmax_nc(const float (&l)[NC], float (&p)[NC])
 }
 
 template <typename T, int NC>
-__global__ void __launch_bounds__(256) head_softmax_c_kernel(const T* __restrict__ y, NormParams np,
-                                                             const float* __restrict__ w_head,   // [NC][C]
-                                                             float* __restrict__ probs, int C, int64_t V) {
+__global__ void __launch_bounds__(256) head_softmax_kernel(const T* __restrict__ y, NormParams np,
+                                                           const float* __restrict__ w_head,   // [NC][C]
+                                                           float* __restrict__ probs, int C, int64_t V) {
   extern __shared__ __align__(16) float sm[];          // a[C], b[C], w[NC][C]
   float* sa = sm; float* sb = sm + C; float* sw = sm + 2 * C;
   const int n = blockIdx.y;
@@ -234,6 +134,9 @@ __global__ void __launch_bounds__(256) head_softmax_c_kernel(const T* __restrict
   for (int i = threadIdx.x; i < NC * C; i += blockDim.x) sw[i] = w_head[i];
   __syncthreads();
   if (C == 32 && (V & 1) == 0) {
+    // the usual head, two voxels per thread (grid sized for V / 2): four 256-bit loads in flight, coefficients read from shared
+    // memory as float4 and used for both voxels -- one voxel per thread with scalar coefficient reads was bound by instruction
+    // issue (~330 instructions per voxel, 4.9 TB/s), not by HBM.  Same arithmetic order per voxel.
     const int64_t v2 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (2 * v2 >= V) return;
     const uint4* yp2 = reinterpret_cast<const uint4*>(y) + (size_t)n * 4 * V + 2 * v2;
@@ -285,9 +188,9 @@ __global__ void __launch_bounds__(256) head_softmax_c_kernel(const T* __restrict
   float l[NC];
 #pragma unroll
   for (int k = 0; k < NC; ++k) l[k] = 0.f;
-  for (int cc = 0; cc < (C >> 3); ++cc) {
+  auto add_chunk = [&](const uint4& q, int cc) {
     float f[8];
-    unpack8<T>(ld_stream(yp + (size_t)cc * V), f);
+    unpack8<T>(q, f);
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
       const int c = cc * 8 + j;
@@ -295,6 +198,15 @@ __global__ void __launch_bounds__(256) head_softmax_c_kernel(const T* __restrict
 #pragma unroll
       for (int k = 0; k < NC; ++k) l[k] = fmaf(sw[k * C + c], x, l[k]);
     }
+  };
+  if (C == 32) {          // all four channel chunks in flight before the first use
+    uint4 q[4];
+#pragma unroll
+    for (int cc = 0; cc < 4; ++cc) q[cc] = ld_stream(yp + (size_t)cc * V);
+#pragma unroll
+    for (int cc = 0; cc < 4; ++cc) add_chunk(q[cc], cc);
+  } else {
+    for (int cc = 0; cc < (C >> 3); ++cc) add_chunk(ld_stream(yp + (size_t)cc * V), cc);
   }
   float p[NC];
   softmax_nc<NC>(l, p);
@@ -304,10 +216,11 @@ __global__ void __launch_bounds__(256) head_softmax_c_kernel(const T* __restrict
 
 // ---------------------------------------------------------------------------------------------
 // a11/a12  One tile: result = sum_m (1/M) * unflip_m(p_m); result *= gaussian; agg[:, tile] += result;
-// wgt[tile] += gaussian.  Same fp32 operation order as the reference.  Tiles are aggregated by
+// wgt[tile] += gaussian.  Same fp32 operation order as the reference, per class.  Tiles are aggregated by
 // consecutive launches on one stream, so the overlap-add is deterministic (no atomics).
-// probs: [M][2][P] for this tile; metas[m].flip gives the mirror of sample m.
+// probs: [M][NC][P] for this tile; metas[m].flip gives the mirror of sample m.
 // ---------------------------------------------------------------------------------------------
+template <int NC>
 __global__ void __launch_bounds__(256) aggregate_tile_kernel(const float* __restrict__ probs,
                                                              const SampleMeta* __restrict__ metas, int M,
                                                              const float* __restrict__ gauss,   // [P] or nullptr
@@ -320,41 +233,9 @@ __global__ void __launch_bounds__(256) aggregate_tile_kernel(const float* __rest
   const int j = (int)((v / pz) % py);
   const int i = (int)(v / ((int64_t)pz * py));
   const float inv = 1.0f / (float)M;
-  float r0 = 0.f, r1 = 0.f;
-  for (int m = 0; m < M; ++m) {
-    const int f = metas[m].flip;
-    const int kk = (f & 1) ? pz - 1 - k : k;
-    const int jj = (f & 2) ? py - 1 - j : j;
-    const int ii = (f & 4) ? px - 1 - i : i;
-    const int64_t src = ((int64_t)ii * py + jj) * pz + kk;
-    r0 += inv * probs[((size_t)m * 2 + 0) * P + src];
-    r1 += inv * probs[((size_t)m * 2 + 1) * P + src];
-  }
-  const float g = gauss ? gauss[v] : 1.0f;
-  if (gauss) { r0 *= g; r1 *= g; }
-  const int64_t V = (int64_t)X * Y * Z;
-  const int64_t dst = ((int64_t)(metas[0].ox + i) * Y + (metas[0].oy + j)) * Z + (metas[0].oz + k);
-  agg[dst] += r0;
-  agg[V + dst] += r1;
-  wgt[dst] += g;
-}
-
-// The same for NC <= 8 classes: probs [M][NC][P]; per class the operation order of aggregate_tile_kernel.
-__global__ void __launch_bounds__(256) aggregate_tile_c_kernel(const float* __restrict__ probs,
-                                                               const SampleMeta* __restrict__ metas, int M, int NC,
-                                                               const float* __restrict__ gauss,   // [P] or nullptr
-                                                               float* __restrict__ agg, float* __restrict__ wgt,
-                                                               int px, int py, int pz, int X, int Y, int Z) {
-  const int64_t P = (int64_t)px * py * pz;
-  const int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (v >= P) return;
-  const int k = (int)(v % pz);
-  const int j = (int)((v / pz) % py);
-  const int i = (int)(v / ((int64_t)pz * py));
-  const float inv = 1.0f / (float)M;
-  float r[8];
+  float r[NC];
 #pragma unroll
-  for (int c = 0; c < 8; ++c) r[c] = 0.f;
+  for (int c = 0; c < NC; ++c) r[c] = 0.f;
   for (int m = 0; m < M; ++m) {
     const int f = metas[m].flip;
     const int kk = (f & 1) ? pz - 1 - k : k;
@@ -362,18 +243,19 @@ __global__ void __launch_bounds__(256) aggregate_tile_c_kernel(const float* __re
     const int ii = (f & 4) ? px - 1 - i : i;
     const int64_t src = ((int64_t)ii * py + jj) * pz + kk;
 #pragma unroll
-    for (int c = 0; c < 8; ++c)
-      if (c < NC) r[c] += inv * probs[((size_t)m * NC + c) * P + src];
+    for (int c = 0; c < NC; ++c) r[c] += inv * probs[((size_t)m * NC + c) * P + src];
   }
   const float g = gauss ? gauss[v] : 1.0f;
   const int64_t V = (int64_t)X * Y * Z;
   const int64_t dst = ((int64_t)(metas[0].ox + i) * Y + (metas[0].oy + j)) * Z + (metas[0].oz + k);
+  // agg += r * g.  Two classes round the product before the add (the reference's `*=` then `+=`); more classes add it with
+  // one rounding, as the separate kernel these counts ran on was compiled to.  The intrinsics pin both, so every class count
+  // keeps its earlier results.  With g = 1 (no Gaussian) both are the plain sum.
 #pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    if (c < NC) {
-      if (gauss) r[c] *= g;
-      agg[(size_t)c * V + dst] += r[c];
-    }
+  for (int c = 0; c < NC; ++c) {
+    float& a = agg[(size_t)c * V + dst];
+    if constexpr (NC == 2) a = __fadd_rn(a, __fmul_rn(r[c], g));
+    else a = __fmaf_rn(r[c], g, a);
   }
   wgt[dst] += g;
 }
@@ -411,59 +293,67 @@ __global__ void __launch_bounds__(256) weight_map_kernel(const float* __restrict
 }
 
 // ---------------------------------------------------------------------------------------------
-// a12 tail: class_probabilities = agg / wgt; seg = argmax (first maximum).  21 B/voxel.
+// a12 tail: class_probabilities = agg / wgt; seg = argmax (first maximum, numpy.argmax).  (8 NC + 5) B/voxel.
 // ---------------------------------------------------------------------------------------------
-// softmax_out may alias agg (in-place normalisation): neither is __restrict__ and every thread reads its own
-// elements before it writes them.
-template <bool VEC>      // VEC: V % 4 == 0 and every buffer 16-byte (seg: 4-byte) aligned
-__global__ void __launch_bounds__(256) finalize_kernel(const float* agg, const float* __restrict__ wgt,
-                                                       float* softmax_out, uint8_t* __restrict__ seg,
-                                                       int64_t V) {
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  if constexpr (VEC) {
-    // 128-bit accesses (four voxels per thread and step): the pass is a pure stream, bound by bytes in flight
-    const int64_t V4 = V >> 2;
-    const float4* a0 = reinterpret_cast<const float4*>(agg); const float4* a1 = reinterpret_cast<const float4*>(agg + V);
-    const float4* w4 = reinterpret_cast<const float4*>(wgt);
-    float4* o0 = reinterpret_cast<float4*>(softmax_out); float4* o1 = softmax_out ? reinterpret_cast<float4*>(softmax_out + V) : nullptr;
-    uchar4* s4 = reinterpret_cast<uchar4*>(seg);
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < V4; i += stride) {
-      const float4 w = w4[i], x = a0[i], y = a1[i];
-      const float4 p0 = make_float4(x.x / w.x, x.y / w.y, x.z / w.z, x.w / w.w);
-      const float4 p1 = make_float4(y.x / w.x, y.y / w.y, y.z / w.z, y.w / w.w);
-      if (softmax_out) { o0[i] = p0; o1[i] = p1; }
-      if (seg) s4[i] = make_uchar4(p1.x > p0.x, p1.y > p0.y, p1.z > p0.z, p1.w > p0.w);
-    }
-    return;
+// p[c] /= w for every class; returns the first class holding the maximum
+template <int NC>
+__device__ __forceinline__ uint8_t divide_argmax(float (&p)[NC], float w) {
+  p[0] = p[0] / w;
+  float best = p[0];
+  int arg = 0;
+#pragma unroll
+  for (int c = 1; c < NC; ++c) {
+    p[c] = p[c] / w;
+    if (p[c] > best) { best = p[c]; arg = c; }
   }
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < V; i += stride) {
-    const float w = wgt[i];
-    const float p0 = agg[i] / w, p1 = agg[V + i] / w;
-    if (softmax_out) { softmax_out[i] = p0; softmax_out[V + i] = p1; }
-    if (seg) seg[i] = p1 > p0 ? 1 : 0;
-  }
+  return (uint8_t)arg;
 }
 
-// NC classes: softmax_out [NC][V] (may alias agg) = agg / wgt; seg = the first class holding the maximum (numpy.argmax).
-__global__ void __launch_bounds__(256) finalize_c_kernel(const float* agg, const float* __restrict__ wgt, float* softmax_out,
-                                                         uint8_t* __restrict__ seg, int NC, int64_t V) {
+// softmax_out [NC][V] may alias agg (in-place normalisation): neither is __restrict__, and every thread reads all of its
+// elements before it writes them.
+template <int NC, bool VEC>      // VEC: V % 4 == 0 and every buffer 16-byte (seg: 4-byte) aligned
+__global__ void __launch_bounds__(256) finalize_kernel(const float* agg, const float* __restrict__ wgt,
+                                                       float* softmax_out, uint8_t* __restrict__ seg, int64_t V) {
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < V; i += stride) {
-    const float w = wgt[i];
-    float best = agg[i] / w;
-    int arg = 0;
-    if (softmax_out) softmax_out[i] = best;
-    for (int c = 1; c < NC; ++c) {
-      const float p = agg[(size_t)c * V + i] / w;
-      if (softmax_out) softmax_out[(size_t)c * V + i] = p;
-      if (p > best) { best = p; arg = c; }
+  if constexpr (VEC) {
+    // 128-bit accesses (four voxels per thread and step): the pass is a pure stream, bound by bytes in flight.  The class
+    // planes are reached by stepping one pointer (a pointer per class, hoisted out of the loop, made ptxas spill at NC = 7).
+    const int64_t V4 = V >> 2;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < V4; i += stride) {
+      const float4 w = reinterpret_cast<const float4*>(wgt)[i];
+      float p[4][NC];
+      const float4* a = reinterpret_cast<const float4*>(agg) + i;
+#pragma unroll
+      for (int c = 0; c < NC; ++c, a += V4) {
+        const float4 x = *a;
+        p[0][c] = x.x; p[1][c] = x.y; p[2][c] = x.z; p[3][c] = x.w;
+      }
+      const uchar4 s = make_uchar4(divide_argmax<NC>(p[0], w.x), divide_argmax<NC>(p[1], w.y), divide_argmax<NC>(p[2], w.z),
+                                   divide_argmax<NC>(p[3], w.w));
+      if (softmax_out) {
+        float4* o = reinterpret_cast<float4*>(softmax_out) + i;
+#pragma unroll
+        for (int c = 0; c < NC; ++c, o += V4) *o = make_float4(p[0][c], p[1][c], p[2][c], p[3][c]);
+      }
+      if (seg) reinterpret_cast<uchar4*>(seg)[i] = s;
     }
-    if (seg) seg[i] = (uint8_t)arg;
+  } else {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < V; i += stride) {
+      float p[NC];
+#pragma unroll
+      for (int c = 0; c < NC; ++c) p[c] = agg[(size_t)c * V + i];
+      const uint8_t s = divide_argmax<NC>(p, wgt[i]);
+      if (softmax_out) {
+#pragma unroll
+        for (int c = 0; c < NC; ++c) softmax_out[(size_t)c * V + i] = p[c];
+      }
+      if (seg) seg[i] = s;
+    }
   }
 }
 
 // argmax over NC classes of p [NC][V], first maximum (numpy.argmax)
-__global__ void __launch_bounds__(256) argmax_c_kernel(const float* __restrict__ p, int NC, uint8_t* __restrict__ seg, int64_t V) {
+__global__ void __launch_bounds__(256) argmax_kernel(const float* __restrict__ p, int NC, uint8_t* __restrict__ seg, int64_t V) {
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < V; i += stride) {
     float best = p[i];
@@ -503,11 +393,6 @@ __global__ void __launch_bounds__(256) ensemble_refine_kernel(float* __restrict_
     acc[i] = f;
     if (label) label[i] = f < 0.5f ? 1 : 0;
   }
-}
-
-__global__ void __launch_bounds__(256) argmax2_kernel(const float* __restrict__ p, uint8_t* __restrict__ seg, int64_t V) {
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < V; i += stride) seg[i] = p[V + i] > p[i] ? 1 : 0;
 }
 
 // chunked T [n][C/8][V][8] -> fp32 NCDHW (debug / layer-level parity tests), optional norm+lrelu

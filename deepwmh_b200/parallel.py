@@ -151,7 +151,7 @@ def predict_volume_ensemble(trainers: Sequence, vol: torch.Tensor, do_mirroring=
     """predict_cases' `for p in params` loop (a13) with every model resident: vol = normalised fp32 [X,Y,Z] (one modality) or
     [M,X,Y,Z] on the device (each extent >= patch) -> (seg uint8 [X,Y,Z], mean softmax fp32 [C,X,Y,Z]), all on the device: per
     model tiled prediction + finalize, running mean by dwmh_axpy (mean = sum_k softmax_k / k in model order), argmax by
-    dwmh_argmax2 (two classes) or dwmh_argmax."""
+    dwmh_argmax."""
     net0 = trainers[0].network
     k = len(trainers)
     with torch.cuda.device(net0.device):

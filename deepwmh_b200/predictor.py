@@ -161,17 +161,9 @@ class SegmentationNetwork:
         assert acc.is_cuda and x.is_cuda and acc.dtype == x.dtype == torch.float32 and acc.is_contiguous() and x.is_contiguous()
         check(self._lib.dwmh_axpy(self._ctx, _ptr(acc), _ptr(x), float(alpha), acc.numel(), self._st()))
 
-    def argmax2(self, softmax: torch.Tensor) -> torch.Tensor:
-        seg = torch.empty(tuple(softmax.shape[1:]), dtype=torch.uint8, device=softmax.device)
-        check(self._lib.dwmh_argmax2(self._ctx, _ptr(softmax), _ptr(seg), seg.numel(), self._st()))
-        return seg
-
     def argmax(self, softmax: torch.Tensor) -> torch.Tensor:
-        """Class map uint8 [x,y,z] of fp32 probabilities [C,x,y,z] on the device; ties go to the lower class (numpy.argmax).
-        Two classes take dwmh_argmax2, more take dwmh_argmax."""
+        """Class map uint8 [x,y,z] of fp32 probabilities [C,x,y,z] on the device; ties go to the lower class (numpy.argmax)."""
         assert softmax.is_cuda and softmax.dtype == torch.float32 and softmax.is_contiguous()
-        if softmax.shape[0] == 2:
-            return self.argmax2(softmax)
         seg = torch.empty(tuple(softmax.shape[1:]), dtype=torch.uint8, device=softmax.device)
         check(self._lib.dwmh_argmax(self._ctx, _ptr(softmax), int(softmax.shape[0]), _ptr(seg), seg.numel(), self._st()))
         return seg

@@ -52,6 +52,7 @@ typedef struct dwmh_net_desc {
 } dwmh_net_desc;
 
 const char* dwmh_last_error(void);
+/* 101: the separate two-class argmax entry point is gone; dwmh_argmax takes two classes like any other count. */
 int dwmh_version(void);
 
 /* --- life cycle (replaces load_model_and_checkpoint_files + trainer.initialize(False)) ----------
@@ -117,9 +118,8 @@ int dwmh_finalize(dwmh_ctx* ctx, const float* agg_dev, const float* wgt_dev, flo
 
 /* a13 ensemble: acc += softmax / k  (k-model mean of predict_cases), n floats. */
 int dwmh_axpy(dwmh_ctx* ctx, float* acc_dev, const float* x_dev, float alpha, int64_t n, void* stream);
-int dwmh_argmax2(dwmh_ctx* ctx, const float* softmax_dev, uint8_t* seg_dev, int64_t nvox, void* stream);
 /* seg = argmax over num_classes (1 .. 255) of softmax_dev fp32 [num_classes][nvox]; the first maximum wins (ties go to the
- * lower class, as numpy.argmax).  dwmh_argmax2 is the same for two classes. */
+ * lower class, as numpy.argmax). */
 int dwmh_argmax(dwmh_ctx* ctx, const float* softmax_dev, int32_t num_classes, uint8_t* seg_dev, int64_t nvox, void* stream);
 
 /* --- SURVEY 8f-3: checkpoint ensemble with softmax masking (deepwmh/pipeline/DCNN_multistage.py:102-125,317-394).
@@ -291,7 +291,7 @@ int dwmh_get_counters(dwmh_ctx* ctx, int64_t* kernel_launches, double* conv_flop
 int dwmh_set_stage_timing(dwmh_ctx* ctx, int32_t on);
 int dwmh_get_stage_timing(dwmh_ctx* ctx, float out_ms[4]);
 /* Per kernel class of the last timed dwmh_predict_3d: out[3k + {0,1,2}] = {device ms, algorithmic bytes, launches} for
- * k = 0 conv3_tc_kernel (bytes not counted here), 1 instnorm_lrelu_kernel, 2 head_softmax_kernel. */
+ * k = 0 conv3_tc_kernel (bytes not counted here), 1 instnorm_lrelu_kernel, 2 head_softmax_kernel (any class count). */
 int dwmh_get_kernel_timing(dwmh_ctx* ctx, double out[9]);
 
 #ifdef __cplusplus

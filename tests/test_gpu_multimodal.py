@@ -11,7 +11,7 @@ Random-init oracle networks for (M, C) in {(2, 3) WMH-challenge layout (T1 + FLA
   * the host-buffer call against normalize_ + predict_3D, bit for bit (padding, re-pitched modalities, crop mask);
   * the resident ensemble, the tile-sharded call in one process and the weight map at C = 3;
   * determinism: two calls are bit-identical, split tile ranges add up to the full run;
-  * argmax over C classes on planted ties picks the lower class;
+  * argmax and both paths of finalize (128-bit and scalar) pick the lower class on planted ties, two classes included;
   * accumulate_tiles / finalize refuse tensors the kernels cannot take;
   * nnUNet_predict end to end on a 2-modality, 3-class model directory against the oracle pipeline.
 """
@@ -172,13 +172,14 @@ def test_bit_identical_repeat_and_split_tile_ranges(kind, M, C):
     dev.close()
 
 
-@pytest.mark.parametrize("C", [3, 5, 8])
-def test_argmax_and_finalize_break_ties_to_the_lower_class(C):
+# (20, 16, 13) takes finalize's 128-bit path, the odd voxel count of (19, 17, 13) its scalar one
+@pytest.mark.parametrize("C,shp", [(C, (20, 16, 13)) for C in (3, 5, 8, 2)] + [(C, (19, 17, 13)) for C in (2, 3, 8)],
+                         ids=["3", "5", "8", "2", "2-odd", "3-odd", "8-odd"])
+def test_argmax_and_finalize_break_ties_to_the_lower_class(C, shp):
     import deepwmh_b200
     plans, net, tr = _pair("cube", 1, C)
     dev = tr.network
     rng = np.random.default_rng(C)
-    shp = (20, 16, 13)
     p = rng.random((C,) + shp).astype(np.float32)
     # plant ties: a random pair of classes shares the maximum at a quarter of the voxels, all classes tie at a few
     tie = rng.random(shp) < 0.25

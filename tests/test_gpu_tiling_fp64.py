@@ -17,8 +17,8 @@ moved by a voxel, its forwards run with modalities 0 and 1 exchanged (M > 1), it
 
 Volumes are [M, X, Y, Z] for M modalities ([X, Y, Z] for one) and the result has C classes: the cases with M > 1 reach
 the first conv's tile fetch with a modality stride (the tcgen05 kernel on the cube plan, conv_first_mm_kernel on the
-anisotropic one), those with C > 2 aggregate_tile_c_kernel and finalize_c_kernel.  A single tile with one mirror axis is
-also checked bit for bit against its two forwards.
+anisotropic one), and each class count reaches the overlap-add and finalize instantiated for it.  A single tile with one
+mirror axis is also checked bit for bit against its two forwards.
 """
 import itertools
 
@@ -284,8 +284,8 @@ SMALL_CASES = [
      for r in range(4) for axes in itertools.combinations(ALL, r)]
 SMALL_IDS = ["shape%d-%s-%s-mirror_axes%d-%s-%d" % (i, c[1], c[2], i, c[4], c[5]) for i, c in enumerate(SMALL_CASES)]
 SMALL_CASES = [c + ("cube", 1, 2, ((0, -1),)) for c in SMALL_CASES]
-# several modalities (the first conv's tile fetch with a modality stride) and classes (aggregate_tile_c_kernel,
-# finalize_c_kernel); (3, 2) feeds three modalities to the two-class overlap-add
+# several modalities (the first conv's tile fetch with a modality stride) and classes (aggregate_tile_kernel<C>,
+# finalize_kernel<C, VEC>); (3, 2) feeds three modalities to the two-class overlap-add
 MC_CASES = [((40, 50, 45), 0.5, True, ALL, True, 8, "cube", M, C, ((0, -1),)) for M, C in ((2, 3), (4, 4), (3, 2), (1, 8))] + [
     ((24, 70, 60), 0.5, True, ALL, True, 8, "aniso", 2, 3, ((0, -1),)),      # conv_first_mm_kernel in tile mode
     ((40, 50, 45), 0.5, True, (0, 1), True, 4, "cube", 2, 3, ((0, -1),)),    # one tile per batch
