@@ -403,9 +403,9 @@ extern "C" int dwmh_commit_weights(dwmh_ctx* c) {
   size_t stat_doubles = 0;
   for (auto& L : c->layers) if (L.has_norm) stat_doubles += (size_t)maxN * L.cout * 2;
   c->stats_bytes = stat_doubles * sizeof(double);
-  // the CUDA-core first-conv kernels leave [n][block][Cout][2] partial statistics (not cleared per forward: every slot is written)
+  // the CUDA-core first conv leaves [n][block][Cout][2] partial statistics (not cleared per forward: every slot is written)
   const Layer& L0 = c->layers[0];
-  const int64_t fc_blocks = std::max((L0.vout() + 256 * FC_VPT - 1) / (256 * FC_VPT), (L0.vout() / 2 + 128 * FC_VPT - 1) / (128 * FC_VPT));
+  const int64_t fc_blocks = (L0.vout() + 256 * FC_VPT - 1) / (256 * FC_VPT);
   const size_t fc_bytes = (size_t)maxN * fc_blocks * 2 * L0.cout * sizeof(float);
   if (!c->buffers_ready && c->lender) {
     dwmh_ctx* o = c->lender;
@@ -668,15 +668,9 @@ static int forward_impl(dwmh_ctx* c, const float* src, int patch_mode, int SX, i
       p.SX = SX; p.SY = SY; p.SZ = SZ; p.px = L.out_sp[0]; p.py = L.out_sp[1]; p.pz = L.out_sp[2];
       p.kd = L.k[0]; p.kh = L.k[1]; p.kw = L.k[2]; p.Cout = L.cout;
       p.Cin = L.c0; p.mstride = (int64_t)SX * SY * SZ; p.partials = c->fc_partials;
-      dim3 grid((unsigned)((L.vout() + 256 * FC_VPT - 1) / (256 * FC_VPT)), nb);
-      const size_t smem = ((size_t)L.c0 * taps * L.cout + 8 * 2 * L.cout) * sizeof(float);     // weights, 8 warps' statistics
-      if (L.c0 > 1) {
-        if (taps == 27) conv_first_mm_kernel<T, true><<<grid, 256, smem, st>>>(p);
-        else conv_first_mm_kernel<T, false><<<grid, 256, smem, st>>>(p);
-      } else if (taps == 27 && L.cout <= 32 && L.out_sp[2] % 2 == 0) {
-        grid.x = (unsigned)((L.vout() / 2 + 128 * FC_VPT - 1) / (128 * FC_VPT));
-        conv_first_k3x2_kernel<T><<<grid, 128, smem, st>>>(p);
-      } else if (taps == 27) conv_first_kernel<T, true><<<grid, 256, smem, st>>>(p);
+      const dim3 grid((unsigned)((L.vout() + 256 * FC_VPT - 1) / (256 * FC_VPT)), nb, (L.cout + 31) / 32);
+      const size_t smem = ((size_t)L.c0 * taps * L.cout + 8 * 2 * 32) * sizeof(float);     // weights, 8 warps' statistics
+      if (taps == 27) conv_first_kernel<T, true><<<grid, 256, smem, st>>>(p);
       else conv_first_kernel<T, false><<<grid, 256, smem, st>>>(p);
       first_stats_reduce_kernel<<<nb, 128, 0, st>>>(c->fc_partials, L.sums, (int)grid.x, 2 * L.cout);
       c->launches += 2;

@@ -45,7 +45,6 @@ constexpr int TC_PLANE_BYTES = TC_PH * TC_PW * 16;     // one 8-channel chunk of
 constexpr int TC_MAX_SA = 4, TC_MAX_NB = 40, TC_MAX_R = 16;
 constexpr int TC_SMEM_MAX = 232448;                    // 227 KB opt-in limit
 constexpr int TC_SMEM_RESERVED = 5120;                 // barriers + TMEM pointer + statistics
-constexpr int TC_SMEM_RESERVED_FIRST = 10240;          // FIRST kernels: + two 4-slot rings of haloed input slices
 constexpr int TC_FIRST_PITCH = 12;                     // words per ring row (10 used): 2 rows apart = 24 words -> conflict-free LDS
 constexpr int TC_FIRST_SLICE = TC_PH * TC_FIRST_PITCH;
 constexpr int TC_FIRST_STAGE_BYTES = 8 * 128 * 16;     // im2col operand of one output plane: 4 hi + 4 lo chunks of 8 taps
@@ -74,8 +73,8 @@ struct TcKParams {
   int G;              // work-item pipelines ("groups") per CTA: 2 = two tiles share the resident weights, each with 256 TMEM columns
   int total_items;
   uint32_t a_stage_bytes, b_tile_bytes, off_b, off_bar;
-  // multi-modality FIRST kernels (MULTI): fc_M input channels fc_mstride floats apart; the slice-ring barriers sit fc_sbar bytes
-  // after off_bar (256 bytes per group)
+  // FIRST kernels: fc_M input channels (modalities) fc_mstride floats apart; the slice-ring barriers sit fc_sbar bytes after
+  // off_bar (256 bytes per group)
   int fc_M; uint32_t fc_sbar; int64_t fc_mstride;
 };
 
@@ -121,8 +120,8 @@ constexpr uint64_t tc_tap_shift_table() {
 constexpr uint64_t kTapShift = tc_tap_shift_table();
 
 // KSTEPS = KC/16 (UMMA K steps per channel chunk); SMALL_CB: CB <= 32 -> per-thread running statistics.
-// MULTI (FIRST only): p.fc_M > 1 input modalities, each plane is fc_M im2col stages accumulated into one TMEM slot.
-template <typename T, int KSTEPS, bool SMALL_CB, bool TCONV, bool DUAL, bool XFORM, bool FIRST = false, bool MULTI = false>
+// FIRST: p.fc_M input modalities, each plane is fc_M im2col stages accumulated into one TMEM slot.
+template <typename T, int KSTEPS, bool SMALL_CB, bool TCONV, bool DUAL, bool XFORM, bool FIRST = false>
 __global__ void __launch_bounds__((DUAL ? 2 : 1) * (TC_THREADS + ((FIRST || XFORM) ? 32 : 0)), 1)
 conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant__ CUtensorMap tmA1, const TcKParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
@@ -183,16 +182,15 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
   uint32_t* tmem_ptr_smem = reinterpret_cast<uint32_t*>(smem + p.off_bar + 8 * nbar * p.G);
   const uint32_t aux_off = (p.off_bar + 8u * nbar * (uint32_t)p.G + 16u + 8u) & ~15u;      // 16-byte aligned (the loaders read coefficients as float4)
   float* s_coef = reinterpret_cast<float*>(smem + aux_off) + (size_t)p.G * 2 * CB + (size_t)g * 2 * 64;   // XFORM: a[64], b[64]
-  // FIRST: ring of haloed input slices, 4 slots (MULTI: 4 per modality)
-  const int NM = MULTI ? p.fc_M : 1;
+  // FIRST: ring of haloed input slices, 4 slots per modality
+  const int NM = p.fc_M;
   float* s_slice = reinterpret_cast<float*>(smem + aux_off) + (size_t)p.G * 2 * CB + (size_t)p.G * 2 * 64 + (size_t)g * 4 * NM * TC_FIRST_SLICE;
   const uint32_t smem_a = smem_base + (uint32_t)g * SA * p.a_stage_bytes;          // this group's activation ring
   // UMMA shared-memory descriptors hold a 14-bit (address >> 4): descriptor arithmetic uses the masked offsets
   const uint32_t smem_a_d = smem_a & 0x3FFFFu, smem_b_d = (smem_base + p.off_b) & 0x3FFFFu;
-  // FIRST: slice ring barriers (MULTI: up to 16 slots of each kind per group)
-  const uint32_t s_full = MULTI ? smem_base + p.off_bar + p.fc_sbar + (uint32_t)g * 256u
-                                : smem_base + p.off_bar + TC_SMEM_RESERVED_FIRST - 128 + (uint32_t)g * 64u;
-  const uint32_t s_empty = s_full + (MULTI ? 128u : 32u);
+  // FIRST: slice ring barriers (up to 16 slots of each kind per group)
+  const uint32_t s_full = smem_base + p.off_bar + p.fc_sbar + (uint32_t)g * 256u;
+  const uint32_t s_empty = s_full + 128u;
 
   if (threadIdx.x == 0) {
     if constexpr (!FIRST) {
@@ -205,17 +203,11 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
       for (uint32_t s_ = 0; s_ < R; ++s_) { tc::mbar_init(bg + 16 * SA + 16 * NB + 8 * s_, 1); tc::mbar_init(bg + 16 * SA + 16 * NB + 8 * (R + s_), 4); }
       for (uint32_t s_ = 0; s_ < SA; ++s_) tc::mbar_init(bg + 16 * SA + 16 * NB + 16 * R + 8 * s_, XFORM ? 3 : 2);
     }
-    if constexpr (FIRST && MULTI)
+    if constexpr (FIRST)
       for (int gg = 0; gg < p.G; ++gg)
         for (int s_ = 0; s_ < 4 * NM; ++s_) {
           tc::mbar_init(smem_base + p.off_bar + p.fc_sbar + gg * 256 + 8 * s_, 1);
           tc::mbar_init(smem_base + p.off_bar + p.fc_sbar + gg * 256 + 128 + 8 * s_, 2);
-        }
-    else if constexpr (FIRST)
-      for (int gg = 0; gg < p.G; ++gg)
-        for (uint32_t s_ = 0; s_ < 4; ++s_) {
-          tc::mbar_init(smem_base + p.off_bar + TC_SMEM_RESERVED_FIRST - 128 + gg * 64 + 8 * s_, 1);
-          tc::mbar_init(smem_base + p.off_bar + TC_SMEM_RESERVED_FIRST - 128 + gg * 64 + 32 + 8 * s_, 2);
         }
     const uint32_t nactive = (uint32_t)min(p.G, p.total_items - (int)blockIdx.x * p.G);      // groups of this CTA that have a tile
     for (uint32_t s_ = 0; s_ < NB; ++s_) { tc::mbar_init(b_full + 8 * s_, 1); tc::mbar_init(b_empty + 8 * s_, nactive); }
@@ -243,9 +235,14 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
   if (idle) {
     // odd item count: the second group of the last CTA has nothing to do
   } else
-  if (FIRST && MULTI && warp == 7) {
-    // ---------------- multi-modality first conv: slice fetcher ---------------------------------------------------------
-    // As below, for NM modalities: slice q = k * NM + m is plane z_lo - 1 + k of modality m, ring slot q % (4 NM).
+  if (FIRST && warp == 7) {
+    // ---------------- first conv: slice fetcher (extra warps 14, 15 of the CTA) ----------------------
+    // Streams the haloed 18 x 10 input slices of this tile (zero outside the patch, tile origin and mirror flip applied
+    // to the source index) into a ring of 4 slots per modality, each value already split x = hi + lo: low half = hi (x
+    // truncated to the 16-bit format, exact), high half = lo = rn(x - hi).  Slice q = k * NM + m is plane z_lo - 1 + k of
+    // modality m and goes to ring slot q % (4 NM).  A warp of its own because the builders' proxy fence
+    // (MEMBAR + FENCE.VIEW.ASYNC) waits for every outstanding global load of the executing warp: with the prefetch in
+    // the builder warps each plane cost one full HBM latency.
     int ox = 0, oy = 0, oz = 0, flip = 0;
     const float* src = p.fc_src;
     int SY = p.fc_SY, SZ = p.fc_SZ;
@@ -264,21 +261,22 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     const float* sbase = src + (size_t)ox * SY * SZ;
     const int zstep = (flip & 4) ? -SY * SZ : SY * SZ;
     if (flip & 4) sbase += (size_t)(p.D - 1) * SY * SZ;
-    const int nq = (z_end - z_lo + 2) * NM, RS = 4 * NM;
+    const int nk = z_end - z_lo + 2, nq = nk * NM;
     constexpr uint32_t kHiMask = ActT<T>::kUmmaFormat == 0 ? 0xFFFFE000u : 0xFFFF0000u;
     uint32_t* ring = reinterpret_cast<uint32_t*>(s_slice);
-    auto fetch = [&](int q, float v[6]) {
-      const int k = q / NM, m = q - k * NM;
-      const int zz = z_lo - 1 + k;
-      const bool zin = q < nq && (unsigned)zz < (unsigned)p.D;
-      const float* sp = sbase + (ptrdiff_t)m * p.fc_mstride + (ptrdiff_t)zz * zstep;
+    int kf = 0, mf = 0;                                         // plane and modality of the next slice to fetch
+    auto fetch = [&](float v[6]) {
+      const int zz = z_lo - 1 + kf;
+      const bool zin = kf < nk && (unsigned)zz < (unsigned)p.D;
+      const float* sp = sbase + (ptrdiff_t)mf * p.fc_mstride + (ptrdiff_t)zz * zstep;
 #pragma unroll
       for (int i = 0; i < 6; ++i) v[i] = (zin && sin_[i]) ? __ldg(sp + sgoff[i]) : 0.f;
+      if (++mf == NM) { mf = 0; ++kf; }
     };
-    auto step = [&](int q, float (&v)[6]) {
-      const int slot = q % RS;
-      if (q >= RS) tc::mbar_wait(s_empty + 8 * slot, ((q / RS) & 1) ^ 1, 10);
-      uint32_t* dst = ring + slot * TC_FIRST_SLICE;
+    RingPos slot;                                               // ring slot of the next slice to store
+    auto step = [&](float (&v)[6]) {
+      tc::mbar_wait(s_empty + 8 * slot.idx, slot.phase ^ 1, 10);
+      uint32_t* dst = ring + slot.idx * TC_FIRST_SLICE;
 #pragma unroll
       for (int i = 0; i < 6; ++i) {
         const float hf = __uint_as_float(__float_as_uint(v[i]) & kHiMask);
@@ -286,21 +284,24 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         if (pos < TC_PH * TC_PW) dst[r * TC_FIRST_PITCH + (pos - r * TC_PW)] = ActT<T>::from_f2(hf, v[i] - hf);
       }
       __syncwarp();
-      if (lane == 0) tc::mbar_arrive(s_full + 8 * slot);
-      fetch(q + 4, v);
+      if (lane == 0) tc::mbar_arrive(s_full + 8 * slot.idx);
+      slot.advance(4 * NM);
+      fetch(v);                                                 // HBM latency is several planes long: 4 slices in flight
     };
     float v0[6], v1[6], v2[6], v3[6];
-    fetch(0, v0); fetch(1, v1); fetch(2, v2); fetch(3, v3);
+    fetch(v0); fetch(v1); fetch(v2); fetch(v3);
     for (int q = 0; q < nq; q += 4) {
-      step(q, v0);
-      if (q + 1 < nq) step(q + 1, v1);
-      if (q + 2 < nq) step(q + 2, v2);
-      if (q + 3 < nq) step(q + 3, v3);
+      step(v0);
+      if (q + 1 < nq) step(v1);
+      if (q + 2 < nq) step(v2);
+      if (q + 3 < nq) step(v3);
     }
-  } else if (FIRST && MULTI && (warp == 0 || warp == 6)) {
-    // ---------------- multi-modality first conv: builder warps -----------------------------------------------------------
-    // One im2col stage per (plane, modality), built exactly as below from that modality's three slices; the MMA issuer
-    // accumulates the NM stages of a plane into one TMEM slot.
+  } else if (FIRST && (warp == 0 || warp == 6)) {
+    // ---------------- first conv: builder warps write the im2col operand ------------------------------
+    // One stage per (plane, modality); the MMA issuer accumulates the NM stages of a plane into one TMEM slot.  Row m of
+    // the operand = output voxel (h0 + m/8, w0 + m%8) of plane t, columns = its 27 neighbours (hi halves in chunks 0..3,
+    // lo halves in chunks 4..7), so that x*w = hi*w_hi + lo*w_hi + hi*w_lo keeps fp32-level accuracy on the tensor cores
+    // (K = 3 x 32).  Stage layout: [8 chunks][128 rows][16 B]  (K-major, SBO = 128 B, LBO = 2048 B).
     const bool leader = tc::elect_one();
     if (warp == 6 && g == 0 && leader) {
       tc::mbar_arrive_expect_tx(b_full, p.b_tile_bytes);
@@ -308,17 +309,17 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     }
     const int l64 = (warp == 0 ? 0 : 32) + lane;
     const uint32_t* ring = reinterpret_cast<const uint32_t*>(s_slice);
-    const int RS = 4 * NM;
     for (int q = 0; q < 2 * NM; ++q) tc::mbar_wait(s_full + 8 * q, 0, 11);
     RingPos xf;
-    for (int j = 0; j < z_end - z_lo; ++j) {
+    for (int j = 0; j < z_end - z_lo; ++j) {                    // plane t = z_lo + j reads slice planes j, j+1, j+2
       for (int m = 0; m < NM; ++m) {
-        const int q2 = (j + 2) * NM + m;
-        tc::mbar_wait(s_full + 8 * (q2 % RS), (q2 / RS) & 1, 11);
+        // slice (k, m) sits in slot (k & 3) * NM + m, in its (k >> 2)-th use of the slot
+        const int s0 = (j & 3) * NM + m, s1 = ((j + 1) & 3) * NM + m, s2 = ((j + 2) & 3) * NM + m;
+        tc::mbar_wait(s_full + 8 * s2, ((j + 2) >> 2) & 1, 11);
         tc::mbar_wait(a_empty + 8 * xf.idx, xf.phase ^ 1, 9);
         uint4* stage = reinterpret_cast<uint4*>(smem + (size_t)g * SA * p.a_stage_bytes + (size_t)xf.idx * p.a_stage_bytes);
-        const uint32_t* sl[3] = {ring + ((j * NM + m) % RS) * TC_FIRST_SLICE, ring + (((j + 1) * NM + m) % RS) * TC_FIRST_SLICE,
-                                 ring + (q2 % RS) * TC_FIRST_SLICE};
+        const uint32_t* sl[3] = {ring + s0 * TC_FIRST_SLICE, ring + s1 * TC_FIRST_SLICE, ring + s2 * TC_FIRST_SLICE};
+        // a lane builds two vertically adjacent rows (hh, ww), (hh + 1, ww): they share 2 of their 3 input rows
         const int hh = (l64 >> 3) * 2, ww = l64 & 7;
         uint32_t val[3][4][3];
 #pragma unroll
@@ -350,121 +351,9 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         }
         tc::fence_proxy_async();
         __syncwarp();
-        if (lane == 0) { tc::mbar_arrive(a_ready + 8 * xf.idx); tc::mbar_arrive(s_empty + 8 * ((j * NM + m) % RS)); }
+        if (lane == 0) { tc::mbar_arrive(a_ready + 8 * xf.idx); tc::mbar_arrive(s_empty + 8 * s0); }
         xf.advance(SA);
       }
-    }
-  } else
-  if (FIRST && warp == 7) {
-    // ---------------- first conv (Cin = 1): slice fetcher (extra warps 14, 15 of the CTA) ------------
-    // Streams the haloed 18 x 10 input slices of this tile (zero outside the patch, tile origin and mirror flip applied
-    // to the source index) into a 4-slot ring, each value already split x = hi + lo: low half = hi (x truncated to the
-    // 16-bit format, exact), high half = lo = rn(x - hi).  A warp of its own because the builders' proxy fence
-    // (MEMBAR + FENCE.VIEW.ASYNC) waits for every outstanding global load of the executing warp: with the prefetch in
-    // the builder warps each plane cost one full HBM latency.
-    int ox = 0, oy = 0, oz = 0, flip = 0;
-    const float* src = p.fc_src;
-    int SY = p.fc_SY, SZ = p.fc_SZ;
-    if (p.fc_patch_mode) { src += (size_t)n * p.D * p.H * p.W; SY = p.H; SZ = p.W; }
-    else { const SampleMeta m_ = p.fc_metas[n]; ox = m_.ox; oy = m_.oy; oz = m_.oz; flip = m_.flip; }
-    int sgoff[6]; bool sin_[6];
-#pragma unroll
-    for (int i = 0; i < 6; ++i) {
-      const int pos = lane + 32 * i;
-      const int r = pos / TC_PW, c = pos - r * TC_PW;
-      const int hh = h0 - 1 + r, ww = w0 - 1 + c;
-      sin_[i] = pos < TC_PH * TC_PW && (unsigned)hh < (unsigned)p.H && (unsigned)ww < (unsigned)p.W;
-      const int sj = oy + ((flip & 2) ? p.H - 1 - hh : hh), sk = oz + ((flip & 1) ? p.W - 1 - ww : ww);
-      sgoff[i] = sin_[i] ? sj * SZ + sk : 0;
-    }
-    const float* sbase = src + (size_t)ox * SY * SZ;
-    const int zstep = (flip & 4) ? -SY * SZ : SY * SZ;
-    if (flip & 4) sbase += (size_t)(p.D - 1) * SY * SZ;
-    const int nslices = z_end - z_lo + 2;                       // slice k = patch plane z_lo - 1 + k
-    constexpr uint32_t kHiMask = ActT<T>::kUmmaFormat == 0 ? 0xFFFFE000u : 0xFFFF0000u;
-    uint32_t* ring = reinterpret_cast<uint32_t*>(s_slice);
-    auto fetch = [&](int k, float v[6]) {
-      const int zz = z_lo - 1 + k;
-      const bool zin = k < nslices && (unsigned)zz < (unsigned)p.D;
-      const float* sp = sbase + (ptrdiff_t)zz * zstep;
-#pragma unroll
-      for (int i = 0; i < 6; ++i) v[i] = (zin && sin_[i]) ? __ldg(sp + sgoff[i]) : 0.f;
-    };
-    auto step = [&](int k, float (&v)[6]) {
-      if (k >= 4) tc::mbar_wait(s_empty + 8 * (k & 3), ((k >> 2) & 1) ^ 1, 10);
-      uint32_t* dst = ring + (k & 3) * TC_FIRST_SLICE;
-#pragma unroll
-      for (int i = 0; i < 6; ++i) {
-        const float hf = __uint_as_float(__float_as_uint(v[i]) & kHiMask);
-        const int pos = lane + 32 * i, r = pos / TC_PW;
-        if (pos < TC_PH * TC_PW) dst[r * TC_FIRST_PITCH + (pos - r * TC_PW)] = ActT<T>::from_f2(hf, v[i] - hf);
-      }
-      __syncwarp();
-      if (lane == 0) tc::mbar_arrive(s_full + 8 * (k & 3));
-      fetch(k + 4, v);                                          // HBM latency is several planes long: 4 slices in flight
-    };
-    float v0[6], v1[6], v2[6], v3[6];
-    fetch(0, v0); fetch(1, v1); fetch(2, v2); fetch(3, v3);
-    for (int k = 0; k < nslices; k += 4) {
-      step(k, v0);
-      if (k + 1 < nslices) step(k + 1, v1);
-      if (k + 2 < nslices) step(k + 2, v2);
-      if (k + 3 < nslices) step(k + 3, v3);
-    }
-  } else if (FIRST && (warp == 0 || warp == 6)) {
-    // ---------------- first conv (Cin = 1): builder warps write the im2col operand -------------------
-    // Row m of the operand = output voxel (h0 + m/8, w0 + m%8) of plane t, columns = its 27 neighbours (hi halves in
-    // chunks 0..3, lo halves in chunks 4..7), so that x*w = hi*w_hi + lo*w_hi + hi*w_lo keeps fp32-level accuracy on
-    // the tensor cores (K = 3 x 32).  Stage layout: [8 chunks][128 rows][16 B]  (K-major, SBO = 128 B, LBO = 2048 B).
-    const bool leader = tc::elect_one();
-    if (warp == 6 && g == 0 && leader) {
-      tc::mbar_arrive_expect_tx(b_full, p.b_tile_bytes);
-      tc::bulk_load(smem_base + p.off_b, p.wpack, p.b_tile_bytes, b_full);
-    }
-    const int l64 = (warp == 0 ? 0 : 32) + lane;
-    const uint32_t* ring = reinterpret_cast<const uint32_t*>(s_slice);
-    tc::mbar_wait(s_full, 0, 11);
-    tc::mbar_wait(s_full + 8, 0, 11);
-    RingPos xf;
-    for (int j = 0; j < z_end - z_lo; ++j) {                    // plane t = z_lo + j reads slices j, j+1, j+2
-      tc::mbar_wait(s_full + 8 * ((j + 2) & 3), ((j + 2) >> 2) & 1, 11);
-      tc::mbar_wait(a_empty + 8 * xf.idx, xf.phase ^ 1, 9);
-      uint4* stage = reinterpret_cast<uint4*>(smem + (size_t)g * SA * p.a_stage_bytes + (size_t)xf.idx * p.a_stage_bytes);
-      const uint32_t* sl[3] = {ring + (j & 3) * TC_FIRST_SLICE, ring + ((j + 1) & 3) * TC_FIRST_SLICE, ring + ((j + 2) & 3) * TC_FIRST_SLICE};
-      // a lane builds two vertically adjacent rows (hh, ww), (hh + 1, ww): they share 2 of their 3 input rows
-      const int hh = (l64 >> 3) * 2, ww = l64 & 7;
-      uint32_t val[3][4][3];
-#pragma unroll
-      for (int dz = 0; dz < 3; ++dz)
-#pragma unroll
-        for (int r = 0; r < 4; ++r)
-#pragma unroll
-          for (int kw = 0; kw < 3; ++kw) val[dz][r][kw] = sl[dz][(hh + r) * TC_FIRST_PITCH + ww + kw];
-#pragma unroll
-      for (int rr = 0; rr < 2; ++rr) {
-        const int m = (hh + rr) * 8 + ww;
-        uint32_t hi[16], lo[16];
-#pragma unroll
-        for (int q = 0; q < 16; ++q) {
-          uint32_t x[2];
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            const int tap = 2 * q + e;
-            x[e] = tap < 27 ? val[tap / 9][(tap / 3) % 3 + rr][tap % 3] : 0u;
-          }
-          hi[q] = __byte_perm(x[0], x[1], 0x5410);
-          lo[q] = __byte_perm(x[0], x[1], 0x7632);
-        }
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          stage[c * 128 + m] = make_uint4(hi[4 * c], hi[4 * c + 1], hi[4 * c + 2], hi[4 * c + 3]);
-          stage[(4 + c) * 128 + m] = make_uint4(lo[4 * c], lo[4 * c + 1], lo[4 * c + 2], lo[4 * c + 3]);
-        }
-      }
-      tc::fence_proxy_async();
-      __syncwarp();
-      if (lane == 0) { tc::mbar_arrive(a_ready + 8 * xf.idx); tc::mbar_arrive(s_empty + 8 * (j & 3)); }
-      xf.advance(SA);
     }
   } else if (XFORM && (warp == 0 || warp == 6 || warp == 7)) {
     // ---------------- norm-on-load: three loader / transform warps per group (roles 0, 6, 7) -----------
@@ -633,10 +522,11 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
     // unrolled burst of 9 taps x KSTEPS per channel chunk in the steady state of a stride-1 layer.
     const bool elected = tc::elect_one();
     const bool leader = elected;
-    if constexpr (FIRST && MULTI) {
-      // one output plane per step: 6 MMAs per modality (weight tile m: 12 k8 chunks of CB rows), all into the plane's slot
+    if constexpr (FIRST) {
+      // one output plane per step, 6 MMAs per modality (hi*w_hi, lo*w_hi, hi*w_lo; K = 32 each; weight tile m: 12 k8 chunks
+      // of CB rows), all into the plane's own slot
       const uint32_t idesc = tc::instr_desc_f16(p.fmt, 128, (int)CB);
-      const uint32_t hi_desc = (128u >> 4) | (1u << 14);
+      const uint32_t hi_desc = (128u >> 4) | (1u << 14);                  // SBO = 128 B for both operands
       const uint32_t a_lbo = (2048u >> 4) << 16, b_lbo = ((CB * 16u) >> 4) << 16;
       const uint32_t b_lo0 = (smem_b_d >> 4) | b_lbo;
       tc::mbar_wait(b_full, 0, 5);
@@ -652,7 +542,7 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
             const uint32_t b_m = b_lo0 + (uint32_t)m * 12u * CB;
 #pragma unroll
             for (int i = 0; i < 6; ++i) {
-              const int achunk = (i == 0 || i == 4) ? 0 : (i == 1 || i == 5) ? 2 : (i == 2 ? 4 : 6);
+              const int achunk = (i == 0 || i == 4) ? 0 : (i == 1 || i == 5) ? 2 : (i == 2 ? 4 : 6);     // hi, hi, lo, lo, hi, hi
               tc::umma_f16(col, tc_desc(hi_desc, a_lo0 + achunk * (2048 >> 4)), tc_desc(hi_desc, b_m + i * 2 * CB), idesc,
                            (m == 0 && i == 0) ? 0u : 1u);
             }
@@ -663,31 +553,6 @@ conv3_tc_kernel(const __grid_constant__ CUtensorMap tmA0, const __grid_constant_
         }
         if (elected) tc::umma_commit(acc_full + 8 * done.idx);
         fresh.advance(R); done.advance(R);
-        __syncwarp();
-      }
-    } else if constexpr (FIRST) {
-      // one output plane per step: 6 MMAs (hi*w_hi, lo*w_hi, hi*w_lo; K = 32 each) into the plane's own slot
-      const uint32_t idesc = tc::instr_desc_f16(p.fmt, 128, (int)CB);
-      const uint32_t hi_desc = (128u >> 4) | (1u << 14);                  // SBO = 128 B for both operands
-      const uint32_t a_lbo = (2048u >> 4) << 16, b_lbo = ((CB * 16u) >> 4) << 16;
-      const uint32_t b_lo0 = (smem_b_d >> 4) | b_lbo;
-      tc::mbar_wait(b_full, 0, 5);
-      RingPos a, fresh, done;
-      for (int t = z_lo; t < z_end; ++t) {
-        tc::mbar_wait(acc_empty + 8 * fresh.idx, fresh.phase ^ 1, 3);
-        tc::mbar_wait(a_mma + 8 * a.idx, a.phase, 4);
-        tc::tc_fence_after();
-        if (leader) {
-          const uint32_t a_lo0 = ((smem_a_d + a.idx * p.a_stage_bytes) >> 4) | a_lbo;
-          const uint32_t col = tmem + fresh.idx * CB;
-#pragma unroll
-          for (int i = 0; i < 6; ++i) {
-            const int achunk = (i == 0 || i == 4) ? 0 : (i == 1 || i == 5) ? 2 : (i == 2 ? 4 : 6);     // hi, hi, lo, lo, hi, hi
-            tc::umma_f16(col, tc_desc(hi_desc, a_lo0 + achunk * (2048 >> 4)), tc_desc(hi_desc, b_lo0 + i * 2 * CB), idesc, i == 0 ? 0u : 1u);
-          }
-        }
-        if (elected) { tc::umma_commit(a_empty + 8 * a.idx); tc::umma_commit(acc_full + 8 * done.idx); }
-        a.advance(SA); fresh.advance(R); done.advance(R);
         __syncwarp();
       }
     } else {
@@ -1594,13 +1459,13 @@ inline int tc_prepare_tconv(TcLayer& t, const std::vector<float>& w, int cin, in
   return 0;
 }
 
-// First conv (Cin = 1, 3x3x3, stride 1): the loader warps of the FIRST kernel build the [128 voxels][32 taps] im2col
-// operand of every output plane from the fp32 volume (tile origin + mirror flip applied on the fly); input and weights
-// are split hi + lo into two fp16 (bf16) values, so the 6 MMAs per plane (hi*w_hi, lo*w_hi, hi*w_lo) reproduce the fp32
-// product to ~2^-22.  w27 = weights as [modality][tap][Cout] (tap = (kd*3 + kh)*3 + kw).
-// nmod > 1 (MULTI kernel): one stage and one 12-chunk weight tile per modality, a 4 * nmod-slot slice ring per group.
+// First conv (Cin = nmod modalities, 3x3x3, stride 1): the loader warps of the FIRST kernel build one [128 voxels][32 taps]
+// im2col operand per modality of every output plane from the fp32 volume (tile origin + mirror flip applied on the fly); input
+// and weights are split hi + lo into two fp16 (bf16) values, so the 6 MMAs per plane and modality (hi*w_hi, lo*w_hi, hi*w_lo)
+// reproduce the fp32 product to ~2^-22.  w27 = weights as [modality][tap][Cout] (tap = (kd*3 + kh)*3 + kw).  One 12-chunk
+// weight tile per modality, a 4 * nmod-slot slice ring per group.
 inline int tc_prepare_first(TcLayer& t, const std::vector<float>& w27, int cout, const int sp[3], bool bf16, void* out, std::string* why,
-                            int nmod = 1) {
+                            int nmod) {
   t.enabled = false;
   why->clear();
   if (cout != 16 && cout != 32) return 0;
@@ -1618,16 +1483,13 @@ inline int tc_prepare_first(TcLayer& t, const std::vector<float>& w27, int cout,
   kp.a_stage_bytes = TC_FIRST_STAGE_BYTES; kp.b_tile_bytes = 12 * cout * 16 * nmod;
   kp.off_b = kp.G * kp.SA * kp.a_stage_bytes;
   kp.off_bar = (kp.off_b + kp.b_tile_bytes + 127) & ~127u;
-  if (nmod == 1) t.smem_bytes = kp.off_bar + TC_SMEM_RESERVED_FIRST;
-  else {
-    // after off_bar (the kernel's layout): G * nbar barriers, TMEM pointer, coefficient area, G * 4 * nmod slices, slice barriers
-    const uint32_t nbar = 3 * kp.SA + 2 * kp.NB + 2 * kp.R;
-    const uint32_t aux = (8u * nbar * kp.G + 24u) & ~15u;
-    const uint32_t slices_end = aux + 4u * (kp.G * 2 * kp.CB + kp.G * 2 * 64 + kp.G * 4 * nmod * TC_FIRST_SLICE);
-    kp.fc_sbar = (slices_end + 7u) & ~7u;
-    kp.fc_M = nmod;
-    t.smem_bytes = kp.off_bar + kp.fc_sbar + kp.G * 256;
-  }
+  // after off_bar (the kernel's layout): G * nbar barriers, TMEM pointer, coefficient area, G * 4 * nmod slices, slice barriers
+  const uint32_t nbar = 3 * kp.SA + 2 * kp.NB + 2 * kp.R;
+  const uint32_t aux = (8u * nbar * kp.G + 24u) & ~15u;
+  const uint32_t slices_end = aux + 4u * (kp.G * 2 * kp.CB + kp.G * 2 * 64 + kp.G * 4 * nmod * TC_FIRST_SLICE);
+  kp.fc_sbar = (slices_end + 7u) & ~7u;
+  kp.fc_M = nmod;
+  t.smem_bytes = kp.off_bar + kp.fc_sbar + kp.G * 256;
   if (t.smem_bytes > TC_SMEM_MAX) { *why = "internal: shared memory plan exceeds 227 KB"; return 1; }
   kp.out = out;
   // B tile of modality m: [12 k8 chunks][cout rows][8]: K blocks of 16 taps = w_hi(0-15), w_hi(16-31), w_hi(0-15), w_hi(16-31),
@@ -1673,7 +1535,6 @@ inline int tc_set_attr_all() {
   if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3_tc_kernel<T, 2, true, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_MAX);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3_tc_kernel<T, 2, true, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_MAX);
   if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3_tc_kernel<T, 2, true, false, true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_MAX);
-  if (e == cudaSuccess) e = cudaFuncSetAttribute(conv3_tc_kernel<T, 2, true, false, true, false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_MAX);
 #undef DWMH_TC_ATTR
   return e == cudaSuccess ? 0 : 1;
 }
@@ -1681,7 +1542,7 @@ inline int tc_set_attr_all() {
 inline int tc_init_attributes(bool bf16) { return bf16 ? tc_set_attr_all<__nv_bfloat16>() : tc_set_attr_all<__half>(); }
 
 struct TcXform { const double* sums; const float* gamma; const float* beta; double inv_count; const void* src; };
-// mstride: floats between two modalities of the source (read only by the multi-modality kernel)
+// mstride: floats between two modalities of the source
 struct TcFirstSrc { const float* src; const SampleMeta* metas; int patch_mode, SY, SZ; int64_t mstride; };
 
 // planes per z-block: split D until the grid fills the machine about twice
@@ -1743,8 +1604,7 @@ int tc_launch(TcLayer& t, int nb, double* sums, StatPartial* partials, int num_s
   const bool small = kp.CB <= 32 && !kp.tconv;
 #define DWMH_TC_LAUNCH(K, S, C, D) conv3_tc_kernel<T, K, S, C, D, false><<<grid, threads, t.smem_bytes, st>>>(t.tm0, t.tm1, kp)
 #define DWMH_TC_LAUNCH_K(S, C, D) do { if (ks == 1) DWMH_TC_LAUNCH(1, S, C, D); else if (ks == 2) DWMH_TC_LAUNCH(2, S, C, D); else DWMH_TC_LAUNCH(4, S, C, D); } while (0)
-  if (kp.first && kp.fc_M > 1) conv3_tc_kernel<T, 2, true, false, true, false, true, true><<<grid, 512, t.smem_bytes, st>>>(t.tm0, t.tm1, kp);
-  else if (kp.first) conv3_tc_kernel<T, 2, true, false, true, false, true><<<grid, 512, t.smem_bytes, st>>>(t.tm0, t.tm1, kp);
+  if (kp.first) conv3_tc_kernel<T, 2, true, false, true, false, true><<<grid, 512, t.smem_bytes, st>>>(t.tm0, t.tm1, kp);
   else if (kp.xform) {
     const unsigned xthreads = (TC_THREADS + 32) * kp.G;
     if (kp.G == 2) conv3_tc_kernel<T, 2, true, false, true, true><<<grid, xthreads, t.smem_bytes, st>>>(t.tm0, t.tm1, kp);

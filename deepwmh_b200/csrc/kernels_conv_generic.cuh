@@ -12,14 +12,15 @@ __host__ __device__ inline int tc_s2d_class(int d, int h, int w, int sd, int sh,
 
 
 // ---------------------------------------------------------------------------------------------
-// First conv (Cin == 1) fused with tile extraction + mirror flip: reads the normalised fp32 volume
-// (or fp32 patches) directly, writes raw [n][Cout/8][P][8] + statistics.  One thread per output
-// voxel, 8 output channels at a time.  w: [taps][Cout] fp32.
+// First conv fused with tile extraction + mirror flip: reads the normalised fp32 volume [Cin][SX][SY][SZ] (patch_mode 0,
+// modalities p.mstride floats apart) or fp32 patches [n][Cin][px][py][pz] (1) directly, writes raw [n][Cout/8][P][8] +
+// statistics.  One thread per output voxel, 8 output channels at a time; per channel the taps of modality 0, 1, ...
+// accumulate in that order into one fp32 sum.  grid.z: blocks of 32 output channels.  w: [Cin][taps][Cout] fp32.
 // ---------------------------------------------------------------------------------------------
 struct FirstConvParams {
-  const float* src;            // volume [SX][SY][SZ] (patch_mode 0) or patches [n][px][py][pz] (1)
+  const float* src;            // volume [Cin][SX][SY][SZ] (patch_mode 0) or patches [n][Cin][px][py][pz] (1)
   const SampleMeta* metas;     // per sample origin + flip (patch_mode 0)
-  const float* w;              // [kd*kh*kw][Cout]
+  const float* w;              // [Cin][kd*kh*kw][Cout]
   void* out;
   double* sums;                // [n][Cout][2]
   int patch_mode;
@@ -27,23 +28,10 @@ struct FirstConvParams {
   int px, py, pz;
   int kd, kh, kw;
   int Cout;
-  int Cin;                     // modalities (conv_first_mm_kernel; the single-modality kernels ignore it)
+  int Cin;                     // modalities
   int64_t mstride;             // floats between two modalities of the volume (patch_mode 0)
   float* partials;             // [n][gridDim.x][Cout][2]: each block's statistics, summed by first_stats_reduce_kernel
 };
-
-// Statistics of the first-conv kernels without atomics, so that a forward gives the same bits on every run: sstat holds
-// one [Cout][2] slot per warp, written by that warp alone; each block sums its warps' slots in warp order into its own
-// slot of p.partials, and first_stats_reduce_kernel adds the blocks of a sample in block order in fp64.
-__device__ __forceinline__ void first_conv_block_partials(const float* sstat, float* partials, int n, int Cout) {
-  __syncthreads();
-  const int nw = blockDim.x >> 5;
-  for (int c = threadIdx.x; c < 2 * Cout; c += blockDim.x) {
-    float s = 0.f;
-    for (int w = 0; w < nw; ++w) s += sstat[w * 2 * Cout + c];
-    partials[((size_t)n * gridDim.x + blockIdx.x) * 2 * Cout + c] = s;
-  }
-}
 
 // grid: one block per sample; sums [n][C2] (C2 = 2 Cout) = sum over the nblk blocks of partials [n][nblk][C2], in order
 __global__ void __launch_bounds__(128) first_stats_reduce_kernel(const float* __restrict__ partials, double* __restrict__ sums,
@@ -57,221 +45,21 @@ __global__ void __launch_bounds__(128) first_stats_reduce_kernel(const float* __
 }
 
 // K3: kernel is 3x3x3 (fully unrolled taps, inputs stay in registers).  Each thread walks FC_VPT voxels
-// (stride = blockDim) and keeps per-channel running statistics in registers (Cout <= 32) so the warp
-// reduction happens once per thread instead of once per voxel.
+// (stride = blockDim) and keeps per-channel running statistics in registers, so the warp reduction happens
+// once per thread instead of once per voxel.  The channel chunk is the outer loop and the modality the inner
+// one, so that only 8 accumulators are live; with one modality the neighbourhood is gathered once per voxel.
 constexpr int FC_VPT = 4;
 
 template <typename T, bool K3>
-__global__ void __launch_bounds__(256) conv_first_kernel(FirstConvParams p) {
-  extern __shared__ float smf[];                 // weights [taps][Cout], then stats [warp][Cout][2]
-  const int kd = K3 ? 3 : p.kd, kh = K3 ? 3 : p.kh, kw = K3 ? 3 : p.kw;
-  const int taps = kd * kh * kw;
-  float* sw = smf;
-  float* sstat = smf + taps * p.Cout;
-  for (int i = threadIdx.x; i < taps * p.Cout; i += blockDim.x) sw[i] = p.w[i];
-  for (int i = threadIdx.x; i < (blockDim.x >> 5) * 2 * p.Cout; i += blockDim.x) sstat[i] = 0.f;
-  __syncthreads();
-  const int n = blockIdx.y;
-  const int64_t P = (int64_t)p.px * p.py * p.pz;
-  int ox = 0, oy = 0, oz = 0, flip = 0;
-  const float* src = p.src;
-  int SY = p.SY, SZ = p.SZ;
-  if (p.patch_mode) { src += (size_t)n * P; SY = p.py; SZ = p.pz; }
-  else { const SampleMeta m = p.metas[n]; ox = m.ox; oy = m.oy; oz = m.oz; flip = m.flip; }
-  const int lane = threadIdx.x & 31;
-  float* wst = sstat + (threadIdx.x >> 5) * 2 * p.Cout;     // this warp's statistics slot
-  const bool reg_stats = p.Cout <= 32;
-  float rs[32], rq[32];
-#pragma unroll
-  for (int q = 0; q < 32; ++q) { rs[q] = 0.f; rq[q] = 0.f; }
-  for (int it = 0; it < FC_VPT; ++it) {
-    const int64_t v = ((int64_t)blockIdx.x * FC_VPT + it) * blockDim.x + threadIdx.x;
-    const bool active = v < P;
-    const int k = (int)(v % p.pz), j = (int)((v / p.pz) % p.py), i = (int)(v / ((int64_t)p.pz * p.py));
-    float xin[27];
-#pragma unroll
-    for (int a = 0; a < (K3 ? 3 : 3); ++a)
-#pragma unroll
-      for (int b = 0; b < 3; ++b)
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-          float val = 0.f;
-          if (a < kd && b < kh && c < kw) {
-            const int ii = i + a - (kd >> 1), jj = j + b - (kh >> 1), kk = k + c - (kw >> 1);
-            if (active && ii >= 0 && ii < p.px && jj >= 0 && jj < p.py && kk >= 0 && kk < p.pz) {
-              const int si = ox + ((flip & 4) ? p.px - 1 - ii : ii);
-              const int sj = oy + ((flip & 2) ? p.py - 1 - jj : jj);
-              const int sk = oz + ((flip & 1) ? p.pz - 1 - kk : kk);
-              val = __ldg(src + ((size_t)si * SY + sj) * SZ + sk);
-            }
-          }
-          xin[(a * 3 + b) * 3 + c] = val;
-        }
-    uint4* outp = reinterpret_cast<uint4*>(p.out) + (size_t)n * (p.Cout >> 3) * P + v;
-    for (int cc = 0; cc < (p.Cout >> 3); ++cc) {
-      float acc[8];
-#pragma unroll
-      for (int q = 0; q < 8; ++q) acc[q] = 0.f;
-#pragma unroll
-      for (int a = 0; a < 3; ++a)
-#pragma unroll
-        for (int b = 0; b < 3; ++b)
-#pragma unroll
-          for (int c = 0; c < 3; ++c) {
-            if (a < kd && b < kh && c < kw) {
-              const int t = (a * kh + b) * kw + c;
-              const float4 w0 = *reinterpret_cast<const float4*>(sw + t * p.Cout + cc * 8);
-              const float4 w1 = *reinterpret_cast<const float4*>(sw + t * p.Cout + cc * 8 + 4);
-              const float x = xin[(a * 3 + b) * 3 + c];
-              acc[0] = fmaf(x, w0.x, acc[0]); acc[1] = fmaf(x, w0.y, acc[1]); acc[2] = fmaf(x, w0.z, acc[2]); acc[3] = fmaf(x, w0.w, acc[3]);
-              acc[4] = fmaf(x, w1.x, acc[4]); acc[5] = fmaf(x, w1.y, acc[5]); acc[6] = fmaf(x, w1.z, acc[6]); acc[7] = fmaf(x, w1.w, acc[7]);
-            }
-          }
-      if (active) outp[(size_t)cc * P] = pack8<T>(acc);
-      if (reg_stats) {
-#pragma unroll
-        for (int q4 = 0; q4 < 4; ++q4) {
-          if (cc == q4 && active) {
-#pragma unroll
-            for (int q = 0; q < 8; ++q) { rs[q4 * 8 + q] += acc[q]; rq[q4 * 8 + q] = fmaf(acc[q], acc[q], rq[q4 * 8 + q]); }
-          }
-        }
-      } else {
-#pragma unroll
-        for (int q = 0; q < 8; ++q) {
-          const float a_ = active ? acc[q] : 0.f;
-          const float s = warp_sum(a_), ss = warp_sum(a_ * a_);
-          if (lane == 0) { wst[(cc * 8 + q) * 2] += s; wst[(cc * 8 + q) * 2 + 1] += ss; }
-        }
-      }
-    }
-  }
-  if (reg_stats) {
-    // transposing butterfly: lane l ends with the warp total of channel l
-#pragma unroll
-    for (int k = 16; k >= 1; k >>= 1) {
-      const bool up = (lane & k) != 0;
-#pragma unroll
-      for (int i = 0; i < k; ++i) {
-        const float sa_ = up ? rs[i] : rs[i + k], ka_ = up ? rs[i + k] : rs[i];
-        const float sb_ = up ? rq[i] : rq[i + k], kb_ = up ? rq[i + k] : rq[i];
-        rs[i] = ka_ + __shfl_xor_sync(0xffffffffu, sa_, k);
-        rq[i] = kb_ + __shfl_xor_sync(0xffffffffu, sb_, k);
-      }
-    }
-    if (lane < p.Cout) { wst[lane * 2] = rs[0]; wst[lane * 2 + 1] = rq[0]; }
-  }
-  first_conv_block_partials(sstat, p.partials, n, p.Cout);
-}
-
-// 3x3x3 specialisation with TWO z-adjacent voxels per thread: one broadcast weight load feeds 16 FMAs
-// (the one-voxel form is bound by the shared-memory port: 1 LDS.128 per 4 FMAs), and the pair shares its
-// 3x3x4 input neighbourhood.  Requires pz even and Cout <= 32.
-template <typename T>
-__global__ void __launch_bounds__(128) conv_first_k3x2_kernel(FirstConvParams p) {
-  extern __shared__ float smf[];                 // weights [27][Cout], then stats [warp][Cout][2]
-  float* sw = smf;
-  float* sstat = smf + 27 * p.Cout;
-  for (int i = threadIdx.x; i < 27 * p.Cout; i += blockDim.x) sw[i] = p.w[i];
-  for (int i = threadIdx.x; i < (blockDim.x >> 5) * 2 * p.Cout; i += blockDim.x) sstat[i] = 0.f;
-  __syncthreads();
-  const int n = blockIdx.y;
-  const int64_t P = (int64_t)p.px * p.py * p.pz, P2 = P >> 1;
-  int ox = 0, oy = 0, oz = 0, flip = 0;
-  const float* src = p.src;
-  int SY = p.SY, SZ = p.SZ;
-  if (p.patch_mode) { src += (size_t)n * P; SY = p.py; SZ = p.pz; }
-  else { const SampleMeta m = p.metas[n]; ox = m.ox; oy = m.oy; oz = m.oz; flip = m.flip; }
-  const int lane = threadIdx.x & 31;
-  float* wst = sstat + (threadIdx.x >> 5) * 2 * p.Cout;     // this warp's statistics slot
-  const int pz2 = p.pz >> 1;
-  float rs[32], rq[32];
-#pragma unroll
-  for (int q = 0; q < 32; ++q) { rs[q] = 0.f; rq[q] = 0.f; }
-  for (int it = 0; it < FC_VPT; ++it) {
-    const int64_t v2 = ((int64_t)blockIdx.x * FC_VPT + it) * blockDim.x + threadIdx.x;      // voxel-pair index
-    const bool active = v2 < P2;
-    const int k = (int)(v2 % pz2) * 2, j = (int)((v2 / pz2) % p.py), i = (int)(v2 / ((int64_t)pz2 * p.py));
-    float xin[9][4];
-#pragma unroll
-    for (int a = 0; a < 3; ++a)
-#pragma unroll
-      for (int b = 0; b < 3; ++b)
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          const int ii = i + a - 1, jj = j + b - 1, kk = k + c - 1;
-          float val = 0.f;
-          if (active && ii >= 0 && ii < p.px && jj >= 0 && jj < p.py && kk >= 0 && kk < p.pz) {
-            const int si = ox + ((flip & 4) ? p.px - 1 - ii : ii);
-            const int sj = oy + ((flip & 2) ? p.py - 1 - jj : jj);
-            const int sk = oz + ((flip & 1) ? p.pz - 1 - kk : kk);
-            val = __ldg(src + ((size_t)si * SY + sj) * SZ + sk);
-          }
-          xin[a * 3 + b][c] = val;
-        }
-    const int64_t v = ((int64_t)i * p.py + j) * p.pz + k;
-    uint4* outp = reinterpret_cast<uint4*>(p.out) + (size_t)n * (p.Cout >> 3) * P + v;
-#pragma unroll
-    for (int cc = 0; cc < 4; ++cc) {
-      if (cc < (p.Cout >> 3)) {
-        float a0[8], a1[8];
-#pragma unroll
-        for (int q = 0; q < 8; ++q) { a0[q] = 0.f; a1[q] = 0.f; }
-#pragma unroll
-        for (int ab = 0; ab < 9; ++ab)
-#pragma unroll
-          for (int c = 0; c < 3; ++c) {
-            const float4 w0 = *reinterpret_cast<const float4*>(sw + (ab * 3 + c) * p.Cout + cc * 8);
-            const float4 w1 = *reinterpret_cast<const float4*>(sw + (ab * 3 + c) * p.Cout + cc * 8 + 4);
-            const float x0 = xin[ab][c], x1 = xin[ab][c + 1];
-            a0[0] = fmaf(x0, w0.x, a0[0]); a0[1] = fmaf(x0, w0.y, a0[1]); a0[2] = fmaf(x0, w0.z, a0[2]); a0[3] = fmaf(x0, w0.w, a0[3]);
-            a0[4] = fmaf(x0, w1.x, a0[4]); a0[5] = fmaf(x0, w1.y, a0[5]); a0[6] = fmaf(x0, w1.z, a0[6]); a0[7] = fmaf(x0, w1.w, a0[7]);
-            a1[0] = fmaf(x1, w0.x, a1[0]); a1[1] = fmaf(x1, w0.y, a1[1]); a1[2] = fmaf(x1, w0.z, a1[2]); a1[3] = fmaf(x1, w0.w, a1[3]);
-            a1[4] = fmaf(x1, w1.x, a1[4]); a1[5] = fmaf(x1, w1.y, a1[5]); a1[6] = fmaf(x1, w1.z, a1[6]); a1[7] = fmaf(x1, w1.w, a1[7]);
-          }
-        if (active) {
-          outp[(size_t)cc * P] = pack8<T>(a0);
-          outp[(size_t)cc * P + 1] = pack8<T>(a1);
-#pragma unroll
-          for (int q = 0; q < 8; ++q) {
-            rs[cc * 8 + q] += a0[q] + a1[q];
-            rq[cc * 8 + q] = fmaf(a0[q], a0[q], fmaf(a1[q], a1[q], rq[cc * 8 + q]));
-          }
-        }
-      }
-    }
-  }
-#pragma unroll
-  for (int k = 16; k >= 1; k >>= 1) {
-    const bool up = (lane & k) != 0;
-#pragma unroll
-    for (int i = 0; i < k; ++i) {
-      const float sa_ = up ? rs[i] : rs[i + k], ka_ = up ? rs[i + k] : rs[i];
-      const float sb_ = up ? rq[i] : rq[i + k], kb_ = up ? rq[i + k] : rq[i];
-      rs[i] = ka_ + __shfl_xor_sync(0xffffffffu, sa_, k);
-      rq[i] = kb_ + __shfl_xor_sync(0xffffffffu, sb_, k);
-    }
-  }
-  if (lane < p.Cout) { wst[lane * 2] = rs[0]; wst[lane * 2 + 1] = rq[0]; }
-  first_conv_block_partials(sstat, p.partials, n, p.Cout);
-}
-
-// ---------------------------------------------------------------------------------------------
-// First conv with Cin = p.Cin > 1 modalities (nnU-Net models with several input images): the volume is [Cin][SX][SY][SZ]
-// (patch_mode 0, modalities p.mstride floats apart) or patches [n][Cin][px][py][pz].  One thread per output voxel; per
-// 8-channel output chunk the taps of modality 0, 1, ... accumulate in that order into one fp32 sum.  w: [Cin][taps][Cout].
-// Statistics as in conv_first_kernel.  Requires Cout <= 32.
-// ---------------------------------------------------------------------------------------------
-template <typename T, bool K3>
-__global__ void __launch_bounds__(256) conv_first_mm_kernel(FirstConvParams p) {
-  extern __shared__ float smf[];                 // weights [Cin][taps][Cout], then stats [warp][Cout][2]
+__global__ void __launch_bounds__(256, 2) conv_first_kernel(FirstConvParams p) {
+  extern __shared__ float smf[];                 // weights [Cin][taps][Cout], then stats [warp][32][2]
   const int kd = K3 ? 3 : p.kd, kh = K3 ? 3 : p.kh, kw = K3 ? 3 : p.kw;
   const int taps = kd * kh * kw;
   float* sw = smf;
   float* sstat = smf + p.Cin * taps * p.Cout;
   for (int i = threadIdx.x; i < p.Cin * taps * p.Cout; i += blockDim.x) sw[i] = p.w[i];
-  for (int i = threadIdx.x; i < (blockDim.x >> 5) * 2 * p.Cout; i += blockDim.x) sstat[i] = 0.f;
   __syncthreads();
+  const int c0 = blockIdx.z * 32, nco = min(32, p.Cout - c0);      // this block's output channels
   const int n = blockIdx.y;
   const int64_t P = (int64_t)p.px * p.py * p.pz;
   int ox = 0, oy = 0, oz = 0, flip = 0;
@@ -281,7 +69,6 @@ __global__ void __launch_bounds__(256) conv_first_mm_kernel(FirstConvParams p) {
   if (p.patch_mode) { src += (size_t)n * p.Cin * P; SY = p.py; SZ = p.pz; mstride = P; }
   else { const SampleMeta m = p.metas[n]; ox = m.ox; oy = m.oy; oz = m.oz; flip = m.flip; }
   const int lane = threadIdx.x & 31;
-  float* wst = sstat + (threadIdx.x >> 5) * 2 * p.Cout;     // this warp's statistics slot
   float rs[32], rq[32];
 #pragma unroll
   for (int q = 0; q < 32; ++q) { rs[q] = 0.f; rq[q] = 0.f; }
@@ -289,65 +76,69 @@ __global__ void __launch_bounds__(256) conv_first_mm_kernel(FirstConvParams p) {
     const int64_t v = ((int64_t)blockIdx.x * FC_VPT + it) * blockDim.x + threadIdx.x;
     const bool active = v < P;
     const int k = (int)(v % p.pz), j = (int)((v / p.pz) % p.py), i = (int)(v / ((int64_t)p.pz * p.py));
-    float acc[4][8];
+    float xin[27];
+    int xm = -1;                                 // the modality whose neighbourhood xin holds
+    uint4* outp = reinterpret_cast<uint4*>(p.out) + ((size_t)n * (p.Cout >> 3) + (c0 >> 3)) * P + v;
+    for (int cc = 0; cc < (nco >> 3); ++cc) {
+      float acc[8];
 #pragma unroll
-    for (int cc = 0; cc < 4; ++cc)
-#pragma unroll
-      for (int q = 0; q < 8; ++q) acc[cc][q] = 0.f;
-    for (int m = 0; m < p.Cin; ++m) {
-      float xin[27];
-#pragma unroll
-      for (int a = 0; a < 3; ++a)
-#pragma unroll
-        for (int b = 0; b < 3; ++b)
-#pragma unroll
-          for (int c = 0; c < 3; ++c) {
-            float val = 0.f;
-            if (a < kd && b < kh && c < kw) {
-              const int ii = i + a - (kd >> 1), jj = j + b - (kh >> 1), kk = k + c - (kw >> 1);
-              if (active && ii >= 0 && ii < p.px && jj >= 0 && jj < p.py && kk >= 0 && kk < p.pz) {
-                const int si = ox + ((flip & 4) ? p.px - 1 - ii : ii);
-                const int sj = oy + ((flip & 2) ? p.py - 1 - jj : jj);
-                const int sk = oz + ((flip & 1) ? p.pz - 1 - kk : kk);
-                val = __ldg(src + (size_t)m * mstride + ((size_t)si * SY + sj) * SZ + sk);
-              }
-            }
-            xin[(a * 3 + b) * 3 + c] = val;
-          }
-      const float* wm = sw + (size_t)m * taps * p.Cout;
-#pragma unroll
-      for (int cc = 0; cc < 4; ++cc) {
-        if (cc < (p.Cout >> 3)) {
+      for (int q = 0; q < 8; ++q) acc[q] = 0.f;
+      const float* wt = sw + c0 + cc * 8;        // the taps of modality 0, 1, ... follow each other, Cout floats apart
+      for (int m = 0; m < p.Cin; ++m) {
+        if (m != xm) {
+          // the coordinates pass through an empty asm so that the tap addresses are recomputed per gather: kept live across
+          // the chunk and modality loops they took the kernel to 180 registers (one block per SM instead of two)
+          int gi = i, gj = j, gk = k;
+          asm volatile("" : "+r"(gi), "+r"(gj), "+r"(gk));
+          xm = m;
 #pragma unroll
           for (int a = 0; a < 3; ++a)
 #pragma unroll
             for (int b = 0; b < 3; ++b)
 #pragma unroll
               for (int c = 0; c < 3; ++c) {
+                float val = 0.f;
                 if (a < kd && b < kh && c < kw) {
-                  const int t = (a * kh + b) * kw + c;
-                  const float4 w0 = *reinterpret_cast<const float4*>(wm + t * p.Cout + cc * 8);
-                  const float4 w1 = *reinterpret_cast<const float4*>(wm + t * p.Cout + cc * 8 + 4);
-                  const float x = xin[(a * 3 + b) * 3 + c];
-                  float* ac = acc[cc];
-                  ac[0] = fmaf(x, w0.x, ac[0]); ac[1] = fmaf(x, w0.y, ac[1]); ac[2] = fmaf(x, w0.z, ac[2]); ac[3] = fmaf(x, w0.w, ac[3]);
-                  ac[4] = fmaf(x, w1.x, ac[4]); ac[5] = fmaf(x, w1.y, ac[5]); ac[6] = fmaf(x, w1.z, ac[6]); ac[7] = fmaf(x, w1.w, ac[7]);
+                  const int ii = gi + a - (kd >> 1), jj = gj + b - (kh >> 1), kk = gk + c - (kw >> 1);
+                  if (active && ii >= 0 && ii < p.px && jj >= 0 && jj < p.py && kk >= 0 && kk < p.pz) {
+                    const int si = ox + ((flip & 4) ? p.px - 1 - ii : ii);
+                    const int sj = oy + ((flip & 2) ? p.py - 1 - jj : jj);
+                    const int sk = oz + ((flip & 1) ? p.pz - 1 - kk : kk);
+                    val = __ldg(src + (size_t)m * mstride + ((size_t)si * SY + sj) * SZ + sk);
+                  }
                 }
+                xin[(a * 3 + b) * 3 + c] = val;
               }
+        }
+#pragma unroll
+        for (int a = 0; a < 3; ++a)
+#pragma unroll
+          for (int b = 0; b < 3; ++b)
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+              if (a < kd && b < kh && c < kw) {
+                const float4 w0 = *reinterpret_cast<const float4*>(wt);
+                const float4 w1 = *reinterpret_cast<const float4*>(wt + 4);
+                wt += p.Cout;
+                const float x = xin[(a * 3 + b) * 3 + c];
+                acc[0] = fmaf(x, w0.x, acc[0]); acc[1] = fmaf(x, w0.y, acc[1]); acc[2] = fmaf(x, w0.z, acc[2]); acc[3] = fmaf(x, w0.w, acc[3]);
+                acc[4] = fmaf(x, w1.x, acc[4]); acc[5] = fmaf(x, w1.y, acc[5]); acc[6] = fmaf(x, w1.z, acc[6]); acc[7] = fmaf(x, w1.w, acc[7]);
+              }
+            }
+      }
+      if (active) {
+        outp[(size_t)cc * P] = pack8<T>(acc);
+#pragma unroll
+        for (int q4 = 0; q4 < 4; ++q4) {
+          if (cc == q4) {
+#pragma unroll
+            for (int q = 0; q < 8; ++q) { rs[q4 * 8 + q] += acc[q]; rq[q4 * 8 + q] = fmaf(acc[q], acc[q], rq[q4 * 8 + q]); }
+          }
         }
       }
     }
-    uint4* outp = reinterpret_cast<uint4*>(p.out) + (size_t)n * (p.Cout >> 3) * P + v;
-#pragma unroll
-    for (int cc = 0; cc < 4; ++cc) {
-      if (cc < (p.Cout >> 3) && active) {
-        outp[(size_t)cc * P] = pack8<T>(acc[cc]);
-#pragma unroll
-        for (int q = 0; q < 8; ++q) { rs[cc * 8 + q] += acc[cc][q]; rq[cc * 8 + q] = fmaf(acc[cc][q], acc[cc][q], rq[cc * 8 + q]); }
-      }
-    }
   }
-  // transposing butterfly: lane l ends with the warp total of channel l
+  // transposing butterfly: lane l ends with the warp total of channel c0 + l
 #pragma unroll
   for (int k = 16; k >= 1; k >>= 1) {
     const bool up = (lane & k) != 0;
@@ -359,8 +150,17 @@ __global__ void __launch_bounds__(256) conv_first_mm_kernel(FirstConvParams p) {
       rq[i] = kb_ + __shfl_xor_sync(0xffffffffu, sb_, k);
     }
   }
-  if (lane < p.Cout) { wst[lane * 2] = rs[0]; wst[lane * 2 + 1] = rq[0]; }
-  first_conv_block_partials(sstat, p.partials, n, p.Cout);
+  // Statistics without atomics, so that a forward gives the same bits on every run: sstat holds one [nco][2] slot per warp,
+  // written by that warp alone; the block sums its warps' slots in warp order into its own slot of p.partials, and
+  // first_stats_reduce_kernel adds the blocks of a sample in block order in fp64.
+  if (lane < nco) { sstat[((threadIdx.x >> 5) * 32 + lane) * 2] = rs[0]; sstat[((threadIdx.x >> 5) * 32 + lane) * 2 + 1] = rq[0]; }
+  __syncthreads();
+  const int nw = blockDim.x >> 5;
+  for (int c = threadIdx.x; c < 2 * nco; c += blockDim.x) {
+    float s = 0.f;
+    for (int w = 0; w < nw; ++w) s += sstat[w * 64 + c];
+    p.partials[((size_t)n * gridDim.x + blockIdx.x) * 2 * p.Cout + 2 * c0 + c] = s;
+  }
 }
 
 // ---------------------------------------------------------------------------------------------

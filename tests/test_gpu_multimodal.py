@@ -90,8 +90,8 @@ def test_forward_patches_match_oracle_and_cuda_core(kind, M, C):
 
 
 # (kind, M, C, base_num_features, activation type).  Every head class count 3..8; (4, 8) is the head's largest shared
-# memory and register footprint; bf16 with several modalities takes the MULTI first conv's bf16 hi / lo split on the cube
-# plan and conv_first_mm_kernel's bf16 instantiation on the anisotropic one; base 64 gives the head a 64-channel input,
+# memory and register footprint; bf16 with several modalities takes the tcgen05 first conv's bf16 hi / lo split on the cube
+# plan and conv_first_kernel's bf16 instantiation on the anisotropic one; base 64 gives the head a 64-channel input,
 # its one-voxel (scalar) branch.
 LAYER_CASES = [
     ("cube", 2, 3, 32, "fp16"), ("aniso", 2, 3, 32, "fp16"), ("cube", 4, 4, 32, "fp16"), ("aniso", 4, 4, 32, "fp16"),
@@ -146,7 +146,7 @@ def test_tiled_predict_3d_with_tta_matches_oracle(M, C):
     tr.network.close()
 
 
-# the anisotropic plan's first conv runs on CUDA cores: conv_first_mm_kernel (M > 1), conv_first_kernel (M = 1)
+# the anisotropic plan's first conv runs on CUDA cores (conv_first_kernel)
 @pytest.mark.parametrize("kind,M,C", [("cube", 2, 3), ("cube", 4, 4), ("aniso", 2, 3), ("aniso", 1, 3)],
                          ids=["2-3", "4-4", "aniso-2-3", "aniso-1-3"])
 def test_bit_identical_repeat_and_split_tile_ranges(kind, M, C):

@@ -16,7 +16,7 @@ moved by a voxel, its forwards run with modalities 0 and 1 exchanged (M > 1), it
 (C > 2) -- must each differ from the device result by 100 times the tolerance, which shows that each would be caught.
 
 Volumes are [M, X, Y, Z] for M modalities ([X, Y, Z] for one) and the result has C classes: the cases with M > 1 reach
-the first conv's tile fetch with a modality stride (the tcgen05 kernel on the cube plan, conv_first_mm_kernel on the
+the first conv's tile fetch with a modality stride (the tcgen05 kernel on the cube plan, conv_first_kernel on the
 anisotropic one), and each class count reaches the overlap-add and finalize instantiated for it.  A single tile with one
 mirror axis is also checked bit for bit against its two forwards.
 """
@@ -287,7 +287,7 @@ SMALL_CASES = [c + ("cube", 1, 2, ((0, -1),)) for c in SMALL_CASES]
 # several modalities (the first conv's tile fetch with a modality stride) and classes (aggregate_tile_kernel<C>,
 # finalize_kernel<C, VEC>); (3, 2) feeds three modalities to the two-class overlap-add
 MC_CASES = [((40, 50, 45), 0.5, True, ALL, True, 8, "cube", M, C, ((0, -1),)) for M, C in ((2, 3), (4, 4), (3, 2), (1, 8))] + [
-    ((24, 70, 60), 0.5, True, ALL, True, 8, "aniso", 2, 3, ((0, -1),)),      # conv_first_mm_kernel in tile mode
+    ((24, 70, 60), 0.5, True, ALL, True, 8, "aniso", 2, 3, ((0, -1),)),      # the CUDA-core first conv in tile mode
     ((40, 50, 45), 0.5, True, (0, 1), True, 4, "cube", 2, 3, ((0, -1),)),    # one tile per batch
     ((40, 50, 45), 0.7, True, ALL, True, 16, "cube", 2, 3, ((0, -1),)),      # two tiles per batch
     ((40, 50, 45), 0.5, True, ALL, True, 8, "cube", 2, 3, ((0, 5), (5, -1))),   # a tile range over two calls

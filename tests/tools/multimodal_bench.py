@@ -53,7 +53,7 @@ def kernel_ms(fn):
 
 
 def _is_first(name):
-    # demangled: conv3_tc_kernel<T, KSTEPS, SMALL_CB, TCONV, DUAL, XFORM, FIRST[, MULTI]>
+    # demangled: conv3_tc_kernel<T, KSTEPS, SMALL_CB, TCONV, DUAL, XFORM, FIRST>
     args = name.split("<", 1)[1].split(">", 1)[0].split(",")
     return len(args) >= 7 and args[6].strip() == "true"
 
