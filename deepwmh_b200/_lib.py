@@ -12,6 +12,10 @@ from . import build as _build
 DWMH_MAX_POOL = 7
 DWMH_MAX_IN_CHANNELS = 4
 DWMH_MAX_CLASSES = 8
+# dwmh_layer_plan's output fields, in order (include/deepwmh_b200.h, enum DWMH_PLAN_*)
+LAYER_PLAN_FIELDS = ("kind", "kd", "sd", "sh", "sw", "KC", "KSTEPS", "CB", "ncb", "resident", "SA", "NB", "R",
+                     "G", "ZB", "nzb", "tiles", "items", "grid", "xform", "s222", "act")
+LAYER_PLAN_KINDS = ("first", "conv", "tconv", "cuda-core")
 
 
 class NetDesc(C.Structure):
@@ -79,7 +83,9 @@ SYMBOLS = {
                                                   C.c_int32, C.c_int32, _P, _P, _P]),
     "dwmh_forward_patches": (C.c_int, [_P, _P, C.c_int32, _P, _P]),
     "dwmh_debug_layer_output": (C.c_int, [_P, C.c_int32, _P, C.c_int64, C.POINTER(C.c_int32), _P]),
+    "dwmh_debug_layer_output_from": (C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int64, C.POINTER(C.c_int32), _P]),
     "dwmh_num_layers": (C.c_int, [_P]),
+    "dwmh_layer_plan": (C.c_int, [_P, C.c_int32, C.c_int32, C.POINTER(C.c_int32)]),
     "dwmh_layer_kernel_kind": (C.c_int, [_P, C.c_int32]),
     "dwmh_layer_norm_on_load": (C.c_int, [_P, C.c_int32]),
     "dwmh_set_force_generic": (C.c_int, [_P, C.c_int32]),

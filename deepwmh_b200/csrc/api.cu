@@ -281,6 +281,29 @@ extern "C" int dwmh_layer_norm_on_load(dwmh_ctx* c, int32_t i) {
   if (!c || i < 0 || i >= (int)c->layers.size()) return -1;
   return (c->layers[i].fused_norm && !c->force_generic) ? 1 : 0;
 }
+extern "C" int dwmh_layer_plan(dwmh_ctx* c, int32_t i, int32_t nb, int32_t out[DWMH_LAYER_PLAN_FIELDS]) {
+  if (!c || !out) return fail("dwmh_layer_plan: null argument");
+  if (i < 0 || i >= (int)c->layers.size()) return fail("dwmh_layer_plan: bad layer index %d", i);
+  if (!c->committed) return fail("dwmh_layer_plan: weights not committed");
+  if (nb < 1 || nb > c->max_batch) return fail("dwmh_layer_plan: batch %d outside 1..%d", nb, c->max_batch);
+  const Layer& L = c->layers[i];
+  for (int f = 0; f < DWMH_LAYER_PLAN_FIELDS; ++f) out[f] = 0;
+  out[DWMH_PLAN_KD] = L.k[0];
+  for (int a = 0; a < 3; ++a) out[DWMH_PLAN_SD + a] = L.s[a];
+  out[DWMH_PLAN_ACT] = c->bf16 ? 1 : 0;
+  if (!L.tc.enabled || c->force_generic) { out[DWMH_PLAN_KIND] = DWMH_PLAN_CUDA_CORE; return 0; }
+  const TcKParams& kp = L.tc.kp;
+  out[DWMH_PLAN_KIND] = L.kind == L_FIRST ? DWMH_PLAN_FIRST : L.kind == L_TCONV ? DWMH_PLAN_TCONV : DWMH_PLAN_CONV;
+  out[DWMH_PLAN_KC] = kp.KC; out[DWMH_PLAN_KSTEPS] = kp.KC / 16; out[DWMH_PLAN_CB] = kp.CB; out[DWMH_PLAN_NCB] = kp.ncb;
+  out[DWMH_PLAN_RESIDENT] = kp.resident; out[DWMH_PLAN_SA] = kp.SA; out[DWMH_PLAN_NB] = kp.NB; out[DWMH_PLAN_R] = kp.R;
+  const TcGrid g = tc_grid(kp, nb, c->num_sms);
+  out[DWMH_PLAN_G] = g.G; out[DWMH_PLAN_ZB] = g.ZB; out[DWMH_PLAN_NZB] = g.nzb; out[DWMH_PLAN_TILES] = g.tiles;
+  out[DWMH_PLAN_ITEMS] = (int32_t)g.items; out[DWMH_PLAN_GRID] = (int32_t)g.grid;
+  // forward_impl hands the transform to the launch when the producer is normalised on load; tc_launch applies it if xform_ok
+  out[DWMH_PLAN_XFORM] = L.kind == L_CONV && c->layers[L.in0].fused_norm && L.tc.xform_ok ? 1 : 0;
+  out[DWMH_PLAN_S222] = kp.s222;
+  return 0;
+}
 extern "C" int dwmh_set_force_generic(dwmh_ctx* c, int32_t on) { if (!c) return fail("null ctx"); c->force_generic = on != 0; return 0; }
 extern "C" int dwmh_get_counters(dwmh_ctx* c, int64_t* k, double* f) { if (!c) return fail("null ctx"); if (k) *k = c->launches; if (f) *f = c->conv_flops; return 0; }
 extern "C" int dwmh_set_stage_timing(dwmh_ctx* c, int32_t on) { if (!c) return fail("null ctx"); c->stage_timing = on != 0; return 0; }
@@ -754,24 +777,33 @@ extern "C" int dwmh_forward_patches(dwmh_ctx* c, const float* patches, int32_t n
   return 0;
 }
 
-extern "C" int dwmh_debug_layer_output(dwmh_ctx* c, int32_t li, float* out, int64_t capacity, int32_t dims[5], void* stream_) {
+extern "C" int dwmh_debug_layer_output_from(dwmh_ctx* c, int32_t li, int32_t first, float* out, int64_t capacity, int32_t dims[5],
+                                            void* stream_) {
   if (!c || li < 0 || li >= (int)c->layers.size()) return fail("dwmh_debug_layer_output: bad layer index");
+  if (first < 0 || first >= c->max_batch) return fail("dwmh_debug_layer_output: first sample %d outside 0..%d", first, c->max_batch - 1);
   Layer& L = c->layers[li];
-  const int n = c->max_batch;
+  const int n = c->max_batch - first;
   dims[0] = n; dims[1] = L.cout; dims[2] = L.out_sp[0]; dims[3] = L.out_sp[1]; dims[4] = L.out_sp[2];
   if (!out) return 0;                         // dims query
-  const int64_t need = (int64_t)n * L.cout * L.vout();
+  const int64_t per = (int64_t)L.cout * L.vout();
   int nn = n;
-  if (capacity < need) { nn = (int)(capacity / ((int64_t)L.cout * L.vout())); dims[0] = nn; if (nn <= 0) return fail("capacity too small"); }
+  if (capacity < (int64_t)n * per) { nn = (int)(capacity / per); dims[0] = nn; if (nn <= 0) return fail("capacity too small"); }
   cudaStream_t st = (cudaStream_t)stream_;
   DEV_GUARD(c->device);
-  // the last conv is kept raw (the head normalises on load): normalise here for a uniform view
+  // the last conv is kept raw (the head normalises on load): normalise here for a uniform view.  Samples from `first` on:
+  // the activations are [n][cout/8][V][8] and the statistics [n][cout][2], so both views start `first` samples in
   NormParams np{nullptr, nullptr, nullptr, 0.0};
-  if ((int)li == c->last_conv || (L.fused_norm && !c->force_generic)) np = NormParams{L.sums, L.gamma_dev, L.beta_dev, L.stats_mean_var ? 0.0 : 1.0 / (double)L.vout()};
-  if (c->bf16) unpack_layer_kernel<__nv_bfloat16><<<c->num_sms * 4, 256, 0, st>>>((const __nv_bfloat16*)L.out, np, out, nn, L.cout, L.vout());
-  else unpack_layer_kernel<__half><<<c->num_sms * 4, 256, 0, st>>>((const __half*)L.out, np, out, nn, L.cout, L.vout());
+  if ((int)li == c->last_conv || (L.fused_norm && !c->force_generic))
+    np = NormParams{L.sums + (size_t)first * L.cout * 2, L.gamma_dev, L.beta_dev, L.stats_mean_var ? 0.0 : 1.0 / (double)L.vout()};
+  const size_t off = (size_t)first * per;
+  if (c->bf16) unpack_layer_kernel<__nv_bfloat16><<<c->num_sms * 4, 256, 0, st>>>((const __nv_bfloat16*)L.out + off, np, out, nn, L.cout, L.vout());
+  else unpack_layer_kernel<__half><<<c->num_sms * 4, 256, 0, st>>>((const __half*)L.out + off, np, out, nn, L.cout, L.vout());
   CU_TRY(cudaGetLastError());
   return 0;
+}
+
+extern "C" int dwmh_debug_layer_output(dwmh_ctx* c, int32_t li, float* out, int64_t capacity, int32_t dims[5], void* stream_) {
+  return dwmh_debug_layer_output_from(c, li, 0, out, capacity, dims, stream_);
 }
 
 // ------------------------------------------------------------------------------------------------

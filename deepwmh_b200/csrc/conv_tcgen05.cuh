@@ -1578,6 +1578,22 @@ inline size_t tc_partials_needed(const TcKParams& kp, int nb, int num_sms) {
   return (size_t)nb * kp.ncb * ((kp.D + ZB - 1) / ZB) * kp.tilesH * kp.tilesW * kp.CB;
 }
 
+// Launch geometry of one layer at batch nb: z-blocks, the tile pipelines per CTA after the pairing rule, work items, CTAs
+struct TcGrid { int ZB, nzb, tiles, G; long long items; unsigned grid; };
+inline TcGrid tc_grid(const TcKParams& kp, int nb, int num_sms) {
+  TcGrid g;
+  g.tiles = kp.tilesH * kp.tilesW;
+  g.ZB = tc_plan_zb(kp, nb, num_sms);
+  g.nzb = (kp.D + g.ZB - 1) / g.ZB;
+  g.items = (long long)nb * kp.ncb * g.nzb * g.tiles;
+  // both groups of a CTA must share the cout block whose weights are resident: pairs (2k, 2k+1) stay inside
+  // one (n, cb) when the tiles x z-blocks count is even
+  g.G = kp.G;
+  if (!kp.first && kp.G == 2 && (kp.resident ? ((long long)g.nzb * g.tiles) % 2 != 0 : g.tiles % 2 != 0)) g.G = 1;    // (streamed weights: same z-block too)
+  g.grid = (unsigned)((g.items + g.G - 1) / g.G);
+  return g;
+}
+
 // sums: the layer's [n][Cout][2] fp64 statistics ({mean, variance} on return); partials: scratch of tc_partials_needed() entries
 template <typename T>
 int tc_launch(TcLayer& t, int nb, double* sums, StatPartial* partials, int num_sms, cudaStream_t st, std::string* err, const TcXform* xf = nullptr, const TcFirstSrc* fs = nullptr) {
@@ -1590,15 +1606,11 @@ int tc_launch(TcLayer& t, int nb, double* sums, StatPartial* partials, int num_s
     kp.fc_mstride = fs->mstride;
   }
   if (xf && t.xform_ok) { kp.xform = 1; kp.xf_sums = xf->sums; kp.xf_gamma = xf->gamma; kp.xf_beta = xf->beta; kp.xf_inv_count = xf->inv_count; kp.xf_src = xf->src; }
-  const int tiles = kp.tilesH * kp.tilesW;
-  const int ZB = tc_plan_zb(kp, nb, num_sms);
-  kp.ZB = ZB; kp.nzb = (kp.D + ZB - 1) / ZB;
-  const long long items = (long long)nb * kp.ncb * kp.nzb * tiles;
-  // both groups of a CTA must share the cout block whose weights are resident: pairs (2k, 2k+1) stay inside
-  // one (n, cb) when the tiles x z-blocks count is even
-  if (!kp.first && kp.G == 2 && (kp.resident ? ((long long)kp.nzb * tiles) % 2 != 0 : tiles % 2 != 0)) kp.G = 1;    // (streamed weights: same z-block too)
-  kp.total_items = (int)items;
-  const unsigned grid = (unsigned)((items + kp.G - 1) / kp.G);
+  const TcGrid tg = tc_grid(kp, nb, num_sms);
+  const int tiles = tg.tiles;
+  kp.ZB = tg.ZB; kp.nzb = tg.nzb; kp.G = tg.G;
+  kp.total_items = (int)tg.items;
+  const unsigned grid = tg.grid;
   const unsigned threads = TC_THREADS * kp.G;
   const int ks = kp.KC / 16;
   const bool small = kp.CB <= 32 && !kp.tconv;

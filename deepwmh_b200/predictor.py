@@ -274,16 +274,32 @@ class SegmentationNetwork:
         check(self._lib.dwmh_forward_patches(self._ctx, _ptr(patches), n, _ptr(out), self._st()))
         return out
 
-    def layer_output(self, index: int, n: int = 1) -> torch.Tensor:
-        """Normalised+activated output of layer `index` for the first n samples of the last forward,
-        as fp32 [n, c, d, h, w] (test hook)."""
+    def layer_output(self, index: int, n: int = 1, samples: "Optional[Sequence[int]]" = None) -> torch.Tensor:
+        """Normalised+activated output of layer `index` for the first n samples of the last forward, or for the listed
+        `samples` (copied one by one: a few samples of a large batch), as fp32 [n, c, d, h, w] (test hook)."""
+        if samples is not None:
+            return torch.cat([self._layer_output_from(index, int(s), 1) for s in samples])
+        return self._layer_output_from(index, 0, n)
+
+    def _layer_output_from(self, index: int, first: int, n: int) -> torch.Tensor:
         dims = (C.c_int32 * 5)()
-        check(self._lib.dwmh_debug_layer_output(self._ctx, index, C.c_void_p(0), 0, dims, self._st()))
+        check(self._lib.dwmh_debug_layer_output_from(self._ctx, index, first, C.c_void_p(0), 0, dims, self._st()))
         per = int(dims[1]) * int(dims[2]) * int(dims[3]) * int(dims[4])
         n = min(n, int(dims[0]))
         buf = torch.empty(n * per, dtype=torch.float32, device=self.device)
-        check(self._lib.dwmh_debug_layer_output(self._ctx, index, _ptr(buf), buf.numel(), dims, self._st()))
+        check(self._lib.dwmh_debug_layer_output_from(self._ctx, index, first, _ptr(buf), buf.numel(), dims, self._st()))
         return buf.view(n, int(dims[1]), int(dims[2]), int(dims[3]), int(dims[4]))
+
+    def layer_plan(self, index: int, nb: int) -> Dict[str, int]:
+        """What the launch of layer `index` at batch nb would run (dwmh_layer_plan): kind, kernel depth, strides, the
+        tcgen05 tiling (KC, KSTEPS, CB, ncb, resident weights, SA, NB, R), the launch geometry (G after the pairing rule,
+        ZB, nzb, tiles, items, grid), norm-on-load (xform), the stride-(2,2,2) issue path (s222) and the activation type."""
+        out = (C.c_int32 * len(_lib.LAYER_PLAN_FIELDS))()
+        check(self._lib.dwmh_layer_plan(self._ctx, index, nb, out))
+        plan = dict(zip(_lib.LAYER_PLAN_FIELDS, (int(v) for v in out)))
+        plan["kind"] = _lib.LAYER_PLAN_KINDS[plan["kind"]]
+        plan["act"] = ("fp16", "bf16")[plan["act"]]
+        return plan
 
     def num_layers(self) -> int:
         return int(self._lib.dwmh_num_layers(self._ctx))

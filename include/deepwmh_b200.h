@@ -275,7 +275,23 @@ int dwmh_forward_patches(dwmh_ctx* ctx, const float* patches_dev, int32_t n, flo
 /* Copy the (normalised, activated) output of layer `layer_index` of the last forward, converted to
  * fp32 NCDHW, into out_dev (capacity in floats); dims_out = {n, c, d, h, w}.  Layer order = execution order. */
 int dwmh_debug_layer_output(dwmh_ctx* ctx, int32_t layer_index, float* out_dev, int64_t capacity, int32_t dims_out[5], void* stream);
+/* The same for samples first, first + 1, ... of the last forward (dims_out[0] = how many were copied). */
+int dwmh_debug_layer_output_from(dwmh_ctx* ctx, int32_t layer_index, int32_t first, float* out_dev, int64_t capacity,
+                                 int32_t dims_out[5], void* stream);
 int dwmh_num_layers(dwmh_ctx* ctx);
+/* What the launch of layer `layer_index` at batch nb (1 .. max_batch) would run, computed by the functions the launch itself
+ * uses; read-only.  Valid after dwmh_commit_weights.  out[DWMH_PLAN_KIND] is one of DWMH_PLAN_FIRST / CONV / TCONV /
+ * CUDA_CORE; for a CUDA-core layer only KIND, KD, the strides and ACT are set (the rest is 0).  G is the tile pipelines per
+ * CTA after the launch's pairing rule, ITEMS = nb * ncb * nzb * tiles, GRID = CTAs. */
+enum {
+  DWMH_PLAN_KIND = 0, DWMH_PLAN_KD, DWMH_PLAN_SD, DWMH_PLAN_SH, DWMH_PLAN_SW,
+  DWMH_PLAN_KC, DWMH_PLAN_KSTEPS, DWMH_PLAN_CB, DWMH_PLAN_NCB, DWMH_PLAN_RESIDENT, DWMH_PLAN_SA, DWMH_PLAN_NB, DWMH_PLAN_R,
+  DWMH_PLAN_G, DWMH_PLAN_ZB, DWMH_PLAN_NZB, DWMH_PLAN_TILES, DWMH_PLAN_ITEMS, DWMH_PLAN_GRID,
+  DWMH_PLAN_XFORM, DWMH_PLAN_S222, DWMH_PLAN_ACT,
+  DWMH_LAYER_PLAN_FIELDS
+};
+enum { DWMH_PLAN_FIRST = 0, DWMH_PLAN_CONV = 1, DWMH_PLAN_TCONV = 2, DWMH_PLAN_CUDA_CORE = 3 };
+int dwmh_layer_plan(dwmh_ctx* ctx, int32_t layer_index, int32_t nb, int32_t out[DWMH_LAYER_PLAN_FIELDS]);
 /* Kernel variant used by a layer: 0 = direct (CUDA cores), 1 = tcgen05 implicit GEMM. */
 int dwmh_layer_kernel_kind(dwmh_ctx* ctx, int32_t layer_index);
 /* 1 when the layer's InstanceNorm + LeakyReLU are applied by its consumer on load (no separate pass, the layer's buffer keeps

@@ -134,13 +134,21 @@ def head_report(net, last, probs):
     return ((probs - p_ref).abs() / tol).max().item(), sens
 
 
-def layer_fp64_reports(net, dev, x, act="fp16", ref_device=None):
+def layer_fp64_reports(net, dev, x, act="fp16", ref_device=None, samples=None):
     """Run `dev` (a SegmentationNetwork, or the CPU emulation below) on x [n, 1, *patch] and compare each of its layers with
     the float64 reference fed the device's previous outputs.  Returns one dict per device layer, in device order (the
-    execution order of the network), and the head's (ratio, sensitivity)."""
+    execution order of the network), and the head's (ratio, sensitivity).  samples: check only these samples of the batch
+    (the device still runs all n; InstanceNorm is per sample, so each sample's layers are independent of the others)."""
     ref_device = ref_device if ref_device is not None else x.device
     n, u = x.shape[0], U[act]
-    probs = dev.forward_patches(x).to(ref_device, torch.float64)
+    probs = dev.forward_patches(x)
+    if samples is None:
+        fetch = lambda i: dev.layer_output(i, n)
+    else:
+        samples = list(samples)
+        probs, x = probs[samples], x[samples]
+        fetch = lambda i: dev.layer_output(i, samples=samples)
+    probs = probs.to(ref_device, torch.float64)
     ref_net = rounded_copy(net, act, torch.float64, ref_device)
     first, last = _first_conv(ref_net), _last_conv(ref_net)
     reports, raw, hooks = [], {}, []
@@ -151,7 +159,7 @@ def layer_fp64_reports(net, dev, x, act="fp16", ref_device=None):
     def on_layer(mod, inp, out):
         i = len(reports)
         x_in = inp[0]
-        got = dev.layer_output(i, n).to(ref_device, torch.float64)
+        got = fetch(i).to(ref_device, torch.float64)
         assert got.shape == out.shape, (i, tuple(got.shape), tuple(out.shape))
         rep = {"layer": i, "shape": tuple(out.shape[1:]), "norm_on_load": dev.layer_norm_on_load(i) == 1}
         if isinstance(mod, O.ConvDropoutNormNonlin):
@@ -176,7 +184,7 @@ def layer_fp64_reports(net, dev, x, act="fp16", ref_device=None):
         with torch.no_grad():
             ref_net(x.to(ref_device, torch.float64))
             assert len(reports) == dev.num_layers(), (len(reports), dev.num_layers())
-            head = head_report(ref_net, dev.layer_output(len(reports) - 1, n).to(ref_device, torch.float64), probs)
+            head = head_report(ref_net, fetch(len(reports) - 1).to(ref_device, torch.float64), probs)
     finally:
         for h in hooks:
             h.remove()
@@ -322,6 +330,19 @@ CASES = {
     "small-bf16": (lambda: small_plans(), 2, "bf16", False),
     "small-generic": (lambda: small_plans(), 2, "fp16", True),
     "partial-generic": (lambda: small_plans(patch=(64, 48, 40)), 2, "fp16", True),
+    # the issue forms tests/test_conv_paths.py found unchecked by the cases above (its REQUIRED set; ADDED_FOR there
+    # names the forms each of these reaches)
+    "dstride-32x64x64-n3": (lambda: small_plans(patch=(32, 64, 64), pools=((2, 1, 1), (2, 2, 2), (2, 2, 2))), 3, "fp16", False),
+    "k133stream-4x64x64": (lambda: small_plans(patch=(4, 64, 64), pools=((1, 2, 2),) * 4, kernels=[[1, 3, 3]] * 5), 2, "fp16", False),
+    "nol32-72x80x40-n1-bf16": (lambda: small_plans(patch=(72, 80, 40), pools=((2, 2, 2),) * 2), 1, "bf16", False),
+}
+
+# The production batch: bench.py and predict_3D run max_batch = 32 forwards per launch, and the last batch of a tile range
+# runs fewer on the same context.  name: (plans factory, batch size, max_batch, activation type, samples checked).  The
+# device runs the whole batch of distinct patches; the float64 reference runs the listed samples only.
+BATCH_CASES = {
+    "bench-128^3-n32": (_bench_plans, 32, 32, "fp16", (0, 13, 31)),
+    "bench-128^3-n17-of-32": (_bench_plans, 17, 32, "fp16", (0, 8, 16)),
 }
 
 
@@ -347,6 +368,27 @@ def test_every_layer_matches_fp64_on_its_own_inputs(case):
             assert any(nw.layer_norm_on_load(i) for i in range(nw.num_layers()))
         x = torch.randn(n, 1, *ps, generator=torch.Generator().manual_seed(7)).cuda()
         reports, head = layer_fp64_reports(net, nw, x, act)
+        check_reports(case, reports, head)
+    finally:
+        nw.close()
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("case", list(BATCH_CASES))
+def test_every_layer_matches_fp64_at_the_production_batch(case):
+    import deepwmh_b200
+    make_plans, n, max_batch, act, samples = BATCH_CASES[case]
+    plans = make_plans()
+    ps = tuple(int(i) for i in plans["plans_per_stage"][0]["patch_size"])
+    net = O.build_benchmark_network(0, plans)
+    tr = deepwmh_b200.nnUNetTrainerV2(plans, device=0, act_dtype=act, max_batch=max_batch)
+    tr.load_checkpoint_ram({"state_dict": net.state_dict()}, False)
+    nw = tr.network
+    try:
+        kinds = [nw.layer_kernel_kind(i) for i in range(nw.num_layers())]
+        assert sum(kinds) >= len(kinds) - 1, kinds
+        x = torch.randn(n, 1, *ps, generator=torch.Generator().manual_seed(7)).cuda()
+        reports, head = layer_fp64_reports(net, nw, x, act, samples=samples)
         check_reports(case, reports, head)
     finally:
         nw.close()
