@@ -24,7 +24,7 @@ class NetDesc(C.Structure):
         ("max_num_features", C.c_int32), ("num_pool", C.c_int32), ("patch_size", C.c_int32 * 3),
         ("pool_op_kernel_sizes", (C.c_int32 * 3) * DWMH_MAX_POOL),
         ("conv_kernel_sizes", (C.c_int32 * 3) * (DWMH_MAX_POOL + 1)),
-        ("act_dtype", C.c_int32), ("max_batch", C.c_int32), ("struct_size", C.c_int32),
+        ("act_dtype", C.c_int32), ("max_batch", C.c_int32), ("head_nonlin", C.c_int32), ("struct_size", C.c_int32),
     ]
 
 
@@ -49,6 +49,7 @@ SYMBOLS = {
     "dwmh_finalize": (C.c_int, [_P, _P, _P, _P, _P, C.c_int32, C.c_int32, C.c_int32, _P]),
     "dwmh_axpy": (C.c_int, [_P, _P, _P, C.c_float, C.c_int64, _P]),
     "dwmh_argmax": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int64, _P]),
+    "dwmh_region_labels": (C.c_int, [_P, _P, C.c_int32, C.POINTER(C.c_int32), _P, C.c_int64, _P]),
     "dwmh_ensemble_masked_add": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P]),
     "dwmh_ensemble_refine": (C.c_int, [_P, _P, C.c_int32, _P, C.c_int64, _P]),
     "dwmh_remove_sparks": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P, _P]),

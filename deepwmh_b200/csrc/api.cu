@@ -50,7 +50,7 @@ struct DevGuard {
 
 extern "C" const char* dwmh_last_error(void) { return g_err.c_str(); }
 extern "C" void dwmh_internal_set_error(const char* msg) { g_err = msg ? msg : ""; }   // for the other translation units (stage1.cu)
-extern "C" int dwmh_version(void) { return 101; }
+extern "C" int dwmh_version(void) { return 102; }
 
 // ------------------------------------------------------------------------------------------------
 // network plan
@@ -210,6 +210,8 @@ static int check_model_bounds(const dwmh_net_desc* d) {
   if (d->num_classes < 2 || d->num_classes > DWMH_MAX_CLASSES)
     return fail("dwmh_create: num_classes=%d unsupported (2 <= num_classes <= %d: the head keeps every class's logits of two "
                 "voxels in registers)", d->num_classes, DWMH_MAX_CLASSES);
+  if (d->head_nonlin != 0 && d->head_nonlin != 1)
+    return fail("dwmh_create: head_nonlin=%d unsupported (0 = softmax over classes, 1 = sigmoid per output)", d->head_nonlin);
   if (d->in_channels > 1 && d->base_num_features > 32)
     return fail("dwmh_create: base_num_features=%d with in_channels=%d unsupported (the multi-modality first conv has at most 32 "
                 "output channels)", d->base_num_features, d->in_channels);
@@ -636,7 +638,8 @@ extern "C" int dwmh_zscore(dwmh_ctx* c, float* vol, const int8_t* seg, int64_t n
 // forward
 // ------------------------------------------------------------------------------------------------
 // The kernels after the last conv (head, overlap-add, finalize) are instantiated for each class count 2 .. DWMH_MAX_CLASSES:
-// f(std::integral_constant<int, NC>) launches them for the model's count.
+// f(std::integral_constant<int, NC>) launches them for the model's count.  The head and the overlap-add have a second
+// instantiation per count for sigmoid-head models (dwmh_net_desc.head_nonlin = 1).
 template <typename F>
 static int with_num_classes(int NC, F&& f) {
   switch (NC) {
@@ -740,7 +743,7 @@ static int forward_impl(dwmh_ctx* c, const float* src, int patch_mode, int SX, i
       c->launches++;
     }
   }
-  // head: norm-on-load + 1x1x1 + softmax
+  // head: norm-on-load + 1x1x1 + softmax / sigmoid
   Layer& L = c->layers[c->last_conv];
   const int64_t head_items = (L.cout == 32 && (L.vout() & 1) == 0) ? L.vout() / 2 : L.vout();      // two voxels per thread in the usual head
   dim3 grid((unsigned)((head_items + 255) / 256), nb);
@@ -748,8 +751,11 @@ static int forward_impl(dwmh_ctx* c, const float* src, int patch_mode, int SX, i
   DW_TRY(cls_timed(2, (double)nb * L.vout() * (2.0 * L.cout + 4.0 * NC), [&] {
     return with_num_classes(NC, [&](auto nc) {
       constexpr int K = decltype(nc)::value;
-      head_softmax_kernel<T, K><<<grid, 256, (2 + K) * L.cout * sizeof(float), st>>>((const T*)L.out, norm_of(L), c->w_head_dev, c->probs,
-                                                                                    L.cout, L.vout());
+      const size_t smem = (2 + K) * L.cout * sizeof(float);
+      if (c->d.head_nonlin == 1)
+        head_softmax_kernel<T, K, true><<<grid, 256, smem, st>>>((const T*)L.out, norm_of(L), c->w_head_dev, c->probs, L.cout, L.vout());
+      else
+        head_softmax_kernel<T, K><<<grid, 256, smem, st>>>((const T*)L.out, norm_of(L), c->w_head_dev, c->probs, L.cout, L.vout());
       return 0; }); }));
   c->launches++;
   c->conv_flops += 2.0 * L.vout() * L.cout * c->d.num_classes * nb;
@@ -873,8 +879,9 @@ extern "C" int dwmh_predict_3d(dwmh_ctx* c, const float* vol, int32_t X, int32_t
     if (c->stage_timing) CU_TRY(cudaEventRecord(c->ev[1], st));
     DW_TRY(with_num_classes(NC, [&](auto nc) {
       constexpr int K = decltype(nc)::value;
+      auto kernel = c->d.head_nonlin == 1 ? aggregate_tile_kernel<K, true> : aggregate_tile_kernel<K>;
       for (int t = 0; t < tb; ++t)
-        aggregate_tile_kernel<K><<<(unsigned)((P + 255) / 256), 256, 0, st>>>(
+        kernel<<<(unsigned)((P + 255) / 256), 256, 0, st>>>(
             c->probs + (size_t)t * M * K * P, c->metas_dev + (size_t)(t0 + t) * M, M, gauss ? c->gauss_dev : nullptr,
             agg, wgt, ps[0], ps[1], ps[2], X, Y, Z);
       return 0; }));
@@ -953,6 +960,26 @@ extern "C" int dwmh_argmax(dwmh_ctx* c, const float* p, int32_t num_classes, uin
   if (num_classes < 1 || num_classes > 255) return fail("dwmh_argmax: num_classes=%d outside 1..255 (uint8 labels)", num_classes);
   DEV_GUARD(c->device);
   argmax_kernel<<<c->num_sms * 8, 256, 0, (cudaStream_t)stream_>>>(p, num_classes, seg, V);
+  c->launches++;
+  CU_TRY(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int dwmh_region_labels(dwmh_ctx* c, const float* p, int32_t num_regions, const int32_t* order, uint8_t* seg, int64_t V,
+                                  void* stream_) {
+  if (!c || !p || !order || !seg) return fail("dwmh_region_labels: null argument");
+  if (num_regions < 1 || num_regions > DWMH_MAX_CLASSES)
+    return fail("dwmh_region_labels: num_regions=%d outside 1..%d", num_regions, DWMH_MAX_CLASSES);
+  RegionTable t{};
+  t.n = num_regions;
+  for (int r = 0; r < num_regions; ++r) {
+    if (order[r] < 0 || order[r] > 255)
+      return fail("dwmh_region_labels: region %d has label %d, outside 0..255 (uint8 labels)", r, order[r]);
+    t.label[r] = (uint8_t)order[r];
+  }
+  if (V <= 0) return fail("dwmh_region_labels: nvox=%lld, must be > 0", (long long)V);
+  DEV_GUARD(c->device);
+  region_labels_kernel<<<c->num_sms * 8, 256, 0, (cudaStream_t)stream_>>>(p, t, seg, V);
   c->launches++;
   CU_TRY(cudaGetLastError());
   return 0;

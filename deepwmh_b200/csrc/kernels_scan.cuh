@@ -1,5 +1,5 @@
-// HBM-bound kernels of the path: masked z-score, fused norm+head+softmax, mirror/Gaussian
-// overlap-add aggregation, finalize (divide + argmax), small vector helpers.
+// HBM-bound kernels of the path: masked z-score, fused norm+head+softmax (or sigmoid), mirror/Gaussian
+// overlap-add aggregation, finalize (divide + argmax), region labels, small vector helpers.
 // Reference semantics: SURVEY.md section 8a rows a2, a11, a12 (nnU-Net v1, un-vendored).
 #pragma once
 #include "common.cuh"
@@ -103,9 +103,12 @@ __global__ void __launch_bounds__(256) zscore_fused_kernel(float* __restrict__ v
 
 // ---------------------------------------------------------------------------------------------
 // Head: InstanceNorm+LeakyReLU of the last decoder conv applied on load, 1x1x1 conv to NC = 2..8 logits
-// (seg_outputs[-1], no bias), softmax over classes (inference_apply_nonlin): l_k = sum_c w[k][c] x_c,
-// p_k = exp(l_k - max) / sum_k' exp(l_k' - max) in fp32, summed in class order.  One thread per voxel (two when
-// C == 32 and V is even), grid.y = sample.  y: [n][C/8][V][8] raw conv output; probs: [n][NC][V] fp32.
+// (seg_outputs[-1], no bias), then the model's inference_apply_nonlin: l_k = sum_c w[k][c] x_c and
+//   SIGMOID = false: softmax over classes, p_k = exp(l_k - max) / sum_k' exp(l_k' - max), summed in class order;
+//   SIGMOID = true:  one sigmoid per output (region-based models), p_k = 1 / (1 + exp(-l_k)) -- IEEE expf and division,
+//                    so exp(-l_k) = inf gives 0 and no finite logit gives NaN;
+// all in fp32.  One thread per voxel (two when C == 32 and V is even), grid.y = sample.  y: [n][C/8][V][8] raw conv
+// output; probs: [n][NC][V] fp32.
 // ---------------------------------------------------------------------------------------------
 template <int NC>
 __device__ __forceinline__ void softmax_nc(const float (&l)[NC], float (&p)[NC]) {
@@ -119,7 +122,17 @@ __device__ __forceinline__ void softmax_nc(const float (&l)[NC], float (&p)[NC])
   for (int k = 0; k < NC; ++k) p[k] = e[k] / s;
 }
 
-template <typename T, int NC>
+template <int NC, bool SIGMOID>
+__device__ __forceinline__ void head_nonlin(const float (&l)[NC], float (&p)[NC]) {
+  if constexpr (SIGMOID) {
+#pragma unroll
+    for (int k = 0; k < NC; ++k) p[k] = 1.f / (1.f + expf(-l[k]));
+  } else {
+    softmax_nc<NC>(l, p);
+  }
+}
+
+template <typename T, int NC, bool SIGMOID = false>
 __global__ void __launch_bounds__(256) head_softmax_kernel(const T* __restrict__ y, NormParams np,
                                                            const float* __restrict__ w_head,   // [NC][C]
                                                            float* __restrict__ probs, int C, int64_t V) {
@@ -175,8 +188,8 @@ __global__ void __launch_bounds__(256) head_softmax_kernel(const T* __restrict__
       }
     }
     float p[2][NC];
-    softmax_nc<NC>(l[0], p[0]);
-    softmax_nc<NC>(l[1], p[1]);
+    head_nonlin<NC, SIGMOID>(l[0], p[0]);
+    head_nonlin<NC, SIGMOID>(l[1], p[1]);
 #pragma unroll
     for (int k = 0; k < NC; ++k)
       *reinterpret_cast<float2*>(probs + ((size_t)n * NC + k) * V + 2 * v2) = make_float2(p[0][k], p[1][k]);
@@ -209,7 +222,7 @@ __global__ void __launch_bounds__(256) head_softmax_kernel(const T* __restrict__
     for (int cc = 0; cc < (C >> 3); ++cc) add_chunk(ld_stream(yp + (size_t)cc * V), cc);
   }
   float p[NC];
-  softmax_nc<NC>(l, p);
+  head_nonlin<NC, SIGMOID>(l, p);
 #pragma unroll
   for (int k = 0; k < NC; ++k) probs[((size_t)n * NC + k) * V + v] = p[k];
 }
@@ -218,9 +231,10 @@ __global__ void __launch_bounds__(256) head_softmax_kernel(const T* __restrict__
 // a11/a12  One tile: result = sum_m (1/M) * unflip_m(p_m); result *= gaussian; agg[:, tile] += result;
 // wgt[tile] += gaussian.  Same fp32 operation order as the reference, per class.  Tiles are aggregated by
 // consecutive launches on one stream, so the overlap-add is deterministic (no atomics).
-// probs: [M][NC][P] for this tile; metas[m].flip gives the mirror of sample m.
+// probs: [M][NC][P] for this tile; metas[m].flip gives the mirror of sample m.  SIGMOID: the instantiation of a
+// sigmoid-head (region-based) model.
 // ---------------------------------------------------------------------------------------------
-template <int NC>
+template <int NC, bool SIGMOID = false>
 __global__ void __launch_bounds__(256) aggregate_tile_kernel(const float* __restrict__ probs,
                                                              const SampleMeta* __restrict__ metas, int M,
                                                              const float* __restrict__ gauss,   // [P] or nullptr
@@ -248,13 +262,14 @@ __global__ void __launch_bounds__(256) aggregate_tile_kernel(const float* __rest
   const float g = gauss ? gauss[v] : 1.0f;
   const int64_t V = (int64_t)X * Y * Z;
   const int64_t dst = ((int64_t)(metas[0].ox + i) * Y + (metas[0].oy + j)) * Z + (metas[0].oz + k);
-  // agg += r * g.  Two classes round the product before the add (the reference's `*=` then `+=`); more classes add it with
-  // one rounding, as the separate kernel these counts ran on was compiled to.  The intrinsics pin both, so every class count
-  // keeps its earlier results.  With g = 1 (no Gaussian) both are the plain sum.
+  // agg += r * g.  Two classes and every sigmoid model round the product before the add (the reference's `*=` then `+=`);
+  // more softmax classes add it with one rounding, as the separate kernel these counts ran on was compiled to.  The
+  // intrinsics pin both, so every softmax class count keeps its earlier results.  With g = 1 (no Gaussian) both are the
+  // plain sum.
 #pragma unroll
   for (int c = 0; c < NC; ++c) {
     float& a = agg[(size_t)c * V + dst];
-    if constexpr (NC == 2) a = __fadd_rn(a, __fmul_rn(r[c], g));
+    if constexpr (NC == 2 || SIGMOID) a = __fadd_rn(a, __fmul_rn(r[c], g));
     else a = __fmaf_rn(r[c], g, a);
   }
   wgt[dst] += g;
@@ -363,6 +378,21 @@ __global__ void __launch_bounds__(256) argmax_kernel(const float* __restrict__ p
       if (x > best) { best = x; arg = c; }
     }
     seg[i] = (uint8_t)arg;
+  }
+}
+
+// Region labels of a sigmoid model (nnU-Net v1 with regions_class_order): seg = 0; for r in order: seg[p[r] > 0.5] =
+// label[r].  A later region overwrites an earlier one; exactly 0.5 and NaN are outside.  p [R][V] fp32.
+struct RegionTable { int n; uint8_t label[DWMH_MAX_CLASSES]; };
+
+__global__ void __launch_bounds__(256) region_labels_kernel(const float* __restrict__ p, RegionTable t, uint8_t* __restrict__ seg,
+                                                            int64_t V) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < V; i += stride) {
+    uint8_t s = 0;
+    for (int r = 0; r < t.n; ++r)
+      if (p[(size_t)r * V + i] > 0.5f) s = t.label[r];
+    seg[i] = s;
   }
 }
 

@@ -16,6 +16,9 @@ modality order of the training data), outputs `<out>/<case>.nii.gz` (uint8 label
 as upstream's predict_cases does (DESIGN §11; DeepWMH passes the flag).  Any failure raises -> non-zero exit, which is what
 `run_shell` turns into `exit(msg)` (deepwmh/utilities/external_call.py:63-72).  Flags of upstream nnUNet_predict that
 DeepWMH never passes and this path does not implement are rejected loudly rather than ignored.
+
+Besides DeepWMH's `-tr nnUNetTrainerV2`, the region-based BraTS trainer `-tr nnUNetTrainerV2BraTSRegions` is served
+(DESIGN §12): sigmoid outputs, labels by its regions_class_order, trainer folder `nnUNetTrainerV2BraTSRegions__<plans>`.
 """
 from __future__ import annotations
 
@@ -27,6 +30,12 @@ from typing import List
 
 from . import cli as _cli
 from . import postprocessing as _pp
+
+
+def served_trainers():
+    """-tr name -> trainer class.  Every other name (the BatchNorm BraTS variants among them) is refused."""
+    from . import predictor
+    return {"nnUNetTrainerV2": predictor.nnUNetTrainerV2, "nnUNetTrainerV2BraTSRegions": predictor.nnUNetTrainerV2BraTSRegions}
 
 
 def _cases_in(folder: str) -> List[str]:
@@ -70,8 +79,15 @@ def main(argv=None) -> int:
     ap.add_argument("--num_threads_nifti_save", type=int, default=2)
     args = ap.parse_args(argv)
 
-    if args.trainer_class_name != _cli.TRAINER or args.model != _cli.CONFIG or args.plans_identifier != _cli.PLANNER:
-        raise NotImplementedError("this entry point serves DeepWMH's model identity only: -tr %s -m %s -p %s" % (_cli.TRAINER, _cli.CONFIG, _cli.PLANNER))
+    trainers = served_trainers()
+    if args.trainer_class_name not in trainers or args.model != _cli.CONFIG or args.plans_identifier != _cli.PLANNER:
+        raise NotImplementedError("this entry point serves -tr %s -m %s -p %s only (got -tr %s -m %s -p %s)"
+                                  % (" | ".join(trainers), _cli.CONFIG, _cli.PLANNER, args.trainer_class_name, args.model,
+                                     args.plans_identifier))
+    trainer_class = trainers[args.trainer_class_name]
+    if args.save_softmax and trainer_class.regions_class_order is not None:
+        raise NotImplementedError("--save_softmax writes the background probability <case>_0.nii.gz; the region-based %s has no "
+                                  "background output" % args.trainer_class_name)
     if list(args.folds) != [_cli.FOLD]:
         raise NotImplementedError("only `-f all` (DeepWMH trains one model on all data, predict.py:148)")
     if args.save_npz or args.lowres_segmentations != "None" or args.mode != "normal" or args.disable_mixed_precision:
@@ -88,7 +104,7 @@ def main(argv=None) -> int:
         if len(hits) != 1:
             raise RuntimeError("cannot resolve task id %s in %s" % (task, cfg_dir))
         task = hits[0]
-    tdir = os.path.join(cfg_dir, task, "%s__%s" % (_cli.TRAINER, _cli.PLANNER))
+    tdir = os.path.join(cfg_dir, task, "%s__%s" % (args.trainer_class_name, _cli.PLANNER))
     plans_path = os.path.join(tdir, "plans.pkl")
     ckpt_path = os.path.join(tdir, _cli.FOLD, args.chk + ".model")
     for pth in (plans_path, ckpt_path):
@@ -128,8 +144,7 @@ def main(argv=None) -> int:
 
     import torch
 
-    import deepwmh_b200
-    trainer = deepwmh_b200.nnUNetTrainerV2(plans, device=0, max_batch=32 if not args.disable_tta else 16)   # CUDA_VISIBLE_DEVICES selects the GPU
+    trainer = trainer_class(plans, device=0, max_batch=32 if not args.disable_tta else 16)   # CUDA_VISIBLE_DEVICES selects the GPU
     trainer.load_checkpoint_ram(torch.load(ckpt_path, map_location="cpu", weights_only=False), False)
     if args.step_size != 0.5:
         raise NotImplementedError("--step_size other than 0.5 is not passed by DeepWMH")

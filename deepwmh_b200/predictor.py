@@ -7,9 +7,10 @@
 
 Same names, argument meaning, defaults and error behaviour as the reference's un-vendored nnunet
 fork (reached from deepwmh/main/predict.py:153-156); all arithmetic runs in libdeepwmh_b200.so
-(hand-written sm_100a CUDA).  PyTorch is used only for device memory and streams.  Combinations
-the reference supports but this path does not (non-tiled, 2-D, regions_class_order, all_in_gpu's
-fp16 buffers) raise NotImplementedError -- there is no CPU fallback by design.
+(hand-written sm_100a CUDA).  PyTorch is used only for device memory and streams.  Region-based
+models (sigmoid outputs, regions_class_order: nnUNetTrainerV2BraTSRegions) run on the same path.
+Combinations the reference supports but this path does not (non-tiled, 2-D, all_in_gpu's fp16
+buffers) raise NotImplementedError -- there is no CPU fallback by design.
 """
 from __future__ import annotations
 
@@ -23,6 +24,7 @@ from . import _lib
 from ._lib import NetDesc, check
 
 ACT_DTYPES = {"fp16": 0, "float16": 0, "half": 0, "bf16": 1, "bfloat16": 1}
+HEAD_NONLINS = {"softmax": 0, "sigmoid": 1}      # dwmh_net_desc.head_nonlin
 
 
 def _ptr(t) -> C.c_void_p:
@@ -60,9 +62,15 @@ class SegmentationNetwork:
     """The `trainer.network` object: Generic_UNet weights resident on one B200 + predict_3D."""
 
     def __init__(self, plans: Dict, device: int = 0, act_dtype: str = "fp16", max_batch: int = 8,
-                 share_workspace_with: "Optional[SegmentationNetwork]" = None):
+                 share_workspace_with: "Optional[SegmentationNetwork]" = None, inference_nonlin: str = "softmax",
+                 num_outputs: Optional[int] = None):
         """share_workspace_with: another network of the same plans on the same device whose activation buffers this one
-        borrows (k resident models of a checkpoint ensemble, dwmh_create_like); the lender must have its weights loaded."""
+        borrows (k resident models of a checkpoint ensemble, dwmh_create_like); the lender must have its weights loaded.
+        inference_nonlin: the network's inference_apply_nonlin, "softmax" over classes (nnUNetTrainerV2) or "sigmoid" per
+        output (region-based trainers).  num_outputs: channels of the last seg_outputs head; None = plans['num_classes'] + 1
+        (a region-based model has one output per region instead)."""
+        if inference_nonlin not in HEAD_NONLINS:
+            raise ValueError("inference_nonlin must be one of %s, not %r" % (sorted(HEAD_NONLINS), inference_nonlin))
         if not torch.cuda.is_available():
             raise _lib.DwmhError("deepwmh_b200 needs a CUDA device (sm_100a); no CPU fallback exists")
         self._lib = _lib.load()
@@ -70,12 +78,13 @@ class SegmentationNetwork:
         pools = [list(map(int, p)) for p in st["pool_op_kernel_sizes"]]
         kers = [list(map(int, k)) for k in st["conv_kernel_sizes"]]
         self.patch_size = tuple(int(i) for i in st["patch_size"])
-        self.num_classes = int(plans["num_classes"]) + 1
+        self.num_classes = int(num_outputs) if num_outputs is not None else int(plans["num_classes"]) + 1
         self.input_channels = int(plans["num_modalities"])
         self.device = torch.device("cuda", device)
         self.do_ds = False
         self.conv_op = "Conv3d"
-        self.inference_apply_nonlin = "softmax(dim=1)"   # fused into the head kernel
+        self.inference_nonlin = inference_nonlin
+        self.inference_apply_nonlin = "softmax(dim=1)" if inference_nonlin == "softmax" else "sigmoid"   # fused into the head kernel
         d = NetDesc()
         d.in_channels, d.num_classes = self.input_channels, self.num_classes
         d.base_num_features, d.max_num_features = int(plans["base_num_features"]), 320
@@ -92,6 +101,7 @@ class SegmentationNetwork:
                 d.conv_kernel_sizes[i][a] = k[a]
         d.act_dtype = ACT_DTYPES[act_dtype]
         d.max_batch = int(max_batch)
+        d.head_nonlin = HEAD_NONLINS[inference_nonlin]
         d.struct_size = C.sizeof(NetDesc)
         self._desc = d
         self._ctx = C.c_void_p()
@@ -168,6 +178,21 @@ class SegmentationNetwork:
         check(self._lib.dwmh_argmax(self._ctx, _ptr(softmax), int(softmax.shape[0]), _ptr(seg), seg.numel(), self._st()))
         return seg
 
+    def region_labels(self, probs: torch.Tensor, order: Sequence[int]) -> torch.Tensor:
+        """Labels uint8 [x,y,z] of a region-based model from its fp32 probabilities [R,x,y,z] on the device: 0, then for each
+        region r in order, label order[r] where probs[r] > 0.5 (later regions overwrite earlier ones)."""
+        if not (isinstance(probs, torch.Tensor) and probs.device == self.device and probs.dtype == torch.float32):
+            raise ValueError("probs must be a float32 tensor on %s" % self.device)
+        if not probs.is_contiguous() or probs.dim() < 2:
+            raise ValueError("probs must be a contiguous [regions, ...] tensor")
+        order = [int(v) for v in order]
+        if len(order) != probs.shape[0]:
+            raise ValueError("%d regions in regions_class_order, %d in probs" % (len(order), probs.shape[0]))
+        seg = torch.empty(tuple(probs.shape[1:]), dtype=torch.uint8, device=probs.device)
+        tab = (C.c_int32 * max(len(order), 1))(*order)
+        check(self._lib.dwmh_region_labels(self._ctx, _ptr(probs), len(order), tab, _ptr(seg), seg.numel(), self._st()))
+        return seg
+
     def normalize_(self, vol: torch.Tensor, seg: Optional[torch.Tensor] = None, mask_mode: int = 2, return_stats: bool = True):
         """In-place z-score of a device fp32 volume (a2).  mask_mode: 0 all, 1 seg>=0, 2 vol!=0.
         return_stats: (mean, std, count) on the host -- this synchronises the stream; False keeps the call asynchronous."""
@@ -211,10 +236,11 @@ class SegmentationNetwork:
                                         mirror_axes_mask(mirror_axes), int(bool(use_gaussian)), _ptr(agg), _ptr(wgt),
                                         int(tile_begin), int(tile_end), self._st()))
 
-    def finalize(self, agg: torch.Tensor, wgt: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor]:
-        """agg [C,X,Y,Z] / wgt [X,Y,Z] in place -> (seg uint8 [X,Y,Z], agg as the probabilities)."""
+    def finalize(self, agg: torch.Tensor, wgt: torch.Tensor, labels: bool = True) -> Tuple[Optional[torch.Tensor], torch.Tensor]:
+        """agg [C,X,Y,Z] / wgt [X,Y,Z] in place -> (seg uint8 [X,Y,Z] = argmax, agg as the probabilities); labels=False
+        skips the argmax and returns None for seg."""
         X, Y, Z = self._check_buffers(agg, wgt)
-        seg = torch.empty((X, Y, Z), dtype=torch.uint8, device=agg.device)
+        seg = torch.empty((X, Y, Z), dtype=torch.uint8, device=agg.device) if labels else None
         check(self._lib.dwmh_finalize(self._ctx, _ptr(agg), _ptr(wgt), _ptr(agg), _ptr(seg), X, Y, Z, self._st()))
         return seg, agg
 
@@ -265,7 +291,7 @@ class SegmentationNetwork:
         return len(s[0]) * len(s[1]) * len(s[2])
 
     def forward_patches(self, patches: torch.Tensor) -> torch.Tensor:
-        """softmax(Generic_UNet(x)) for x [n,M,px,py,pz] fp32 on device -> [n,C,px,py,pz] fp32."""
+        """inference_apply_nonlin(Generic_UNet(x)) for x [n,M,px,py,pz] fp32 on device -> [n,C,px,py,pz] fp32."""
         assert patches.is_cuda and patches.dtype == torch.float32 and patches.is_contiguous()
         n = patches.shape[0]
         if patches.numel() != n * self.input_channels * int(np.prod(self.patch_size)):
@@ -328,7 +354,9 @@ class SegmentationNetwork:
                    return_device_tensors: bool = False):
         """[U:SegmentationNetwork.predict_3D].  x: (M, x, y, z) numpy fp32 or CUDA tensor, M = input modalities.
         Returns (seg int64 [x,y,z], class_probabilities fp32 [classes,x,y,z]) as numpy arrays, or -- additive flag
-        return_device_tensors -- (seg uint8, probabilities fp32) as CUDA tensors without the device-to-host copies."""
+        return_device_tensors -- (seg uint8, probabilities fp32) as CUDA tensors without the device-to-host copies.
+        regions_class_order (sigmoid networks only): seg is the region rule of region_labels instead of the argmax, float32
+        as upstream returns it (uint8 with return_device_tensors)."""
         assert step_size <= 1, "step_size must be smaller than 1. Otherwise there will be a gap between consecutive predictions"
         assert len(x.shape) == 4, "data must have shape (c,x,y,z)"
         if not self._weights_loaded:
@@ -340,8 +368,11 @@ class SegmentationNetwork:
                 raise ValueError("mirror axes")
         if not use_sliding_window:
             raise NotImplementedError("only the tiled (use_sliding_window=True) branch is on DeepWMH's path")
-        if regions_class_order is not None:
-            raise NotImplementedError("regions_class_order is not used by DeepWMH")
+        if regions_class_order is not None and self.inference_nonlin != "sigmoid":
+            raise NotImplementedError("regions_class_order needs a sigmoid network (inference_nonlin='sigmoid'); no nnU-Net v1 "
+                                      "trainer pairs it with a softmax")
+        if regions_class_order is not None and len(regions_class_order) != self.num_classes:
+            raise ValueError("regions_class_order has %d entries, the network %d outputs" % (len(regions_class_order), self.num_classes))
         if patch_size is not None and tuple(int(i) for i in patch_size) != self.patch_size:
             raise NotImplementedError("patch_size must equal the plans' patch size %s" % (self.patch_size,))
         if pad_border_mode != "constant" or pad_kwargs.get("constant_values", 0) != 0:
@@ -367,11 +398,13 @@ class SegmentationNetwork:
             agg = torch.zeros((self.num_classes, X, Y, Z), dtype=torch.float32, device=self.device)
             wgt = torch.zeros((X, Y, Z), dtype=torch.float32, device=self.device)
             self.accumulate_tiles(vol, agg, wgt, step_size, do_mirroring, mirror_axes, use_gaussian)
-            seg, probs = self.finalize(agg, wgt)
+            seg, probs = self.finalize(agg, wgt, labels=regions_class_order is None)
+            if regions_class_order is not None:
+                seg = self.region_labels(probs, regions_class_order)
             sl = tuple(slicer[1:])
             if return_device_tensors:
                 return seg[sl], probs[(slice(None),) + sl]
-            seg_np = seg[sl].cpu().numpy().astype(np.int64)
+            seg_np = seg[sl].cpu().numpy().astype(np.int64 if regions_class_order is None else np.float32)
             probs_np = probs[(slice(None),) + sl].cpu().numpy()
         return seg_np, probs_np
 
@@ -379,13 +412,17 @@ class SegmentationNetwork:
 class nnUNetTrainerV2:
     """The slice of the trainer surface `predict_cases` uses [U:nnUNetTrainerV2.py], B200-backed."""
 
+    inference_nonlin = "softmax"
+    regions_class_order = None
+
     def __init__(self, plans: Dict, device: int = 0, act_dtype: str = "fp16", max_batch: int = 8,
                  exact_scipy_gaussian: bool = True, share_workspace_with: "Optional[nnUNetTrainerV2]" = None):
         self.plans = plans
         self.process_plans(plans)
         self.data_aug_params = {"do_mirror": True, "mirror_axes": (0, 1, 2)}
         self.network = SegmentationNetwork(plans, device, act_dtype, max_batch,
-                                           share_workspace_with.network if share_workspace_with is not None else None)
+                                           share_workspace_with.network if share_workspace_with is not None else None,
+                                           inference_nonlin=self.inference_nonlin, num_outputs=self.num_classes)
         if exact_scipy_gaussian:
             self.network.install_scipy_gaussian()
 
@@ -438,7 +475,7 @@ class nnUNetTrainerV2:
         self.network.eval()
         ret = self.network.predict_3D(data, do_mirroring=do_mirroring, mirror_axes=mirror_axes or (),
                                       use_sliding_window=use_sliding_window, step_size=step_size,
-                                      patch_size=self.patch_size, regions_class_order=None,
+                                      patch_size=self.patch_size, regions_class_order=self.regions_class_order,
                                       use_gaussian=use_gaussian, pad_border_mode=pad_border_mode,
                                       pad_kwargs=pad_kwargs, all_in_gpu=all_in_gpu, verbose=verbose,
                                       mixed_precision=mixed_precision, return_device_tensors=return_device_tensors)
@@ -474,3 +511,17 @@ class nnUNetTrainerV2:
                 int(bool(do_mirroring)), mirror_axes_mask(mirror_axes), int(bool(use_gaussian)),
                 sm.ctypes.data_as(C.c_void_p), sg.ctypes.data_as(C.c_void_p), net._st()))
         return sg, sm
+
+
+class nnUNetTrainerV2BraTSRegions(nnUNetTrainerV2):
+    """[U:training/network_training/competitions_with_custom_Trainers/BraTS2020/nnUNetTrainerV2BraTSRegions.py]: the BraTS
+    region trainer -- four modalities, one sigmoid output per overlapping tumour region, labels by regions_class_order.
+    Otherwise nnUNetTrainerV2 (Generic_UNet with InstanceNorm, same predict wrappers)."""
+
+    regions = {"whole tumor": (1, 2, 3), "tumor core": (2, 3), "enhancing tumor": (3,)}     # get_brats_regions()
+    regions_class_order = (1, 2, 3)
+    inference_nonlin = "sigmoid"
+
+    def process_plans(self, plans: Dict):
+        super().process_plans(plans)
+        self.num_classes = len(self.regions)      # network outputs; plans['num_classes'] stays the label count

@@ -224,7 +224,7 @@ def preprocess_test_case(network, plans: Dict, input_files: Sequence[str], force
 
 def save_segmentation_nifti_from_softmax(network, softmax, out_fname: str, properties: Dict, order: int = 1, force_separate_z=None,
                                          softmax_fname: Optional[str] = None, post3mm_fname: Optional[str] = None,
-                                         for_which_classes=None, min_valid_object_sizes=None):
+                                         for_which_classes=None, min_valid_object_sizes=None, region_class_order=None):
     """[U:inference/segmentation_export.py::save_segmentation_nifti_from_softmax]: softmax [classes, x, y, z] (ALREADY
     transposed back; CUDA tensor or numpy) -> resample back to the cropped grid (order 1, device) -> argmax (labels
     0 .. classes-1, ties to the lower class) -> paste into
@@ -233,6 +233,8 @@ def save_segmentation_nifti_from_softmax(network, softmax, out_fname: str, prope
     post3mm_fname: `remove_3mm_sparks` of the label map on the device (deepwmh/main/predict.py:19-26,158-163).
     for_which_classes / min_valid_object_sizes: a postprocessing.json (deepwmh_b200/postprocessing.py), applied on the
     device to the label file only, as upstream's predict_cases rewrites that file; the other outputs do not see it.
+    region_class_order: a region-based model's order (softmax then holds its sigmoid probabilities); the labels are the
+    region rule of SegmentationNetwork.region_labels on the resampled probabilities instead of the argmax.
     Returns the label map as written."""
     import torch
 
@@ -243,7 +245,7 @@ def save_segmentation_nifti_from_softmax(network, softmax, out_fname: str, prope
         sm = sm.to(device=network.device, dtype=torch.float32).contiguous()
         sm = resample_softmax_back_device(sm, properties["size_after_cropping"], properties["original_spacing"],
                                           properties["spacing_after_resampling"], force_separate_z, order)
-        seg = network.argmax(sm.contiguous())
+        seg = network.argmax(sm.contiguous()) if region_class_order is None else network.region_labels(sm.contiguous(), region_class_order)
         full_shape = tuple(int(v) for v in properties["original_size_of_raw_data"])
         sl = tuple(slice(b[0], b[1]) for b in properties["crop_bbox"])
         full = torch.zeros(full_shape, dtype=torch.uint8, device=network.device)

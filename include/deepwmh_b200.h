@@ -37,7 +37,8 @@ typedef struct dwmh_ctx dwmh_ctx;
  * (SURVEY.md Appendix A1/A6).  Replaces nnUNetTrainerV2.initialize_network [U]. */
 typedef struct dwmh_net_desc {
   int32_t in_channels;                        /* plans['num_modalities']: 1 .. DWMH_MAX_IN_CHANNELS  */
-  int32_t num_classes;                        /* plans['num_classes'] + 1: 2 .. DWMH_MAX_CLASSES     */
+  int32_t num_classes;                        /* network outputs, 2 .. DWMH_MAX_CLASSES: plans['num_classes'] + 1 for a
+                                               * softmax model, the number of regions for a sigmoid one          */
   int32_t base_num_features;                  /* 32                                                  */
   int32_t max_num_features;                   /* 320                                                 */
   int32_t num_pool;                           /* len(pool_op_kernel_sizes)                           */
@@ -46,18 +47,21 @@ typedef struct dwmh_net_desc {
   int32_t conv_kernel_sizes[DWMH_MAX_POOL + 1][3];     /* each entry 1 or 3                          */
   int32_t act_dtype;                          /* 0 = fp16 operands/storage (default), 1 = bf16       */
   int32_t max_batch;                          /* patch forwards per batch (multiple of the mirror count), 0 = default 8 */
+  int32_t head_nonlin;                        /* the model's inference_apply_nonlin: 0 = softmax over classes (default),
+                                               * 1 = sigmoid per output (region-based trainers, e.g. nnUNetTrainerV2BraTSRegions) */
   int32_t struct_size;                        /* MUST be sizeof(dwmh_net_desc): dwmh_create rejects any other value, so a
                                                * binding built against another layout of this struct fails loudly instead
                                                * of being read past its end                                           */
 } dwmh_net_desc;
 
 const char* dwmh_last_error(void);
-/* 101: the separate two-class argmax entry point is gone; dwmh_argmax takes two classes like any other count. */
+/* 101: the separate two-class argmax entry point is gone; dwmh_argmax takes two classes like any other count.
+ * 102: dwmh_net_desc.head_nonlin (sigmoid-head models) and dwmh_region_labels. */
 int dwmh_version(void);
 
 /* --- life cycle (replaces load_model_and_checkpoint_files + trainer.initialize(False)) ----------
- * dwmh_create fails for in_channels or num_classes outside the bounds above, and for in_channels > 1 with
- * base_num_features > 32. */
+ * dwmh_create fails for in_channels or num_classes outside the bounds above, for head_nonlin other than 0 or 1, and for
+ * in_channels > 1 with base_num_features > 32. */
 int dwmh_create(dwmh_ctx** out, int device, const dwmh_net_desc* desc);
 int dwmh_destroy(dwmh_ctx* ctx);
 /* A further model on the same device that BORROWS the activation workspaces of `parent` (k resident models of the
@@ -96,7 +100,9 @@ int dwmh_set_importance_map(dwmh_ctx* ctx, const float* map_host);
 /* --- a7/a11/a12: SegmentationNetwork.predict_3D, tiled branch -----------------------------------
  * vol_dev: normalised fp32 [M][X][Y][Z], each extent >= patch (caller pads, a10).
  * Accumulates into agg_dev fp32 [C][X][Y][Z] and wgt_dev fp32 [X][Y][Z] (caller zero-initialises):
- *   agg[:, tile] += gaussian * sum_m (1/M) unflip_m(softmax(net(flip_m(tile)))),  wgt[tile] += gaussian
+ *   agg[:, tile] += gaussian * sum_m (1/M) unflip_m(nonlin(net(flip_m(tile)))),  wgt[tile] += gaussian
+ * with nonlin the model's inference nonlinearity (softmax over classes, or a sigmoid per output for head_nonlin = 1; the
+ * latter rounds the product before the add, as the reference's `*=` then `+=` do)
  * for the tiles with linear index in [tile_begin, tile_end) in x-outer / y / z-inner order
  * (tile_end < 0 = all).  mirror_axes_mask: bit a set = axis a in mirror_axes; do_mirroring = 0 -> M = 1.
  * use_gaussian = 0 (or a single tile) -> weights of 1.  Tile-sharded multi-GPU runs reduce agg and
@@ -112,7 +118,9 @@ int dwmh_weight_map(dwmh_ctx* ctx, int32_t X, int32_t Y, int32_t Z, double step_
                     float* wgt_dev, void* stream);
 
 /* class_probabilities = agg / wgt ; seg = argmax over classes (first maximum wins).
- * softmax_dev fp32 [C][X][Y][Z] (may alias agg_dev), seg_dev uint8 [X][Y][Z] with values 0 .. C-1; either may be NULL. */
+ * softmax_dev fp32 [C][X][Y][Z] (may alias agg_dev), seg_dev uint8 [X][Y][Z] with values 0 .. C-1; either may be NULL.
+ * The same for a sigmoid-head model (upstream's regions_class_order = None); its region labels come from
+ * dwmh_region_labels on the probabilities, with seg_dev NULL here. */
 int dwmh_finalize(dwmh_ctx* ctx, const float* agg_dev, const float* wgt_dev, float* softmax_dev,
                   uint8_t* seg_dev, int32_t X, int32_t Y, int32_t Z, void* stream);
 
@@ -121,6 +129,13 @@ int dwmh_axpy(dwmh_ctx* ctx, float* acc_dev, const float* x_dev, float alpha, in
 /* seg = argmax over num_classes (1 .. 255) of softmax_dev fp32 [num_classes][nvox]; the first maximum wins (ties go to the
  * lower class, as numpy.argmax). */
 int dwmh_argmax(dwmh_ctx* ctx, const float* softmax_dev, int32_t num_classes, uint8_t* seg_dev, int64_t nvox, void* stream);
+/* Labels of a region-based model (nnU-Net v1 with regions_class_order): seg = 0, then for r = 0 .. num_regions-1 in order
+ * seg[probs[r] > 0.5] = region_class_order_host[r] -- a later region overwrites an earlier one, exactly 0.5 and NaN are
+ * outside.  probs_dev fp32 [num_regions][nvox] (the sigmoid probabilities), region_class_order_host HOST int32
+ * [num_regions], seg_dev uint8 [nvox].  Refused before any device work: a null pointer, num_regions outside
+ * 1 .. DWMH_MAX_CLASSES, a label outside 0 .. 255, nvox <= 0. */
+int dwmh_region_labels(dwmh_ctx* ctx, const float* probs_dev, int32_t num_regions, const int32_t* region_class_order_host,
+                       uint8_t* seg_dev, int64_t nvox, void* stream);
 
 /* --- SURVEY 8f-3: checkpoint ensemble with softmax masking (deepwmh/pipeline/DCNN_multistage.py:102-125,317-394).
  * dwmh_ensemble_masked_add: acc += 1 - m (1 - x) for one checkpoint's BACKGROUND probability x (the fork's
@@ -256,7 +271,9 @@ int dwmh_n4(int32_t device, const float* in_dev, int32_t X, int32_t Y, int32_t Z
 
 /* --- a6 end to end with HOST buffers (what predict_preprocessed_data_return_seg_and_softmax does):
  * raw fp32 volume [M][X][Y][Z] in host memory -> (optional z-score of every modality, mask_mode as above, <0 = skip)
- * -> tiled prediction -> host softmax fp32 [C][X][Y][Z] and seg uint8 [X][Y][Z].  H2D/D2H inside. */
+ * -> tiled prediction -> host softmax fp32 [C][X][Y][Z] and seg uint8 [X][Y][Z].  H2D/D2H inside.  The probabilities are
+ * those of the model's inference nonlinearity; seg is always the argmax (region labels: dwmh_region_labels on device
+ * buffers). */
 int dwmh_predict_volume_host(dwmh_ctx* ctx, const float* vol_host, int32_t X, int32_t Y, int32_t Z,
                              int32_t zscore_mask_mode, double step_size, int32_t do_mirroring,
                              int32_t mirror_axes_mask, int32_t use_gaussian,
@@ -270,7 +287,8 @@ int dwmh_predict_volume_host_masked(dwmh_ctx* ctx, const float* vol_host, const 
                                     float* softmax_host, uint8_t* seg_host, void* stream);
 
 /* --- test / profiling hooks ----------------------------------------------------------------------
- * Generic_UNet.forward + softmax on n patches: patches_dev fp32 [n][M][px][py][pz] -> probs_dev fp32 [n][C][px][py][pz]. */
+ * Generic_UNet.forward + the model's inference nonlinearity (softmax, or sigmoid for head_nonlin = 1) on n patches:
+ * patches_dev fp32 [n][M][px][py][pz] -> probs_dev fp32 [n][C][px][py][pz]. */
 int dwmh_forward_patches(dwmh_ctx* ctx, const float* patches_dev, int32_t n, float* probs_dev, void* stream);
 /* Copy the (normalised, activated) output of layer `layer_index` of the last forward, converted to
  * fp32 NCDHW, into out_dev (capacity in floats); dims_out = {n, c, d, h, w}.  Layer order = execution order. */
