@@ -7,6 +7,8 @@ surface (`nnUNetTrainerV2.predict_preprocessed_data_return_seg_and_softmax`,
 """
 from . import _lib  # noqa: F401
 from .plans import benchmark_plans  # noqa: F401
-from .predictor import SegmentationNetwork, nnUNetTrainerV2, nnUNetTrainerV2BraTSRegions, pad_nd_image  # noqa: F401
+from .predictor import (SegmentationNetwork, nnUNetTrainerV2, nnUNetTrainerV2BraTSRegions,  # noqa: F401
+                        nnUNetTrainerV2CascadeFullRes, pad_nd_image)
 
-__all__ = ["SegmentationNetwork", "nnUNetTrainerV2", "nnUNetTrainerV2BraTSRegions", "benchmark_plans", "pad_nd_image"]
+__all__ = ["SegmentationNetwork", "nnUNetTrainerV2", "nnUNetTrainerV2BraTSRegions", "nnUNetTrainerV2CascadeFullRes", "benchmark_plans",
+           "pad_nd_image"]

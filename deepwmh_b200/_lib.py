@@ -12,6 +12,8 @@ from . import build as _build
 DWMH_MAX_POOL = 7
 DWMH_MAX_IN_CHANNELS = 4
 DWMH_MAX_CLASSES = 8
+DWMH_NORM_CT, DWMH_NORM_CT2 = 1, 2
+DWMH_CT_WORKSPACE_BYTES = 65536
 # dwmh_layer_plan's output fields, in order (include/deepwmh_b200.h, enum DWMH_PLAN_*)
 LAYER_PLAN_FIELDS = ("kind", "kd", "sd", "sh", "sw", "KC", "KSTEPS", "CB", "ncb", "resident", "SA", "NB", "R",
                      "G", "ZB", "nzb", "tiles", "items", "grid", "xform", "s222", "act")
@@ -76,6 +78,9 @@ SYMBOLS = {
     "dwmh_s1_apply_priors": (C.c_int, [C.c_int32, _P, _P, _P, _P, C.c_int32, C.c_int64, _P]),
     "dwmh_resample_workspace": (C.c_int, [C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.POINTER(C.c_int64)]),
     "dwmh_resample": (C.c_int, [C.c_int32, _P, C.POINTER(C.c_int32), _P, C.POINTER(C.c_int32), C.c_int32, C.c_int32, C.c_int32, _P, _P]),
+    "dwmh_ct_normalize": (C.c_int, [C.c_int32, _P, _P, C.c_int64, C.c_int32, C.c_double, C.c_double, C.c_double, C.c_double,
+                                    C.POINTER(C.c_double), _P, _P]),
+    "dwmh_cascade_onehot": (C.c_int, [C.c_int32, _P, C.POINTER(C.c_int32), _P, C.POINTER(C.c_int32), C.c_int32, _P]),
     "dwmh_n4_workspace": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int64)]),
     "dwmh_n4": (C.c_int, [C.c_int32, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_int32), _P, _P, _P, _P]),
     "dwmh_predict_volume_host": (C.c_int, [_P, _P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_int32,

@@ -74,14 +74,18 @@ def _check_cases(case_names: List[str], images: List[str]):
 
 
 def predict_case(trainer, plans: Dict, in_file, out_file: str, softmax_file: str = None, post3mm_file: str = None,
-                 do_mirroring: bool = True, for_which_classes=None, min_valid_object_sizes=None):
+                 do_mirroring: bool = True, for_which_classes=None, min_valid_object_sizes=None, segs_from_prev_stage: str = None):
     """One case the way nnUNet_predict's predict_cases does it (SURVEY.md A7/A10): preprocess_patient (crop -> transpose ->
     resample -> z-score), tiled prediction, transpose back, resample back, argmax (the region rule for a trainer with a
     regions_class_order), paste back, NIfTI.  in_file: the image, or
     the list of its modality files in channel order.  Everything between the file read and the file write stays on the device.
-    for_which_classes / min_valid_object_sizes: a loaded postprocessing.json for the label file (postprocessing.py)."""
+    for_which_classes / min_valid_object_sizes: a loaded postprocessing.json for the label file (postprocessing.py).
+    segs_from_prev_stage: the previous stage's label file of a cascade's full-resolution trainer."""
     files = [in_file] if isinstance(in_file, str) else list(in_file)
-    data, _, props = trainer.preprocess_patient(files, as_numpy=False)
+    if segs_from_prev_stage is None:
+        data, _, props = trainer.preprocess_patient(files, as_numpy=False)
+    else:
+        data, _, props = trainer.preprocess_patient(files, as_numpy=False, segs_from_prev_stage=segs_from_prev_stage)
     _, softmax = trainer.predict_preprocessed_data_return_seg_and_softmax(
         data, do_mirroring=do_mirroring, mirror_axes=trainer.data_aug_params["mirror_axes"], use_sliding_window=True,
         step_size=0.5, use_gaussian=True, all_in_gpu=False, mixed_precision=True, return_device_tensors=True)

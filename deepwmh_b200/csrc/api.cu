@@ -16,6 +16,7 @@
 
 #include "common.cuh"
 #include "kernels_scan.cuh"
+#include "kernels_ct.cuh"
 #include "kernels_ccl.cuh"
 #include "kernels_conv_generic.cuh"
 #include "conv_tcgen05.cuh"
@@ -50,7 +51,7 @@ struct DevGuard {
 
 extern "C" const char* dwmh_last_error(void) { return g_err.c_str(); }
 extern "C" void dwmh_internal_set_error(const char* msg) { g_err = msg ? msg : ""; }   // for the other translation units (stage1.cu)
-extern "C" int dwmh_version(void) { return 102; }
+extern "C" int dwmh_version(void) { return 103; }
 
 // ------------------------------------------------------------------------------------------------
 // network plan
@@ -626,6 +627,68 @@ extern "C" int dwmh_zscore(dwmh_ctx* c, float* vol, const int8_t* seg, int64_t n
   if (stats_out) {
     double h[3];
     CU_TRY(cudaMemcpyAsync(h, c->zs_acc, sizeof h, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    const double cnt = h[2] > 0 ? h[2] : 1.0, m = h[0] / cnt;
+    double var = h[1] / cnt - m * m; if (var < 0) var = 0;
+    stats_out[0] = m; stats_out[1] = std::sqrt(var); stats_out[2] = h[2];
+  }
+  return 0;
+}
+
+// ------------------------------------------------------------------------------------------------
+// CT / CT2 normalisation (context-free)
+// ------------------------------------------------------------------------------------------------
+static bool finite_f32(double v) { return std::isfinite(v) && std::isfinite((float)v); }
+
+extern "C" int dwmh_ct_normalize(int32_t device, float* vol, const int8_t* seg, int64_t n, int32_t scheme, double lb, double ub,
+                                 double mean, double sd, double* stats_out, void* workspace, void* stream_) {
+  if (!vol) return fail("dwmh_ct_normalize: null vol");
+  if (n <= 0) return fail("dwmh_ct_normalize: n=%lld (must be > 0)", (long long)n);
+  if (scheme != DWMH_NORM_CT && scheme != DWMH_NORM_CT2)
+    return fail("dwmh_ct_normalize: unknown scheme %d (DWMH_NORM_CT = %d, DWMH_NORM_CT2 = %d)", scheme, DWMH_NORM_CT, DWMH_NORM_CT2);
+  if (!finite_f32(lb) || !finite_f32(ub)) return fail("dwmh_ct_normalize: lb=%g, ub=%g must be finite in fp32", lb, ub);
+  if ((float)lb > (float)ub) return fail("dwmh_ct_normalize: lb=%g > ub=%g", lb, ub);
+  if (scheme == DWMH_NORM_CT) {
+    if (!finite_f32(mean) || !finite_f32(sd)) return fail("dwmh_ct_normalize: CT mean=%g, sd=%g must be finite in fp32", mean, sd);
+    if (!((float)sd > 0.f)) return fail("dwmh_ct_normalize: CT sd=%g must be > 0 in fp32", sd);
+    if (stats_out) return fail("dwmh_ct_normalize: CT takes mean and sd from the plans; stats_out is for CT2 only");
+  } else {
+    if (!workspace) return fail("dwmh_ct_normalize: CT2 needs a workspace of DWMH_CT_WORKSPACE_BYTES");
+    if ((reinterpret_cast<uintptr_t>(vol) & 15) || (seg && (reinterpret_cast<uintptr_t>(seg) & 3)) || (reinterpret_cast<uintptr_t>(workspace) & 7))
+      return fail("dwmh_ct_normalize: CT2 buffers must be 16-byte (vol) / 4-byte (seg) / 8-byte (workspace) aligned");
+  }
+  DEV_GUARD(device);
+  cudaStream_t st = (cudaStream_t)stream_;
+  int sms = 148;
+  CU_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+  const float lbf = (float)lb, ubf = (float)ub;
+  if (scheme == DWMH_NORM_CT) {
+    const bool vec = !(reinterpret_cast<uintptr_t>(vol) & 15) && !(seg && (reinterpret_cast<uintptr_t>(seg) & 3));
+    const int64_t items = vec ? std::max<int64_t>(n >> 2, 1) : n;
+    const int grid = (int)std::min<int64_t>((items + 255) / 256, (int64_t)sms * 8);
+    if (vec) ct_normalize_kernel<true><<<grid, 256, 0, st>>>(vol, seg, n, lbf, ubf, (float)mean, (float)sd);
+    else ct_normalize_kernel<false><<<grid, 256, 0, st>>>(vol, seg, n, lbf, ubf, (float)mean, (float)sd);
+    CU_TRY(cudaGetLastError());
+    return 0;
+  }
+  // workspace: [0] barrier counter, [1..3] totals, [4 ...] one slot of three doubles per CTA
+  int per_sm = 0;
+  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ct2_fused_kernel, 256, 0));
+  if (per_sm < 1) return fail("dwmh_ct_normalize: the CT2 kernel does not fit an SM");
+  const int max_ctas = (int)((DWMH_CT_WORKSPACE_BYTES / sizeof(double) - 4) / 3);
+  int grid = std::min(sms * std::min(per_sm, 4), max_ctas);
+  unsigned long long* barrier = reinterpret_cast<unsigned long long*>(workspace);
+  double* totals = reinterpret_cast<double*>(workspace) + 1;
+  double* slots = reinterpret_cast<double*>(workspace) + 4;
+  unsigned long long target = (unsigned long long)grid;
+  CU_TRY(cudaMemsetAsync(barrier, 0, sizeof(unsigned long long), st));
+  void* args[] = {(void*)&vol, (void*)&seg, (void*)&n, (void*)&lbf, (void*)&ubf, (void*)&slots, (void*)&barrier, (void*)&target,
+                  (void*)&totals};
+  CU_TRY(cudaLaunchCooperativeKernel((const void*)ct2_fused_kernel, dim3(grid), dim3(256), args, 0, st));
+  CU_TRY(cudaGetLastError());
+  if (stats_out) {
+    double h[3];
+    CU_TRY(cudaMemcpyAsync(h, totals, sizeof h, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     const double cnt = h[2] > 0 ? h[2] : 1.0, m = h[0] / cnt;
     double var = h[1] / cnt - m * m; if (var < 0) var = 0;

@@ -193,6 +193,47 @@ __global__ void __launch_bounds__(256) rs_gather_kernel(const double* __restrict
   }
 }
 
+// The cascade's previous-stage input [U:predict.py::preprocess_save_to_queue]: resize_segmentation(labels, out shape,
+// order 1) then one-hot over classes 1 .. C-1, written straight into C-1 fp32 planes of the network input.  Per voxel and
+// class c (ascending), the order-1 resize of the 0/1 indicator of c is rs_gather_kernel's sum over the 2 x 2 x 2 taps of
+// rs_taps; a tap of value 0 adds an exact 0 and a tap of value 1 adds w0 * w1 * w2, so only the taps holding c are added,
+// in the same order.  Where that sum is >= 0.5, c is written (later classes overwrite earlier ones).  The clip to the
+// indicator's range cannot move a sum across 0.5, so it is left out.
+__global__ void __launch_bounds__(256) rs_onehot_kernel(const uint8_t* __restrict__ labels, float* __restrict__ dst, RsParams p,
+                                                        int num_classes) {
+  const int N0 = p.ax[0].n_in, N1 = p.ax[1].n_in, N2 = p.ax[2].n_in;
+  const int O0 = p.ax[0].n_out, O1 = p.ax[1].n_out, O2 = p.ax[2].n_out;
+  const int64_t V = (int64_t)O0 * O1 * O2;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; v < V; v += stride) {
+    const int o2 = (int)(v % O2), o1 = (int)((v / O2) % O1), o0 = (int)(v / ((int64_t)O2 * O1));
+    int b0, b1, b2, s0, s1, s2;
+    double w0[4], w1[4], w2[4];
+    rs_taps(p.ax[0], o0, b0, w0, s0); rs_taps(p.ax[1], o1, b1, w1, s1); rs_taps(p.ax[2], o2, b2, w2, s2);
+    uint8_t lab[2][2][2];
+#pragma unroll
+    for (int a = 0; a < 2; ++a)
+#pragma unroll
+      for (int b = 0; b < 2; ++b)
+#pragma unroll
+        for (int c = 0; c < 2; ++c)
+          lab[a][b][c] = labels[((int64_t)min(b0 + a, N0 - 1) * N1 + min(b1 + b, N1 - 1)) * N2 + min(b2 + c, N2 - 1)];
+    int out = 0;
+    for (int k = 1; k < num_classes; ++k) {
+      double t = 0.0;
+#pragma unroll
+      for (int a = 0; a < 2; ++a)
+#pragma unroll
+        for (int b = 0; b < 2; ++b)
+#pragma unroll
+          for (int c = 0; c < 2; ++c)
+            if (lab[a][b][c] == k) t = __dadd_rn(t, __dmul_rn(__dmul_rn(w0[a], w1[b]), w2[c]));
+      if (t >= 0.5) out = k;
+    }
+    for (int k = 1; k < num_classes; ++k) dst[(size_t)(k - 1) * V + v] = out == k ? 1.f : 0.f;
+  }
+}
+
 int grid_for(int device) {
   int sms = 148;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
@@ -278,6 +319,30 @@ extern "C" int dwmh_resample(int32_t device, const float* src, const int32_t in_
   p.out_mode = out_mode;
   if (order == 0) p.clip_axis = -1;
   rs_gather_kernel<<<grid, 256, 0, st>>>(coef, dst, p, range);
+  RS_CU(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int dwmh_cascade_onehot(int32_t device, const uint8_t* labels, const int32_t in_shape[3], float* dst, const int32_t out_shape[3],
+                                   int32_t num_classes, void* stream_) {
+  if (!labels || !dst || !in_shape || !out_shape) return fail("dwmh_cascade_onehot: null argument");
+  if (num_classes < 2 || num_classes > DWMH_MAX_CLASSES)
+    return fail("dwmh_cascade_onehot: num_classes=%d unsupported (2 <= num_classes <= %d)", num_classes, DWMH_MAX_CLASSES);
+  for (int a = 0; a < 3; ++a)
+    if (in_shape[a] <= 0 || out_shape[a] <= 0)
+      return fail("dwmh_cascade_onehot: empty extent on axis %d (in %d, out %d)", a, in_shape[a], out_shape[a]);
+  RsDevGuard dg(device);
+  if (!dg.ok) return fail("cudaSetDevice(%d) failed", device);
+  RsParams p;
+  for (int a = 0; a < 3; ++a) {
+    RsAxis& x = p.ax[a];
+    x.n_in = in_shape[a]; x.n_out = out_shape[a];
+    x.mode = 1; x.margin = 0;
+    x.scale = (double)in_shape[a] / (double)out_shape[a];
+  }
+  p.clip_axis = -1;
+  p.out_mode = 0;
+  rs_onehot_kernel<<<grid_for(device), 256, 0, (cudaStream_t)stream_>>>(labels, dst, p, num_classes);
   RS_CU(cudaGetLastError());
   return 0;
 }

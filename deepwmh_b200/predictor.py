@@ -63,23 +63,25 @@ class SegmentationNetwork:
 
     def __init__(self, plans: Dict, device: int = 0, act_dtype: str = "fp16", max_batch: int = 8,
                  share_workspace_with: "Optional[SegmentationNetwork]" = None, inference_nonlin: str = "softmax",
-                 num_outputs: Optional[int] = None):
+                 num_outputs: Optional[int] = None, stage: Optional[int] = None, in_channels: Optional[int] = None):
         """share_workspace_with: another network of the same plans on the same device whose activation buffers this one
         borrows (k resident models of a checkpoint ensemble, dwmh_create_like); the lender must have its weights loaded.
         inference_nonlin: the network's inference_apply_nonlin, "softmax" over classes (nnUNetTrainerV2) or "sigmoid" per
         output (region-based trainers).  num_outputs: channels of the last seg_outputs head; None = plans['num_classes'] + 1
-        (a region-based model has one output per region instead)."""
+        (a region-based model has one output per region instead).  stage: the plans_per_stage key whose network this is;
+        None = the largest (3d_fullres; 3d_lowres is the smallest).  in_channels: network inputs; None =
+        plans['num_modalities'] (a cascade's full-resolution stage adds the previous stage's classes)."""
         if inference_nonlin not in HEAD_NONLINS:
             raise ValueError("inference_nonlin must be one of %s, not %r" % (sorted(HEAD_NONLINS), inference_nonlin))
         if not torch.cuda.is_available():
             raise _lib.DwmhError("deepwmh_b200 needs a CUDA device (sm_100a); no CPU fallback exists")
         self._lib = _lib.load()
-        st = plans["plans_per_stage"][max(plans["plans_per_stage"].keys())]
+        st = plans["plans_per_stage"][max(plans["plans_per_stage"].keys()) if stage is None else stage]
         pools = [list(map(int, p)) for p in st["pool_op_kernel_sizes"]]
         kers = [list(map(int, k)) for k in st["conv_kernel_sizes"]]
         self.patch_size = tuple(int(i) for i in st["patch_size"])
         self.num_classes = int(num_outputs) if num_outputs is not None else int(plans["num_classes"]) + 1
-        self.input_channels = int(plans["num_modalities"])
+        self.input_channels = int(plans["num_modalities"]) if in_channels is None else int(in_channels)
         self.device = torch.device("cuda", device)
         self.do_ds = False
         self.conv_op = "Conv3d"
@@ -416,20 +418,26 @@ class nnUNetTrainerV2:
     regions_class_order = None
 
     def __init__(self, plans: Dict, device: int = 0, act_dtype: str = "fp16", max_batch: int = 8,
-                 exact_scipy_gaussian: bool = True, share_workspace_with: "Optional[nnUNetTrainerV2]" = None):
+                 exact_scipy_gaussian: bool = True, share_workspace_with: "Optional[nnUNetTrainerV2]" = None,
+                 stage: Optional[int] = None):
+        """stage: the plans_per_stage key to run; None = the largest (3d_fullres), the smallest is 3d_lowres."""
         self.plans = plans
+        self.stage = stage
         self.process_plans(plans)
         self.data_aug_params = {"do_mirror": True, "mirror_axes": (0, 1, 2)}
         self.network = SegmentationNetwork(plans, device, act_dtype, max_batch,
                                            share_workspace_with.network if share_workspace_with is not None else None,
-                                           inference_nonlin=self.inference_nonlin, num_outputs=self.num_classes)
+                                           inference_nonlin=self.inference_nonlin, num_outputs=self.num_classes, stage=self.stage,
+                                           in_channels=self.num_input_channels)
         if exact_scipy_gaussian:
             self.network.install_scipy_gaussian()
 
     def process_plans(self, plans: Dict):
-        stage = max(plans["plans_per_stage"].keys())
-        st = plans["plans_per_stage"][stage]
-        self.stage = stage
+        if getattr(self, "stage", None) is None:
+            self.stage = max(plans["plans_per_stage"].keys())
+        elif self.stage not in plans["plans_per_stage"]:
+            raise ValueError("stage %r is not in the plans (stages %s)" % (self.stage, sorted(plans["plans_per_stage"])))
+        st = plans["plans_per_stage"][self.stage]
         self.patch_size = np.array(st["patch_size"]).astype(int)
         self.net_num_pool_op_kernel_sizes = st["pool_op_kernel_sizes"]
         self.net_conv_kernel_sizes = st["conv_kernel_sizes"]
@@ -448,12 +456,14 @@ class nnUNetTrainerV2:
         sd = {(k[7:] if k.startswith("module.") else k): v for k, v in checkpoint["state_dict"].items()}
         self.network.load_state_dict(sd)
 
-    def preprocess_patient(self, input_files, as_numpy: bool = True):
+    def preprocess_patient(self, input_files, as_numpy: bool = True, segs_from_prev_stage: Optional[str] = None):
         """[U:nnUNetTrainer.preprocess_patient] -> (data [c, x, y, z] fp32, seg [1, x, y, z], properties): crop_to_nonzero,
-        transpose_forward, resample to the plans' spacing and z-score (the last two on the device).  as_numpy=False keeps
-        data / seg on the device (the predictor accepts CUDA tensors)."""
+        transpose_forward, resample to the spacing of this trainer's stage and normalise (the last two on the device).
+        as_numpy=False keeps data / seg on the device (the predictor accepts CUDA tensors).  segs_from_prev_stage: a cascade
+        case's previous-stage label file (preprocess.preprocess_test_case)."""
         from . import preprocess
-        d, s, props = preprocess.preprocess_test_case(self.network, self.plans, list(input_files))
+        d, s, props = preprocess.preprocess_test_case(self.network, self.plans, list(input_files), stage=self.stage,
+                                                      segs_from_prev_stage=segs_from_prev_stage)
         if as_numpy:
             return d.cpu().numpy(), s.cpu().numpy(), props
         return d, s, props
@@ -525,3 +535,27 @@ class nnUNetTrainerV2BraTSRegions(nnUNetTrainerV2):
     def process_plans(self, plans: Dict):
         super().process_plans(plans)
         self.num_classes = len(self.regions)      # network outputs; plans['num_classes'] stays the label count
+
+
+class nnUNetTrainerV2CascadeFullRes(nnUNetTrainerV2):
+    """[U:training/network_training/nnUNetTrainerV2_CascadeFullRes.py] the full-resolution stage of nnU-Net's cascade: the
+    largest plans stage, with the 3d_lowres stage's labels as C-1 one-hot input channels after the M modalities
+    (preprocess_patient's segs_from_prev_stage).  Otherwise nnUNetTrainerV2."""
+
+    @staticmethod
+    def input_channels(plans: Dict) -> int:
+        """num_modalities + num_classes - 1; raises NotImplementedError above DWMH_MAX_IN_CHANNELS (before any GPU work)."""
+        n = int(plans["num_modalities"]) + int(plans["num_classes"])
+        if n > _lib.DWMH_MAX_IN_CHANNELS:
+            raise NotImplementedError("the cascade's full-resolution network takes num_modalities + num_classes - 1 = %d input "
+                                      "channels; at most DWMH_MAX_IN_CHANNELS = %d are supported" % (n, _lib.DWMH_MAX_IN_CHANNELS))
+        return n
+
+    def process_plans(self, plans: Dict):
+        super().process_plans(plans)
+        self.num_input_channels = self.input_channels(plans)
+
+    def preprocess_patient(self, input_files, as_numpy: bool = True, segs_from_prev_stage: Optional[str] = None):
+        if segs_from_prev_stage is None:
+            raise ValueError("the cascade's full-resolution stage needs the previous stage's segmentation (segs_from_prev_stage)")
+        return super().preprocess_patient(input_files, as_numpy, segs_from_prev_stage)

@@ -11,6 +11,7 @@ Restates, for DeepWMH's single modality and for models with up to four, what nnU
 """
 from __future__ import annotations
 
+import os
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -166,24 +167,126 @@ def read_modalities(input_files: Sequence[str]):
     return np.ascontiguousarray(np.stack(vols)).astype(np.float32), hdr0
 
 
-def preprocess_test_case(network, plans: Dict, input_files: Sequence[str], force_separate_z=None):
+NORMALIZATION_SCHEMES = ("nonCT", "CT", "CT2", "noNorm")
+
+
+def normalization_schemes(plans: Dict) -> List[Tuple[str, Optional[Dict[str, float]]]]:
+    """[U:GenericPreprocessor.resample_and_normalize] each modality's scheme and, for CT / CT2, its constants from
+    plans['dataset_properties']['intensityproperties'][c] as floats.  Raises NotImplementedError for a scheme other than
+    nonCT, CT, CT2 or noNorm and for a CT / CT2 modality whose plans lack one of the constants; ValueError for constants
+    the CT kernels refuse (non-finite, lb > ub, sd <= 0).  Reads nothing but the plans."""
+    M = int(plans.get("num_modalities", 1))
+    schemes = plans.get("normalization_schemes") or {}
+    props = (plans.get("dataset_properties") or {}).get("intensityproperties") or {}
+    out = []
+    for m in range(M):
+        scheme = schemes.get(m, "nonCT")
+        if scheme not in NORMALIZATION_SCHEMES:
+            raise NotImplementedError("normalization scheme %r of modality %d: nnU-Net's %s are implemented"
+                                      % (scheme, m, ", ".join(NORMALIZATION_SCHEMES)))
+        if scheme not in ("CT", "CT2"):
+            out.append((scheme, None))
+            continue
+        keys = ("percentile_00_5", "percentile_99_5") + (("mean", "sd") if scheme == "CT" else ())
+        ip = props.get(m)
+        missing = [k for k in keys if ip is None or k not in ip]
+        if missing:
+            raise NotImplementedError("normalization scheme %r of modality %d needs plans['dataset_properties']['intensityproperties'][%d]"
+                                      "[%s]; these plans lack it" % (scheme, m, m, "], [".join(repr(k) for k in missing)))
+        c = {k: float(ip[k]) for k in keys}
+        with np.errstate(over="ignore"):
+            f32 = {k: np.float32(v) for k, v in c.items()}
+        if not all(np.isfinite(v) for v in f32.values()) or f32["percentile_00_5"] > f32["percentile_99_5"]:
+            raise ValueError("intensityproperties[%d] of scheme %r: %s (finite in float32, percentile_00_5 <= percentile_99_5)"
+                             % (m, scheme, c))
+        if scheme == "CT" and not f32["sd"] > 0:
+            raise ValueError("intensityproperties[%d]['sd'] = %r: the CT scheme divides by it" % (m, c["sd"]))
+        out.append((scheme, c))
+    return out
+
+
+def ct_normalize_device(vol, seg, scheme: str, constants: Dict[str, float]):
+    """nnU-Net's CT or CT2 scheme in place on one fp32 CUDA volume (dwmh_ct_normalize); seg: int8 crop mask (zeroed where
+    < 0) or None.  Returns CT2's (mean, sd, mask count) -- which synchronises the stream -- and None for CT."""
+    import ctypes as C
+
+    import torch
+
+    from . import _lib
+    lib = _lib.load()
+    assert vol.is_cuda and vol.dtype == torch.float32 and vol.is_contiguous()
+    assert seg is None or (seg.dtype == torch.int8 and seg.is_contiguous() and seg.numel() == vol.numel())
+    ct2 = scheme == "CT2"
+    code = _lib.DWMH_NORM_CT2 if ct2 else _lib.DWMH_NORM_CT
+    stats = (C.c_double * 3)() if ct2 else None
+    with torch.cuda.device(vol.device):
+        ws = torch.empty(_lib.DWMH_CT_WORKSPACE_BYTES, dtype=torch.uint8, device=vol.device) if ct2 else None
+        _lib.check(lib.dwmh_ct_normalize(vol.device.index, C.c_void_p(vol.data_ptr()), C.c_void_p(seg.data_ptr() if seg is not None else 0),
+                                         vol.numel(), code, constants["percentile_00_5"], constants["percentile_99_5"],
+                                         constants.get("mean", 0.0), constants.get("sd", 1.0), stats,
+                                         C.c_void_p(ws.data_ptr() if ws is not None else 0),
+                                         C.c_void_p(torch.cuda.current_stream(vol.device).cuda_stream)))
+    return tuple(stats) if ct2 else None
+
+
+def cascade_onehot_device(labels, out, num_classes: int):
+    """The cascade's previous-stage channels (dwmh_cascade_onehot): uint8 CUDA labels [x, y, z] -> resize_segmentation(order
+    1) onto out's grid -> one-hot over classes 1 .. num_classes-1 written into out, fp32 CUDA [num_classes-1, X, Y, Z]."""
+    import ctypes as C
+
+    import torch
+
+    from . import _lib
+    lib = _lib.load()
+    assert labels.is_cuda and labels.dtype == torch.uint8 and labels.dim() == 3
+    assert out.is_cuda and out.dtype == torch.float32 and out.is_contiguous() and out.dim() == 4 and out.shape[0] == num_classes - 1
+    labels = labels.contiguous()
+    ins = (C.c_int32 * 3)(*labels.shape)
+    outs = (C.c_int32 * 3)(*out.shape[1:])
+    with torch.cuda.device(out.device):
+        _lib.check(lib.dwmh_cascade_onehot(out.device.index, C.c_void_p(labels.data_ptr()), ins, C.c_void_p(out.data_ptr()), outs,
+                                           int(num_classes), C.c_void_p(torch.cuda.current_stream(out.device).cuda_stream)))
+    return out
+
+
+def read_prev_stage_labels(label_file: str, image_shape: Sequence[int], num_classes: int) -> np.ndarray:
+    """[U:inference/predict.py::preprocess_save_to_queue] the previous stage's label map of a cascade case in SimpleITK
+    axis order (z, y, x), uint8.  Its NIfTI shape must be image_shape (the first modality file's) and its values labels
+    0 .. num_classes-1."""
+    from . import nifti
+    if not os.path.isfile(label_file):
+        raise RuntimeError("the previous stage's segmentation %s does not exist" % label_file)
+    lab, _ = nifti.read_nifti(label_file)
+    if tuple(lab.shape) != tuple(image_shape):
+        raise ValueError("the previous stage's segmentation %s has shape %s, the case's images %s"
+                         % (label_file, tuple(lab.shape), tuple(image_shape)))
+    bad = ~np.isin(lab, np.arange(num_classes))
+    if bad.any():
+        raise ValueError("the previous stage's segmentation %s holds values %s outside the labels 0 .. %d of the model"
+                         % (label_file, ", ".join("%g" % v for v in np.unique(lab[bad])[:8]), num_classes - 1))
+    return np.ascontiguousarray(np.transpose(lab, (2, 1, 0))).astype(np.uint8)
+
+
+def preprocess_test_case(network, plans: Dict, input_files: Sequence[str], force_separate_z=None, stage=None,
+                         segs_from_prev_stage: Optional[str] = None):
     """[U:GenericPreprocessor.preprocess_test_case] for M = plans['num_modalities'] modalities (`<case>_0000 ...`; DeepWMH: one
     FLAIR): read (SimpleITK axis order z, y, x) -> crop_to_nonzero (nonzero mask over all modalities, holes filled) ->
-    transpose_forward -> NaN -> 0 -> resample every modality to the plans' spacing (device) -> z-score of every modality with
-    its own use_mask_for_norm (device).  Only the non-CT scheme exists here.  Returns (data fp32 CUDA [M, x, y, z],
-    seg int8 CUDA [1, x, y, z], properties)."""
+    transpose_forward -> NaN -> 0 -> resample every modality to the spacing of plans stage `stage` (default: the largest
+    key; device) -> normalise every modality by its scheme with its own use_mask_for_norm (device): nonCT (z-score), CT, CT2
+    or noNorm (normalization_schemes).  segs_from_prev_stage: a 3d_cascade_fullres case's previous-stage label file
+    (read_prev_stage_labels): after transpose_forward, resize_segmentation(order 1) of the UNCROPPED map onto the cropped,
+    resampled grid, one-hot over classes 1 .. C-1, appended after the M modalities without normalisation.  Returns (data
+    fp32 CUDA [M (+ C-1), x, y, z], seg int8 CUDA [1, x, y, z], properties)."""
     import torch
 
     M = int(plans.get("num_modalities", 1))
     if len(input_files) != M:
         raise ValueError("the model takes %d modalities; got %d input files" % (M, len(input_files)))
-    schemes = plans.get("normalization_schemes") or {}
-    for m in range(M):
-        if schemes.get(m, "nonCT") != "nonCT":
-            raise NotImplementedError("normalization scheme %r of modality %d: only nnU-Net's non-CT z-score is implemented"
-                                      % (schemes.get(m), m))
+    norm = normalization_schemes(plans)
+    stage = max(plans["plans_per_stage"].keys()) if stage is None else stage
+    num_classes = int(plans["num_classes"]) + 1
     data, hdr = read_modalities(input_files)
-    stage = max(plans["plans_per_stage"].keys())
+    prev = read_prev_stage_labels(segs_from_prev_stage, hdr["shape"], num_classes) if segs_from_prev_stage is not None else None
     target_spacing = np.array(plans["plans_per_stage"][stage]["current_spacing"], dtype=np.float64)
     tf = list(plans.get("transpose_forward", [0, 1, 2]))
     props = {"original_size_of_raw_data": np.array(data.shape[1:]), "original_spacing": np.array(hdr["spacing"][::-1], dtype=np.float64),
@@ -198,6 +301,18 @@ def preprocess_test_case(network, plans: Dict, input_files: Sequence[str], force
     original_spacing_transposed = props["original_spacing"][tf]
     mask_for_norm = plans.get("use_mask_for_norm", {0: False})
     use_mask = [bool(mask_for_norm[m]) for m in range(M)]
+    case = os.path.basename(input_files[0])
+
+    def normalize(v, mask, m):
+        scheme, constants = norm[m]
+        if scheme == "nonCT":
+            network.normalize_(v, mask if use_mask[m] else None, 1 if use_mask[m] else 0, return_stats=False)
+        elif scheme in ("CT", "CT2"):
+            stats = ct_normalize_device(v, mask if use_mask[m] else None, scheme, constants)
+            if stats is not None and stats[2] == 0:
+                raise ValueError("%s, modality %d: no voxel lies strictly between the CT2 bounds %r and %r, so the scheme has no "
+                                 "mean or standard deviation" % (case, m, constants["percentile_00_5"], constants["percentile_99_5"]))
+
     with torch.cuda.device(network.device):
         d = torch.from_numpy(cropped).to(network.device)
         sg = torch.from_numpy(seg).to(network.device)
@@ -207,7 +322,7 @@ def preprocess_test_case(network, plans: Dict, input_files: Sequence[str], force
         props["use_nonzero_mask_for_norm"] = {m: use_mask[m] for m in range(M)}
         if M == 1:
             v = d[0].contiguous()
-            network.normalize_(v, sg[0].contiguous() if use_mask[0] else None, 1 if use_mask[0] else 0, return_stats=False)
+            normalize(v, sg[0].contiguous(), 0)
             d = v[None]
         else:
             d = d.contiguous()
@@ -216,9 +331,15 @@ def preprocess_test_case(network, plans: Dict, input_files: Sequence[str], force
             chans = []
             for m in range(M):
                 v = d[m].clone() if d[0].numel() % 4 else d[m]
-                network.normalize_(v, mask if use_mask[m] else None, 1 if use_mask[m] else 0, return_stats=False)
+                normalize(v, mask, m)
                 chans.append(v)
             d = torch.stack(chans) if d[0].numel() % 4 else d
+        if prev is not None:
+            x = torch.empty((M + num_classes - 1,) + tuple(d.shape[1:]), dtype=torch.float32, device=network.device)
+            x[:M] = d
+            labels = torch.from_numpy(np.ascontiguousarray(prev.transpose(tf))).to(network.device)
+            cascade_onehot_device(labels, x[M:], num_classes)
+            d = x
     return d, sg, props
 
 

@@ -258,6 +258,34 @@ int dwmh_resample_workspace(const int32_t in_shape[3], int32_t order, int32_t se
 int dwmh_resample(int32_t device, const float* src_dev, const int32_t in_shape[3], void* dst_dev, const int32_t out_shape[3],
                   int32_t order, int32_t separate_axis, int32_t out_mode, void* workspace_dev, void* stream);
 
+/* --- nnU-Net's CT intensity normalisation [U:GenericPreprocessor.resample_and_normalize] of one modality, in place on the
+ * device, context-free.  vol_dev fp32 [n]; lb / ub = intensityproperties' percentile_00_5 / percentile_99_5.  Every constant
+ * is rounded to fp32 and the arithmetic is fp32 with IEEE division:
+ *   DWMH_NORM_CT:  x = (clip(x, lb, ub) - mean) / sd, mean / sd from the plans (> 0).  No synchronisation; any alignment
+ *                  (128-bit accesses when vol is 16-byte and seg 4-byte aligned).  stats_host must be NULL.
+ *   DWMH_NORM_CT2: mask = lb < x < ub on the unclipped values; x = (clip(x, lb, ub) - mn) / sd with mn / sd the mean and
+ *                  population std of x over the mask, accumulated in fp64 (deterministic, one cooperative launch; mean / sd
+ *                  are ignored).  vol 16-byte, seg 4-byte aligned; workspace_dev: DWMH_CT_WORKSPACE_BYTES of 8-byte aligned
+ *                  device memory, not shared with a call in flight.  stats_host (may be NULL) = {mn, sd, mask count} in fp64,
+ *                  which synchronises the stream; an empty mask leaves NaN in vol and a count of 0.
+ * seg_dev (may be NULL): int8 crop mask [n]; x = 0 where seg < 0 (use_mask_for_norm).  Refused before any device work: a
+ * null vol, n <= 0, another scheme, a non-finite lb / ub (or, for CT, mean / sd), lb > ub, sd <= 0 for CT.
+ * "noNorm" needs no call; "nonCT" is dwmh_zscore.  The host-buffer calls (dwmh_predict_volume_host*) normalise with the
+ * z-score only. */
+#define DWMH_NORM_CT 1
+#define DWMH_NORM_CT2 2
+#define DWMH_CT_WORKSPACE_BYTES 65536
+int dwmh_ct_normalize(int32_t device, float* vol_dev, const int8_t* seg_dev, int64_t n, int32_t scheme, double lb, double ub,
+                      double mean, double sd, double* stats_host, void* workspace_dev, void* stream);
+
+/* --- The 3d_cascade_fullres input [U:inference/predict.py::preprocess_save_to_queue], context-free: labels_dev uint8
+ * [in_shape] (the previous stage's labels after transpose_forward, values 0 .. num_classes-1) -> resize_segmentation(labels,
+ * out_shape, order=1) -> one-hot over classes 1 .. num_classes-1 as fp32 0 / 1 planes dst_dev [num_classes-1][out_shape]
+ * (the network input's channels after the modalities).  Bit-exact: the order-1 taps of dwmh_resample in fp64.  Refused
+ * before any device work: a null pointer, an extent <= 0, num_classes outside 2 .. DWMH_MAX_CLASSES. */
+int dwmh_cascade_onehot(int32_t device, const uint8_t* labels_dev, const int32_t in_shape[3], float* dst_dev,
+                        const int32_t out_shape[3], int32_t num_classes, void* stream);
+
 /* --- N4 bias-field correction (the `N4BiasFieldCorrection -d 3 -c [50x50x50x50,0.0] -s 2` step of DeepWMH_predict,
  * deepwmh/main/predict.py:117-126) on the device, context-free.  Restated from Tustison et al. 2010 with 200 bins, FWHM 0.15,
  * Wiener noise 0.01, cubic B-splines on an initial 1 x 1 x 1 mesh doubled per level, convergence threshold 0
