@@ -138,6 +138,17 @@ def check(rc: int):
         raise DwmhError(msg.decode() if msg else f"libdeepwmh_b200 error {rc}")
 
 
+def ptr(t) -> C.c_void_p:
+    """Device address of a tensor's data; None gives a null pointer."""
+    return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
+
+
+def stream(device=None) -> C.c_void_p:
+    """The caller's current stream on `device` (a stream handle is only valid on its own device)."""
+    import torch      # here, so that this module imports without torch's CUDA runtime
+    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
+
+
 def compute_steps(patch, image, step_size):
     """_compute_steps_for_sliding_window through the C ABI (host only, no GPU needed)."""
     lib = load()

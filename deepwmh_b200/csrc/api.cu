@@ -5,7 +5,6 @@
 #include <algorithm>
 #include <array>
 #include <cmath>
-#include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -14,6 +13,7 @@
 #include <type_traits>
 #include <vector>
 
+#include "host.cuh"
 #include "common.cuh"
 #include "kernels_scan.cuh"
 #include "kernels_ct.cuh"
@@ -23,34 +23,7 @@
 
 using namespace dwmh;
 
-// ------------------------------------------------------------------------------------------------
-// error plumbing
-// ------------------------------------------------------------------------------------------------
-static thread_local std::string g_err;
-static int fail(const char* fmt, ...) {
-  char buf[1024];
-  va_list ap; va_start(ap, fmt); vsnprintf(buf, sizeof buf, fmt, ap); va_end(ap);
-  g_err = buf;
-  return 1;
-}
-#define CU_TRY(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) \
-  return fail("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e__), __FILE__, __LINE__); } while (0)
-#define DW_TRY(expr) do { int r__ = (expr); if (r__) return r__; } while (0)
-
-// Entry points run on the context's device and leave the caller's current device as they found it.
-struct DevGuard {
-  int prev = -1; bool ok = false;
-  explicit DevGuard(int dev) {
-    if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
-    ok = (prev == dev) || cudaSetDevice(dev) == cudaSuccess;
-    if (prev == dev) prev = -1;
-  }
-  ~DevGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
-#define DEV_GUARD(dev) DevGuard dev_guard__(dev); if (!dev_guard__.ok) return fail("cudaSetDevice(%d) failed", (int)(dev))
-
 extern "C" const char* dwmh_last_error(void) { return g_err.c_str(); }
-extern "C" void dwmh_internal_set_error(const char* msg) { g_err = msg ? msg : ""; }   // for the other translation units (stage1.cu)
 extern "C" int dwmh_version(void) { return 103; }
 
 // ------------------------------------------------------------------------------------------------
@@ -369,14 +342,6 @@ static float round_act(float v, bool bf16) {
   return bf16 ? __bfloat162float(__float2bfloat16_rn(v)) : __half2float(__float2half_rn(v));
 }
 
-template <typename V>
-static int upload(V** dst, const std::vector<V>& src) {
-  if (*dst) { cudaFree(*dst); *dst = nullptr; }
-  CU_TRY(cudaMalloc((void**)dst, src.size() * sizeof(V)));
-  CU_TRY(cudaMemcpy(*dst, src.data(), src.size() * sizeof(V), cudaMemcpyHostToDevice));
-  return 0;
-}
-
 extern "C" int dwmh_commit_weights(dwmh_ctx* c) {
   if (!c) return fail("null ctx");
   DEV_GUARD(c->device);
@@ -595,8 +560,28 @@ extern "C" int dwmh_gaussian_map(const int32_t patch[3], double sigma_scale, flo
 }
 
 // ------------------------------------------------------------------------------------------------
-// a2 z-score
+// a2 z-score, CT2: cooperative statistics kernels (grid_ordered_totals)
 // ------------------------------------------------------------------------------------------------
+// Grid of one cooperative launch of `kernel` (256 threads) on `device`: every CTA must be resident at once, at most 4 per SM.
+static int coop_grid(const void* kernel, int device, const char* what, int* grid) {
+  int per_sm = 0;
+  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, 256, 0));
+  if (per_sm < 1) return fail("%s does not fit an SM", what);
+  *grid = sm_count(device) * std::min(per_sm, 4);
+  return 0;
+}
+
+// Waits for `st` and turns the kernel's {sum, sum of squares, count} totals into {mean, population std, count}.
+static int read_stats(const double* totals, double* stats_out, cudaStream_t st) {
+  double h[3];
+  CU_TRY(cudaMemcpyAsync(h, totals, sizeof h, cudaMemcpyDeviceToHost, st));
+  CU_TRY(cudaStreamSynchronize(st));
+  const double cnt = h[2] > 0 ? h[2] : 1.0, m = h[0] / cnt;
+  double var = h[1] / cnt - m * m; if (var < 0) var = 0;
+  stats_out[0] = m; stats_out[1] = std::sqrt(var); stats_out[2] = h[2];
+  return 0;
+}
+
 extern "C" int dwmh_zscore(dwmh_ctx* c, float* vol, const int8_t* seg, int64_t n, int32_t mask_mode, double* stats_out, void* stream_) {
   if (!c || !vol) return fail("dwmh_zscore: null argument");
   if (mask_mode < 0 || mask_mode > 2) return fail("dwmh_zscore: mask_mode %d", mask_mode);
@@ -605,11 +590,7 @@ extern "C" int dwmh_zscore(dwmh_ctx* c, float* vol, const int8_t* seg, int64_t n
   cudaStream_t st = (cudaStream_t)stream_;
   DEV_GUARD(c->device);
   if (!c->zs_acc) {
-    // one cooperative launch: every CTA must be resident at once
-    int per_sm = 0;
-    CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, zscore_fused_kernel, 256, 0));
-    if (per_sm < 1) return fail("dwmh_zscore: the fused kernel does not fit an SM");
-    c->zs_grid = c->num_sms * std::min(per_sm, 4);
+    DW_TRY(coop_grid((const void*)zscore_fused_kernel, c->device, "dwmh_zscore: the fused kernel", &c->zs_grid));
     CU_TRY(cudaMalloc((void**)&c->zs_acc, (4 + 3 * (size_t)c->zs_grid) * sizeof(double)));
     CU_TRY(cudaMalloc((void**)&c->zs_barrier, sizeof(unsigned long long)));
     CU_TRY(cudaMemset(c->zs_barrier, 0, sizeof(unsigned long long)));
@@ -624,14 +605,7 @@ extern "C" int dwmh_zscore(dwmh_ctx* c, float* vol, const int8_t* seg, int64_t n
   }
   c->launches += 1;
   CU_TRY(cudaGetLastError());
-  if (stats_out) {
-    double h[3];
-    CU_TRY(cudaMemcpyAsync(h, c->zs_acc, sizeof h, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaStreamSynchronize(st));
-    const double cnt = h[2] > 0 ? h[2] : 1.0, m = h[0] / cnt;
-    double var = h[1] / cnt - m * m; if (var < 0) var = 0;
-    stats_out[0] = m; stats_out[1] = std::sqrt(var); stats_out[2] = h[2];
-  }
+  if (stats_out) DW_TRY(read_stats(c->zs_acc, stats_out, st));
   return 0;
 }
 
@@ -659,24 +633,21 @@ extern "C" int dwmh_ct_normalize(int32_t device, float* vol, const int8_t* seg, 
   }
   DEV_GUARD(device);
   cudaStream_t st = (cudaStream_t)stream_;
-  int sms = 148;
-  CU_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
   const float lbf = (float)lb, ubf = (float)ub;
   if (scheme == DWMH_NORM_CT) {
     const bool vec = !(reinterpret_cast<uintptr_t>(vol) & 15) && !(seg && (reinterpret_cast<uintptr_t>(seg) & 3));
     const int64_t items = vec ? std::max<int64_t>(n >> 2, 1) : n;
-    const int grid = (int)std::min<int64_t>((items + 255) / 256, (int64_t)sms * 8);
+    const int grid = (int)std::min<int64_t>((items + 255) / 256, (int64_t)sm_count(device) * 8);
     if (vec) ct_normalize_kernel<true><<<grid, 256, 0, st>>>(vol, seg, n, lbf, ubf, (float)mean, (float)sd);
     else ct_normalize_kernel<false><<<grid, 256, 0, st>>>(vol, seg, n, lbf, ubf, (float)mean, (float)sd);
     CU_TRY(cudaGetLastError());
     return 0;
   }
   // workspace: [0] barrier counter, [1..3] totals, [4 ...] one slot of three doubles per CTA
-  int per_sm = 0;
-  CU_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ct2_fused_kernel, 256, 0));
-  if (per_sm < 1) return fail("dwmh_ct_normalize: the CT2 kernel does not fit an SM");
   const int max_ctas = (int)((DWMH_CT_WORKSPACE_BYTES / sizeof(double) - 4) / 3);
-  int grid = std::min(sms * std::min(per_sm, 4), max_ctas);
+  int grid = 0;
+  DW_TRY(coop_grid((const void*)ct2_fused_kernel, device, "dwmh_ct_normalize: the CT2 kernel", &grid));
+  grid = std::min(grid, max_ctas);
   unsigned long long* barrier = reinterpret_cast<unsigned long long*>(workspace);
   double* totals = reinterpret_cast<double*>(workspace) + 1;
   double* slots = reinterpret_cast<double*>(workspace) + 4;
@@ -686,14 +657,7 @@ extern "C" int dwmh_ct_normalize(int32_t device, float* vol, const int8_t* seg, 
                   (void*)&totals};
   CU_TRY(cudaLaunchCooperativeKernel((const void*)ct2_fused_kernel, dim3(grid), dim3(256), args, 0, st));
   CU_TRY(cudaGetLastError());
-  if (stats_out) {
-    double h[3];
-    CU_TRY(cudaMemcpyAsync(h, totals, sizeof h, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaStreamSynchronize(st));
-    const double cnt = h[2] > 0 ? h[2] : 1.0, m = h[0] / cnt;
-    double var = h[1] / cnt - m * m; if (var < 0) var = 0;
-    stats_out[0] = m; stats_out[1] = std::sqrt(var); stats_out[2] = h[2];
-  }
+  if (stats_out) DW_TRY(read_stats(totals, stats_out, st));
   return 0;
 }
 

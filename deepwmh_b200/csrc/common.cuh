@@ -56,6 +56,48 @@ __device__ __forceinline__ double warp_sum_d(double v) {
   return v;
 }
 
+// Ordered grid reduction of the cooperative statistics kernels (256 threads, every CTA resident) over each thread's
+// (s, ss, cnt).  Every CTA leaves its {sum, sum of squares, count} in its slot (slots: [gridDim.x][3] doubles), arrives at
+// `barrier` and waits until the counter reaches `target`; warp 0 then adds the slots in index order -- deterministic, no
+// atomics on the data, the same totals in every CTA.  Returns the totals, in shared memory; out_stats (may be null)
+// receives them from CTA 0.
+__device__ __forceinline__ const double* grid_ordered_totals(double s, double ss, double cnt, double* __restrict__ slots,
+                                                             unsigned long long* __restrict__ barrier, unsigned long long target,
+                                                             double* __restrict__ out_stats) {
+  s = warp_sum_d(s); ss = warp_sum_d(ss); cnt = warp_sum_d(cnt);
+  __shared__ double sh[3][8];
+  __shared__ double tot[3];
+  const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
+  if (l == 0) { sh[0][w] = s; sh[1][w] = ss; sh[2][w] = cnt; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int k = 1; k < 8; ++k) { sh[0][0] += sh[0][k]; sh[1][0] += sh[1][k]; sh[2][0] += sh[2][k]; }
+    double* my = slots + (size_t)blockIdx.x * 3;
+    my[0] = sh[0][0]; my[1] = sh[1][0]; my[2] = sh[2][0];
+    __threadfence();
+    atomicAdd(barrier, 1ull);
+    while (*reinterpret_cast<volatile unsigned long long*>(barrier) < target) { }
+    __threadfence();
+  }
+  __syncthreads();
+  if (w == 0) {      // ordered total: lane l adds slots l, l + 32, ...; the 32 lane sums are combined in lane order
+    double a = 0.0, b = 0.0, c = 0.0;
+    const volatile double* vs = slots;
+    for (int k = l; k < (int)gridDim.x; k += 32) { a += vs[3 * k]; b += vs[3 * k + 1]; c += vs[3 * k + 2]; }
+    for (int k = 0; k < 32; ++k) {
+      const double ak = __shfl_sync(0xffffffffu, a, k), bk = __shfl_sync(0xffffffffu, b, k), ck = __shfl_sync(0xffffffffu, c, k);
+      if (l == 0) { if (k == 0) { tot[0] = ak; tot[1] = bk; tot[2] = ck; } else { tot[0] += ak; tot[1] += bk; tot[2] += ck; } }
+    }
+  }
+  __syncthreads();
+  if (out_stats && blockIdx.x == 0 && threadIdx.x < 3) out_stats[threadIdx.x] = tot[threadIdx.x];
+  return tot;
+}
+
+// order-preserving float <-> unsigned key (atomicMin / atomicMax on floats)
+__device__ __forceinline__ unsigned float_key(float f) { const unsigned u = __float_as_uint(f); return (u & 0x80000000u) ? ~u : (u | 0x80000000u); }
+__device__ __forceinline__ float key_float(unsigned k) { return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k); }
+
 __device__ __forceinline__ float lrelu(float v) { return v > 0.f ? v : 0.01f * v; }
 
 // streaming 128-bit accesses that do not pollute L1

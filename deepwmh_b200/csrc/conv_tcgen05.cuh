@@ -33,6 +33,7 @@
 #include <type_traits>
 #include <vector>
 #include "common.cuh"
+#include "host.cuh"
 #include "tc_primitives.cuh"
 
 namespace dwmh {
@@ -1169,7 +1170,7 @@ struct TcLayer {
   bool map_bf16 = false;
   bool xform_ok = false;          // layer shape supports norm-on-load of its (single) input: plain stride-1, 32-channel chunks, resident weights
   CUtensorMap tm0, tm1;
-  void* wpack = nullptr;
+  uint16_t* wpack = nullptr;      // packed fp16 / bf16 weights
   TcKParams kp{};
   size_t smem_bytes = 0;
 };
@@ -1381,8 +1382,7 @@ inline int tc_prepare(TcLayer& t, const std::vector<float>& w, int c0, int c1, i
                   tile[((size_t)k8 * kp.jmax * CB + (size_t)r * CB + co_) * 8 + e] = tc_to_bits(v, bf16);
                 }
         }
-  if (cudaMalloc(&t.wpack, pk.size() * 2) != cudaSuccess) { *why = "cudaMalloc(wpack) failed"; return 1; }
-  if (cudaMemcpy(t.wpack, pk.data(), pk.size() * 2, cudaMemcpyHostToDevice) != cudaSuccess) { *why = "cudaMemcpy(wpack) failed"; return 1; }
+  if (upload(&t.wpack, pk)) { *why = g_err; return 1; }
   kp.wpack = t.wpack;
   // input maps: the (possibly parity-split) producer tensor has nclass * C0 channels at the reduced resolution
   t.map_bf16 = bf16;
@@ -1448,8 +1448,7 @@ inline int tc_prepare_tconv(TcLayer& t, const std::vector<float>& w, int cin, in
               tile[((size_t)k8 * CB + (size_t)q * CBt + co_) * 8 + e] = tc_to_bits(w[((size_t)ci * cout + co) * taps + q], bf16);
             }
     }
-  if (cudaMalloc(&t.wpack, pk.size() * 2) != cudaSuccess) { *why = "cudaMalloc(wpack) failed"; return 1; }
-  if (cudaMemcpy(t.wpack, pk.data(), pk.size() * 2, cudaMemcpyHostToDevice) != cudaSuccess) { *why = "cudaMemcpy(wpack) failed"; return 1; }
+  if (upload(&t.wpack, pk)) { *why = g_err; return 1; }
   kp.wpack = t.wpack;
   t.map_bf16 = bf16;
   { const int a0[6] = {maxN, cin, in_sp[0], in_sp[1], in_sp[2], KC}; for (int i = 0; i < 6; ++i) t.ms0[i] = a0[i]; }
@@ -1513,8 +1512,7 @@ inline int tc_prepare_first(TcLayer& t, const std::vector<float>& w27, int cout,
           }
           pk[(((size_t)m * 12 + kb * 2 + k8) * cout + co) * 8 + e] = v;
         }
-  if (cudaMalloc(&t.wpack, pk.size() * 2) != cudaSuccess) { *why = "cudaMalloc(wpack) failed"; return 1; }
-  if (cudaMemcpy(t.wpack, pk.data(), pk.size() * 2, cudaMemcpyHostToDevice) != cudaSuccess) { *why = "cudaMemcpy(wpack) failed"; return 1; }
+  if (upload(&t.wpack, pk)) { *why = g_err; return 1; }
   kp.wpack = t.wpack;
   t.map_bf16 = bf16;
   t.ms0[0] = 0; t.ms1[0] = 0;

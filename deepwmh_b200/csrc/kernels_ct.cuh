@@ -58,9 +58,9 @@ __device__ __forceinline__ void ct2_add(float x, float lb, float ub, double& s, 
 
 // "CT2": one cooperative launch, as zscore_fused_kernel: every thread sums its voxels inside (lb, ub) in fp64, the CTAs
 // leave {sum, sum of squares, count} in their slots, a grid-wide barrier, every CTA adds the slots in index order
-// (deterministic, no atomics on the data) and normalises the share it read.  vol 16-byte, seg 4-byte aligned.  slots:
-// [gridDim.x][3] doubles; barrier: a counter that is `target` once every CTA of this launch has arrived; out_stats (may be
-// null) = the totals.  An empty mask gives NaN (0 / 0), as upstream; the caller refuses it from the count.
+// (grid_ordered_totals: deterministic, no atomics on the data) and normalises the share it read.  vol 16-byte, seg 4-byte
+// aligned.  slots: [gridDim.x][3] doubles; barrier: a counter that is `target` once every CTA of this launch has arrived;
+// out_stats (may be null) = the totals.  An empty mask gives NaN (0 / 0), as upstream; the caller refuses it from the count.
 __global__ void __launch_bounds__(256) ct2_fused_kernel(float* __restrict__ vol, const int8_t* __restrict__ seg, int64_t n,
                                                         float lb, float ub, double* __restrict__ slots,
                                                         unsigned long long* __restrict__ barrier, unsigned long long target,
@@ -77,33 +77,7 @@ __global__ void __launch_bounds__(256) ct2_fused_kernel(float* __restrict__ vol,
   }
   if (blockIdx.x == 0 && threadIdx.x == 0)
     for (int64_t i = n4 << 2; i < n; ++i) ct2_add(vol[i], lb, ub, s, ss, cnt);
-  s = warp_sum_d(s); ss = warp_sum_d(ss); cnt = warp_sum_d(cnt);
-  __shared__ double sh[3][8];
-  __shared__ double tot[3];
-  const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
-  if (l == 0) { sh[0][w] = s; sh[1][w] = ss; sh[2][w] = cnt; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    for (int k = 1; k < 8; ++k) { sh[0][0] += sh[0][k]; sh[1][0] += sh[1][k]; sh[2][0] += sh[2][k]; }
-    double* my = slots + (size_t)blockIdx.x * 3;
-    my[0] = sh[0][0]; my[1] = sh[1][0]; my[2] = sh[2][0];
-    __threadfence();
-    atomicAdd(barrier, 1ull);
-    while (*reinterpret_cast<volatile unsigned long long*>(barrier) < target) { }
-    __threadfence();
-  }
-  __syncthreads();
-  if (w == 0) {      // ordered total: lane l adds slots l, l + 32, ...; the 32 lane sums are combined in lane order
-    double a = 0.0, b = 0.0, c = 0.0;
-    const volatile double* vs = slots;
-    for (int k = l; k < (int)gridDim.x; k += 32) { a += vs[3 * k]; b += vs[3 * k + 1]; c += vs[3 * k + 2]; }
-    for (int k = 0; k < 32; ++k) {
-      const double ak = __shfl_sync(0xffffffffu, a, k), bk = __shfl_sync(0xffffffffu, b, k), ck = __shfl_sync(0xffffffffu, c, k);
-      if (l == 0) { if (k == 0) { tot[0] = ak; tot[1] = bk; tot[2] = ck; } else { tot[0] += ak; tot[1] += bk; tot[2] += ck; } }
-    }
-  }
-  __syncthreads();
-  if (out_stats && blockIdx.x == 0 && threadIdx.x < 3) out_stats[threadIdx.x] = tot[threadIdx.x];
+  const double* tot = grid_ordered_totals(s, ss, cnt, slots, barrier, target, out_stats);
   const double m = tot[0] / tot[2];
   double var = tot[1] / tot[2] - m * m;
   var = var > 0.0 ? var : 0.0;

@@ -22,11 +22,11 @@ __device__ __forceinline__ void zscore_stats(const double* acc, float& mean, flo
 
 // One cooperative launch for the whole z-score (volumes of DeepWMH's size are launch-latency bound: 29 MB is 4 us of
 // HBM time).  Every CTA reduces its share in fp64 and leaves {sum, sum of squares, count} in its own slot; a grid-wide
-// barrier (all CTAs are co-resident: cudaLaunchCooperativeKernel); every CTA then adds the slots in index order --
-// deterministic, no atomics on the data, no memset -- and applies the normalisation to the share it already read (the
-// second read is served by L2 for volumes below its 126 MB).  slots: [gridDim.x][3] doubles; barrier: one monotonically
-// increasing counter, `target` = its value once every CTA of THIS launch has arrived; out_stats (may be null) = the
-// totals for the host.
+// barrier (all CTAs are co-resident: cudaLaunchCooperativeKernel); every CTA then adds the slots in index order
+// (grid_ordered_totals: deterministic, no atomics on the data, no memset) and applies the normalisation to the share it
+// already read (the second read is served by L2 for volumes below its 126 MB).  slots: [gridDim.x][3] doubles; barrier:
+// one monotonically increasing counter, `target` = its value once every CTA of THIS launch has arrived; out_stats (may be
+// null) = the totals for the host.
 __global__ void __launch_bounds__(256) zscore_fused_kernel(float* __restrict__ vol, const int8_t* __restrict__ seg, int64_t n, int mask_mode,
                                                            double* __restrict__ slots, unsigned long long* __restrict__ barrier,
                                                            unsigned long long target, double* __restrict__ out_stats) {
@@ -52,35 +52,8 @@ __global__ void __launch_bounds__(256) zscore_fused_kernel(float* __restrict__ v
       if (m) { s += v; ss += (double)v * v; cnt += 1.0; }
     }
   }
-  s = warp_sum_d(s); ss = warp_sum_d(ss); cnt = warp_sum_d(cnt);
-  __shared__ double sh[3][8];
-  __shared__ double tot[3];
-  const int w = threadIdx.x >> 5, l = threadIdx.x & 31;
-  if (l == 0) { sh[0][w] = s; sh[1][w] = ss; sh[2][w] = cnt; }
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    for (int k = 1; k < 8; ++k) { sh[0][0] += sh[0][k]; sh[1][0] += sh[1][k]; sh[2][0] += sh[2][k]; }
-    double* my = slots + (size_t)blockIdx.x * 3;
-    my[0] = sh[0][0]; my[1] = sh[1][0]; my[2] = sh[2][0];
-    __threadfence();
-    atomicAdd(barrier, 1ull);
-    while (*reinterpret_cast<volatile unsigned long long*>(barrier) < target) { }
-    __threadfence();
-  }
-  __syncthreads();
-  if (w == 0) {      // ordered total: lane l adds slots l, l + 32, ...; the 32 lane sums are combined in lane order
-    double a = 0.0, b = 0.0, c = 0.0;
-    const volatile double* vs = slots;
-    for (int k = l; k < (int)gridDim.x; k += 32) { a += vs[3 * k]; b += vs[3 * k + 1]; c += vs[3 * k + 2]; }
-    for (int k = 0; k < 32; ++k) {
-      const double ak = __shfl_sync(0xffffffffu, a, k), bk = __shfl_sync(0xffffffffu, b, k), ck = __shfl_sync(0xffffffffu, c, k);
-      if (l == 0) { if (k == 0) { tot[0] = ak; tot[1] = bk; tot[2] = ck; } else { tot[0] += ak; tot[1] += bk; tot[2] += ck; } }
-    }
-  }
-  __syncthreads();
-  if (out_stats && blockIdx.x == 0 && threadIdx.x < 3) out_stats[threadIdx.x] = tot[threadIdx.x];
   float mean, denom;
-  zscore_stats(tot, mean, denom);
+  zscore_stats(grid_ordered_totals(s, ss, cnt, slots, barrier, target, out_stats), mean, denom);
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
     float4 v = v4[i];
     bool m0 = true, m1 = true, m2 = true, m3 = true;

@@ -17,33 +17,19 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdarg>
 #include <cstdint>
-#include <cstdio>
 #include <cuda_runtime.h>
 
-extern "C" void dwmh_internal_set_error(const char* msg);
+#include "host.cuh"
+#include "common.cuh"
+
+using dwmh::fail;
+using dwmh::sm_count;
 
 namespace {
 
-int fail(const char* fmt, ...) {
-  char buf[1024];
-  va_list ap; va_start(ap, fmt); vsnprintf(buf, sizeof buf, fmt, ap); va_end(ap);
-  dwmh_internal_set_error(buf);
-  return 1;
-}
-#define N4_CU(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) \
-  return fail("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e__), __FILE__, __LINE__); } while (0)
-
-struct N4DevGuard {
-  int prev = -1; bool ok = false;
-  explicit N4DevGuard(int dev) {
-    if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
-    ok = (prev == dev) || cudaSetDevice(dev) == cudaSuccess;
-    if (prev == dev) prev = -1;
-  }
-  ~N4DevGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
+using dwmh::float_key;
+using dwmh::key_float;
 
 constexpr int N4_BINS = 200;
 constexpr int N4_PAD = 512;                          // 2^(ceil(log2 200) + 1)
@@ -76,9 +62,6 @@ struct N4Args {
   unsigned* keys;              // [2] order-preserving keys of min / max of U over the valid points
   double* table;               // [203] sharpening table
 };
-
-__device__ __forceinline__ unsigned n4_key(float f) { const unsigned u = __float_as_uint(f); return (u & 0x80000000u) ? ~u : (u | 0x80000000u); }
-__device__ __forceinline__ float n4_unkey(unsigned k) { return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k); }
 
 // Cubic B-spline weights of full-resolution index t on the domain [0, n_full - 1] -> [0, mesh]; returns the span.
 __device__ __forceinline__ int n4_bspline(int t, int n_full, int mesh, double w[4]) {
@@ -188,7 +171,7 @@ __global__ void __launch_bounds__(256) n4_field_kernel(N4Args a) {
       const float l = a.logi[base + k];
       const float uv = (float)((double)l - b);               // NaN stays NaN
       a.u[base + k] = uv;
-      if (!isnan(uv)) { const unsigned key = n4_key(uv); mn = min(mn, key); mx = max(mx, key); }
+      if (!isnan(uv)) { const unsigned key = float_key(uv); mn = min(mn, key); mx = max(mx, key); }
     }
     __syncwarp();
   }
@@ -208,7 +191,7 @@ __global__ void __launch_bounds__(256) n4_hist_kernel(N4Args a) {
   __shared__ unsigned long long sh[N4_BINS];
   for (int b = threadIdx.x; b < N4_BINS; b += blockDim.x) sh[b] = 0ull;
   __syncthreads();
-  const double lo = (double)n4_unkey(a.keys[0]), hi = (double)n4_unkey(a.keys[1]);
+  const double lo = (double)key_float(a.keys[0]), hi = (double)key_float(a.keys[1]);
   const double slope = (hi - lo) / (N4_BINS - 1);
   if (a.keys[0] <= a.keys[1] && slope > 0.0) {
     const int64_t n = (int64_t)a.nx * a.ny * a.nz;
@@ -262,7 +245,7 @@ __global__ void __launch_bounds__(N4_PAD) n4_sharpen_kernel(N4Args a) {
   const int t = threadIdx.x, tid = t & 255;
   const bool upper = t >= 256;
   const unsigned k0 = a.keys[0], k1 = a.keys[1];
-  const double lo = (double)n4_unkey(k0), hi = (double)n4_unkey(k1);
+  const double lo = (double)key_float(k0), hi = (double)key_float(k1);
   const double slope = (hi - lo) / (N4_BINS - 1);
   const bool identity = !(k0 <= k1) || !(slope > 0.0);
   const double sfwhm = N4_FWHM / slope;
@@ -501,21 +484,18 @@ extern "C" int dwmh_n4(int32_t device, const float* in, int32_t X, int32_t Y, in
   if (n4_check(X, Y, Z, shrink, num_levels)) return 1;
   for (int l = 0; l < num_levels; ++l)
     if (iterations[l] < 0) return fail("dwmh_n4: %d iterations on level %d", iterations[l], l);
-  N4DevGuard dg(device);
-  if (!dg.ok) return fail("cudaSetDevice(%d) failed", device);
+  DEV_GUARD(device);
   cudaStream_t st = (cudaStream_t)stream_;
-  int sms = 148;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-  const int grid = sms * 4;
+  const int grid = sm_count(device) * 4;
   N4Args a;
   n4_layout(X, Y, Z, shrink, num_levels, (char*)workspace, &a);
   const int warps_z = std::max(1, std::min(8, (48 * 1024) / (a.nz * (int)sizeof(double))));
 
   a.mesh = 1; a.C = 4;
   n4_shrink_log_kernel<<<grid, 256, 0, st>>>(in, a);
-  N4_CU(cudaGetLastError());
+  CU_TRY(cudaGetLastError());
   cudaStream_t cs = nullptr;                 // private stream, used only to capture the per-level graph
-  N4_CU(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
+  CU_TRY(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
   int rc = 0;
   for (int level = 0; level < num_levels && rc == 0; ++level) {
     if (level > 0) {
@@ -549,6 +529,6 @@ extern "C" int dwmh_n4(int32_t device, const float* in, int32_t X, int32_t Y, in
   cudaStreamDestroy(cs);
   if (rc) return rc;
   n4_output_kernel<<<grid, 256, (size_t)8 * a.C * sizeof(double), st>>>(in, out, log_field, a);
-  N4_CU(cudaGetLastError());
+  CU_TRY(cudaGetLastError());
   return 0;
 }

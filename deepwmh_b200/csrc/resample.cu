@@ -15,33 +15,19 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdarg>
 #include <cstdint>
-#include <cstdio>
 #include <cuda_runtime.h>
 
-extern "C" void dwmh_internal_set_error(const char* msg);
+#include "host.cuh"
+#include "common.cuh"
+
+using dwmh::fail;
+using dwmh::sm_count;
 
 namespace {
 
-int fail(const char* fmt, ...) {
-  char buf[1024];
-  va_list ap; va_start(ap, fmt); vsnprintf(buf, sizeof buf, fmt, ap); va_end(ap);
-  dwmh_internal_set_error(buf);
-  return 1;
-}
-#define RS_CU(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) \
-  return fail("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e__), __FILE__, __LINE__); } while (0)
-
-struct RsDevGuard {
-  int prev = -1; bool ok = false;
-  explicit RsDevGuard(int dev) {
-    if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
-    ok = (prev == dev) || cudaSetDevice(dev) == cudaSuccess;
-    if (prev == dev) prev = -1;
-  }
-  ~RsDevGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
+using dwmh::float_key;
+using dwmh::key_float;
 
 constexpr int RS_NPAD = 12;        // scipy's _prepad_for_spline_filter for mode 'nearest'
 constexpr int RS_RADIUS = 24;      // FIR radius of the prefilter
@@ -59,10 +45,6 @@ __device__ __forceinline__ int rs_ext(int i, int n) {
   return p < 0 ? 0 : (p > n - 1 ? n - 1 : p);
 }
 
-// order-preserving float <-> uint for atomicMin / atomicMax
-__device__ __forceinline__ unsigned rs_key(float f) { const unsigned u = __float_as_uint(f); return (u & 0x80000000u) ? ~u : (u | 0x80000000u); }
-__device__ __forceinline__ float rs_unkey(unsigned k) { return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k); }
-
 // min / max of every slice along `axis` (axis < 0: the whole volume is one slice): grid (nslices, chunks); a block reduces its
 // share of one slice and issues one atomicMin / atomicMax.  range[2 s] = min key, range[2 s + 1] = max key.
 __global__ void __launch_bounds__(256) rs_range_kernel(const float* __restrict__ src, int n0, int n1, int n2, int axis, unsigned* __restrict__ range) {
@@ -74,7 +56,7 @@ __global__ void __launch_bounds__(256) rs_range_kernel(const float* __restrict__
     if (axis <= 0) idx = (int64_t)s * M + e;                                  // axis 0 (or whole volume, s = 0): contiguous
     else if (axis == 1) idx = ((e / n2) * n1 + s) * n2 + e % n2;              // (i0, i2) with i2 fastest
     else idx = e * n2 + s;                                                    // (i0, i1), strided
-    const unsigned k = rs_key(src[idx]);
+    const unsigned k = float_key(src[idx]);
     mn = min(mn, k); mx = max(mx, k);
   }
 #pragma unroll
@@ -186,7 +168,7 @@ __global__ void __launch_bounds__(256) rs_gather_kernel(const double* __restrict
       }
     }
     const int s = p.clip_axis < 0 ? 0 : (p.clip_axis == 0 ? s0 : (p.clip_axis == 1 ? s1 : s2));
-    const double lo = (double)rs_unkey(range[2 * s]), hi = (double)rs_unkey(range[2 * s + 1]);
+    const double lo = (double)key_float(range[2 * s]), hi = (double)key_float(range[2 * s + 1]);
     t = t < lo ? lo : (t > hi ? hi : t);
     if (p.out_mode == 1) reinterpret_cast<int8_t*>(out)[v] = t >= 0.5 ? 0 : -1;
     else reinterpret_cast<float*>(out)[v] = (float)t;
@@ -234,12 +216,6 @@ __global__ void __launch_bounds__(256) rs_onehot_kernel(const uint8_t* __restric
   }
 }
 
-int grid_for(int device) {
-  int sms = 148;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-  return sms * 8;
-}
-
 bool fir_ready[64] = {false};
 
 }  // namespace
@@ -266,18 +242,17 @@ extern "C" int dwmh_resample(int32_t device, const float* src, const int32_t in_
   if (out_mode != 0 && out_mode != 1) return fail("dwmh_resample: out_mode %d", out_mode);
   for (int a = 0; a < 3; ++a)
     if (in_shape[a] <= 0 || out_shape[a] <= 0) return fail("dwmh_resample: empty extent on axis %d", a);
-  RsDevGuard dg(device);
-  if (!dg.ok) return fail("cudaSetDevice(%d) failed", device);
+  DEV_GUARD(device);
   cudaStream_t st = (cudaStream_t)stream_;
   if (device >= 0 && device < 64 && !fir_ready[device]) {
     double h[RS_RADIUS + 1];
     const double z = std::sqrt(3.0) - 2.0;
     double zk = 1.0;
     for (int k = 0; k <= RS_RADIUS; ++k) { h[k] = std::sqrt(3.0) * zk; zk *= z; }
-    RS_CU(cudaMemcpyToSymbol(c_fir, h, sizeof h));
+    CU_TRY(cudaMemcpyToSymbol(c_fir, h, sizeof h));
     fir_ready[device] = true;
   }
-  const int grid = grid_for(device);
+  const int grid = sm_count(device) * 8;
   const int64_t wsd = rs_ws_doubles(in_shape, order, separate_axis);
   double* bufA = reinterpret_cast<double*>(workspace);
   double* bufB = bufA + wsd;
@@ -319,7 +294,7 @@ extern "C" int dwmh_resample(int32_t device, const float* src, const int32_t in_
   p.out_mode = out_mode;
   if (order == 0) p.clip_axis = -1;
   rs_gather_kernel<<<grid, 256, 0, st>>>(coef, dst, p, range);
-  RS_CU(cudaGetLastError());
+  CU_TRY(cudaGetLastError());
   return 0;
 }
 
@@ -331,8 +306,7 @@ extern "C" int dwmh_cascade_onehot(int32_t device, const uint8_t* labels, const 
   for (int a = 0; a < 3; ++a)
     if (in_shape[a] <= 0 || out_shape[a] <= 0)
       return fail("dwmh_cascade_onehot: empty extent on axis %d (in %d, out %d)", a, in_shape[a], out_shape[a]);
-  RsDevGuard dg(device);
-  if (!dg.ok) return fail("cudaSetDevice(%d) failed", device);
+  DEV_GUARD(device);
   RsParams p;
   for (int a = 0; a < 3; ++a) {
     RsAxis& x = p.ax[a];
@@ -342,7 +316,7 @@ extern "C" int dwmh_cascade_onehot(int32_t device, const uint8_t* labels, const 
   }
   p.clip_axis = -1;
   p.out_mode = 0;
-  rs_onehot_kernel<<<grid_for(device), 256, 0, (cudaStream_t)stream_>>>(labels, dst, p, num_classes);
-  RS_CU(cudaGetLastError());
+  rs_onehot_kernel<<<sm_count(device) * 8, 256, 0, (cudaStream_t)stream_>>>(labels, dst, p, num_classes);
+  CU_TRY(cudaGetLastError());
   return 0;
 }

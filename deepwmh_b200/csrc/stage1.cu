@@ -14,46 +14,18 @@
 //   dwmh_s1_label_vote / _apply_priors   average_contiguous_labels (image_ops.py:23-38) and the tissue priors (:213-243)
 #include "../../include/deepwmh_b200.h"
 
-#include <cstdarg>
 #include <cstdint>
-#include <cstdio>
 #include <cstring>
 #include <cuda_runtime.h>
 
+#include "host.cuh"
 #include "common.cuh"
 #include "kernels_ccl.cuh"
 
-extern "C" void dwmh_internal_set_error(const char* msg);   // api.cu (thread-local message behind dwmh_last_error)
+using dwmh::fail;
+using dwmh::sm_count;
 
 namespace {
-
-int fail(const char* fmt, ...) {
-  char buf[1024];
-  va_list ap; va_start(ap, fmt); vsnprintf(buf, sizeof buf, fmt, ap); va_end(ap);
-  dwmh_internal_set_error(buf);
-  return 1;
-}
-#define S1_CU(expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) \
-  return fail("%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e__), __FILE__, __LINE__); } while (0)
-
-// Entry points run on `device` and leave the caller's current device as they found it.
-struct S1DevGuard {
-  int prev = -1; bool ok = false;
-  explicit S1DevGuard(int dev) {
-    if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
-    ok = (prev == dev) || cudaSetDevice(dev) == cudaSuccess;
-    if (prev == dev) prev = -1;
-  }
-  ~S1DevGuard() { if (prev >= 0) cudaSetDevice(prev); }
-};
-#define S1_DEV(dev) S1DevGuard dev_guard__(dev); if (!dev_guard__.ok) return fail("cudaSetDevice(%d) failed", (int)(dev))
-
-int grid_for(int device) {
-  static int sms[64] = {0};
-  if (device < 0 || device >= 64) return 148 * 8;
-  if (!sms[device]) cudaDeviceGetAttribute(&sms[device], cudaDevAttrMultiProcessorCount, device);
-  return (sms[device] > 0 ? sms[device] : 148) * 8;
-}
 
 using dwmh::warp_sum_d;
 
@@ -717,10 +689,10 @@ int cs_threads(int Z) { const int t = (Z + 31) & ~31; return t < 256 ? t : 256; 
 static int zscore_launch(int device, VolPtrs vols, int nvol, const float* mask, int64_t n, int fill_outside, void* workspace,
                          bool aligned, cudaStream_t st) {
   double* ws = (double*)workspace;
-  S1_CU(cudaMemsetAsync(ws, 0, (size_t)nvol * ZS_SLOT * sizeof(double), st));
+  CU_TRY(cudaMemsetAsync(ws, 0, (size_t)nvol * ZS_SLOT * sizeof(double), st));
   // min slot <- 0x7f7f7f7f (above the key of every float below 3.39e38): one strided 2-D memset over the slots
-  S1_CU(cudaMemset2DAsync((char*)workspace + 32, ZS_SLOT * sizeof(double), 0x7f, 4, nvol, st));
-  const dim3 grid((grid_for(device) + nvol - 1) / nvol, nvol);
+  CU_TRY(cudaMemset2DAsync((char*)workspace + 32, ZS_SLOT * sizeof(double), 0x7f, 4, nvol, st));
+  const dim3 grid((sm_count(device) * 8 + nvol - 1) / nvol, nvol);
   if (aligned) {
     s1_stats_kernel<true><<<grid, 256, 0, st>>>(vols, mask, n, ws);
     s1_zscore_apply_kernel<true><<<grid, 256, 0, st>>>(vols, mask, n, ws, fill_outside);
@@ -728,7 +700,7 @@ static int zscore_launch(int device, VolPtrs vols, int nvol, const float* mask, 
     s1_stats_kernel<false><<<grid, 256, 0, st>>>(vols, mask, n, ws);
     s1_zscore_apply_kernel<false><<<grid, 256, 0, st>>>(vols, mask, n, ws, fill_outside);
   }
-  S1_CU(cudaGetLastError());
+  CU_TRY(cudaGetLastError());
   return 0;
 }
 
@@ -738,13 +710,13 @@ extern "C" int dwmh_s1_zscore(int32_t device, float* x, const float* mask, int64
   if (n <= 0) return fail("dwmh_s1_zscore: empty volume");
   if (fill_outside && !mask) return fail("dwmh_s1_zscore: fill_outside needs a mask");
   cudaStream_t st = (cudaStream_t)stream_;
-  S1_DEV(device);
+  DEV_GUARD(device);
   VolPtrs vols{}; vols.p[0] = x;
   if (zscore_launch(device, vols, 1, mask, n, fill_outside, workspace, (((uintptr_t)x | (uintptr_t)mask) & 15) == 0, st)) return 1;
   if (stats_out) {
     double h[4];
-    S1_CU(cudaMemcpyAsync(h, workspace, sizeof h, cudaMemcpyDeviceToHost, st));
-    S1_CU(cudaStreamSynchronize(st));
+    CU_TRY(cudaMemcpyAsync(h, workspace, sizeof h, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
     const double cnt = h[2] > 0 ? h[2] : 1.0, m = h[0] / cnt;
     double var = h[1] / cnt - m * m; if (var < 0) var = 0;
     stats_out[0] = m; stats_out[1] = sqrt(var); stats_out[2] = h[2];
@@ -761,7 +733,7 @@ extern "C" int dwmh_s1_zscore_batch(int32_t device, float* const* xs, int32_t nv
   VolPtrs vols{};
   uintptr_t al = (uintptr_t)mask;
   for (int i = 0; i < nvol; ++i) { if (!xs[i]) return fail("dwmh_s1_zscore_batch: xs[%d] is null", i); vols.p[i] = xs[i]; al |= (uintptr_t)xs[i]; }
-  S1_DEV(device);
+  DEV_GUARD(device);
   return zscore_launch(device, vols, nvol, mask, n, fill_outside, workspace, (al & 15) == 0, (cudaStream_t)stream_);
 }
 
@@ -780,12 +752,12 @@ extern "C" int dwmh_s1_mean_std_grid(int32_t device, const float* x, const float
   GridGeom q;
   if (geom(X, Y, Z, patch_size, &q)) return 1;
   cudaStream_t st = (cudaStream_t)stream_;
-  S1_DEV(device);
+  DEV_GUARD(device);
   const size_t ncell = (size_t)q.g[0] * q.g[1] * q.g[2], ngrid = (size_t)(q.g[0] + 2) * (q.g[1] + 2) * (q.g[2] + 2);
   double* cells = (double*)workspace;
   double* mg = (double*)((char*)workspace + align256(ncell * 3 * sizeof(double)));
   double* sg = (double*)((char*)mg + align256(ngrid * sizeof(double)));
-  S1_CU(cudaMemsetAsync(workspace, 0, align256(ncell * 3 * sizeof(double)) + 2 * align256(ngrid * sizeof(double)), st));
+  CU_TRY(cudaMemsetAsync(workspace, 0, align256(ncell * 3 * sizeof(double)) + 2 * align256(ngrid * sizeof(double)), st));
   const int slabs = (q.st[0] + CS_SLAB - 1) / CS_SLAB;
   if (q.g[2] > 300) return fail("dwmh_s1_mean_std_grid: %d cells along z exceed the shared-memory tables (300)", q.g[2]);
   VolPtrs vols{}; vols.p[0] = const_cast<float*>(x);
@@ -793,7 +765,7 @@ extern "C" int dwmh_s1_mean_std_grid(int32_t device, const float* x, const float
   s1_grid_stats_kernel<<<(unsigned)((ncell + 127) / 128), 128, 0, st>>>(cells, q, mask ? 1 : 0, mg, sg, 0);
   if ((Y + 7) / 8 > 65535) return fail("dwmh_s1_mean_std_grid: volume too large");
   s1_grid_zoom_kernel<<<dim3(X, (Y + 7) / 8), 256, 16 * (q.g[2] + 2) * sizeof(double), st>>>(mg, sg, q, mean_out, std_out);
-  S1_CU(cudaGetLastError());
+  CU_TRY(cudaGetLastError());
   return 0;
 }
 
@@ -819,29 +791,29 @@ extern "C" int dwmh_s1_local_mean_align(int32_t device, const float* target, flo
   VolPtrs vols{}; vols.p[0] = const_cast<float*>(target);
   for (int i = 0; i < k; ++i) { if (!refs[i]) return fail("dwmh_s1_local_mean_align: refs[%d] is null", i); vols.p[i + 1] = refs[i]; }
   cudaStream_t st = (cudaStream_t)stream_;
-  S1_DEV(device);
+  DEV_GUARD(device);
   const int nvol = k + 1;
   const size_t ncell = (size_t)q.g[0] * q.g[1] * q.g[2], gstride = align256((size_t)(q.g[0] + 2) * (q.g[1] + 2) * (q.g[2] + 2) * sizeof(double)) / sizeof(double);
   const size_t cells_bytes = align256((size_t)nvol * ncell * 3 * sizeof(double));
   double* cells = (double*)workspace;
   double* mg = (double*)((char*)workspace + cells_bytes);
   double* sg = mg + (size_t)nvol * gstride;
-  S1_CU(cudaMemsetAsync(workspace, 0, cells_bytes + 2 * (size_t)nvol * gstride * sizeof(double), st));
+  CU_TRY(cudaMemsetAsync(workspace, 0, cells_bytes + 2 * (size_t)nvol * gstride * sizeof(double), st));
   const int slabs = (q.st[0] + CS_SLAB - 1) / CS_SLAB;
   s1_cell_sums_kernel<<<dim3((unsigned)(q.g[0] * q.g[1] * slabs), nvol), cs_threads(Z), 3 * cs_threads(Z) * sizeof(double), st>>>(vols, mask, q, slabs, cells);
   s1_grid_stats_kernel<<<dim3((unsigned)((ncell + 127) / 128), nvol), 128, 0, st>>>(cells, q, mask ? 1 : 0, mg, sg, gstride);
   const size_t za_smem = 16 * (size_t)(q.g[2] + 2) * sizeof(double) + (size_t)Z * (sizeof(double) + sizeof(int));
   if (za_smem > 48 * 1024) return fail("dwmh_s1_local_mean_align: Z = %d exceeds the shared-memory z table", Z);
   s1_zoom_align_kernel<<<dim3(X, (Y + 7) / 8), 256, za_smem, st>>>(mg, gstride, q, vols, nvol, target_local_mu_out);
-  S1_CU(cudaGetLastError());
+  CU_TRY(cudaGetLastError());
   return 0;
 }
 
 extern "C" int dwmh_s1_align_local_mean(int32_t device, float* x, const float* local_mu, const float* target_local_mu, int64_t n, void* stream_) {
   if (!x || !local_mu || !target_local_mu) return fail("dwmh_s1_align_local_mean: null argument");
-  S1_DEV(device);
-  s1_align_kernel<<<grid_for(device), 256, 0, (cudaStream_t)stream_>>>(x, local_mu, target_local_mu, n);
-  S1_CU(cudaGetLastError());
+  DEV_GUARD(device);
+  s1_align_kernel<<<sm_count(device) * 8, 256, 0, (cudaStream_t)stream_>>>(x, local_mu, target_local_mu, n);
+  CU_TRY(cudaGetLastError());
   return 0;
 }
 
@@ -857,18 +829,18 @@ static int group_nll_impl(const char* who, int32_t device, const float* x_prime,
     rp.p[i] = refs[i];
     if (masks) mp.p[i] = masks[i];
   }
-  S1_DEV(device);
+  DEV_GUARD(device);
   const NllParams q{min_std, side, k};
   cudaStream_t st = (cudaStream_t)stream_;
   if (masks) {
-    s1_group_nll_masked_kernel<<<grid_for(device), 256, 0, st>>>(x_prime, rp, mp, q, mul_mask, anomaly, mu_out, sigma_out, n);
+    s1_group_nll_masked_kernel<<<sm_count(device) * 8, 256, 0, st>>>(x_prime, rp, mp, q, mul_mask, anomaly, mu_out, sigma_out, n);
   } else {
     uintptr_t al = (uintptr_t)x_prime | (uintptr_t)mul_mask | (uintptr_t)anomaly | (uintptr_t)mu_out | (uintptr_t)sigma_out;
     for (int i = 0; i < k; ++i) al |= (uintptr_t)refs[i];
-    if ((al & 15) == 0) s1_group_nll_kernel<true><<<grid_for(device), 256, 0, st>>>(x_prime, rp, q, mul_mask, anomaly, mu_out, sigma_out, n);
-    else s1_group_nll_kernel<false><<<grid_for(device), 256, 0, st>>>(x_prime, rp, q, mul_mask, anomaly, mu_out, sigma_out, n);
+    if ((al & 15) == 0) s1_group_nll_kernel<true><<<sm_count(device) * 8, 256, 0, st>>>(x_prime, rp, q, mul_mask, anomaly, mu_out, sigma_out, n);
+    else s1_group_nll_kernel<false><<<sm_count(device) * 8, 256, 0, st>>>(x_prime, rp, q, mul_mask, anomaly, mu_out, sigma_out, n);
   }
-  S1_CU(cudaGetLastError());
+  CU_TRY(cudaGetLastError());
   return 0;
 }
 
@@ -891,7 +863,7 @@ extern "C" int dwmh_s1_median_filter(int32_t device, const float* in, float* out
   if (X <= 0 || Y <= 0 || Z <= 0) return fail("dwmh_s1_median_filter: empty volume");
   const int kx = kernel_size[0], ky = kernel_size[1], kz = kernel_size[2];
   if (kx < 1 || ky < 1 || kz < 1 || kx > 9 || ky > 9 || kz > 9) return fail("dwmh_s1_median_filter: kernel %dx%dx%d (1..9 per axis supported)", kx, ky, kz);
-  S1_DEV(device);
+  DEV_GUARD(device);
   const size_t smem = (size_t)(MT_X + kx - 1) * (MT_Y + ky - 1) * (MT_Z + kz - 1) * sizeof(uint32_t);
   dim3 grid((Z + MT_Z - 1) / MT_Z, (Y + MT_Y - 1) / MT_Y, (X + MT_X - 1) / MT_X);
   if (grid.y > 65535 || grid.z > 65535) return fail("dwmh_s1_median_filter: volume too large");
@@ -903,7 +875,7 @@ extern "C" int dwmh_s1_median_filter(int32_t device, const float* in, float* out
                     MS(1, 5, 5) || MS(5, 1, 5) || MS(5, 5, 1) || MS(1, 6, 6) || MS(6, 1, 6) || MS(6, 6, 1);
 #undef MS
   if (!done) s1_median_kernel<<<grid, 256, smem, st>>>(in, out, X, Y, Z, kx, ky, kz);
-  S1_CU(cudaGetLastError());
+  CU_TRY(cudaGetLastError());
   return 0;
 }
 
@@ -930,17 +902,17 @@ extern "C" int dwmh_s1_component_filtering(int32_t device, const float* mask, in
     for (int a = 0; a < 3; ++a) filt[a] = a == am;
   }
   cudaStream_t st = (cudaStream_t)stream_;
-  S1_DEV(device);
+  DEV_GUARD(device);
   int* L = (int*)workspace;
   int* size = (int*)((char*)workspace + align256((size_t)V * 4));
   float* acc = (float*)((char*)workspace + 2 * align256((size_t)V * 4));
   unsigned long long* best = (unsigned long long*)((char*)workspace + 3 * align256((size_t)V * 4));
   const Dims d{{X, Y, Z}, {(int64_t)Y * Z, (int64_t)Z, 1}};
-  const int grid = grid_for(device);
-  S1_CU(cudaMemsetAsync(acc, 0, (size_t)V * 4, st));
+  const int grid = sm_count(device) * 8;
+  CU_TRY(cudaMemsetAsync(acc, 0, (size_t)V * 4, st));
   for (int ax = 0; ax < 3; ++ax) {
     if (!filt[ax]) { cf_passthrough_kernel<<<grid, 256, 0, st>>>(mask, acc, V); continue; }
-    S1_CU(cudaMemsetAsync(best, 0, (size_t)d.n[ax] * 8, st));
+    CU_TRY(cudaMemsetAsync(best, 0, (size_t)d.n[ax] * 8, st));
     cf_erode_init_kernel<<<grid, 256, 0, st>>>(mask, L, size, d, ax, V);
     cf_merge_kernel<<<grid, 256, 0, st>>>(L, d, ax, V);
     dwmh::ccl_count_kernel<<<grid, 256, 0, st>>>(L, size, V);
@@ -948,7 +920,7 @@ extern "C" int dwmh_s1_component_filtering(int32_t device, const float* mask, in
     cf_accum_kernel<<<grid, 256, 0, st>>>(L, best, acc, d, ax, V);
   }
   cf_final_kernel<<<grid, 256, 0, st>>>(acc, out, V);
-  S1_CU(cudaGetLastError());
+  CU_TRY(cudaGetLastError());
   return 0;
 }
 
@@ -956,15 +928,15 @@ extern "C" int dwmh_s1_minmax(int32_t device, const float* x, const float* mask,
   if (!x || !workspace || !out_minmax) return fail("dwmh_s1_minmax: null argument");
   if (n <= 0) return fail("dwmh_s1_minmax: empty volume");
   cudaStream_t st = (cudaStream_t)stream_;
-  S1_DEV(device);
+  DEV_GUARD(device);
   const int init[2] = {0x7fffffff, (int)0x80000000};
   int* mm = (int*)workspace;
-  S1_CU(cudaMemcpyAsync(mm, init, sizeof init, cudaMemcpyHostToDevice, st));
-  s1_minmax_kernel<<<grid_for(device), 256, 0, st>>>(x, mask, n, mm);
-  S1_CU(cudaGetLastError());
+  CU_TRY(cudaMemcpyAsync(mm, init, sizeof init, cudaMemcpyHostToDevice, st));
+  s1_minmax_kernel<<<sm_count(device) * 8, 256, 0, st>>>(x, mask, n, mm);
+  CU_TRY(cudaGetLastError());
   int h[2];
-  S1_CU(cudaMemcpyAsync(h, mm, sizeof h, cudaMemcpyDeviceToHost, st));
-  S1_CU(cudaStreamSynchronize(st));
+  CU_TRY(cudaMemcpyAsync(h, mm, sizeof h, cudaMemcpyDeviceToHost, st));
+  CU_TRY(cudaStreamSynchronize(st));
   if (h[0] == 0x7fffffff) return fail("dwmh_s1_minmax: the mask selects no voxel");
   for (int i = 0; i < 2; ++i) { const int o = h[i] >= 0 ? h[i] : h[i] ^ 0x7fffffff; memcpy(&out_minmax[i], &o, 4); }
   return 0;
@@ -976,20 +948,20 @@ extern "C" int dwmh_s1_histogram(int32_t device, const float* x, const float* ma
   if (n <= 0) return fail("dwmh_s1_histogram: empty volume");
   if (nbins < 1 || nbins > 2048) return fail("dwmh_s1_histogram: nbins = %d (1..2048 supported)", nbins);
   cudaStream_t st = (cudaStream_t)stream_;
-  S1_DEV(device);
-  S1_CU(cudaMemsetAsync(counts, 0, (size_t)nbins * sizeof(uint64_t), st));
+  DEV_GUARD(device);
+  CU_TRY(cudaMemsetAsync(counts, 0, (size_t)nbins * sizeof(uint64_t), st));
   const size_t smem = (size_t)(nbins + 1) * sizeof(double) + (size_t)nbins * sizeof(unsigned int);
-  s1_histogram_kernel<<<grid_for(device) / 2, 256, smem, st>>>(x, mask, n, fill_outside, fill_value, edges, nbins,
+  s1_histogram_kernel<<<sm_count(device) * 4, 256, smem, st>>>(x, mask, n, fill_outside, fill_value, edges, nbins,
                                                                  reinterpret_cast<unsigned long long*>(counts));
-  S1_CU(cudaGetLastError());
+  CU_TRY(cudaGetLastError());
   return 0;
 }
 
 extern "C" int dwmh_s1_threshold_mask(int32_t device, const float* x, float threshold, const float* mul_mask, float* out, int64_t n, void* stream_) {
   if (!x || !out) return fail("dwmh_s1_threshold_mask: null argument");
-  S1_DEV(device);
-  s1_threshold_kernel<<<grid_for(device), 256, 0, (cudaStream_t)stream_>>>(x, threshold, mul_mask, out, n);
-  S1_CU(cudaGetLastError());
+  DEV_GUARD(device);
+  s1_threshold_kernel<<<sm_count(device) * 8, 256, 0, (cudaStream_t)stream_>>>(x, threshold, mul_mask, out, n);
+  CU_TRY(cudaGetLastError());
   return 0;
 }
 
@@ -1002,17 +974,17 @@ extern "C" int dwmh_s1_masked_sums(int32_t device, const float* const* xs, int32
   uintptr_t al = (uintptr_t)mask;
   for (int i = 0; i < nvol; ++i) { if (!xs[i]) return fail("dwmh_s1_masked_sums: xs[%d] is null", i); vols.p[i] = const_cast<float*>(xs[i]); al |= (uintptr_t)xs[i]; }
   cudaStream_t st = (cudaStream_t)stream_;
-  S1_DEV(device);
+  DEV_GUARD(device);
   double* ws = (double*)workspace;
-  S1_CU(cudaMemsetAsync(ws, 0, (size_t)nvol * ZS_SLOT * sizeof(double), st));
-  S1_CU(cudaMemset2DAsync((char*)workspace + 32, ZS_SLOT * sizeof(double), 0x7f, 4, nvol, st));
-  const dim3 grid((grid_for(device) + nvol - 1) / nvol, nvol);
+  CU_TRY(cudaMemsetAsync(ws, 0, (size_t)nvol * ZS_SLOT * sizeof(double), st));
+  CU_TRY(cudaMemset2DAsync((char*)workspace + 32, ZS_SLOT * sizeof(double), 0x7f, 4, nvol, st));
+  const dim3 grid((sm_count(device) * 8 + nvol - 1) / nvol, nvol);
   if ((al & 15) == 0) s1_stats_kernel<true><<<grid, 256, 0, st>>>(vols, mask, n, ws, positive_only);
   else s1_stats_kernel<false><<<grid, 256, 0, st>>>(vols, mask, n, ws, positive_only);
-  S1_CU(cudaGetLastError());
+  CU_TRY(cudaGetLastError());
   double h[S1_MAX_VOLS * ZS_SLOT];
-  S1_CU(cudaMemcpyAsync(h, ws, (size_t)nvol * ZS_SLOT * sizeof(double), cudaMemcpyDeviceToHost, st));
-  S1_CU(cudaStreamSynchronize(st));
+  CU_TRY(cudaMemcpyAsync(h, ws, (size_t)nvol * ZS_SLOT * sizeof(double), cudaMemcpyDeviceToHost, st));
+  CU_TRY(cudaStreamSynchronize(st));
   for (int i = 0; i < nvol; ++i) for (int j = 0; j < 3; ++j) out_host[i * 3 + j] = h[i * ZS_SLOT + j];
   return 0;
 }
@@ -1024,9 +996,9 @@ extern "C" int dwmh_s1_label_vote(int32_t device, const float* const* labels, in
   if (num_labels < 1 || num_labels > S1_MAX_LABELS) return fail("dwmh_s1_label_vote: %d label ids (1..%d supported)", num_labels, S1_MAX_LABELS);
   RefPtrs rp{};
   for (int i = 0; i < k; ++i) { if (!labels[i]) return fail("dwmh_s1_label_vote: labels[%d] is null", i); rp.p[i] = labels[i]; }
-  S1_DEV(device);
-  s1_label_vote_kernel<<<grid_for(device), 256, 0, (cudaStream_t)stream_>>>(rp, k, num_labels, averaged_label, tissue_majority, n);
-  S1_CU(cudaGetLastError());
+  DEV_GUARD(device);
+  s1_label_vote_kernel<<<sm_count(device) * 8, 256, 0, (cudaStream_t)stream_>>>(rp, k, num_labels, averaged_label, tissue_majority, n);
+  CU_TRY(cudaGetLastError());
   return 0;
 }
 
@@ -1035,8 +1007,8 @@ extern "C" int dwmh_s1_apply_priors(int32_t device, float* anomaly, const float*
   if (!anomaly || !averaged_label) return fail("dwmh_s1_apply_priors: null argument");
   if (stage != 1 && stage != 2) return fail("dwmh_s1_apply_priors: stage must be 1 or 2");
   if (stage == 2 && (!anomaly_median || !tissue_majority)) return fail("dwmh_s1_apply_priors: stage 2 needs the median-filtered score and the tissue mask");
-  S1_DEV(device);
-  s1_apply_priors_kernel<<<grid_for(device), 256, 0, (cudaStream_t)stream_>>>(anomaly, anomaly_median, averaged_label, tissue_majority, stage, n);
-  S1_CU(cudaGetLastError());
+  DEV_GUARD(device);
+  s1_apply_priors_kernel<<<sm_count(device) * 8, 256, 0, (cudaStream_t)stream_>>>(anomaly, anomaly_median, averaged_label, tissue_majority, stage, n);
+  CU_TRY(cudaGetLastError());
   return 0;
 }

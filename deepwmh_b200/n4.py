@@ -45,9 +45,8 @@ def n4_bias_field_correction(volume, shrink_factor: int = 2, iterations: Sequenc
         ws = torch.empty(int(nbytes.value), dtype=torch.uint8, device=vol.device)
         out = torch.empty_like(vol)
         field = torch.empty_like(vol) if return_log_field else None
-        _lib.check(lib.dwmh_n4(vol.device.index, C.c_void_p(vol.data_ptr()), X, Y, Z, int(shrink_factor), len(iters), it,
-                               C.c_void_p(out.data_ptr()), C.c_void_p(field.data_ptr() if field is not None else None),
-                               C.c_void_p(ws.data_ptr()), C.c_void_p(torch.cuda.current_stream(vol.device).cuda_stream)))
+        _lib.check(lib.dwmh_n4(vol.device.index, _lib.ptr(vol), X, Y, Z, int(shrink_factor), len(iters), it, _lib.ptr(out),
+                               _lib.ptr(field), _lib.ptr(ws), _lib.stream(vol.device)))
     if is_numpy:
         out = out.cpu().numpy()
         field = field.cpu().numpy() if field is not None else None

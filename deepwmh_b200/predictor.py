@@ -21,19 +21,10 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import NetDesc, check
+from ._lib import NetDesc, check, ptr, stream
 
 ACT_DTYPES = {"fp16": 0, "float16": 0, "half": 0, "bf16": 1, "bfloat16": 1}
 HEAD_NONLINS = {"softmax": 0, "sigmoid": 1}      # dwmh_net_desc.head_nonlin
-
-
-def _ptr(t) -> C.c_void_p:
-    return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
-
-
-def _stream(device=None) -> C.c_void_p:
-    """The caller's current stream ON `device` (a stream handle is only valid on its own device)."""
-    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
 def pad_nd_image(image: np.ndarray, new_shape, mode="constant", kwargs=None):
@@ -158,26 +149,26 @@ class SegmentationNetwork:
         self._gaussian_installed = True
 
     def _st(self) -> C.c_void_p:
-        return _stream(self.device)
+        return stream(self.device)
 
     # ---- device-level pieces (used by the sharded drivers) ---------------------------------------
     def weight_map(self, shape: Sequence[int], step_size: float, use_gaussian: bool, out: Optional[torch.Tensor] = None) -> torch.Tensor:
         """wgt [X,Y,Z] of the complete tile set (dwmh_weight_map): data-independent, computed locally by every rank."""
         X, Y, Z = (int(v) for v in shape)
         wgt = out if out is not None else torch.empty((X, Y, Z), dtype=torch.float32, device=self.device)
-        check(self._lib.dwmh_weight_map(self._ctx, X, Y, Z, float(step_size), int(bool(use_gaussian)), _ptr(wgt), self._st()))
+        check(self._lib.dwmh_weight_map(self._ctx, X, Y, Z, float(step_size), int(bool(use_gaussian)), ptr(wgt), self._st()))
         return wgt
 
     def axpy_(self, acc: torch.Tensor, x: torch.Tensor, alpha: float):
         """acc += alpha * x on the device (a13: running mean of the k models' softmax)."""
         assert acc.is_cuda and x.is_cuda and acc.dtype == x.dtype == torch.float32 and acc.is_contiguous() and x.is_contiguous()
-        check(self._lib.dwmh_axpy(self._ctx, _ptr(acc), _ptr(x), float(alpha), acc.numel(), self._st()))
+        check(self._lib.dwmh_axpy(self._ctx, ptr(acc), ptr(x), float(alpha), acc.numel(), self._st()))
 
     def argmax(self, softmax: torch.Tensor) -> torch.Tensor:
         """Class map uint8 [x,y,z] of fp32 probabilities [C,x,y,z] on the device; ties go to the lower class (numpy.argmax)."""
         assert softmax.is_cuda and softmax.dtype == torch.float32 and softmax.is_contiguous()
         seg = torch.empty(tuple(softmax.shape[1:]), dtype=torch.uint8, device=softmax.device)
-        check(self._lib.dwmh_argmax(self._ctx, _ptr(softmax), int(softmax.shape[0]), _ptr(seg), seg.numel(), self._st()))
+        check(self._lib.dwmh_argmax(self._ctx, ptr(softmax), int(softmax.shape[0]), ptr(seg), seg.numel(), self._st()))
         return seg
 
     def region_labels(self, probs: torch.Tensor, order: Sequence[int]) -> torch.Tensor:
@@ -192,7 +183,7 @@ class SegmentationNetwork:
             raise ValueError("%d regions in regions_class_order, %d in probs" % (len(order), probs.shape[0]))
         seg = torch.empty(tuple(probs.shape[1:]), dtype=torch.uint8, device=probs.device)
         tab = (C.c_int32 * max(len(order), 1))(*order)
-        check(self._lib.dwmh_region_labels(self._ctx, _ptr(probs), len(order), tab, _ptr(seg), seg.numel(), self._st()))
+        check(self._lib.dwmh_region_labels(self._ctx, ptr(probs), len(order), tab, ptr(seg), seg.numel(), self._st()))
         return seg
 
     def normalize_(self, vol: torch.Tensor, seg: Optional[torch.Tensor] = None, mask_mode: int = 2, return_stats: bool = True):
@@ -200,10 +191,10 @@ class SegmentationNetwork:
         return_stats: (mean, std, count) on the host -- this synchronises the stream; False keeps the call asynchronous."""
         assert vol.is_cuda and vol.dtype == torch.float32 and vol.is_contiguous()
         if not return_stats:
-            check(self._lib.dwmh_zscore(self._ctx, _ptr(vol), _ptr(seg), vol.numel(), mask_mode, None, self._st()))
+            check(self._lib.dwmh_zscore(self._ctx, ptr(vol), ptr(seg), vol.numel(), mask_mode, None, self._st()))
             return None
         stats = (C.c_double * 3)()
-        check(self._lib.dwmh_zscore(self._ctx, _ptr(vol), _ptr(seg), vol.numel(), mask_mode, stats, self._st()))
+        check(self._lib.dwmh_zscore(self._ctx, ptr(vol), ptr(seg), vol.numel(), mask_mode, stats, self._st()))
         return tuple(stats)
 
     def _check_buffers(self, agg: torch.Tensor, wgt: torch.Tensor, vol: Optional[torch.Tensor] = None):
@@ -234,8 +225,8 @@ class SegmentationNetwork:
         """dwmh_predict_3d on device tensors: vol [M,X,Y,Z] fp32 (or [X,Y,Z] for one modality), agg [C,X,Y,Z], wgt [X,Y,Z]
         (accumulated into)."""
         X, Y, Z = self._check_buffers(agg, wgt, vol)
-        check(self._lib.dwmh_predict_3d(self._ctx, _ptr(vol), X, Y, Z, float(step_size), int(bool(do_mirroring)),
-                                        mirror_axes_mask(mirror_axes), int(bool(use_gaussian)), _ptr(agg), _ptr(wgt),
+        check(self._lib.dwmh_predict_3d(self._ctx, ptr(vol), X, Y, Z, float(step_size), int(bool(do_mirroring)),
+                                        mirror_axes_mask(mirror_axes), int(bool(use_gaussian)), ptr(agg), ptr(wgt),
                                         int(tile_begin), int(tile_end), self._st()))
 
     def finalize(self, agg: torch.Tensor, wgt: torch.Tensor, labels: bool = True) -> Tuple[Optional[torch.Tensor], torch.Tensor]:
@@ -243,7 +234,7 @@ class SegmentationNetwork:
         skips the argmax and returns None for seg."""
         X, Y, Z = self._check_buffers(agg, wgt)
         seg = torch.empty((X, Y, Z), dtype=torch.uint8, device=agg.device) if labels else None
-        check(self._lib.dwmh_finalize(self._ctx, _ptr(agg), _ptr(wgt), _ptr(agg), _ptr(seg), X, Y, Z, self._st()))
+        check(self._lib.dwmh_finalize(self._ctx, ptr(agg), ptr(wgt), ptr(agg), ptr(seg), X, Y, Z, self._st()))
         return seg, agg
 
     def ensemble_masked_add_(self, acc: torch.Tensor, bg_softmax: torch.Tensor, valid_mask: Optional[torch.Tensor] = None):
@@ -253,12 +244,12 @@ class SegmentationNetwork:
         assert bg_softmax.dtype == torch.float32 and bg_softmax.is_contiguous()
         if valid_mask is not None:
             assert valid_mask.dtype == torch.float32 and valid_mask.is_contiguous() and valid_mask.shape == acc.shape
-        check(self._lib.dwmh_ensemble_masked_add(self._ctx, _ptr(acc), _ptr(bg_softmax), _ptr(valid_mask), acc.numel(), self._st()))
+        check(self._lib.dwmh_ensemble_masked_add(self._ctx, ptr(acc), ptr(bg_softmax), ptr(valid_mask), acc.numel(), self._st()))
 
     def ensemble_refine_(self, acc: torch.Tensor, k: int) -> torch.Tensor:
         """acc /= k in place (the ensembled field) -> uint8 label `field < 0.5` (DCNN_multistage.py:118-119)."""
         label = torch.empty(acc.shape, dtype=torch.uint8, device=acc.device)
-        check(self._lib.dwmh_ensemble_refine(self._ctx, _ptr(acc), int(k), _ptr(label), acc.numel(), self._st()))
+        check(self._lib.dwmh_ensemble_refine(self._ctx, ptr(acc), int(k), ptr(label), acc.numel(), self._st()))
         return label
 
     def remove_sparks(self, seg: torch.Tensor, min_volume: int = 3) -> torch.Tensor:
@@ -267,7 +258,7 @@ class SegmentationNetwork:
         assert seg.is_cuda and seg.dtype == torch.uint8 and seg.is_contiguous() and seg.dim() == 3
         out = torch.empty_like(seg)
         X, Y, Z = seg.shape
-        check(self._lib.dwmh_remove_sparks(self._ctx, _ptr(seg), X, Y, Z, int(min_volume), _ptr(out), self._st()))
+        check(self._lib.dwmh_remove_sparks(self._ctx, ptr(seg), X, Y, Z, int(min_volume), ptr(out), self._st()))
         return out
 
     def keep_largest_components_(self, seg: torch.Tensor, class_mask: int, volume_per_voxel: float, min_valid_mm3: float = -1.0) -> torch.Tensor:
@@ -276,7 +267,7 @@ class SegmentationNetwork:
         least min_valid_mm3 (if >= 0); the voxels of every other one become 0."""
         assert seg.is_cuda and seg.dtype == torch.uint8 and seg.is_contiguous() and seg.dim() == 3
         X, Y, Z = seg.shape
-        check(self._lib.dwmh_keep_largest_components(self._ctx, _ptr(seg), X, Y, Z, int(class_mask), float(volume_per_voxel),
+        check(self._lib.dwmh_keep_largest_components(self._ctx, ptr(seg), X, Y, Z, int(class_mask), float(volume_per_voxel),
                                                      float(min_valid_mm3), self._st()))
         return seg
 
@@ -299,7 +290,7 @@ class SegmentationNetwork:
         if patches.numel() != n * self.input_channels * int(np.prod(self.patch_size)):
             raise ValueError("patches must be [n, %d, %d, %d, %d]" % ((self.input_channels,) + self.patch_size))
         out = torch.empty((n, self.num_classes) + tuple(self.patch_size), dtype=torch.float32, device=patches.device)
-        check(self._lib.dwmh_forward_patches(self._ctx, _ptr(patches), n, _ptr(out), self._st()))
+        check(self._lib.dwmh_forward_patches(self._ctx, ptr(patches), n, ptr(out), self._st()))
         return out
 
     def layer_output(self, index: int, n: int = 1, samples: "Optional[Sequence[int]]" = None) -> torch.Tensor:
@@ -315,7 +306,7 @@ class SegmentationNetwork:
         per = int(dims[1]) * int(dims[2]) * int(dims[3]) * int(dims[4])
         n = min(n, int(dims[0]))
         buf = torch.empty(n * per, dtype=torch.float32, device=self.device)
-        check(self._lib.dwmh_debug_layer_output_from(self._ctx, index, first, _ptr(buf), buf.numel(), dims, self._st()))
+        check(self._lib.dwmh_debug_layer_output_from(self._ctx, index, first, ptr(buf), buf.numel(), dims, self._st()))
         return buf.view(n, int(dims[1]), int(dims[2]), int(dims[3]), int(dims[4]))
 
     def layer_plan(self, index: int, nb: int) -> Dict[str, int]:

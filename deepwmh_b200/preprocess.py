@@ -85,8 +85,8 @@ def resample_device(vol, new_shape, order: int, separate_axis: Optional[int] = N
     with torch.cuda.device(vol.device):
         ws = torch.empty(int(nbytes.value), dtype=torch.uint8, device=vol.device)
         out = torch.empty(new_shape, dtype=torch.int8 if out_mode == 1 else torch.float32, device=vol.device)
-        _lib.check(lib.dwmh_resample(vol.device.index, C.c_void_p(vol.data_ptr()), ins, C.c_void_p(out.data_ptr()), outs, int(order), sep,
-                                     int(out_mode), C.c_void_p(ws.data_ptr()), C.c_void_p(torch.cuda.current_stream(vol.device).cuda_stream)))
+        _lib.check(lib.dwmh_resample(vol.device.index, _lib.ptr(vol), ins, _lib.ptr(out), outs, int(order), sep, int(out_mode),
+                                     _lib.ptr(ws), _lib.stream(vol.device)))
     return out
 
 
@@ -221,11 +221,10 @@ def ct_normalize_device(vol, seg, scheme: str, constants: Dict[str, float]):
     stats = (C.c_double * 3)() if ct2 else None
     with torch.cuda.device(vol.device):
         ws = torch.empty(_lib.DWMH_CT_WORKSPACE_BYTES, dtype=torch.uint8, device=vol.device) if ct2 else None
-        _lib.check(lib.dwmh_ct_normalize(vol.device.index, C.c_void_p(vol.data_ptr()), C.c_void_p(seg.data_ptr() if seg is not None else 0),
+        _lib.check(lib.dwmh_ct_normalize(vol.device.index, _lib.ptr(vol), _lib.ptr(seg),
                                          vol.numel(), code, constants["percentile_00_5"], constants["percentile_99_5"],
-                                         constants.get("mean", 0.0), constants.get("sd", 1.0), stats,
-                                         C.c_void_p(ws.data_ptr() if ws is not None else 0),
-                                         C.c_void_p(torch.cuda.current_stream(vol.device).cuda_stream)))
+                                         constants.get("mean", 0.0), constants.get("sd", 1.0), stats, _lib.ptr(ws),
+                                         _lib.stream(vol.device)))
     return tuple(stats) if ct2 else None
 
 
@@ -244,8 +243,8 @@ def cascade_onehot_device(labels, out, num_classes: int):
     ins = (C.c_int32 * 3)(*labels.shape)
     outs = (C.c_int32 * 3)(*out.shape[1:])
     with torch.cuda.device(out.device):
-        _lib.check(lib.dwmh_cascade_onehot(out.device.index, C.c_void_p(labels.data_ptr()), ins, C.c_void_p(out.data_ptr()), outs,
-                                           int(num_classes), C.c_void_p(torch.cuda.current_stream(out.device).cuda_stream)))
+        _lib.check(lib.dwmh_cascade_onehot(out.device.index, _lib.ptr(labels), ins, _lib.ptr(out), outs, int(num_classes),
+                                           _lib.stream(out.device)))
     return out
 
 

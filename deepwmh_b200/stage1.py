@@ -22,6 +22,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from ._lib import ptr, stream
 
 Array = Union[np.ndarray, torch.Tensor]
 
@@ -34,14 +35,6 @@ def _dev(t: Array, device: int, copy: bool = False) -> torch.Tensor:
     if copy and out.data_ptr() == t.data_ptr():
         out = out.clone()
     return out
-
-
-def _ptr(t: Optional[torch.Tensor]) -> C.c_void_p:
-    return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(0)
-
-
-def _stream(device: int) -> C.c_void_p:
-    return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
 def _i3(v: Sequence[int]):
@@ -67,7 +60,7 @@ def z_score(data: Array, mask: Optional[Array] = None, fill_outside: bool = Fals
     ws = torch.empty(16, dtype=torch.float64, device=x.device)
     stats = (C.c_double * 3)() if return_stats else None
     with torch.cuda.device(x.device):
-        _lib.check(lib.dwmh_s1_zscore(device, _ptr(x), _ptr(m), x.numel(), int(bool(fill_outside)), _ptr(ws), stats, _stream(device)))
+        _lib.check(lib.dwmh_s1_zscore(device, ptr(x), ptr(m), x.numel(), int(bool(fill_outside)), ptr(ws), stats, stream(device)))
     return (x, tuple(stats)) if return_stats else x
 
 
@@ -86,8 +79,8 @@ def z_score_batch_(volumes: Sequence[torch.Tensor], mask: Optional[Array] = None
     ws = torch.empty(8 * len(volumes), dtype=torch.float64, device=dev)
     ptrs = (C.c_void_p * len(volumes))(*[v.data_ptr() for v in volumes])
     with torch.cuda.device(dev):
-        _lib.check(lib.dwmh_s1_zscore_batch(dev.index, ptrs, len(volumes), _ptr(m), volumes[0].numel(), int(bool(fill_outside)),
-                                            _ptr(ws), _stream(dev.index)))
+        _lib.check(lib.dwmh_s1_zscore_batch(dev.index, ptrs, len(volumes), ptr(m), volumes[0].numel(), int(bool(fill_outside)),
+                                            ptr(ws), stream(dev.index)))
     return volumes
 
 
@@ -110,8 +103,8 @@ def local_mean_align_(target: torch.Tensor, refs: Sequence[torch.Tensor], patch_
     mu = torch.empty_like(target) if return_local_mean else None
     ptrs = (C.c_void_p * max(1, len(refs)))(*[r.data_ptr() for r in refs])
     with torch.cuda.device(dev):
-        _lib.check(lib.dwmh_s1_local_mean_align(dev.index, _ptr(target), ptrs, len(refs), _ptr(m), X, Y, Z, ps, _ptr(mu), _ptr(ws),
-                                                _stream(dev.index)))
+        _lib.check(lib.dwmh_s1_local_mean_align(dev.index, ptr(target), ptrs, len(refs), ptr(m), X, Y, Z, ps, ptr(mu), ptr(ws),
+                                                stream(dev.index)))
     return mu
 
 
@@ -133,7 +126,7 @@ def mean_std_grid(data: Array, patch_size: Sequence[int], order: int = 1, mask: 
     ws = torch.empty(nbytes.value, dtype=torch.uint8, device=x.device)
     mean, std = torch.empty_like(x), torch.empty_like(x)
     with torch.cuda.device(x.device):
-        _lib.check(lib.dwmh_s1_mean_std_grid(device, _ptr(x), _ptr(m), X, Y, Z, ps, _ptr(mean), _ptr(std), _ptr(ws), _stream(device)))
+        _lib.check(lib.dwmh_s1_mean_std_grid(device, ptr(x), ptr(m), X, Y, Z, ps, ptr(mean), ptr(std), ptr(ws), stream(device)))
     return mean, std
 
 
@@ -142,7 +135,7 @@ def align_local_mean_(x: torch.Tensor, local_mu: torch.Tensor, target_local_mu: 
     lib = _lib.load()
     device = x.device.index
     with torch.cuda.device(x.device):
-        _lib.check(lib.dwmh_s1_align_local_mean(device, _ptr(x), _ptr(local_mu), _ptr(target_local_mu), x.numel(), _stream(device)))
+        _lib.check(lib.dwmh_s1_align_local_mean(device, ptr(x), ptr(local_mu), ptr(target_local_mu), x.numel(), stream(device)))
     return x
 
 
@@ -166,12 +159,12 @@ def _group_nll(x: torch.Tensor, refs: Sequence[torch.Tensor], masks: Optional[Se
     ptrs = (C.c_void_p * len(refs))(*[r.data_ptr() for r in refs])
     with torch.cuda.device(x.device):
         if masks is None:
-            _lib.check(lib.dwmh_s1_group_nll(device, _ptr(x), ptrs, len(refs), min_std, side, _ptr(mul_mask), _ptr(an), _ptr(mu), _ptr(sg),
-                                             x.numel(), _stream(device)))
+            _lib.check(lib.dwmh_s1_group_nll(device, ptr(x), ptrs, len(refs), min_std, side, ptr(mul_mask), ptr(an), ptr(mu), ptr(sg),
+                                             x.numel(), stream(device)))
         else:
             mptrs = (C.c_void_p * len(masks))(*[m.data_ptr() for m in masks])
-            _lib.check(lib.dwmh_s1_group_nll_masked(device, _ptr(x), ptrs, mptrs, len(refs), min_std, side, _ptr(mul_mask), _ptr(an),
-                                                    _ptr(mu), _ptr(sg), x.numel(), _stream(device)))
+            _lib.check(lib.dwmh_s1_group_nll_masked(device, ptr(x), ptrs, mptrs, len(refs), min_std, side, ptr(mul_mask), ptr(an),
+                                                    ptr(mu), ptr(sg), x.numel(), stream(device)))
     return an, mu, sg
 
 
@@ -215,7 +208,7 @@ def median_filter(data: Array, kernel_size: Sequence[int], device: int = 0) -> t
     out = torch.empty_like(x)
     X, Y, Z = (int(v) for v in x.shape)
     with torch.cuda.device(x.device):
-        _lib.check(lib.dwmh_s1_median_filter(device, _ptr(x), _ptr(out), X, Y, Z, _i3(kernel_size), _stream(device)))
+        _lib.check(lib.dwmh_s1_median_filter(device, ptr(x), ptr(out), X, Y, Z, _i3(kernel_size), stream(device)))
     return out
 
 
@@ -251,7 +244,7 @@ def component_filtering(mask: Array, voxel_size: Sequence[float], return_type: s
     ws = torch.empty(nbytes.value, dtype=torch.uint8, device=m.device)
     out = torch.empty_like(m)
     with torch.cuda.device(m.device):
-        _lib.check(lib.dwmh_s1_component_filtering(device, _ptr(m), X, Y, Z, vs, _ptr(out), _ptr(ws), _stream(device)))
+        _lib.check(lib.dwmh_s1_component_filtering(device, ptr(m), X, Y, Z, vs, ptr(out), ptr(ws), stream(device)))
     return out
 
 
@@ -262,7 +255,7 @@ def minmax(data: Array, mask: Optional[Array] = None, device: int = 0) -> Tuple[
     ws = torch.empty(2, dtype=torch.int32, device=x.device)
     out = (C.c_float * 2)()
     with torch.cuda.device(x.device):
-        _lib.check(lib.dwmh_s1_minmax(device, _ptr(x), _ptr(m), x.numel(), _ptr(ws), out, _stream(device)))
+        _lib.check(lib.dwmh_s1_minmax(device, ptr(x), ptr(m), x.numel(), ptr(ws), out, stream(device)))
     return float(out[0]), float(out[1])
 
 
@@ -277,8 +270,8 @@ def histogram(data: Array, bin_edges: np.ndarray, mask: Optional[Array] = None, 
     nbins = int(edges.numel()) - 1
     counts = torch.empty(nbins, dtype=torch.int64, device=x.device)
     with torch.cuda.device(x.device):
-        _lib.check(lib.dwmh_s1_histogram(device, _ptr(x), _ptr(m), x.numel(), int(fill_value is not None),
-                                         float(fill_value if fill_value is not None else 0.0), _ptr(edges), nbins, _ptr(counts), _stream(device)))
+        _lib.check(lib.dwmh_s1_histogram(device, ptr(x), ptr(m), x.numel(), int(fill_value is not None),
+                                         float(fill_value if fill_value is not None else 0.0), ptr(edges), nbins, ptr(counts), stream(device)))
     return counts.cpu().numpy()
 
 
@@ -324,7 +317,7 @@ def threshold_mask(data: Array, threshold: float, mul_mask: Optional[Array] = No
     mm = _dev(mul_mask, device) if mul_mask is not None else None
     out = torch.empty_like(x)
     with torch.cuda.device(x.device):
-        _lib.check(lib.dwmh_s1_threshold_mask(device, _ptr(x), float(threshold), _ptr(mm), _ptr(out), x.numel(), _stream(device)))
+        _lib.check(lib.dwmh_s1_threshold_mask(device, ptr(x), float(threshold), ptr(mm), ptr(out), x.numel(), stream(device)))
     return out
 
 
@@ -382,8 +375,8 @@ def masked_sums(volumes: Sequence[torch.Tensor], mask: Optional[Array] = None, p
     out = (C.c_double * (3 * len(volumes)))()
     ptrs = (C.c_void_p * len(volumes))(*[v.data_ptr() for v in volumes])
     with torch.cuda.device(dev):
-        _lib.check(lib.dwmh_s1_masked_sums(dev.index, ptrs, len(volumes), _ptr(m), volumes[0].numel(), int(bool(positive_only)), _ptr(ws),
-                                           out, _stream(dev.index)))
+        _lib.check(lib.dwmh_s1_masked_sums(dev.index, ptrs, len(volumes), ptr(m), volumes[0].numel(), int(bool(positive_only)), ptr(ws),
+                                           out, stream(dev.index)))
     return np.array(out, dtype=np.float64).reshape(len(volumes), 3)
 
 
@@ -440,7 +433,7 @@ def label_vote(labels: Sequence[Array], device: int = 0) -> Tuple[torch.Tensor, 
     avg, tissue = torch.empty_like(ls[0]), torch.empty_like(ls[0])
     ptrs = (C.c_void_p * len(ls))(*[l.data_ptr() for l in ls])
     with torch.cuda.device(ls[0].device):
-        _lib.check(lib.dwmh_s1_label_vote(device, ptrs, len(ls), num, _ptr(avg), _ptr(tissue), avg.numel(), _stream(device)))
+        _lib.check(lib.dwmh_s1_label_vote(device, ptrs, len(ls), num, ptr(avg), ptr(tissue), avg.numel(), stream(device)))
     return avg, tissue
 
 
@@ -455,8 +448,8 @@ def apply_priors_(anomaly: torch.Tensor, averaged_label: torch.Tensor, tissue_ma
     lib = _lib.load()
     dev = anomaly.device
     with torch.cuda.device(dev):
-        _lib.check(lib.dwmh_s1_apply_priors(dev.index, _ptr(anomaly), _ptr(anomaly_median), _ptr(averaged_label), _ptr(tissue_majority),
-                                            1 if anomaly_median is None else 2, anomaly.numel(), _stream(dev.index)))
+        _lib.check(lib.dwmh_s1_apply_priors(dev.index, ptr(anomaly), ptr(anomaly_median), ptr(averaged_label), ptr(tissue_majority),
+                                            1 if anomaly_median is None else 2, anomaly.numel(), stream(dev.index)))
     return anomaly
 
 
